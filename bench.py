@@ -221,6 +221,14 @@ def _rel_l2(a, b):
     return float(np.linalg.norm(a - b) / max(np.linalg.norm(b), 1e-30))
 
 
+def dump_outputs(out_dir, arrays):
+    """Writes each array as out_dir/<name>.npy in float32, so that two builds run with the same arguments can be compared
+    output for output."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float32))
+
+
 def parity_vs_oracle(local_rank):
     """The kernels the benchmark times, checked against the CPU oracle inside the benchmark process: (i) a 2-block prefix of
     the model at the config-2 shapes (N=1536, S=1024, D=4096 -- same tile fits, fused q|k|v, attention shapes as the timed
@@ -377,16 +385,18 @@ def run_ours(args, rank, world, local_rank):
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    l0 = ctx.launch_count
-    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    e0.record(stream)
-    for _ in range(args.steps):
-        resident_step()
-    e1.record(stream)
-    barrier()
+    try:     # the sampler's nvidia-smi child must not outlive a failed run
+        l0 = ctx.launch_count
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record(stream)
+        for _ in range(args.steps):
+            resident_step()
+        e1.record(stream)
+        barrier()
+    finally:
+        clocks = sampler.stop() if rank == 0 else None
     launches = (ctx.launch_count - l0) // args.steps
     ms_per_step = max_over_ranks(e0.elapsed_time(e1)) / args.steps
-    clocks = sampler.stop() if rank == 0 else None
     value = 1e3 / ms_per_step
     timed_latent = ctx.denoise_get_latent()
     parity["timed_latent_finite"] = all_ok(bool(np.isfinite(timed_latent).all() and np.abs(timed_latent).max() > 0))
@@ -446,6 +456,11 @@ def run_ours(args, rank, world, local_rank):
     torch.cuda.synchronize()
     vae_ms = ev_time(ctx, stream, lambda: ctx.vae_decode_dev(lat_dev.data_ptr(), (F, H, W), frames_dev.data_ptr()),
                      max(3, min(args.steps, 10)), warm=3)
+    frames_sample = None
+    if args.dump_outputs:
+        # 2^20 of the 29.5 M frame values (118 MB in fp32) at fixed, seeded positions
+        pick = np.sort(np.random.default_rng(0).choice(frames_dev.numel(), 1 << 20, replace=False))
+        frames_sample = frames_dev.view(-1)[torch.from_numpy(pick).cuda()].cpu().numpy()
     ctx.set_profiling(True)
     ctx.vae_decode_dev(lat_dev.data_ptr(), (F, H, W), frames_dev.data_ptr())
     vprof = ctx.get_profile()
@@ -725,6 +740,9 @@ def run_ours(args, rank, world, local_rank):
         if dist is not None:
             dist.destroy_process_group()
         return
+    if args.dump_outputs:
+        # the latent ltx_denoise_get_latent returns after the last timed step, and the frames of the last timed VAE decode
+        dump_outputs(args.dump_outputs, dict(latent=timed_latent, vae_frames_sample=frames_sample))
 
     pk = peaks()
     # DRAM traffic of the dominant kernel: bytes of ONE FFN-in launch from the newest committed `ncu --set full` capture
@@ -795,17 +813,29 @@ def run_ours(args, rank, world, local_rank):
         dist.destroy_process_group()
 
 
+def _positive_int(s):
+    v = int(s)
+    if v < 1:
+        raise argparse.ArgumentTypeError(f"must be at least 1, got {v}")
+    return v
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=16)
+    ap.add_argument("--steps", type=_positive_int, default=16, help="timed steps")
     ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what they computed to DIR/<name>.npy (float32): the denoised latent "
+                         "and a seeded sample of the decoded frames")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cfg5", action="store_true", help="skip the two-stage 1536x1024x257 extra")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-cpu-full-step", action="store_true", help="skip the one true 48-block CPU step (~26 s)")
     ap.add_argument("--no-parity", action="store_true", help="skip the in-process oracle checks (N = 1)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs --impl ours (the reference arm times one block of the CPU port and keeps no outputs)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -40,6 +40,15 @@ def test_reference_arm_other_ranks_exit_quietly():
     assert r.stdout.strip() == ""
 
 
+def test_bad_arguments_are_refused_before_any_work():
+    """--steps is the number of timed steps, so it must be at least 1; --dump-outputs writes the product arm's outputs only."""
+    for args in (("--steps", "0"), ("--steps", "-3"), ("--dump-outputs", "unused")):
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--warmup", "0", *args],
+                           capture_output=True, text=True, timeout=300, cwd=ROOT)
+        assert r.returncode == 2 and r.stdout.strip() == "", (args, r.returncode, r.stdout[-500:])
+        assert "--steps" in r.stderr or "--dump-outputs" in r.stderr, r.stderr[-500:]
+
+
 def test_product_arm_refuses_to_run_without_a_gpu():
     """No CPU fallback: on a host without a CUDA device the product arm exits non-zero and prints no result line."""
     import torch

@@ -1,5 +1,5 @@
 import math, sys, os, torch
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import ltx_video_swift_mlx_b200  # noqa
 from ltx_video_swift_mlx_b200.context import LtxContext, LTXTransformerConfig
 ctx = LtxContext(LTXTransformerConfig(num_layers=1, num_attention_heads=1), 0)
