@@ -405,6 +405,23 @@ int ltx_conv3d_plan(int T, int H, int W, int Cin, int Cout, int mode, int ntaps,
 /* 3x3x3 conv on a channels-last fp32 volume [T,H,W,Cin] -> [T,H,W,Cout] fp32 with reflect/replicate padding. */
 int ltx_op_conv3d(ltx_ctx* ctx, const float* x, const void* w_bf16_27_O_I, const float* bias, float* out, int T, int H,
                   int W, int Cin, int Cout, int causal);
+/* The convolution's padding prologue: fp32 [T,H,W,C] -> bf16 [T+2,H+2,W+2,C] with the padding materialised.  mode 0 copy,
+ * 1 x*a[c] + b[c], 2 silu(pixel_norm(x) * (1 + a[c]) + b[c]) (a, b both NULL: no modulation), 3 silu(x*a[c] + b[c]).
+ * pad bits: 1 causal (two leading frame copies), 2 zero padding in H, W instead of reflect, 4 zero padding in T instead of
+ * frame replication. */
+int ltx_op_vae_prep(ltx_ctx* ctx, const float* x, void* out_pad_bf16, int T, int H, int W, int C, int mode, const float* a,
+                    const float* b, int pad);
+/* Rewrites the padding voxels of a bf16 [T+2,H+2,W+2,C] volume from its interior, as ltx_op_vae_prep pads (same pad bits). */
+int ltx_op_vae_halo_fill(ltx_ctx* ctx, void* vol_bf16, int T, int H, int W, int C, int pad);
+/* The implicit-GEMM conv on an already padded bf16 volume [T+2,H+2,W+2,Cin] with weights bf16 [ntaps][Cout][Cin] (27: 3x3x3,
+ * 9: the per-frame 3x3 taps dt = 1) and one of its epilogues: 0 out = conv + bias (+ resid, nullable; out == resid allowed)
+ * [T,H,W,Cout]; 1 depth-to-space into out [2T-1+t_shift,2H,2W,Cout/8] plus the 4x tiled depth-to-space of resid [T,H,W,Cin];
+ * 2 unpatchify 4x4 + (x+1)/2 (clipped to [0,1] unless no_clip) into out [T,4H,4W,3] (Cout = 48); 3 pixel-norm,
+ * * (1 + next_scale) + next_shift (both nullable), SiLU of conv + bias into the interior of next_pad [T+2,H+2,W+2,Cout] at frame
+ * offset next_tshift (1 or 2); 4 as 0 with resid, and its output also as in 3. */
+int ltx_op_conv3d_epi(ltx_ctx* ctx, const void* x_pad_bf16, const void* w_bf16, const float* bias, int T, int H, int W, int Cin,
+                      int Cout, int ntaps, int mode, float* out, const float* resid, int t_shift, int no_clip, void* next_pad_bf16,
+                      const float* next_scale, const float* next_shift, int next_tshift);
 
 #if defined(__GNUC__)
 #pragma GCC visibility pop

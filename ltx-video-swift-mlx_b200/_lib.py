@@ -115,6 +115,9 @@ SIGNATURES = {
     "ltx_op_qknorm_rope": (_I, [_P, _P, _I, _I, _P, _P, _P, _I, _F]),
     "ltx_op_conv3d": (_I, [_P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I]),
     "ltx_conv3d_plan": (_I, [_I, _I, _I, _I, _I, _I, _I, _I, C.POINTER(C.c_int32)]),
+    "ltx_op_vae_prep": (_I, [_P, _P, _P, _I, _I, _I, _I, _I, _P, _P, _I]),
+    "ltx_op_vae_halo_fill": (_I, [_P, _P, _I, _I, _I, _I, _I]),
+    "ltx_op_conv3d_epi": (_I, [_P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _P, _P, _I, _I, _P, _P, _P, _I]),
 }
 
 _lib = None

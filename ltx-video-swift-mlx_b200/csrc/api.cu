@@ -1317,4 +1317,39 @@ int ltx_op_conv3d(ltx_ctx* c, const float* x, const void* w, const float* bias, 
   });
 }
 
+int ltx_op_vae_prep(ltx_ctx* c, const float* x, void* out_pad, int T, int H, int W, int C, int mode, const float* a, const float* b,
+                    int pad) {
+  return guarded(c, [&] {
+    launch_vae_prep(x, reinterpret_cast<bf16*>(out_pad), T, H, W, C, mode, a, b, pad, c->stream);
+    c->launches++;
+  });
+}
+
+int ltx_op_vae_halo_fill(ltx_ctx* c, void* vol, int T, int H, int W, int C, int pad) {
+  return guarded(c, [&] {
+    launch_vae_halo_fill(reinterpret_cast<bf16*>(vol), T, H, W, C, pad, c->stream);
+    c->launches++;
+  });
+}
+
+int ltx_op_conv3d_epi(ltx_ctx* c, const void* x_pad, const void* w, const float* bias, int T, int H, int W, int Cin, int Cout,
+                      int ntaps, int mode, float* out, const float* resid, int t_shift, int no_clip, void* next_pad,
+                      const float* next_scale, const float* next_shift, int next_tshift) {
+  return guarded(c, [&] {
+    ConvEpi e;
+    e.mode = mode; e.out = out; e.bias = bias; e.resid = resid; e.Cin = Cin; e.t_shift = t_shift; e.no_clip = no_clip;
+    e.next_pad = reinterpret_cast<bf16*>(next_pad); e.next_scale = next_scale; e.next_shift = next_shift; e.next_tshift = next_tshift;
+    // the split-K scratch as vae_conv reserves it, so that every shape gets the plan the decoder gets
+    float* scratch = nullptr;
+    const size_t slab3 = static_cast<size_t>(3) * T * H * W * Cout * 4;
+    if (mode == 0 && ntaps == 27 && conv3d_wants_tap_split(H, W, Cin, Cout)) {
+      c->v_split.reserve(slab3);
+      scratch = c->v_split.as<float>();
+    }
+    launch_conv3d(reinterpret_cast<const bf16*>(x_pad), reinterpret_cast<const bf16*>(w), T, H, W, Cin, Cout, e, c->stream, ntaps,
+                  scratch, scratch ? slab3 : 0);
+    c->launches++;
+  });
+}
+
 }  // extern "C"

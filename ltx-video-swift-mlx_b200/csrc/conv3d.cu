@@ -805,15 +805,25 @@ void launch_conv3d(const bf16* x_pad, const bf16* w, int T, int H, int W, int Ci
   ConvEpi epi = epi_in;
   LTX_CHECK(T > 0 && H > 1 && W > 1, 2, "conv3d: bad volume (reflect padding needs H, W >= 2)");
   LTX_CHECK(ntaps == 27 || ntaps == 9, 2, "conv3d: 27 taps (3x3x3) or 9 taps (per-frame 3x3)");
-  LTX_CHECK(Cin % 64 == 0, 2, "conv3d: Cin must be a multiple of 64");
+  LTX_CHECK(Cin > 0 && Cin % 64 == 0 && Cout > 0, 2, "conv3d: Cin must be a positive multiple of 64");
+  LTX_CHECK(epi.mode >= 0 && epi.mode <= 4, 2, "bad conv epilogue mode");
+  LTX_CHECK(epi.mode == 3 || epi.out != nullptr, 2, "conv3d: no output buffer");
   LTX_CHECK(epi.mode != 0 || Cout % 4 == 0, 2, "conv3d: Cout must be a multiple of 4");
-  LTX_CHECK(epi.mode != 1 || (Cout % 32 == 0 && Cin % 8 == 0 && epi.resid != nullptr), 2, "conv3d: bad d2s configuration");
+  LTX_CHECK(epi.mode != 1 || (Cout % 32 == 0 && Cin % 8 == 0 && epi.resid != nullptr && (epi.t_shift == 0 || epi.t_shift == 1)), 2,
+            "conv3d: bad d2s configuration");
+  // the unpatchify store writes frame channel co >> 4 of a 3-channel frame
+  LTX_CHECK(epi.mode != 2 || Cout == 48, 2, "conv3d: the unpatchify epilogue needs Cout = 48 (3 channels x 4 x 4)");
   LTX_CHECK(epi.mode != 4 || (epi.resid != nullptr && epi.out != nullptr), 2, "conv3d: mode 4 needs the residual stream");
   LTX_CHECK((epi.mode != 3 && epi.mode != 4) || (Cout % 32 == 0 && Cout <= 256 && Cout > 64 && epi.next_pad != nullptr && ntaps == 27), 2,
             "conv3d: the fused-prologue epilogue needs 64 < Cout <= 256 (one tile = all channels of a voxel)");
+  LTX_CHECK((epi.mode != 3 && epi.mode != 4) ||
+                ((epi.next_tshift == 1 || epi.next_tshift == 2) && (epi.next_scale == nullptr) == (epi.next_shift == nullptr)),
+            2, "conv3d: fused-prologue epilogue needs next_tshift 1 or 2 and both or neither of next_scale / next_shift");
   const size_t slab = static_cast<size_t>(T) * H * W * Cout * 4;
   const bool scratch_ok = splitk_scratch != nullptr && 3 * slab <= splitk_scratch_bytes;
   const ConvPlan pl = conv3d_plan(T, H, W, Cin, Cout, epi.mode, ntaps, scratch_ok, device_sm_count(), conv_pair_enabled(), conv_slab_enabled());
+  // only the mode-0 / mode-4 store of an unsplit conv can do without a bias
+  LTX_CHECK(epi.bias != nullptr || ((epi.mode == 0 || epi.mode == 4) && pl.ksplit == 1), 2, "conv3d: no bias");
   ConvGeom g;
   g.T = T; g.H = H; g.W = W; g.Cin = Cin; g.Cout = Cout;
   g.bt = pl.bt; g.bh = pl.bh; g.bw = pl.bw;
@@ -847,7 +857,8 @@ void launch_conv3d(const bf16* x_pad, const bf16* w, int T, int H, int W, int Ci
 }
 
 void launch_vae_halo_fill(bf16* vol, int T, int H, int W, int C, int pad, cudaStream_t s) {
-  LTX_CHECK(C % 8 == 0 && H > 1 && W > 1, 2, "vae_halo_fill: bad shape");
+  LTX_CHECK(C % 8 == 0 && T > 0 && H > 1 && W > 1, 2, "vae_halo_fill: bad shape");
+  LTX_CHECK(pad >= 0 && pad <= 7, 2, "vae_halo_fill: pad takes the VAE_PAD_* bits only");
   // work = the padding voxels only; a warp per voxel
   const int64_t nvox = 2 * static_cast<int64_t>(H + 2) * (W + 2) + static_cast<int64_t>(T) * (2 * (W + 2) + 2 * H);
   LTX_CHECK(nvox < (1ll << 30), 2, "vae_halo_fill: volume too large");
@@ -860,7 +871,10 @@ void launch_vae_halo_fill(bf16* vol, int T, int H, int W, int C, int pad, cudaSt
 
 void launch_vae_prep(const float* x, bf16* out, int T, int H, int W, int C, int mode, const float* a, const float* b,
                      int pad, cudaStream_t s) {
-  LTX_CHECK(C % 4 == 0 && C <= 2048 && H > 1 && W > 1, 2, "vae_prep: bad shape (C must be a multiple of 4, at most 2048)");
+  LTX_CHECK(C % 4 == 0 && C <= 2048 && T > 0 && H > 1 && W > 1, 2, "vae_prep: bad shape (C must be a multiple of 4, at most 2048)");
+  LTX_CHECK(mode >= 0 && mode <= 3 && pad >= 0 && pad <= 7, 2, "vae_prep: bad mode or pad bits");
+  // modes 1 / 3 read both tables; mode 2 reads both or neither (a != NULL selects the modulation)
+  LTX_CHECK(mode == 0 || (a != nullptr && b != nullptr) || (mode == 2 && a == nullptr && b == nullptr), 2, "vae_prep: bad scale / shift tables");
   const int64_t nvox = static_cast<int64_t>(T + 2) * (H + 2) * (W + 2);
   LTX_CHECK(nvox < (1ll << 31), 2, "vae_prep: volume too large");
   int64_t blocks = (nvox + 7) / 8;

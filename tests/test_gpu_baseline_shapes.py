@@ -5,7 +5,7 @@ projection, the 3-way tap split or the 256-wide conv tiles that the benchmarked 
     a 4-block prefix of the 48-block model against the oracle (C/LTXConfig.swift:122-139, T/LTXTransformer.swift:235-486);
     the same prefix with int8 group-64 weights (P/LTXPipeline.swift:323-333) against the bf16 model;
   * config 4's decoder: the real channel plan (base 1024, 5 res blocks per stage, V/VideoDecoder.swift:331-355) on the
-    config-2 latent 4x16x24 (25 frames of 512x768) against the oracle, PSNR >= 40 dB.
+    config-2 latent 4x16x24 (25 frames of 512x768) against the oracle, PSNR >= 50 dB (57.8 dB measured on a B200 at 1000 W).
 The oracle needs a few seconds of CPU per case at these sizes."""
 import numpy as np
 import pytest
@@ -115,5 +115,5 @@ def test_full_vae_plan_at_cfg2_latent():
     assert out.shape == tuple(ref.shape) == (25, 512, 768, 3)
     assert np.isfinite(out).all() and out.min() >= 0 and out.max() <= 1
     p = O.psnr(torch.from_numpy(out), ref)
-    assert p >= 40.0, p
+    assert p >= 50.0, p
     ctx.close()

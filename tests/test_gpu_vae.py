@@ -1,4 +1,5 @@
-"""Video-VAE decode parity against the CPU oracle: PSNR >= 40 dB on [0,1] frames (bf16 activations into the convs)."""
+"""Video-VAE decode parity against the CPU oracle: PSNR >= 50 dB on [0,1] frames (bf16 activations into the convs; every case
+measured 58.4-61.4 dB on a B200 at 1000 W)."""
 import numpy as np
 import pytest
 import torch
@@ -19,7 +20,7 @@ def test_vae_decode_matches_oracle(base, blocks, fhw):
     assert out.shape == tuple(ref.shape) == (8 * (fhw[0] - 1) + 1, 32 * fhw[1], 32 * fhw[2], 3)
     assert np.isfinite(out).all() and out.min() >= 0 and out.max() <= 1
     p = O.psnr(torch.from_numpy(out), ref)
-    assert p >= 40.0, p
+    assert p >= 50.0, p
     ctx.close()
 
 
@@ -33,7 +34,7 @@ def test_vae_decode_timestep_conditioned():
     nz = torch.randn(1, 128, 2, 3, 4, generator=g)
     ref = O.decode_video(w, ocfg, z, timestep=0.05, decode_noise=nz)
     out = ctx.vae_decode(z[0].numpy(), timestep=0.05, decode_noise=nz[0].numpy())
-    assert O.psnr(torch.from_numpy(out), ref) >= 40.0
+    assert O.psnr(torch.from_numpy(out), ref) >= 50.0
     plain = ctx.vae_decode(z[0].numpy())
     assert O.psnr(torch.from_numpy(plain), ref) < 35.0      # the conditioning really changes the frames
     ctx.close()
@@ -48,7 +49,7 @@ def test_vae_decode_causal():
     z = torch.randn(1, 128, 3, 3, 4, generator=torch.Generator().manual_seed(53))
     ref = O.decode_video(w, ocfg, z)
     out = ctx.vae_decode(z[0].numpy(), causal=True)
-    assert O.psnr(torch.from_numpy(out), ref) >= 40.0
+    assert O.psnr(torch.from_numpy(out), ref) >= 50.0
     noncausal = ctx.vae_decode(z[0].numpy(), causal=False)
     assert O.psnr(torch.from_numpy(noncausal), ref) < 35.0
     ctx.close()
@@ -73,7 +74,7 @@ def test_vae_decode_temporal_tiling(frames, tile, overlap, timed):
     assert out.shape == tuple(ref.shape), (out.shape, ref.shape)
     assert out.shape[0] == ctx.lib.ltx_vae_tiled_frames(frames, tile, overlap)
     assert np.isfinite(out).all() and out.min() >= 0 and out.max() <= 1
-    assert O.psnr(torch.from_numpy(out), ref) >= 40.0
+    assert O.psnr(torch.from_numpy(out), ref) >= 50.0
     # (ii) the same chunk schedule on the host; interior frames of a chunk (never clipped away) must agree to fp32 rounding
     stride, po = tile - overlap, 8 * overlap
     chunks, start = [], 0
