@@ -165,7 +165,8 @@ int ltx_dit_forward_dev(ltx_ctx* ctx, const void* latent, ltx_dtype latent_dtype
  *   video_latent [1, N, in_channels], audio_latent [1, Ta, audio_in_channels] (bf16 or fp32), contexts [1, S, caption_channels],
  *   one sigma per stream, masks [1, S] int32 or NULL; out_video [1, N, out_channels], out_audio [1, Ta, audio_in_channels] fp32.
  * context_key != 0 caches the text K / V of both streams.  Weights: bf16, or int8 / int4 after ltx_finalize_weights(ctx, 8 | 4, 64)
- * (quantize(model: ltx2, groupSize: 64, bits:), Pipeline/LTXPipeline.swift:491).  This version: B = 1, one GPU. */
+ * (quantize(model: ltx2, groupSize: 64, bits:), Pipeline/LTXPipeline.swift:491).  One GPU; B = 1 here, B = 2 through
+ * ltx_av_forward_batch. */
 int ltx_av_forward(ltx_ctx* ctx, const void* video_latent, ltx_dtype video_dtype, const void* audio_latent, ltx_dtype audio_dtype,
                    const void* video_context, const void* audio_context, ltx_dtype context_dtype, float video_sigma,
                    float audio_sigma, const int32_t* video_mask, const int32_t* audio_mask, int N, int Ta, int S, int F, int H,
@@ -187,6 +188,24 @@ int ltx_av_forward_tokens_dev(ltx_ctx* ctx, const void* video_latent, ltx_dtype 
                               const float* video_sigmas, const float* audio_sigma, const int32_t* video_mask,
                               const int32_t* audio_mask, int N, int Ta, int S, int F, int H, int W, uint64_t context_key,
                               float* out_video, float* out_audio);
+/* LTX2Transformer.callAsFunction (Models/Transformer/LTX2Transformer.swift:240-392) on a batch, with the conventions of
+ * ltx_dit_forward: B items (1 or 2, e.g. the conditional and unconditional passes of a CFG step) in one forward.
+ *   video_latent [B, N, in_channels], audio_latent [B, Ta, audio_in_channels] (bf16 or fp32), contexts [B, S, caption_channels];
+ *   video_sigmas [B], or [B, N] when video_ts_per_token != 0; audio_sigmas [B]; masks [B, S] int32 or NULL;
+ *   out_video [B, N, out_channels], out_audio [B, Ta, audio_in_channels] fp32.
+ * Each item attends within itself only, and its outputs equal those of the B = 1 call on that item alone, bit for bit.
+ * B > 2, and B = 2 on a sequence-parallel (Ulysses) context, return LTX_ERR_UNSUPPORTED; bad sizes or NULL tensors
+ * LTX_ERR_INVALID_ARGUMENT.  Refused calls write nothing.  Host-pointer variant copies in/out and synchronises. */
+int ltx_av_forward_batch(ltx_ctx* ctx, const void* video_latent, ltx_dtype video_dtype, const void* audio_latent,
+                         ltx_dtype audio_dtype, const void* video_context, const void* audio_context, ltx_dtype context_dtype,
+                         const float* video_sigmas, int video_ts_per_token, const float* audio_sigmas, const int32_t* video_mask,
+                         const int32_t* audio_mask, int B, int N, int Ta, int S, int F, int H, int W, uint64_t context_key,
+                         float* out_video, float* out_audio);
+int ltx_av_forward_batch_dev(ltx_ctx* ctx, const void* video_latent, ltx_dtype video_dtype, const void* audio_latent,
+                             ltx_dtype audio_dtype, const void* video_context, const void* audio_context, ltx_dtype context_dtype,
+                             const float* video_sigmas, int video_ts_per_token, const float* audio_sigmas,
+                             const int32_t* video_mask, const int32_t* audio_mask, int B, int N, int Ta, int S, int F, int H, int W,
+                             uint64_t context_key, float* out_video, float* out_audio);
 /* LTXTransformer.clearRoPECache (:202) + drops the cached text K/V. */
 int ltx_dit_clear_caches(ltx_ctx* ctx);
 
@@ -218,8 +237,10 @@ typedef struct {
   int32_t disable_stg_prefix_sharing; /* 0 (default): the STG pass reuses the conditional pass's blocks before the first
                                          perturbed block (identical inputs -> identical values); 1: recompute them */
   int32_t disable_batched_cfg;        /* 0 (default): on one GPU the conditional and unconditional passes run as ONE B = 2
-                                         forward, as denoise() batches them (Pipeline/LTXPipeline.swift:2234-2269); 1: as two
-                                         B = 1 forwards, the way generateVideo issues them (:829-848).  Same values per pass. */
+                                         forward, as denoise() batches them (Pipeline/LTXPipeline.swift:2234-2269) -- in both
+                                         ltx_denoise_step and ltx_av_denoise_step; 1: as two B = 1 forwards, the way
+                                         generateVideo / generateVideoWithAudio issue them (:829-848, :1300-1362).  Same values
+                                         per pass.  LTX_BATCHED_CFG=0 in the environment also selects two forwards. */
 } ltx_step_params;
 /* noise [in_channels, F, H, W] fp32 host; latent = noise * sigma0 (:793).  neg_context may be NULL. */
 int ltx_denoise_begin(ltx_ctx* ctx, const float* noise, int F, int H, int W, float sigma0, const void* context,
@@ -235,7 +256,9 @@ int ltx_denoise_latent_dev(ltx_ctx* ctx, float** latent_dev);
  *   begin : video_noise [in_channels, F, H, W], audio_noise [Ta, audio_in_channels] (the packed audio latent) fp32 host; both
  *           are scaled by sigma0 (:1255-1259); contexts [S, caption_channels]; one mask serves both streams (textMask); the
  *           negative contexts (a pair, or both NULL) enable CFG.
- *   step  : per pass one LTX2Transformer forward (two with CFG, :1300-1362); video = applyCFG (+ rescale) + scheduler.step,
+ *   step  : per pass one LTX2Transformer forward (two with CFG, :1300-1362; on one GPU without Ulysses both passes run as
+ *           one B = 2 forward, item 0 conditional, unless disable_batched_cfg or LTX_BATCHED_CFG=0 -- same values per pass);
+ *           video = applyCFG (+ rescale) + scheduler.step,
  *           audio = applyCFG + latent += (sigma_next - sigma) * velocity (:1402).  Reads sigma, sigma_next, cfg_scale,
  *           rescale_phi and i2v_frame0_conditioned of ltx_step_params (per-token video timesteps sigma * (1 - mask) and an
  *           untouched frame 0, :1293-1298, 1381-1391; set the frame with ltx_denoise_set_frame0); STG / GE are not part of
@@ -374,6 +397,14 @@ int ltx_op_gemm_blocked(ltx_ctx* ctx, const void* A, const void* B, const float*
 /* x[M,N] (fp32) += (A B^T + bias) * (gate_a[n] + gate_b[n]) * scale ; shadow (bf16, nullable) = new x. */
 int ltx_op_gemm_resid(ltx_ctx* ctx, const void* A, const void* B, const float* bias, float* x, const float* gate_a,
                       const float* gate_b, void* shadow, int M, int N, int K, float scale);
+/* The weight-streaming kernel on a batch of `items` (1 or 2) items of up to 32 rows each (M <= 32 * items; two items take its
+ * 64-row form, the dual model's batched audio stream), or an error: C[M,N] = A[M,K] B[N,K]^T + bias[N] with
+ *   mode 0 / 1 / 3 / 4 as ltx_op_gemm (out [M,N]); mode 0 with vt_item_ld > 0: out is V^T [N, items * vt_item_ld], row m of
+ *   item i = m / (M / items) in column i * vt_item_ld + m % (M / items);
+ *   mode 2: x[M,N] += (A B^T + bias) * (gate_a[(m / rows_per_gate) * N + n] + gate_b[n]) (one gate row per item: rows_per_gate
+ *   = M / items; gate_b nullable). */
+int ltx_op_gemm_skinny(ltx_ctx* ctx, const void* A, const void* B, const float* bias, void* out, float* x, const float* gate_a,
+                       const float* gate_b, int rows_per_gate, int M, int N, int K, int mode, int items, int64_t vt_item_ld);
 /* per-64-group affine quantiser / dequantiser and the dequant-fused GEMM (codes [N,K] bytes or [N,K/2] nibbles;
  * scales, biases fp32 [K/64, N]); mode / force_bn as in ltx_op_gemm. */
 int ltx_op_quantize(ltx_ctx* ctx, const void* w_bf16, int N, int K, int bits, void* q_out, float* scales_out, float* biases_out);

@@ -64,6 +64,8 @@ SIGNATURES = {
     "ltx_av_forward_dev": (_I, [_P, _P, _I, _P, _I, _P, _P, _I, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _U64, _P, _P]),
     "ltx_av_forward_tokens": (_I, [_P, _P, _I, _P, _I, _P, _P, _I, _P, _F, _P, _P, _I, _I, _I, _I, _I, _I, _U64, _P, _P]),
     "ltx_av_forward_tokens_dev": (_I, [_P, _P, _I, _P, _I, _P, _P, _I, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _U64, _P, _P]),
+    "ltx_av_forward_batch": (_I, [_P, _P, _I, _P, _I, _P, _P, _I, _P, _I, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _U64, _P, _P]),
+    "ltx_av_forward_batch_dev": (_I, [_P, _P, _I, _P, _I, _P, _P, _I, _P, _I, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _U64, _P, _P]),
     "ltx_dit_clear_caches": (_I, [_P]),
     "ltx_guided_euler_step": (_I, [_P, _P, _P, _P, _P, _P, _I, _SZ, _F, _F, _F, _F, _F, _F]),
     "ltx_guided_euler_step_dev": (_I, [_P, _P, _P, _P, _P, _P, _I, _SZ, _F, _F, _F, _F, _F, _F]),
@@ -105,6 +107,7 @@ SIGNATURES = {
     "ltx_op_gemm": (_I, [_P, _P, _P, _P, _P, _I, _I, _I, _I, _I]),
     "ltx_op_gemm_blocked": (_I, [_P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, C.c_int64, _I]),
     "ltx_op_gemm_resid": (_I, [_P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _F]),
+    "ltx_op_gemm_skinny": (_I, [_P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, C.c_int64]),
     "ltx_op_quantize": (_I, [_P, _P, _I, _I, _I, _P, _P, _P]),
     "ltx_op_dequantize": (_I, [_P, _P, _P, _P, _I, _I, _I, _P]),
     "ltx_op_gemm_q": (_I, [_P, _P, _P, _P, _P, _I, _P, _P, _I, _I, _I, _I, _I]),

@@ -265,21 +265,39 @@ class LtxContext:
                                                  mask_ptr, B, N, S, F, H, W,
                                                  C.byref(flags) if flags is not None else None, out_ptr))
 
-    def av_forward(self, video_latent, audio_latent, video_context, audio_context, video_sigma, audio_sigma: float,
+    def av_forward(self, video_latent, audio_latent, video_context, audio_context, video_sigma, audio_sigma,
                    fhw: Tuple[int, int, int], video_mask=None, audio_mask=None, context_key: int = 0):
-        """LTX2Transformer.callAsFunction: video_latent [1,N,C], audio_latent [1,Ta,Ca], contexts [1,S,Cc] ->
-        (video velocity [1,N,C], audio velocity [1,Ta,Ca]) fp32.  video_sigma: a float, or an array [1,N] / [N] of per-token
-        sigmas (videoTimesteps of the image-to-video mode)."""
+        """LTX2Transformer.callAsFunction: video_latent [B,N,C], audio_latent [B,Ta,Ca], contexts [B,S,Cc], B = 1 or 2 ->
+        (video velocity [B,N,C], audio velocity [B,Ta,Ca]) fp32.  video_sigma: a float, or an array [B] / [1,N] / [N] / [B,N]
+        (per-token sigmas: videoTimesteps of the image-to-video mode); audio_sigma: a float or [B]; masks [B,S] or None.
+        Mismatched batch tensors raise LtxError code 2; B > 2 code 5 (the library's refusal)."""
         vc, ac, cc = _dtype_code(video_latent), _dtype_code(audio_latent), _dtype_code(video_context)
         assert _dtype_code(audio_context) == cc, "both contexts must have the same dtype"
         vl, al, vx, axx = _host(video_latent), _host(audio_latent), _host(video_context), _host(audio_context)
-        assert vl.shape[0] == 1 and al.shape[0] == 1, "the dual model takes B = 1"
-        N, Ta, S = vl.shape[1], al.shape[1], vx.shape[1]
+        B, N, Ta, S = vl.shape[0], vl.shape[1], al.shape[1], vx.shape[1]
         vm = None if video_mask is None else _host(video_mask, np.int32)
         am = None if audio_mask is None else _host(audio_mask, np.int32)
+        F, H, W = fhw
+        if B != 1:
+            vs = _host(np.asarray(video_sigma, dtype=np.float32).reshape(-1), np.float32)
+            as_ = _host(np.asarray(audio_sigma, dtype=np.float32).reshape(-1), np.float32)
+            per_token = vs.size == B * N and vs.size != B
+            ok = (al.shape[0] == B and vx.shape[0] == B and _host(audio_context).shape[:2] == (B, S) and as_.size == B
+                  and (vs.size == B or per_token)
+                  and all(m is None or m.size == B * S for m in (vm, am)))
+            if not ok:
+                raise LtxError(2, "dual forward: batch tensors must all have B items ([B,N,C], [B,Ta,Ca], [B,S,Cc], "
+                                  "sigmas [B] / [B,N], masks [B,S])")
+            ov = np.full((B, N, self.config.out_channels), np.nan, dtype=np.float32)
+            oa = np.full((B, Ta, self.config.audio_in_channels), np.nan, dtype=np.float32)
+            self._check(self.lib.ltx_av_forward_batch(self.handle, _ptr(vl), vc, _ptr(al), ac, _ptr(vx), _ptr(axx), cc, _ptr(vs),
+                                                      int(per_token), _ptr(as_), _ptr(vm), _ptr(am), B, N, Ta, S, F, H, W,
+                                                      int(context_key), _ptr(ov), _ptr(oa)))
+            return ov, oa
+        assert al.shape[0] == 1, "video and audio latents must have the same batch"
         ov = np.empty((1, N, self.config.out_channels), dtype=np.float32)
         oa = np.empty((1, Ta, self.config.audio_in_channels), dtype=np.float32)
-        F, H, W = fhw
+        audio_sigma = float(np.asarray(audio_sigma).reshape(-1)[0])
         if not np.isscalar(video_sigma) and np.asarray(video_sigma).size > 1:
             vs = np.ascontiguousarray(_host(video_sigma, np.float32).reshape(-1))
             assert vs.size == N, "per-token video sigmas must have N entries"
@@ -398,9 +416,11 @@ class LtxContext:
         self._av_session_audio_shape = (Ta, self.config.audio_in_channels)
 
     def av_denoise_step(self, sigma: float, sigma_next: float, step_index: int = 0, cfg_scale: float = 1.0,
-                        rescale_phi: float = 0.0, i2v_frame0_conditioned: bool = False):
+                        rescale_phi: float = 0.0, i2v_frame0_conditioned: bool = False, batched_cfg: bool = True):
+        """batched_cfg: with CFG on one GPU, run the conditional and unconditional passes as one B = 2 forward (same values)."""
         p = LtxStepParams()
         p.i2v_frame0_conditioned = int(i2v_frame0_conditioned)
+        p.disable_batched_cfg = 0 if batched_cfg else 1
         p.sigma, p.sigma_next, p.cfg_scale, p.rescale_phi, p.step_index = sigma, sigma_next, cfg_scale, rescale_phi, step_index
         self._check(self.lib.ltx_av_denoise_step(self.handle, C.byref(p)))
 

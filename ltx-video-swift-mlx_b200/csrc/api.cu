@@ -253,7 +253,7 @@ int ltx_ctx_destroy(ltx_ctx* c) {
                     &c->v_lat, &c->v_noise, &c->v_frames, &c->v_mix, &c->v_te, &c->v_split, &c->v_pad2, &c->snap_x, &c->s_ts, &c->f_asplit, &c->f_wsplit, &c->f_h,
                     &c->f_q, &c->f_k, &c->f_v, &c->f_att, &c->f_ffh, &c->f_ctx, &c->f_c1, &c->f_c2, &c->f_tk, &c->f_tv, &c->f_lat,
                     &c->f_bias, &c->q_panel, &c->gemm_ws, &c->u_part, &c->u_ab, &c->u_stats, &c->u_in, &c->u_out, &c->u_ref, &c->av.ws, &c->av.a_cos, &c->av.a_sin, &c->av.xv_cos, &c->av.xv_sin, &c->av_in[0], &c->av_in[1], &c->av_in[2], &c->av_in[3], &c->av_in[4], &c->av_in[5], &c->av_in[6], &c->av_in[7],
-                    &c->v_tile_lat, &c->v_tile_noise, &c->v_tile_frames, &c->s_alat, &c->s_avc, &c->s_avu, &c->s_actx_pos, &c->s_actx_neg};
+                    &c->v_tile_lat, &c->v_tile_noise, &c->v_tile_frames, &c->s_alat, &c->s_avc, &c->s_avu, &c->s_actx_pos, &c->s_actx_neg, &c->s_alat_pair, &c->s_actx_pair};
   for (DevBuf* b : bufs) b->release();
   for (auto& t : c->text) { t.k.release(); t.vt.release(); t.bias.release(); }
   for (auto& t : c->av.text) { t.k.release(); t.vt.release(); t.bias.release(); }
@@ -535,51 +535,73 @@ int ltx_av_forward_tokens_dev(ltx_ctx* c, const void* video_latent, ltx_dtype vi
   });
 }
 
-// host-buffer form of the dual forward; video_sigmas holds one value, or N when per_token
+// refusals of the batched dual forward that come before any work: B outside 1..2, B = 2 under Ulysses, null tensors
+static void av_batch_check(ltx_ctx* c, int B, const void* vl, const void* al, const void* vc, const void* ac, const float* vs,
+                           const float* as, const void* ov, const void* oa) {
+  LTX_CHECK(B >= 1, LTX_ERR_INVALID_ARGUMENT, "dual forward: B must be >= 1");
+  LTX_CHECK(B <= 2, LTX_ERR_UNSUPPORTED, "dual forward: batches of 1 or 2 items");
+  LTX_CHECK(B == 1 || !(c->dist.comm_world && c->dist.sp > 1), LTX_ERR_UNSUPPORTED, "the batched dual forward is single-GPU");
+  LTX_CHECK(vl && al && vc && ac && vs && as && ov && oa, LTX_ERR_INVALID_ARGUMENT, "null tensor");
+}
+
+int ltx_av_forward_batch_dev(ltx_ctx* c, const void* video_latent, ltx_dtype video_dtype, const void* audio_latent,
+                             ltx_dtype audio_dtype, const void* video_context, const void* audio_context, ltx_dtype context_dtype,
+                             const float* video_sigmas, int video_ts_per_token, const float* audio_sigmas,
+                             const int32_t* video_mask, const int32_t* audio_mask, int B, int N, int Ta, int S, int F, int H, int W,
+                             uint64_t context_key, float* out_video, float* out_audio) {
+  return guarded(c, [&] {
+    av_batch_check(c, B, video_latent, audio_latent, video_context, audio_context, video_sigmas, audio_sigmas, out_video, out_audio);
+    dit_av_forward_dev(c, video_latent, video_dtype, audio_latent, audio_dtype, video_context, audio_context, context_dtype,
+                       video_sigmas, video_ts_per_token ? 1 : 0, audio_sigmas, video_mask, audio_mask, B, N, Ta, S, F, H, W,
+                       context_key, out_video, out_audio);
+  });
+}
+
+// host-buffer form of the dual forward for B items; video_sigmas holds B values, or B * N when per_token; audio_sigmas B
 static int av_forward_host(ltx_ctx* c, const void* video_latent, ltx_dtype video_dtype, const void* audio_latent,
                            ltx_dtype audio_dtype, const void* video_context, const void* audio_context, ltx_dtype context_dtype,
-                           const float* video_sigmas, int per_token, float audio_sigma, const int32_t* video_mask,
-                           const int32_t* audio_mask, int N, int Ta, int S, int F, int H, int W, uint64_t context_key,
+                           const float* video_sigmas, int per_token, const float* audio_sigmas, const int32_t* video_mask,
+                           const int32_t* audio_mask, int B, int N, int Ta, int S, int F, int H, int W, uint64_t context_key,
                            float* out_video, float* out_audio) {
   return guarded(c, [&] {
-    LTX_CHECK(video_latent && audio_latent && video_context && audio_context && video_sigmas && out_video && out_audio, LTX_ERR_INVALID_ARGUMENT,
-              "null tensor");
+    av_batch_check(c, B, video_latent, audio_latent, video_context, audio_context, video_sigmas, audio_sigmas, out_video, out_audio);
     LTX_CHECK(N >= 1 && Ta >= 1 && S >= 1 && c->av.ready, LTX_ERR_INVALID_ARGUMENT, "bad sizes, or dual-model weights not finalized");
     const ltx_config& g = c->cfg;
     const int Ca = c->av.Cin;
     DevBuf* b = c->av_in;   // staged host inputs: video latent, audio latent, contexts, sigmas, masks, outputs
-    h2d(c, b[0], video_latent, static_cast<size_t>(N) * g.in_channels * dsize(video_dtype));
-    h2d(c, b[1], audio_latent, static_cast<size_t>(Ta) * Ca * dsize(audio_dtype));
-    const size_t cbytes = static_cast<size_t>(S) * g.caption_channels * dsize(context_dtype);
+    h2d(c, b[0], video_latent, static_cast<size_t>(B) * N * g.in_channels * dsize(video_dtype));
+    h2d(c, b[1], audio_latent, static_cast<size_t>(B) * Ta * Ca * dsize(audio_dtype));
+    const size_t cbytes = static_cast<size_t>(B) * S * g.caption_channels * dsize(context_dtype), nm = static_cast<size_t>(B) * S;
     h2d(c, b[2], video_context, cbytes);
     h2d(c, b[3], audio_context, cbytes);
-    // sigmas: [audio, video...] so the video values start 4-byte aligned right behind the audio one
-    const size_t nvs = per_token ? static_cast<size_t>(N) : 1;
-    b[4].reserve((1 + nvs) * 4);
-    LTX_CUDA(cudaMemcpyAsync(b[4].ptr, &audio_sigma, 4, cudaMemcpyHostToDevice, c->stream));
-    LTX_CUDA(cudaMemcpyAsync(b[4].as<float>() + 1, video_sigmas, nvs * 4, cudaMemcpyHostToDevice, c->stream));
+    // sigmas: [audio x B, video...] so the video values start 4-byte aligned right behind the audio ones
+    const size_t nvs = static_cast<size_t>(B) * (per_token ? N : 1);
+    b[4].reserve((B + nvs) * 4);
+    LTX_CUDA(cudaMemcpyAsync(b[4].ptr, audio_sigmas, B * 4, cudaMemcpyHostToDevice, c->stream));
+    LTX_CUDA(cudaMemcpyAsync(b[4].as<float>() + B, video_sigmas, nvs * 4, cudaMemcpyHostToDevice, c->stream));
     const int32_t *vm = nullptr, *am = nullptr;
-    b[5].reserve(static_cast<size_t>(2) * S * 4);
+    b[5].reserve(2 * nm * 4);
     if (video_mask) {
-      LTX_CUDA(cudaMemcpyAsync(b[5].ptr, video_mask, static_cast<size_t>(S) * 4, cudaMemcpyHostToDevice, c->stream));
+      LTX_CUDA(cudaMemcpyAsync(b[5].ptr, video_mask, nm * 4, cudaMemcpyHostToDevice, c->stream));
       vm = b[5].as<int32_t>();
     }
     if (audio_mask) {
-      LTX_CUDA(cudaMemcpyAsync(b[5].as<int32_t>() + S, audio_mask, static_cast<size_t>(S) * 4, cudaMemcpyHostToDevice, c->stream));
-      am = b[5].as<int32_t>() + S;
+      LTX_CUDA(cudaMemcpyAsync(b[5].as<int32_t>() + nm, audio_mask, nm * 4, cudaMemcpyHostToDevice, c->stream));
+      am = b[5].as<int32_t>() + nm;
     }
-    b[6].reserve(static_cast<size_t>(N) * g.out_channels * 4);
-    b[7].reserve(static_cast<size_t>(Ta) * Ca * 4);
-    const uint64_t fpv = context_key ? host_text_fingerprint(video_context, cbytes, video_mask, static_cast<size_t>(S)) : 0;
-    const uint64_t fpa = context_key ? host_text_fingerprint(audio_context, cbytes, audio_mask, static_cast<size_t>(S)) : 0;
+    const size_t nov = static_cast<size_t>(B) * N * g.out_channels, noa = static_cast<size_t>(B) * Ta * Ca;
+    b[6].reserve(nov * 4);
+    b[7].reserve(noa * 4);
+    const uint64_t fpv = context_key ? host_text_fingerprint(video_context, cbytes, video_mask, nm) : 0;
+    const uint64_t fpa = context_key ? host_text_fingerprint(audio_context, cbytes, audio_mask, nm) : 0;
     text_cache_guard(c->text, context_key, fpv);
     text_cache_guard(c->av.text, context_key, fpa);
-    dit_av_forward_dev(c, b[0].ptr, video_dtype, b[1].ptr, audio_dtype, b[2].ptr, b[3].ptr, context_dtype, b[4].as<float>() + 1,
-                       per_token, b[4].as<float>(), vm, am, 1, N, Ta, S, F, H, W, context_key, b[6].as<float>(), b[7].as<float>());
+    dit_av_forward_dev(c, b[0].ptr, video_dtype, b[1].ptr, audio_dtype, b[2].ptr, b[3].ptr, context_dtype, b[4].as<float>() + B,
+                       per_token, b[4].as<float>(), vm, am, B, N, Ta, S, F, H, W, context_key, b[6].as<float>(), b[7].as<float>());
     text_cache_stamp(c->text, context_key, fpv);
     text_cache_stamp(c->av.text, context_key, fpa);
-    LTX_CUDA(cudaMemcpyAsync(out_video, b[6].ptr, static_cast<size_t>(N) * g.out_channels * 4, cudaMemcpyDeviceToHost, c->stream));
-    LTX_CUDA(cudaMemcpyAsync(out_audio, b[7].ptr, static_cast<size_t>(Ta) * Ca * 4, cudaMemcpyDeviceToHost, c->stream));
+    LTX_CUDA(cudaMemcpyAsync(out_video, b[6].ptr, nov * 4, cudaMemcpyDeviceToHost, c->stream));
+    LTX_CUDA(cudaMemcpyAsync(out_audio, b[7].ptr, noa * 4, cudaMemcpyDeviceToHost, c->stream));
     LTX_CUDA(cudaStreamSynchronize(c->stream));
   });
 }
@@ -589,7 +611,17 @@ int ltx_av_forward(ltx_ctx* c, const void* video_latent, ltx_dtype video_dtype, 
                    float audio_sigma, const int32_t* video_mask, const int32_t* audio_mask, int N, int Ta, int S, int F, int H,
                    int W, uint64_t context_key, float* out_video, float* out_audio) {
   return av_forward_host(c, video_latent, video_dtype, audio_latent, audio_dtype, video_context, audio_context, context_dtype,
-                         &video_sigma, 0, audio_sigma, video_mask, audio_mask, N, Ta, S, F, H, W, context_key, out_video, out_audio);
+                         &video_sigma, 0, &audio_sigma, video_mask, audio_mask, 1, N, Ta, S, F, H, W, context_key, out_video, out_audio);
+}
+
+int ltx_av_forward_batch(ltx_ctx* c, const void* video_latent, ltx_dtype video_dtype, const void* audio_latent,
+                         ltx_dtype audio_dtype, const void* video_context, const void* audio_context, ltx_dtype context_dtype,
+                         const float* video_sigmas, int video_ts_per_token, const float* audio_sigmas, const int32_t* video_mask,
+                         const int32_t* audio_mask, int B, int N, int Ta, int S, int F, int H, int W, uint64_t context_key,
+                         float* out_video, float* out_audio) {
+  return av_forward_host(c, video_latent, video_dtype, audio_latent, audio_dtype, video_context, audio_context, context_dtype,
+                         video_sigmas, video_ts_per_token ? 1 : 0, audio_sigmas, video_mask, audio_mask, B, N, Ta, S, F, H, W,
+                         context_key, out_video, out_audio);
 }
 
 int ltx_av_forward_tokens(ltx_ctx* c, const void* video_latent, ltx_dtype video_dtype, const void* audio_latent,
@@ -597,7 +629,7 @@ int ltx_av_forward_tokens(ltx_ctx* c, const void* video_latent, ltx_dtype video_
                           const float* video_sigmas, float audio_sigma, const int32_t* video_mask, const int32_t* audio_mask, int N,
                           int Ta, int S, int F, int H, int W, uint64_t context_key, float* out_video, float* out_audio) {
   return av_forward_host(c, video_latent, video_dtype, audio_latent, audio_dtype, video_context, audio_context, context_dtype,
-                         video_sigmas, 1, audio_sigma, video_mask, audio_mask, N, Ta, S, F, H, W, context_key, out_video, out_audio);
+                         video_sigmas, 1, &audio_sigma, video_mask, audio_mask, 1, N, Ta, S, F, H, W, context_key, out_video, out_audio);
 }
 
 int ltx_dit_clear_caches(ltx_ctx* c) {
@@ -701,6 +733,11 @@ int ltx_denoise_begin(ltx_ctx* c, const float* noise, int F, int H, int W, float
 }
 
 namespace {
+// LTX_BATCHED_CFG=0: the guidance passes of both denoise loops run as separate B = 1 forwards
+bool batched_cfg_env() {
+  static const bool on = [] { const char* e = getenv("LTX_BATCHED_CFG"); return e ? atoi(e) != 0 : true; }();
+  return on;
+}
 // (re)sizes the per-session work buffers for a [C, F, H, W] latent and records the geometry
 void session_resize(ltx_ctx* c, int F, int H, int W) {
   const size_t n = static_cast<size_t>(c->cfg.in_channels) * F * H * W;
@@ -825,8 +862,7 @@ int ltx_denoise_step(ltx_ctx* c, const ltx_step_params* p) {
     // better (N = 4096 GEMMs: 192 tiles instead of 2 x 96 on 74 CTA pairs; attention: 768 CTAs instead of 2 x 384 on 296
     // slots) and the weights are read once.  Batch row 0 is the conditional pass, so the STG pass can still resume from its
     // stream.  Per batch row the arithmetic is that of the separate passes.
-    static const bool batched_on = [] { const char* e = getenv("LTX_BATCHED_CFG"); return e ? atoi(e) != 0 : true; }();
-    const bool batched = batched_on && use_cfg && groups == 1 && !(c->dist.comm_world && c->dist.sp > 1) && c->precision == 16 &&
+    const bool batched = batched_cfg_env() && use_cfg && groups == 1 && !(c->dist.comm_world && c->dist.sp > 1) && c->precision == 16 &&
                          !p->disable_batched_cfg;
     const int stg_idx = use_stg ? n_pass - 1 : -1;
     const bool share = use_stg && !p->disable_stg_prefix_sharing && first_stg > 0 && first_stg < g.num_layers &&
@@ -953,8 +989,26 @@ int ltx_av_denoise_begin(ltx_ctx* c, const float* video_noise, const float* audi
       h2d(c, c->s_actx_neg, neg_audio_context, cbytes);
       c->s_has_mask_neg = neg_mask != nullptr;
       if (neg_mask) h2d(c, c->s_mask_neg, neg_mask, static_cast<size_t>(S) * 4);
+      // inputs of the batched guidance forward: both prompts of each stream in one [2, S, Cc] buffer, one [2, S] mask when
+      // either prompt has one (all ones for the other), room for two latents / velocities of each stream
+      c->s_ctx_pair.reserve(2 * cbytes);
+      c->s_actx_pair.reserve(2 * cbytes);
+      LTX_CUDA(cudaMemcpyAsync(c->s_ctx_pair.ptr, c->s_ctx_pos.ptr, cbytes, cudaMemcpyDeviceToDevice, c->stream));
+      LTX_CUDA(cudaMemcpyAsync(c->s_ctx_pair.as<uint8_t>() + cbytes, c->s_ctx_neg.ptr, cbytes, cudaMemcpyDeviceToDevice, c->stream));
+      LTX_CUDA(cudaMemcpyAsync(c->s_actx_pair.ptr, c->s_actx_pos.ptr, cbytes, cudaMemcpyDeviceToDevice, c->stream));
+      LTX_CUDA(cudaMemcpyAsync(c->s_actx_pair.as<uint8_t>() + cbytes, c->s_actx_neg.ptr, cbytes, cudaMemcpyDeviceToDevice, c->stream));
+      if (mask || neg_mask) {
+        std::vector<int32_t> pm(static_cast<size_t>(2) * S, 1);
+        if (mask) memcpy(pm.data(), mask, static_cast<size_t>(S) * 4);
+        if (neg_mask) memcpy(pm.data() + S, neg_mask, static_cast<size_t>(S) * 4);
+        h2d(c, c->s_mask_pair, pm.data(), pm.size() * 4);
+        LTX_CUDA(cudaStreamSynchronize(c->stream));   // pm goes out of scope
+      }
+      c->s_tok.reserve(2 * n * 2);
+      c->vel.reserve(2 * n * 4);
+      c->s_alat_pair.reserve(2 * na * 4);
     }
-    c->s_avc.reserve(na * 4);
+    c->s_avc.reserve((c->s_has_neg ? 2 : 1) * na * 4);   // batched: [conditional | unconditional] audio velocities
     c->s_avu.reserve(na * 4);
     c->scratch.reserve(64 * sizeof(double));
     c->s_serial += 2;
@@ -978,17 +1032,26 @@ int ltx_av_denoise_step(ltx_ctx* c, const ltx_step_params* p) {
       ProfScope ps(c, PROF_OTHER, 0.0, 6.0 * n);
       launch_patchify(c->s_latent.as<float>(), c->s_tok.as<bf16>(), nullptr, C, T, st);
     }
-    LTX_CUDA(cudaMemcpyAsync(c->s_sigma.ptr, &p->sigma, 4, cudaMemcpyHostToDevice, st));
+    const bool use_cfg = p->cfg_scale > 1.0f && c->s_has_neg;
+    // Conditional + unconditional as ONE B = 2 forward on one GPU (as ltx_denoise_step does): the audio stream's Linears read
+    // their weights once for both prompts and the video stream's GEMMs / attention fill their waves better.  Item 0 is the
+    // conditional pass; per item the arithmetic is that of the separate passes.
+    const bool batched = batched_cfg_env() && use_cfg && c->dist.groups == 1 && !(c->dist.comm_world && c->dist.sp > 1) &&
+                         !p->disable_batched_cfg;
+    const int nb = batched ? 2 : 1;
+    const float sig2[2] = {p->sigma, p->sigma};   // one sigma per item, for both streams
+    LTX_CUDA(cudaMemcpyAsync(c->s_sigma.ptr, sig2, 8, cudaMemcpyHostToDevice, st));
     // image-to-video (:1293-1298): video timesteps sigma * (1 - conditioningMask) per token; the audio stream keeps sigma
     const bool i2v = p->i2v_frame0_conditioned != 0;
     const float* ts_dev = c->s_sigma.as<float>();
     if (i2v) {
-      c->s_ts.reserve(static_cast<size_t>(T) * 4);
-      ProfScope ps(c, PROF_OTHER, 0.0, 4.0 * T);
-      launch_fill_token_timesteps(c->s_ts.as<float>(), T, T, H * W, c->s_sigma.as<float>(), st);
+      c->s_ts.reserve(static_cast<size_t>(nb) * T * 4);
+      ProfScope ps(c, PROF_OTHER, 0.0, 4.0 * nb * T);
+      launch_fill_token_timesteps(c->s_ts.as<float>(), nb * T, T, H * W, c->s_sigma.as<float>(), st);
       ts_dev = c->s_ts.as<float>();
     }
     const uint64_t key_pos = 0x6000000000000000ull + c->s_serial, key_neg = key_pos + 1;
+    const uint64_t key_pair = 0x6800000000000000ull + c->s_serial;
     auto pass = [&](bool neg, float* v_lat, float* a_vel) {
       const int32_t* mk = neg ? (c->s_has_mask_neg ? c->s_mask_neg.as<int32_t>() : nullptr)
                               : (c->s_has_mask_pos ? c->s_mask_pos.as<int32_t>() : nullptr);
@@ -998,9 +1061,24 @@ int ltx_av_denoise_step(ltx_ctx* c, const ltx_step_params* p) {
       ProfScope ps(c, PROF_OTHER, 0.0, 8.0 * n);
       launch_unpatchify(c->vel.as<float>(), v_lat, C, T, st);
     };
-    const bool use_cfg = p->cfg_scale > 1.0f && c->s_has_neg;
-    pass(false, c->s_vc.as<float>(), c->s_avc.as<float>());
-    if (use_cfg) pass(true, c->s_vu.as<float>(), c->s_avu.as<float>());
+    float* avu = c->s_avu.as<float>();
+    if (batched) {
+      bf16* tok = c->s_tok.as<bf16>();
+      float* alat2 = c->s_alat_pair.as<float>();
+      LTX_CUDA(cudaMemcpyAsync(tok + n, tok, n * 2, cudaMemcpyDeviceToDevice, st));   // the same latents under both prompts
+      LTX_CUDA(cudaMemcpyAsync(alat2, c->s_alat.ptr, na * 4, cudaMemcpyDeviceToDevice, st));
+      LTX_CUDA(cudaMemcpyAsync(alat2 + na, c->s_alat.ptr, na * 4, cudaMemcpyDeviceToDevice, st));
+      const int32_t* mk = (c->s_has_mask_pos || c->s_has_mask_neg) ? c->s_mask_pair.as<int32_t>() : nullptr;
+      avu = c->s_avc.as<float>() + na;
+      dit_av_forward_dev(c, tok, LTX_BF16, alat2, LTX_F32, c->s_ctx_pair.ptr, c->s_actx_pair.ptr, c->s_ctx_dtype, ts_dev, i2v ? 1 : 0,
+                         c->s_sigma.as<float>(), mk, mk, 2, T, Ta, S, F, H, W, key_pair, c->vel.as<float>(), c->s_avc.as<float>());
+      ProfScope ps(c, PROF_OTHER, 0.0, 16.0 * n, 2);
+      launch_unpatchify(c->vel.as<float>(), c->s_vc.as<float>(), C, T, st);
+      launch_unpatchify(c->vel.as<float>() + n, c->s_vu.as<float>(), C, T, st);
+    } else {
+      pass(false, c->s_vc.as<float>(), c->s_avc.as<float>());
+      if (use_cfg) pass(true, c->s_vu.as<float>(), avu);
+    }
     // video: applyCFG (+ rescale) + scheduler.step, frame 0 untouched in the image-to-video mode (:1364-1391)
     GuidedEulerArgs a;
     a.latent = c->s_latent.as<float>(); a.v_cond = c->s_vc.as<float>();
@@ -1014,7 +1092,7 @@ int ltx_av_denoise_step(ltx_ctx* c, const ltx_step_params* p) {
     launch_guided_euler(a, st);
     // audio: applyCFG + a += (sigma' - sigma) v (:1402)
     const float dt = static_cast<float>(static_cast<double>(p->sigma_next) - static_cast<double>(p->sigma));
-    launch_audio_cfg_euler(c->s_alat.as<float>(), c->s_avc.as<float>(), use_cfg ? c->s_avu.as<float>() : nullptr, p->cfg_scale, dt,
+    launch_audio_cfg_euler(c->s_alat.as<float>(), c->s_avc.as<float>(), use_cfg ? avu : nullptr, p->cfg_scale, dt,
                            static_cast<int64_t>(na), st);
   });
 }
@@ -1200,7 +1278,31 @@ int ltx_op_gemm_resid(ltx_ctx* c, const void* A, const void* B, const float* bia
     e.rows_per_gate = M > 0 ? M : 1; e.shadow = reinterpret_cast<bf16*>(shadow); e.lds = N; e.scale = scale;
     if (M > 32 && M <= 512) gemm_attach_workspace(c, e);   // as the DiT forward does for few-row problems (swap-AB kernel)
     launch_gemm(reinterpret_cast<const bf16*>(A), K, reinterpret_cast<const bf16*>(B), K, M, N, K, e, c->stream, 0, 0, 0,
-                1 /* M <= 32: the weight-streaming kernel, as on the dual model's audio stream */);
+                32 /* M <= 32: the weight-streaming kernel, as on the dual model's audio stream */);
+    c->launches++;
+  });
+}
+
+int ltx_op_gemm_skinny(ltx_ctx* c, const void* A, const void* B, const float* bias, void* out, float* x, const float* gate_a,
+                       const float* gate_b, int rows_per_gate, int M, int N, int K, int mode, int items, int64_t vt_item_ld) {
+  return guarded(c, [&] {
+    LTX_CHECK(A && B && (mode == EPI_GATE_RESID ? x != nullptr : out != nullptr) && (items == 1 || items == 2) &&
+                  (vt_item_ld == 0 || (M % items == 0 && vt_item_ld >= M / items)),
+              LTX_ERR_INVALID_ARGUMENT, "bad skinny GEMM arguments");
+    LTX_CHECK(mode >= EPI_BF16 && mode <= EPI_SILU_BF16 && (vt_item_ld == 0 || mode == EPI_BF16), LTX_ERR_INVALID_ARGUMENT, "bad mode");
+    GemmEpi e;
+    e.mode = mode; e.bias = bias;
+    if (mode == EPI_GATE_RESID) {
+      e.resid = x; e.ldr = N; e.gate_a = gate_a; e.gate_b = gate_b; e.gate_ld = N;
+      e.rows_per_gate = rows_per_gate > 0 ? rows_per_gate : M;
+    } else if (vt_item_ld > 0) {
+      e.out = out; e.ldo = items * vt_item_ld; e.transpose_out = 1;
+      if (items > 1) { e.t_item_rows = M / items; e.t_item_ld = vt_item_ld; }
+    } else {
+      e.out = out; e.ldo = N;
+    }
+    LTX_CHECK(gemm_skinny_eligible(K, K, M, N, K, e, 0, 32 * items), LTX_ERR_INVALID_ARGUMENT, "shape not eligible for the skinny GEMM");
+    launch_gemm(reinterpret_cast<const bf16*>(A), K, reinterpret_cast<const bf16*>(B), K, M, N, K, e, c->stream, 0, 0, 0, 32 * items);
     c->launches++;
   });
 }

@@ -266,6 +266,7 @@ struct ltx_ctx {
   uint64_t s_serial = 0;
   // audio + video session (ltx_av_denoise_*): audio latent / velocities [Ta, Ca] fp32, audio contexts
   ltx::DevBuf s_alat, s_avc, s_avu, s_actx_pos, s_actx_neg;
+  ltx::DevBuf s_alat_pair, s_actx_pair;   // [2, Ta, Ca] / [2, S, Cc]: inputs of the batched guidance forward
   int s_Ta = 0;
 
   // ---- VAE workspaces

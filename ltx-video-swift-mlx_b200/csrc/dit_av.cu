@@ -4,14 +4,17 @@
 // RMSNorms in front of every sub-layer, and two cross-modal attentions per block (audio -> video, video -> audio) whose
 // queries / keys carry temporal-only RoPE and whose modulation comes from four extra AdaLN-single embedders.
 //
-// Streams (token-major rows):  video x fp32 [N, D] (D = 4096),  audio ax fp32 [Ta, Da] (Da = 2048).
+// Streams (token-major rows):  video x fp32 [B*N, D] (D = 4096),  audio ax fp32 [B*Ta, Da] (Da = 2048), B = 1 or 2 items
+// (the conditional and unconditional passes of a CFG step as one batched forward).
 // Everything GEMM-shaped runs on gemm_bf16_tcgen05 / gemm_bf16_2cta, every attention on attention_fwd_tcgen05 (head_dim 128
 // for the video stream, 64 for audio and cross-modal); the learned-weight norm + modulation and the head_dim-generic q/k
 // norm + RoPE are the two row kernels below.  Text K / V of both streams are step-invariant and cached like the video-only
 // model's.  The video sigma is one scalar, or one value per video token (the image-to-video mode feeds sigma * (1 - mask),
 // Pipeline/LTXPipeline.swift:1293-1298; every video-side embedder then runs per token, LTX2Transformer.swift:273-298).
 // Weights: bf16, or int8 / int4 codes through the dequant-fused GEMM (quantize(model: ltx2, ...), Pipeline/LTXPipeline.swift:491).
-// Restrictions of this version: B = 1, single GPU.
+// Every per-row kernel and GEMM row gives each item the arithmetic of its B = 1 forward: at B = 2 the audio stream's
+// 2 x Ta <= 64 rows take the 64-row form of the weight-streaming GEMM, and every modulation / gate / RoPE row is looked
+// up per item (or per token).  Restrictions of this version: B <= 2, single GPU.
 #include <algorithm>
 #include <cmath>
 
@@ -38,12 +41,15 @@ __device__ __forceinline__ float block_sum_256(float v, float* red) {
 // T/LTX2TransformerBlock.swift:208-281; one row per CTA.
 __global__ void __launch_bounds__(256) rmsnorm_w_mod_kernel(const float* x, bf16* out, int D, const float* w, const float* sc_t,
                                                              const float* sc_a, const float* sh_t, const float* sh_a, int64_t a_ld,
-                                                             float eps) {
+                                                             int a_rpr, float eps) {
   __shared__ float red[8];
   griddep_launch();
   griddep_wait();
   const int row = blockIdx.x;
-  if (sc_a) { sc_a += row * a_ld; sh_a += row * a_ld; }   // a_ld > 0: one modulation row per token (per-token sigmas)
+  if (sc_a) {   // a_ld > 0: one modulation row per a_rpr rows (1: per token, N / Ta: per batch item)
+    sc_a += (row / a_rpr) * a_ld;
+    sh_a += (row / a_rpr) * a_ld;
+  }
   const float4* xr = reinterpret_cast<const float4*>(x + static_cast<int64_t>(row) * D);
   const int nv = D >> 2;
   float ss = 0.f;
@@ -74,7 +80,8 @@ __global__ void __launch_bounds__(256) rmsnorm_w_mod_kernel(const float* x, bf16
 struct ModSet {
   const float *sc_t, *sc_a, *sh_t, *sh_a;
   bf16* out;
-  int64_t a_ld;   // 0: sc_a / sh_a are one vector shared by all rows; > 0: row r uses sc_a + r * a_ld (per-token sigmas)
+  int64_t a_ld;   // 0: sc_a / sh_a are one vector shared by all rows; > 0: row r uses sc_a + (r / rpr) * a_ld
+  int rpr;        // rows per modulation row: 1 (per-token sigmas) or the rows of one batch item
 };
 template <int VPT, int ROWS, int NOUT>
 __global__ void __launch_bounds__(256) rmsnorm_w_mod_fast_kernel(const float* x, int M, const float* w, const ModSet m0,
@@ -138,7 +145,8 @@ __global__ void __launch_bounds__(256) rmsnorm_w_mod_fast_kernel(const float* x,
     for (int rr = 0; rr < ROWS; ++rr) {
       const int row = row0 + rr;
       if (row >= M) break;
-      if (m.a_ld != 0) combine(static_cast<int64_t>(row) * m.a_ld);
+      // a new modulation row: the first row of the CTA, and every row whose token (rpr = 1) or batch item differs
+      if (m.a_ld != 0 && (rr == 0 || row / m.rpr != (row - 1) / m.rpr)) combine(static_cast<int64_t>(row / m.rpr) * m.a_ld);
       uint2* orow = reinterpret_cast<uint2*>(m.out + static_cast<int64_t>(row) * D);
 #pragma unroll
       for (int k = 0; k < VPT; ++k)
@@ -211,7 +219,10 @@ __global__ void __launch_bounds__(256) qknorm_rope_hd_kernel(bf16* x, int64_t ld
 }
 
 // ---------------------------------------------------------------- profiled launch helpers
-void gemm(ltx_ctx* c, const bf16* A, int64_t lda, const bf16* B, int64_t ldb, int M, int N, int K, const GemmEpi& e) {
+// items: batch items whose rows make up M (1 or 2).  The weight-streaming kernel takes up to 32 rows per item, so a row of a
+// two-item product runs on the kernel its one-item product runs on.
+void gemm(ltx_ctx* c, const bf16* A, int64_t lda, const bf16* B, int64_t ldb, int M, int N, int K, const GemmEpi& e,
+          int items = 1) {
   auto it = c->qw.empty() ? c->qw.end() : c->qw.find(B);
   const bool panel = it != c->qw.end() && it->second.scratch != nullptr && M >= 257;
   ProfScope ps(c, PROF_GEMM, 2.0 * M * N * K, 2.0 * (static_cast<double>(M) * K + static_cast<double>(N) * K + static_cast<double>(M) * N),
@@ -220,67 +231,85 @@ void gemm(ltx_ctx* c, const bf16* A, int64_t lda, const bf16* B, int64_t ldb, in
     launch_gemm_q(A, lda, it->second, M, N, K, e, c->stream);
     return;
   }
-  launch_gemm(A, lda, B, ldb, M, N, K, e, c->stream, 0, 0, 0, 1);   // the audio stream's M <= 32 Linears stream their weights
+  launch_gemm(A, lda, B, ldb, M, N, K, e, c->stream, 0, 0, 0, 32 * items);   // the audio stream's Linears stream their weights
 }
 // out_bf16[M, N] = A W^T + b
-void linear(ltx_ctx* c, const bf16* A, int M, int K, const bf16* W, const float* b, int N, bf16* out, int mode = EPI_BF16) {
+void linear(ltx_ctx* c, const bf16* A, int M, int K, const bf16* W, const float* b, int N, bf16* out, int mode = EPI_BF16,
+            int items = 1) {
   GemmEpi e;
   e.mode = mode; e.out = out; e.ldo = N; e.bias = b;
-  gemm(c, A, K, W, K, M, N, K, e);
+  gemm(c, A, K, W, K, M, N, K, e, items);
 }
-// x[M, N] (fp32) += (A W^T + b) * (gate_a[n] + gate_b[n])   (null gates: 1)
+// x[M, N] (fp32) += (A W^T + b) * (gate_a[(m / gate_rows) * gate_ld + n] + gate_b[n])   (null gates: 1); gate_ld = 0: one
+// gate row for all M rows
 void linear_resid(ltx_ctx* c, const bf16* A, int M, int K, const bf16* W, const float* b, int N, float* x, const float* gate_a,
-                  const float* gate_b, int64_t gate_ld = 0) {
+                  const float* gate_b, int64_t gate_ld = 0, int gate_rows = 1, int items = 1) {
   GemmEpi e;
   e.mode = EPI_GATE_RESID; e.resid = x; e.ldr = N; e.bias = b; e.gate_a = gate_a; e.gate_b = gate_b; e.gate_ld = gate_ld;
-  e.rows_per_gate = gate_ld > 0 ? 1 : (M > 0 ? M : 1);   // gate_ld > 0: one gate row per token
-  gemm(c, A, K, W, K, M, N, K, e);
+  e.rows_per_gate = gate_ld > 0 ? gate_rows : (M > 0 ? M : 1);
+  gemm(c, A, K, W, K, M, N, K, e, items);
 }
-// V^T [Nout, rows] (row pitch ld_out) = (h W^T + b)^T: the weight is the A operand, so the product lands transposed.
-// Quantised weights must be the B operand: project into `tmp` [rows, Nout], then transpose.
-void linear_t(ltx_ctx* c, const bf16* W, const float* b, int Nout, int K, const bf16* hrows, int rows, bf16* out, int64_t ld_out,
-              bf16* tmp) {
+// V^T of `items` batch items: item i's [Nout, rows] block starts at column i * item_ld of `out` (row pitch items * item_ld)
+// = (h W^T + b)^T.  The weight is the A operand, so the product lands transposed.  Quantised weights must be the B operand:
+// project into `tmp` [items * rows, Nout], then transpose.
+void linear_t(ltx_ctx* c, const bf16* W, const float* b, int Nout, int K, const bf16* hrows, int rows, int items, bf16* out,
+              int64_t item_ld, bf16* tmp) {
+  const int64_t ld_out = items * item_ld;
   if (c->qw.empty() || c->qw.find(W) == c->qw.end()) {
     GemmEpi e;
     e.mode = EPI_BF16; e.out = out; e.ldo = ld_out; e.bias = b;
-    if (rows <= 32 && gemm_skinny_eligible(K, K, rows, Nout, K, e, 0)) {   // audio rows: stream the weight, store transposed
+    if (items > 1) { e.t_item_rows = rows; e.t_item_ld = item_ld; }
+    if (rows <= 32 && gemm_skinny_eligible(K, K, items * rows, Nout, K, e, 0, 32 * items)) {   // audio rows: stream the weight
       e.transpose_out = 1;
-      gemm(c, hrows, K, W, K, rows, Nout, K, e);
+      gemm(c, hrows, K, W, K, items * rows, Nout, K, e, items);
       return;
     }
+    e.t_item_rows = 0;
     e.bias_per_row = 1;
-    gemm(c, W, K, hrows, K, Nout, rows, K, e);
+    if (items == 1 || rows == item_ld) {   // the items' column blocks are contiguous
+      gemm(c, W, K, hrows, K, Nout, items * rows, K, e);
+      return;
+    }
+    for (int i = 0; i < items; ++i) {
+      e.out = out + i * item_ld;
+      gemm(c, W, K, hrows + static_cast<int64_t>(i) * rows * K, K, Nout, rows, K, e);
+    }
     return;
   }
   GemmEpi e;
   e.mode = EPI_BF16; e.out = tmp; e.ldo = Nout; e.bias = b;
-  gemm(c, hrows, K, W, K, rows, Nout, K, e);
-  ProfScope ps(c, PROF_OTHER, 0.0, 4.0 * rows * Nout);
-  launch_transpose_bf16(tmp, Nout, rows, Nout, out, ld_out, c->stream);
+  gemm(c, hrows, K, W, K, items * rows, Nout, K, e, items);
+  ProfScope ps(c, PROF_OTHER, 0.0, 4.0 * items * rows * Nout, items);
+  for (int i = 0; i < items; ++i)
+    launch_transpose_bf16(tmp + static_cast<int64_t>(i) * rows * Nout, Nout, rows, Nout, out + i * item_ld, ld_out, c->stream);
 }
+// B items: Q [B*Nq, D], K [B*Nk, ldk], V^T [D, B*ldv] (item b at column b * ldv), key bias [B, Nk]
 void attention(ltx_ctx* c, const bf16* Q, const bf16* K, int64_t ldk, const bf16* Vt, int64_t ldv, const float* bias, bf16* O, int H,
-               int hd, int Nq, int Nk) {
+               int hd, int B, int Nq, int Nk) {
   const int D = H * hd;
-  ProfScope ps(c, PROF_ATTN, 4.0 * H * static_cast<double>(Nq) * Nk * hd, 2.0 * (2.0 * Nq + 2.0 * Nk) * D);
-  launch_attention(Q, D, K, ldk, Vt, ldv, bias, O, D, 1, H, Nq, Nk, D, 1.0f / sqrtf(static_cast<float>(hd)), c->stream);
+  ProfScope ps(c, PROF_ATTN, 4.0 * B * H * static_cast<double>(Nq) * Nk * hd, 2.0 * B * (2.0 * Nq + 2.0 * Nk) * D);
+  launch_attention(Q, D, K, ldk, Vt, ldv, bias, O, D, B, H, Nq, Nk, D, 1.0f / sqrtf(static_cast<float>(hd)), c->stream);
 }
+// a_ld > 0: row r takes its modulation rows sc_a / sh_a + (r / a_rpr) * a_ld (one per token, or one per batch item)
 void normw(ltx_ctx* c, const float* x, bf16* out, int M, int D, const float* w, const float* sc_t, const float* sc_a,
-           const float* sh_t, const float* sh_a, float eps, int64_t a_ld = 0) {
+           const float* sh_t, const float* sh_a, float eps, int64_t a_ld = 0, int a_rpr = 1) {
   ProfScope ps(c, PROF_ROW, 0.0, static_cast<double>(M) * D * 6.0);
-  const ModSet m{sc_t, sc_a, sh_t, sh_a, out, a_ld};
+  const ModSet m{sc_t, sc_a, sh_t, sh_a, out, a_ld, a_rpr};
   if (D == 4096)
     launch_pdl(PDL_ROWS, rmsnorm_w_mod_fast_kernel<4, 4, 1>, dim3((M + 3) / 4), dim3(256), 0, c->stream, x, M, w, m, m, eps);
   else if (D == 2048)
     launch_pdl(PDL_ROWS, rmsnorm_w_mod_fast_kernel<2, 4, 1>, dim3((M + 3) / 4), dim3(256), 0, c->stream, x, M, w, m, m, eps);
   else
-    launch_pdl(PDL_ROWS, rmsnorm_w_mod_kernel, dim3(M), dim3(256), 0, c->stream, x, out, D, w, sc_t, sc_a, sh_t, sh_a, a_ld, eps);
+    launch_pdl(PDL_ROWS, rmsnorm_w_mod_kernel, dim3(M), dim3(256), 0, c->stream, x, out, D, w, sc_t, sc_a, sh_t, sh_a, a_ld, a_rpr,
+               eps);
   LTX_CUDA(cudaGetLastError());
 }
 // two modulations of the same normalised rows: out0 with (sc0, sh0), out1 with (sc1, sh1); tbl rows r*D of `tbl`, `ada`
 void normw2(ltx_ctx* c, const float* x, bf16* out0, bf16* out1, int M, int D, const float* w, const float* tbl, const float* ada,
-            float eps, int64_t a_ld = 0) {
+            float eps, int64_t a_ld = 0, int a_rpr = 1) {
   // rows: 0 a2v scale, 1 a2v shift, 2 v2a scale, 3 v2a shift
-  const ModSet m0{tbl, ada, tbl + D, ada + D, out0, a_ld}, m1{tbl + 2 * D, ada + 2 * D, tbl + 3 * D, ada + 3 * D, out1, a_ld};
+  const ModSet m0{tbl, ada, tbl + D, ada + D, out0, a_ld, a_rpr},
+      m1{tbl + 2 * D, ada + 2 * D, tbl + 3 * D, ada + 3 * D, out1, a_ld, a_rpr};
   if (D == 4096 || D == 2048) {
     ProfScope ps(c, PROF_ROW, 0.0, static_cast<double>(M) * D * 8.0);
     if (D == 4096)
@@ -290,8 +319,8 @@ void normw2(ltx_ctx* c, const float* x, bf16* out0, bf16* out1, int M, int D, co
     LTX_CUDA(cudaGetLastError());
     return;
   }
-  normw(c, x, out0, M, D, w, m0.sc_t, m0.sc_a, m0.sh_t, m0.sh_a, eps, a_ld);
-  normw(c, x, out1, M, D, w, m1.sc_t, m1.sc_a, m1.sh_t, m1.sh_a, eps, a_ld);
+  normw(c, x, out0, M, D, w, m0.sc_t, m0.sc_a, m0.sh_t, m0.sh_a, eps, a_ld, a_rpr);
+  normw(c, x, out1, M, D, w, m1.sc_t, m1.sc_a, m1.sh_t, m1.sh_a, eps, a_ld, a_rpr);
 }
 void qknorm_hd(ltx_ctx* c, bf16* x, int M, int D, int hd, const float* w, const float* cs, const float* sn, int rpr, float eps) {
   ProfScope ps(c, PROF_ROW, 0.0, static_cast<double>(M) * D * (4.0 + (cs ? 4.0 : 0.0)));
@@ -330,32 +359,33 @@ AdaLnW adaln_w(ltx_ctx* c, const std::string& p, int64_t dim, int n) {
   return a;
 }
 
-// AdaLayerNormSingle (T/LTXTimestepEmbedding.swift:96-124) for one sigma: se = sincos(sigma * mult) is shared by every
-// embedder of the same stream; emb = L2(silu(L1(se))), lin = L(silu(emb)).
-void adaln_single(ltx_ctx* c, const AdaLnW& a, const float* se, float* t1, float* emb, float* lin) {
-  ProfScope ps(c, PROF_OTHER, 2.0 * a.dim * (256.0 + (1.0 + a.n) * a.dim), 2.0 * a.dim * (256.0 + (1.0 + a.n) * a.dim), 3);
-  launch_gemv(a.w1, a.b1, se, t1, 1, a.dim, 256, 0, c->stream);
-  launch_gemv(a.w2, a.b2, t1, emb, 1, a.dim, a.dim, 1, c->stream);
-  launch_gemv(a.wl, a.bl, emb, lin, 1, a.n * a.dim, a.dim, 1, c->stream);
+// AdaLayerNormSingle (T/LTXTimestepEmbedding.swift:96-124) for one sigma per batch item (B rows): se = sincos(sigma * mult)
+// is shared by every embedder of the same stream; emb = L2(silu(L1(se))), lin = L(silu(emb)), row pitches dim and n * dim.
+void adaln_single(ltx_ctx* c, const AdaLnW& a, const float* se, float* t1, float* emb, float* lin, int B = 1) {
+  ProfScope ps(c, PROF_OTHER, 2.0 * B * a.dim * (256.0 + (1.0 + a.n) * a.dim), 2.0 * a.dim * (256.0 + (1.0 + a.n) * a.dim), 3);
+  launch_gemv(a.w1, a.b1, se, t1, B, a.dim, 256, 0, c->stream);
+  launch_gemv(a.w2, a.b2, t1, emb, B, a.dim, a.dim, 1, c->stream);
+  launch_gemv(a.wl, a.bl, emb, lin, B, a.n * a.dim, a.dim, 1, c->stream);
 }
 
 // The same for R sigmas (one per video token): the three Linears as tensor-core GEMMs over the R rows, bf16 operands, the
 // SiLUs in the first epilogue / a cast pass (the video-only model's per-token path, dit.cu).  se_bf [R, 256] bf16;
 // t1_bf [R, dim] bf16 scratch; emb [R, dim] fp32; lin [R, n * dim] fp32 with row pitch ld_lin.
-void adaln_single_rows(ltx_ctx* c, const AdaLnW& a, const bf16* se_bf, int R, bf16* t1_bf, float* emb, float* lin, int64_t ld_lin) {
+void adaln_single_rows(ltx_ctx* c, const AdaLnW& a, const bf16* se_bf, int R, bf16* t1_bf, float* emb, float* lin, int64_t ld_lin,
+                       int items) {
   GemmEpi e1;
   e1.mode = EPI_SILU_BF16; e1.out = t1_bf; e1.ldo = a.dim; e1.bias = a.b1;
-  gemm(c, se_bf, 256, a.w1, 256, R, a.dim, 256, e1);
+  gemm(c, se_bf, 256, a.w1, 256, R, a.dim, 256, e1, items);
   GemmEpi e2;
   e2.mode = EPI_F32; e2.out = emb; e2.ldo = a.dim; e2.bias = a.b2;
-  gemm(c, t1_bf, a.dim, a.w2, a.dim, R, a.dim, a.dim, e2);
+  gemm(c, t1_bf, a.dim, a.w2, a.dim, R, a.dim, a.dim, e2, items);
   {
     ProfScope ps(c, PROF_OTHER, 0.0, 6.0 * R * a.dim);
     launch_silu_cast(emb, t1_bf, static_cast<int64_t>(R) * a.dim, c->stream);
   }
   GemmEpi e3;
   e3.mode = EPI_F32; e3.out = lin; e3.ldo = ld_lin; e3.bias = a.bl;
-  gemm(c, t1_bf, a.dim, a.wl, a.dim, R, a.n * a.dim, a.dim, e3);
+  gemm(c, t1_bf, a.dim, a.wl, a.dim, R, a.n * a.dim, a.dim, e3, items);
 }
 
 // 1-D RoPE table, token-major [T, dim/2] (precomputeFreqsCis with a [1, T] grid, T/LTXRoPE.swift:375-488): all dim/2
@@ -440,8 +470,9 @@ void dit_av_forward_dev(ltx_ctx* c, const void* v_latent, int v_dtype, const voi
   AvWeights& av = c->av;
   LTX_CHECK(av.ready, LTX_ERR_WEIGHTS, "dual audio/video weights not loaded / finalized");
   LTX_CHECK(!(c->dist.comm_world && c->dist.sp > 1), LTX_ERR_UNSUPPORTED, "the dual model is single-GPU in this version");
-  LTX_CHECK(B == 1 && N >= 1 && Ta >= 1 && S >= 1 && static_cast<int64_t>(F) * H * W == N, LTX_ERR_INVALID_ARGUMENT,
-            "dual forward: B must be 1 and N = F*H*W");
+  LTX_CHECK(B >= 1 && B <= 2, LTX_ERR_UNSUPPORTED, "dual forward: batches of 1 or 2 items");
+  LTX_CHECK(N >= 1 && Ta >= 1 && S >= 1 && static_cast<int64_t>(F) * H * W == N, LTX_ERR_INVALID_ARGUMENT,
+            "dual forward: N = F*H*W");
   LTX_CHECK(v_latent && a_latent && v_context && a_context && v_ts_dev && a_ts_dev && out_v_dev && out_a_dev,
             LTX_ERR_INVALID_ARGUMENT, "null tensor");
   LTX_CHECK((v_dtype == LTX_BF16 || v_dtype == LTX_F32) && (a_dtype == LTX_BF16 || a_dtype == LTX_F32), LTX_ERR_UNSUPPORTED,
@@ -451,38 +482,49 @@ void dit_av_forward_dev(ltx_ctx* c, const void* v_latent, int v_dtype, const voi
   const int Da = av.Da, Ha = av.Ha, hda = av.hd, FFa = g.ffn_mult * Da, Cv = g.in_channels, Ca = av.Cin;
   const float eps = g.norm_eps;
   cudaStream_t st = c->stream;
-  const int64_t ldv = round_up8(N), lda = round_up8(Ta);
+  const int64_t ldv = round_up8(N), lda = round_up8(Ta);   // per-item column pitches of the V^T operands
+  const int R = B * N, Ra = B * Ta;                         // rows of the two streams
 
   // ---- workspaces: the video stream reuses the video-only model's buffers
-  c->x.reserve(static_cast<size_t>(N) * D * 4);
-  c->h.reserve(static_cast<size_t>(N) * D * 2);
-  c->q2.reserve(static_cast<size_t>(N) * D * 2);
-  c->qk.reserve(static_cast<size_t>(N) * 2 * D * 2);
-  c->vt.reserve(static_cast<size_t>(D) * ldv * 2);
-  c->att.reserve(static_cast<size_t>(N) * D * 2);
-  c->ffh.reserve(static_cast<size_t>(N) * FFD * 2);
-  c->xb.reserve(static_cast<size_t>(N) * D * 2);
+  c->x.reserve(static_cast<size_t>(R) * D * 4);
+  c->h.reserve(static_cast<size_t>(R) * D * 2);
+  c->q2.reserve(static_cast<size_t>(R) * D * 2);
+  c->qk.reserve(static_cast<size_t>(R) * 2 * D * 2);
+  c->vt.reserve(static_cast<size_t>(D) * B * ldv * 2);
+  c->att.reserve(static_cast<size_t>(R) * D * 2);
+  c->ffh.reserve(static_cast<size_t>(R) * FFD * 2);
+  c->xb.reserve(static_cast<size_t>(R) * D * 2);
   DevBuf& wsb = av.ws;
-  // rows of the video-side modulation tensors: one, or one per token (per-token sigmas); their row pitches
-  const int VR = v_ts_per_token ? N : 1;
-  const int64_t vada_ld = v_ts_per_token ? 6 * static_cast<int64_t>(D) : 0, cv_ld = v_ts_per_token ? 5 * static_cast<int64_t>(D) : 0;
+  // rows of the video-side modulation tensors: one per item, or one per token (per-token sigmas)
+  const int VR = v_ts_per_token ? R : B;
+  // Modulation / gate rows and their pitches.  Row r of a stream reads row r / *_rpr; a pitch of 0 (B = 1 with one sigma)
+  // shares one row among all rows.  The cross-modal tables are [scale/shift rows 0-3 | gate row 4]: interleaved per token
+  // ([R, 5, D]) with per-token sigmas, otherwise all items' rows 0-3 ([B, 4, D]) followed by all items' gates ([B, D]).
+  const bool per_item = B > 1;
+  const int v_rpr = v_ts_per_token ? 1 : N;
+  const int64_t vada_ld = (v_ts_per_token || per_item) ? 6 * static_cast<int64_t>(D) : 0;
+  const int64_t cv_ld = v_ts_per_token ? 5 * static_cast<int64_t>(D) : per_item ? 4 * static_cast<int64_t>(D) : 0;
+  const int64_t cvg_ld = v_ts_per_token ? 5 * static_cast<int64_t>(D) : per_item ? static_cast<int64_t>(D) : 0;
+  const int64_t aada_ld = per_item ? 6 * static_cast<int64_t>(Da) : 0, ca_ld = per_item ? 4 * static_cast<int64_t>(Da) : 0,
+                cag_ld = per_item ? static_cast<int64_t>(Da) : 0;
   // audio / cross-modal workspace carved out of one allocation
   size_t off = 0;
   auto carve = [&](size_t bytes) { const size_t o = off; off += (bytes + 255) / 256 * 256; return o; };
-  const size_t o_ax = carve(static_cast<size_t>(Ta) * Da * 4), o_ah = carve(static_cast<size_t>(Ta) * Da * 2),
-               o_ah2 = carve(static_cast<size_t>(Ta) * Da * 2), o_aq = carve(static_cast<size_t>(Ta) * Da * 2),
-               o_ak = carve(static_cast<size_t>(Ta) * Da * 2), o_avt = carve(static_cast<size_t>(Da) * lda * 2),
-               o_aatt = carve(static_cast<size_t>(Ta) * Da * 2), o_affh = carve(static_cast<size_t>(Ta) * FFa * 2),
-               o_cq = carve(static_cast<size_t>(N) * Da * 2), o_catt = carve(static_cast<size_t>(N) * Da * 2),
-               o_vt2 = carve(static_cast<size_t>(Da) * ldv * 2), o_lat = carve(static_cast<size_t>(std::max(N * Cv, Ta * Ca)) * 2),
-               o_se = carve(2 * 256 * 4), o_t1 = carve(static_cast<size_t>(D) * 4),
-               o_vemb = carve(static_cast<size_t>(VR) * D * 4), o_aemb = carve(static_cast<size_t>(Da) * 4),
-               o_vada = carve(static_cast<size_t>(VR) * 6 * D * 4), o_aada = carve(static_cast<size_t>(6) * Da * 4),
-               o_cv = carve(static_cast<size_t>(VR) * 5 * D * 4), o_ca = carve(static_cast<size_t>(5) * Da * 4),
+  const size_t o_ax = carve(static_cast<size_t>(Ra) * Da * 4), o_ah = carve(static_cast<size_t>(Ra) * Da * 2),
+               o_ah2 = carve(static_cast<size_t>(Ra) * Da * 2), o_aq = carve(static_cast<size_t>(Ra) * Da * 2),
+               o_ak = carve(static_cast<size_t>(Ra) * Da * 2), o_avt = carve(static_cast<size_t>(Da) * B * lda * 2),
+               o_aatt = carve(static_cast<size_t>(Ra) * Da * 2), o_affh = carve(static_cast<size_t>(Ra) * FFa * 2),
+               o_cq = carve(static_cast<size_t>(R) * Da * 2), o_catt = carve(static_cast<size_t>(R) * Da * 2),
+               o_vt2 = carve(static_cast<size_t>(Da) * B * ldv * 2),
+               o_lat = carve(static_cast<size_t>(std::max(R * Cv, Ra * Ca)) * 2),
+               o_se = carve(static_cast<size_t>(B) * 2 * 256 * 4), o_t1 = carve(static_cast<size_t>(B) * D * 4),
+               o_vemb = carve(static_cast<size_t>(VR) * D * 4), o_aemb = carve(static_cast<size_t>(B) * Da * 4),
+               o_vada = carve(static_cast<size_t>(VR) * 6 * D * 4), o_aada = carve(static_cast<size_t>(B) * 6 * Da * 4),
+               o_cv = carve(static_cast<size_t>(VR) * 5 * D * 4), o_ca = carve(static_cast<size_t>(B) * 5 * Da * 4),
                o_scr = carve(static_cast<size_t>(VR) * D * 4),
-               o_tq = carve(c->qw.empty() ? 0 : static_cast<size_t>(std::max(N, Ta)) * D * 2),   // projection before the V^T transpose
-               o_sev = carve(v_ts_per_token ? static_cast<size_t>(N) * 256 * 2 : 0),
-               o_t1v = carve(v_ts_per_token ? static_cast<size_t>(N) * D * 2 : 0);
+               o_tq = carve(c->qw.empty() ? 0 : static_cast<size_t>(std::max(R, Ra)) * D * 2),   // projection before the V^T transpose
+               o_sev = carve(v_ts_per_token ? static_cast<size_t>(R) * 256 * 2 : 0),
+               o_t1v = carve(v_ts_per_token ? static_cast<size_t>(R) * D * 2 : 0);
   wsb.reserve(off);
   uint8_t* wbase = wsb.as<uint8_t>();
   float* x = c->x.as<float>();
@@ -528,11 +570,11 @@ void dit_av_forward_dev(ltx_ctx* c, const void* v_latent, int v_dtype, const voi
   TextProjW vsrc;
   vsrc.w_c1 = c->w_c1; vsrc.w_c2 = c->w_c2; vsrc.b_c1 = c->b_c1; vsrc.b_c2 = c->b_c2; vsrc.D = D; vsrc.user = c;
   vsrc.layer = [](const void* u, int i) -> const AttnWeights& { return static_cast<const ltx_ctx*>(u)->blocks[i].a2; };
-  TextCache& tcv = dit_prepare_text(c, c->text, &c->text_rr, vsrc, v_context, ctx_dtype, v_mask_dev, 1, S, context_key);
+  TextCache& tcv = dit_prepare_text(c, c->text, &c->text_rr, vsrc, v_context, ctx_dtype, v_mask_dev, B, S, context_key);
   TextProjW asrc;
   asrc.w_c1 = av.w_c1; asrc.w_c2 = av.w_c2; asrc.b_c1 = av.b_c1; asrc.b_c2 = av.b_c2; asrc.D = Da; asrc.user = c;
   asrc.layer = audio_text_layer;
-  TextCache& tca = dit_prepare_text(c, av.text, &av.text_rr, asrc, a_context, ctx_dtype, a_mask_dev, 1, S, context_key);
+  TextCache& tca = dit_prepare_text(c, av.text, &av.text_rr, asrc, a_context, ctx_dtype, a_mask_dev, B, S, context_key);
   const float* vbias = tcv.has_bias ? tcv.bias.as<float>() : nullptr;
   const float* abias = tca.has_bias ? tca.bias.as<float>() : nullptr;
 
@@ -545,124 +587,128 @@ void dit_av_forward_dev(ltx_ctx* c, const void* v_latent, int v_dtype, const voi
       launch_cast_f32_bf16(reinterpret_cast<const float*>(lat), lat_bf, static_cast<int64_t>(rows) * Cin, st);
       src = lat_bf;
     }
-    linear(c, src, rows, Cin, w, b, Dout, tmp);
+    linear(c, src, rows, Cin, w, b, Dout, tmp, EPI_BF16, B);
     ProfScope ps(c, PROF_OTHER, 0.0, 6.0 * rows * Dout);
     launch_cast_bf16_f32(tmp, xout, static_cast<int64_t>(rows) * Dout, st);
   };
-  embed(v_latent, v_dtype, N, Cv, c->w_patch, c->b_patch, D, x, h);
-  embed(a_latent, a_dtype, Ta, Ca, av.w_patch, av.b_patch, Da, ax, ah);
+  embed(v_latent, v_dtype, R, Cv, c->w_patch, c->b_patch, D, x, h);
+  embed(a_latent, a_dtype, Ra, Ca, av.w_patch, av.b_patch, Da, ax, ah);
 
-  // ---- timestep embedders: one sinusoidal embedding per stream feeds that stream's three AdaLN-singles (:256-298)
+  // ---- timestep embedders: one sinusoidal embedding per stream and item feeds that stream's three AdaLN-singles (:256-298)
+  float* se_a = se + B * 256;
   {
-    ProfScope ps(c, PROF_OTHER, 0.0, 2048.0, 2);
-    launch_sincos_embed(v_ts_dev, g.timestep_scale_multiplier, se, 1, 256, st);
-    launch_sincos_embed(a_ts_dev, g.timestep_scale_multiplier, se + 256, 1, 256, st);
+    ProfScope ps(c, PROF_OTHER, 0.0, 2048.0 * B, 2);
+    launch_sincos_embed(v_ts_dev, g.timestep_scale_multiplier, se, B, 256, st);
+    launch_sincos_embed(a_ts_dev, g.timestep_scale_multiplier, se_a, B, 256, st);
   }
   AdaLnW vmain;
   vmain.w1 = c->w_t1; vmain.b1 = c->b_t1; vmain.w2 = c->w_t2; vmain.b2 = c->b_t2; vmain.wl = c->w_ada; vmain.bl = c->b_ada;
   vmain.dim = D; vmain.n = 6;
+  float* cvg = v_ts_per_token ? cv + 4 * D : cv + static_cast<int64_t>(B) * 4 * D;   // gate rows (see the pitches above)
+  float* cag = ca + static_cast<int64_t>(B) * 4 * Da;
   if (!v_ts_per_token) {
-    adaln_single(c, vmain, se, t1, vemb, vada);
-    adaln_single(c, av.cv_ss, se, t1, scr, cv);                 // rows 0-3: a2v scale, a2v shift, v2a scale, v2a shift
-    adaln_single(c, av.cv_g, se, t1, scr, cv + 4 * D);          // row 4: a2v gate
+    adaln_single(c, vmain, se, t1, vemb, vada, B);
+    adaln_single(c, av.cv_ss, se, t1, scr, cv, B);              // rows 0-3: a2v scale, a2v shift, v2a scale, v2a shift
+    adaln_single(c, av.cv_g, se, t1, scr, cvg, B);              // row 4: a2v gate
   } else {
     bf16 *sev = reinterpret_cast<bf16*>(wbase + o_sev), *t1v = reinterpret_cast<bf16*>(wbase + o_t1v);
     {
-      ProfScope ps(c, PROF_OTHER, 0.0, 4.0 * N + 512.0 * N);
-      launch_sincos_embed(v_ts_dev, g.timestep_scale_multiplier, nullptr, N, 256, st, sev);
+      ProfScope ps(c, PROF_OTHER, 0.0, 4.0 * R + 512.0 * R);
+      launch_sincos_embed(v_ts_dev, g.timestep_scale_multiplier, nullptr, R, 256, st, sev);
     }
-    adaln_single_rows(c, vmain, sev, N, t1v, vemb, vada, vada_ld);
-    adaln_single_rows(c, av.cv_ss, sev, N, t1v, scr, cv, cv_ld);            // [N, 5, D]: rows 0-3 of every token
-    adaln_single_rows(c, av.cv_g, sev, N, t1v, scr, cv + 4 * D, cv_ld);     // row 4 of every token
+    adaln_single_rows(c, vmain, sev, R, t1v, vemb, vada, vada_ld, B);
+    adaln_single_rows(c, av.cv_ss, sev, R, t1v, scr, cv, cv_ld, B);         // [R, 5, D]: rows 0-3 of every token
+    adaln_single_rows(c, av.cv_g, sev, R, t1v, scr, cvg, cvg_ld, B);        // row 4 of every token
   }
-  adaln_single(c, av.ada_a, se + 256, t1, aemb, aada);
-  adaln_single(c, av.ca_ss, se + 256, t1, scr, ca);
-  adaln_single(c, av.ca_g, se + 256, t1, scr, ca + 4 * Da);
+  adaln_single(c, av.ada_a, se_a, t1, aemb, aada, B);
+  adaln_single(c, av.ca_ss, se_a, t1, scr, ca, B);
+  adaln_single(c, av.ca_g, se_a, t1, scr, cag, B);
 
   for (int i = 0; i < L; ++i) {
     const BlockWeights& bv = c->blocks[i];
     const AvBlockW& ba = av.blocks[i];
     // ---- 1: video self-attention (T/LTX2TransformerBlock.swift:208-211)
-    normw(c, x, h, N, D, ba.norm1, bv.sst + D, vada + D, bv.sst, vada, eps, vada_ld);
+    normw(c, x, h, R, D, ba.norm1, bv.sst + D, vada + D, bv.sst, vada, eps, vada_ld, v_rpr);
     {
       GemmEpi e;
       e.mode = EPI_BF16; e.out = qk; e.ldo = 2 * D; e.bias = bv.a1.bq;
-      gemm(c, h, D, bv.a1.wq, D, N, 2 * D, D, e);   // packed q|k projection
+      gemm(c, h, D, bv.a1.wq, D, R, 2 * D, D, e, B);   // packed q|k projection
     }
-    linear_t(c, bv.a1.wv, bv.a1.bv, D, D, h, N, vt, ldv, tq);
+    linear_t(c, bv.a1.wv, bv.a1.bv, D, D, h, N, B, vt, ldv, tq);
     {
-      ProfScope ps(c, PROF_ROW, 0.0, 2.0 * N * D * 8.0, (D == 4096) ? 1 : 2);
-      launch_qknorm_rope(qk, 2 * D, N, D, bv.a1.q_norm, cos_v, sin_v, N, eps, st, bv.a1.k_norm);
+      ProfScope ps(c, PROF_ROW, 0.0, 2.0 * R * D * 8.0, (D == 4096) ? 1 : 2);
+      launch_qknorm_rope(qk, 2 * D, R, D, bv.a1.q_norm, cos_v, sin_v, N, eps, st, bv.a1.k_norm);
     }
     {
-      ProfScope ps(c, PROF_ATTN, 4.0 * Hv * static_cast<double>(N) * N * hdv, 2.0 * 4.0 * N * D);
-      launch_attention(qk, 2 * D, qk + D, 2 * D, vt, ldv, nullptr, att, D, 1, Hv, N, N, D, 1.0f / sqrtf(static_cast<float>(hdv)), st);
+      ProfScope ps(c, PROF_ATTN, 4.0 * B * Hv * static_cast<double>(N) * N * hdv, 2.0 * 4.0 * R * D);
+      launch_attention(qk, 2 * D, qk + D, 2 * D, vt, ldv, nullptr, att, D, B, Hv, N, N, D, 1.0f / sqrtf(static_cast<float>(hdv)), st);
     }
-    linear_resid(c, att, N, D, bv.a1.wo, bv.a1.bo, D, x, vada + 2 * D, bv.sst + 2 * D, vada_ld);
+    linear_resid(c, att, R, D, bv.a1.wo, bv.a1.bo, D, x, vada + 2 * D, bv.sst + 2 * D, vada_ld, v_rpr, B);
     // ---- 2: audio self-attention (:213-216)
-    normw(c, ax, ah, Ta, Da, ba.anorm1, ba.asst + Da, aada + Da, ba.asst, aada, eps);
-    linear(c, ah, Ta, Da, ba.aa1.wq, ba.aa1.bq, Da, aq);
-    linear(c, ah, Ta, Da, ba.aa1.wk, ba.aa1.bk, Da, ak);
-    linear_t(c, ba.aa1.wv, ba.aa1.bv, Da, Da, ah, Ta, avt, lda, tq);
-    qknorm_hd(c, aq, Ta, Da, hda, ba.aa1.q_norm, cos_a, sin_a, Ta, eps);
-    qknorm_hd(c, ak, Ta, Da, hda, ba.aa1.k_norm, cos_a, sin_a, Ta, eps);
-    attention(c, aq, ak, Da, avt, lda, nullptr, aatt, Ha, hda, Ta, Ta);
-    linear_resid(c, aatt, Ta, Da, ba.aa1.wo, ba.aa1.bo, Da, ax, aada + 2 * Da, ba.asst + 2 * Da);
+    normw(c, ax, ah, Ra, Da, ba.anorm1, ba.asst + Da, aada + Da, ba.asst, aada, eps, aada_ld, Ta);
+    linear(c, ah, Ra, Da, ba.aa1.wq, ba.aa1.bq, Da, aq, EPI_BF16, B);
+    linear(c, ah, Ra, Da, ba.aa1.wk, ba.aa1.bk, Da, ak, EPI_BF16, B);
+    linear_t(c, ba.aa1.wv, ba.aa1.bv, Da, Da, ah, Ta, B, avt, lda, tq);
+    qknorm_hd(c, aq, Ra, Da, hda, ba.aa1.q_norm, cos_a, sin_a, Ta, eps);
+    qknorm_hd(c, ak, Ra, Da, hda, ba.aa1.k_norm, cos_a, sin_a, Ta, eps);
+    attention(c, aq, ak, Da, avt, lda, nullptr, aatt, Ha, hda, B, Ta, Ta);
+    linear_resid(c, aatt, Ra, Da, ba.aa1.wo, ba.aa1.bo, Da, ax, aada + 2 * Da, ba.asst + 2 * Da, aada_ld, Ta, B);
     // ---- 3: video text cross-attention on norm2(x), no RoPE, no gate (:218-221)
-    normw(c, x, h, N, D, ba.norm2, nullptr, nullptr, nullptr, nullptr, eps);
-    linear(c, h, N, D, bv.a2.wq, bv.a2.bq, D, q2);
-    qknorm_hd(c, q2, N, D, hdv, bv.a2.q_norm, nullptr, nullptr, 1, eps);
-    attention(c, q2, tcv.k.as<bf16>() + static_cast<int64_t>(i) * S * D, D, tcv.vt.as<bf16>() + static_cast<int64_t>(i) * D * tcv.ldv,
-              tcv.ldv, vbias, att, Hv, hdv, N, S);
-    linear_resid(c, att, N, D, bv.a2.wo, bv.a2.bo, D, x, nullptr, nullptr);
+    normw(c, x, h, R, D, ba.norm2, nullptr, nullptr, nullptr, nullptr, eps);
+    linear(c, h, R, D, bv.a2.wq, bv.a2.bq, D, q2, EPI_BF16, B);
+    qknorm_hd(c, q2, R, D, hdv, bv.a2.q_norm, nullptr, nullptr, 1, eps);
+    attention(c, q2, tcv.k.as<bf16>() + static_cast<int64_t>(i) * B * S * D, D,
+              tcv.vt.as<bf16>() + static_cast<int64_t>(i) * D * B * tcv.ldv, tcv.ldv, vbias, att, Hv, hdv, B, N, S);
+    linear_resid(c, att, R, D, bv.a2.wo, bv.a2.bo, D, x, nullptr, nullptr, 0, 1, B);
     // ---- 4: audio text cross-attention (:223-226)
-    normw(c, ax, ah, Ta, Da, ba.anorm2, nullptr, nullptr, nullptr, nullptr, eps);
-    linear(c, ah, Ta, Da, ba.aa2.wq, ba.aa2.bq, Da, aq);
-    qknorm_hd(c, aq, Ta, Da, hda, ba.aa2.q_norm, nullptr, nullptr, 1, eps);
-    attention(c, aq, tca.k.as<bf16>() + static_cast<int64_t>(i) * S * Da, Da, tca.vt.as<bf16>() + static_cast<int64_t>(i) * Da * tca.ldv,
-              tca.ldv, abias, aatt, Ha, hda, Ta, S);
-    linear_resid(c, aatt, Ta, Da, ba.aa2.wo, ba.aa2.bo, Da, ax, nullptr, nullptr);
+    normw(c, ax, ah, Ra, Da, ba.anorm2, nullptr, nullptr, nullptr, nullptr, eps);
+    linear(c, ah, Ra, Da, ba.aa2.wq, ba.aa2.bq, Da, aq, EPI_BF16, B);
+    qknorm_hd(c, aq, Ra, Da, hda, ba.aa2.q_norm, nullptr, nullptr, 1, eps);
+    attention(c, aq, tca.k.as<bf16>() + static_cast<int64_t>(i) * B * S * Da, Da,
+              tca.vt.as<bf16>() + static_cast<int64_t>(i) * Da * B * tca.ldv, tca.ldv, abias, aatt, Ha, hda, B, Ta, S);
+    linear_resid(c, aatt, Ra, Da, ba.aa2.wo, ba.aa2.bo, Da, ax, nullptr, nullptr, 0, 1, B);
     // ---- 5-6: cross-modal attention; both directions read the streams as they are here (:228-271).  Table / embedding
-    // rows: 0 a2v scale, 1 a2v shift, 2 v2a scale, 3 v2a shift, 4 gate.
-    normw2(c, x, h, h2, N, D, ba.a2v_norm, ba.sst_ca_v, cv, eps, cv_ld);      // video as a2v query (h) and as v2a context (h2)
-    normw2(c, ax, ah, ah2, Ta, Da, ba.v2a_norm, ba.sst_ca_a, ca, eps);   // audio as a2v context (ah) and as v2a query (ah2)
+    // rows: 0 a2v scale, 1 a2v shift, 2 v2a scale, 3 v2a shift, 4 gate.  Each item attends within itself only.
+    normw2(c, x, h, h2, R, D, ba.a2v_norm, ba.sst_ca_v, cv, eps, cv_ld, v_rpr);   // video as a2v query (h) and v2a context (h2)
+    normw2(c, ax, ah, ah2, Ra, Da, ba.v2a_norm, ba.sst_ca_a, ca, eps, ca_ld, Ta);  // audio as a2v context (ah) and v2a query (ah2)
     // A2V: Q from video (temporal RoPE of the video frames), K / V from audio
-    linear(c, h, N, D, ba.a2v.wq, ba.a2v.bq, Da, cq);
-    linear(c, ah, Ta, Da, ba.a2v.wk, ba.a2v.bk, Da, ak);
-    linear_t(c, ba.a2v.wv, ba.a2v.bv, Da, Da, ah, Ta, avt, lda, tq);
-    qknorm_hd(c, cq, N, Da, hda, ba.a2v.q_norm, cos_xv, sin_xv, N, eps);
-    qknorm_hd(c, ak, Ta, Da, hda, ba.a2v.k_norm, cos_a, sin_a, Ta, eps);
-    attention(c, cq, ak, Da, avt, lda, nullptr, catt, Ha, hda, N, Ta);
+    linear(c, h, R, D, ba.a2v.wq, ba.a2v.bq, Da, cq, EPI_BF16, B);
+    linear(c, ah, Ra, Da, ba.a2v.wk, ba.a2v.bk, Da, ak, EPI_BF16, B);
+    linear_t(c, ba.a2v.wv, ba.a2v.bv, Da, Da, ah, Ta, B, avt, lda, tq);
+    qknorm_hd(c, cq, R, Da, hda, ba.a2v.q_norm, cos_xv, sin_xv, N, eps);
+    qknorm_hd(c, ak, Ra, Da, hda, ba.a2v.k_norm, cos_a, sin_a, Ta, eps);
+    attention(c, cq, ak, Da, avt, lda, nullptr, catt, Ha, hda, B, N, Ta);
     // V2A: Q from audio, K / V from video (projected before the a2v update lands in x: h2 was taken above)
-    linear(c, ah2, Ta, Da, ba.v2a.wq, ba.v2a.bq, Da, aq);
-    linear(c, h2, N, D, ba.v2a.wk, ba.v2a.bk, Da, cq);
-    linear_t(c, ba.v2a.wv, ba.v2a.bv, Da, D, h2, N, vt2, ldv, tq);
-    qknorm_hd(c, aq, Ta, Da, hda, ba.v2a.q_norm, cos_a, sin_a, Ta, eps);
-    qknorm_hd(c, cq, N, Da, hda, ba.v2a.k_norm, cos_xv, sin_xv, N, eps);
-    attention(c, aq, cq, Da, vt2, ldv, nullptr, aatt, Ha, hda, Ta, N);
-    linear_resid(c, catt, N, Da, ba.a2v.wo, ba.a2v.bo, D, x, cv + 4 * D, ba.sst_ca_v + 4 * D, cv_ld);
-    linear_resid(c, aatt, Ta, Da, ba.v2a.wo, ba.v2a.bo, Da, ax, ca + 4 * Da, ba.sst_ca_a + 4 * Da);
+    linear(c, ah2, Ra, Da, ba.v2a.wq, ba.v2a.bq, Da, aq, EPI_BF16, B);
+    linear(c, h2, R, D, ba.v2a.wk, ba.v2a.bk, Da, cq, EPI_BF16, B);
+    linear_t(c, ba.v2a.wv, ba.v2a.bv, Da, D, h2, N, B, vt2, ldv, tq);
+    qknorm_hd(c, aq, Ra, Da, hda, ba.v2a.q_norm, cos_a, sin_a, Ta, eps);
+    qknorm_hd(c, cq, R, Da, hda, ba.v2a.k_norm, cos_xv, sin_xv, N, eps);
+    attention(c, aq, cq, Da, vt2, ldv, nullptr, aatt, Ha, hda, B, Ta, N);
+    linear_resid(c, catt, R, Da, ba.a2v.wo, ba.a2v.bo, D, x, cvg, ba.sst_ca_v + 4 * D, cvg_ld, v_rpr, B);
+    linear_resid(c, aatt, Ra, Da, ba.v2a.wo, ba.v2a.bo, Da, ax, cag, ba.sst_ca_a + 4 * Da, cag_ld, Ta, B);
     // ---- 7-8: feed-forward on both streams (:273-281)
-    normw(c, x, h, N, D, ba.norm3, bv.sst + 4 * D, vada + 4 * D, bv.sst + 3 * D, vada + 3 * D, eps, vada_ld);
-    linear(c, h, N, D, bv.w_in, bv.b_in, FFD, ffh, EPI_GELU_BF16);
-    linear_resid(c, ffh, N, FFD, bv.w_out, bv.b_out, D, x, vada + 5 * D, bv.sst + 5 * D, vada_ld);
-    normw(c, ax, ah, Ta, Da, ba.anorm3, ba.asst + 4 * Da, aada + 4 * Da, ba.asst + 3 * Da, aada + 3 * Da, eps);
-    linear(c, ah, Ta, Da, ba.w_in, ba.b_in, FFa, affh, EPI_GELU_BF16);
-    linear_resid(c, affh, Ta, FFa, ba.w_out, ba.b_out, Da, ax, aada + 5 * Da, ba.asst + 5 * Da);
+    normw(c, x, h, R, D, ba.norm3, bv.sst + 4 * D, vada + 4 * D, bv.sst + 3 * D, vada + 3 * D, eps, vada_ld, v_rpr);
+    linear(c, h, R, D, bv.w_in, bv.b_in, FFD, ffh, EPI_GELU_BF16, B);
+    linear_resid(c, ffh, R, FFD, bv.w_out, bv.b_out, D, x, vada + 5 * D, bv.sst + 5 * D, vada_ld, v_rpr, B);
+    normw(c, ax, ah, Ra, Da, ba.anorm3, ba.asst + 4 * Da, aada + 4 * Da, ba.asst + 3 * Da, aada + 3 * Da, eps, aada_ld, Ta);
+    linear(c, ah, Ra, Da, ba.w_in, ba.b_in, FFa, affh, EPI_GELU_BF16, B);
+    linear_resid(c, affh, Ra, FFa, ba.w_out, ba.b_out, Da, ax, aada + 5 * Da, ba.asst + 5 * Da, aada_ld, Ta, B);
   }
   // ---- output heads (T/LTX2Transformer.swift:370-388): LayerNorm(no affine) * (1 + scale) + shift ; proj_out
-  auto head = [&](const float* xs, int rows, int Dx, const float* sst, const float* emb, int emb_per_row, bf16* tmp, const bf16* w,
+  // emb: one row per item (rpr = rows of an item) or per token (rpr = 1)
+  auto head = [&](const float* xs, int rows, int Dx, const float* sst, const float* emb, int rpr, bf16* tmp, const bf16* w,
                   const float* b, int Cout, float* out) {
     {
       ProfScope ps(c, PROF_ROW, 0.0, static_cast<double>(rows) * Dx * 6.0);
-      launch_rmsnorm_mod(xs, tmp, rows, Dx, sst, sst + Dx, emb, emb, Dx, emb_per_row ? 1 : rows, eps, 1, st);
+      launch_rmsnorm_mod(xs, tmp, rows, Dx, sst, sst + Dx, emb, emb, Dx, rpr, eps, 1, st);
     }
     GemmEpi e;
     e.mode = EPI_F32; e.out = out; e.ldo = Cout; e.bias = b;
-    gemm(c, tmp, Dx, w, Dx, rows, Cout, Dx, e);
+    gemm(c, tmp, Dx, w, Dx, rows, Cout, Dx, e, B);
   };
-  head(x, N, D, c->sst_out, vemb, v_ts_per_token, h, c->w_out, c->b_out, g.out_channels, out_v_dev);
-  head(ax, Ta, Da, av.sst_out, aemb, 0, ah, av.w_out, av.b_out, Ca, out_a_dev);
+  head(x, R, D, c->sst_out, vemb, v_rpr, h, c->w_out, c->b_out, g.out_channels, out_v_dev);
+  head(ax, Ra, Da, av.sst_out, aemb, Ta, ah, av.w_out, av.b_out, Ca, out_a_dev);
 }
 
 }  // namespace ltx

@@ -214,9 +214,9 @@ void launch_gemm(const bf16* A, int64_t lda, const bf16* B, int64_t ldb, int M, 
     const char* e = getenv("LTX_GEMM_FORCE_BN");
     if (e) force_bn = atoi(e);
   }
-  LTX_CHECK(epi.transpose_out == 0 || (allow_skinny && force_bn == 0 && gemm_skinny_eligible(lda, ldb, M, N, K, epi, a_kblock)), 2,
-            "GEMM: transpose_out is served by the weight-streaming kernel only");
-  if (allow_skinny && force_bn == 0 && gemm_skinny_eligible(lda, ldb, M, N, K, epi, a_kblock)) {
+  const bool skinny = allow_skinny && force_bn == 0 && gemm_skinny_eligible(lda, ldb, M, N, K, epi, a_kblock, allow_skinny);
+  LTX_CHECK(epi.transpose_out == 0 || skinny, 2, "GEMM: transpose_out is served by the weight-streaming kernel only");
+  if (skinny) {
     launch_gemm_skinny(A, lda, B, ldb, M, N, K, epi, stream);
     return;
   }

@@ -118,6 +118,10 @@ struct GemmEpi {
   int64_t ldt = 0;
   // weight-streaming kernel only (gemm_skinny.cu), EPI_BF16: element (m, n) is stored at out[n * ldo + m] -- V^T for the PV MMA
   int transpose_out = 0;
+  // with transpose_out, a batch of items (64-row form): row m of item m / t_item_rows lands in column
+  // (m / t_item_rows) * t_item_ld + m % t_item_rows, so each item's V^T block starts at a padded column.  0 = off.
+  int t_item_rows = 0;
+  int64_t t_item_ld = 0;
   int debug = 0;  // bit 0: skip the epilogue's global traffic (LTX_GEMM_DEBUG, timing experiments only)
   // Optional split-K workspace of the weight-streaming kernel for M <= 512 (gemm_swapab.cu): fp32 partial tiles + one zeroed
   // arrival counter per (weight tile, CTA).  Owned by the caller's context (one per stream); giving it is also the opt-in to
@@ -131,12 +135,13 @@ struct GemmEpi {
 // C[M,N] = A[M,K] * B[N,K]^T ; A, B bf16 K-major (row pitch lda / ldb elements, multiples of 8).
 // a_kblock > 0: A is K-blocked (Ulysses receive layout): element (m, k) lives at A[(k / a_kblock) * a_kblock_stride +
 // m * lda + k % a_kblock] (a_kblock % 64 == 0, lda = a_kblock).
-// allow_skinny: M <= 32 problems may take the weight-streaming kernel (gemm_skinny.cu) -- opt-in, because its summation
-// order differs from the tile kernels' and the sequence-parallel path promises results bit-identical to one GPU.
+// allow_skinny: problems of up to that many rows may take the weight-streaming kernel (gemm_skinny.cu) -- opt-in, because its
+// summation order differs from the tile kernels' and the sequence-parallel path promises results bit-identical to one GPU.
+// 0: never; 32; 64 only for a batch of two items of <= 32 rows each, whose one-item calls take the kernel too.
 void launch_gemm(const bf16* A, int64_t lda, const bf16* B, int64_t ldb, int M, int N, int K, const GemmEpi& epi,
                  cudaStream_t stream, int force_bn = 0, int a_kblock = 0, int64_t a_kblock_stride = 0, int allow_skinny = 0);
-// weight-streaming Linear for M <= 32 (gemm_skinny.cu): HBM-bound, mma.sync on 16-byte coalesced weight rows
-bool gemm_skinny_eligible(int64_t lda, int64_t ldb, int M, int N, int K, const GemmEpi& epi, int a_kblock);
+// weight-streaming Linear for M <= max_rows (32 or 64, gemm_skinny.cu): HBM-bound, mma.sync on 16-byte coalesced weight rows
+bool gemm_skinny_eligible(int64_t lda, int64_t ldb, int M, int N, int K, const GemmEpi& epi, int a_kblock, int max_rows = 32);
 void launch_gemm_skinny(const bf16* A, int64_t lda, const bf16* W, int64_t ldb, int M, int N, int K, const GemmEpi& epi,
                         cudaStream_t stream);
 int gemm_fit_tile_width(int M, int N);

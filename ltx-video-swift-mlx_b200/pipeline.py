@@ -129,10 +129,11 @@ def denoise_av_host_seam(ctx: LtxContext, video_noise: np.ndarray, audio_noise: 
 def denoise_av_resident(ctx: LtxContext, video_noise: np.ndarray, audio_noise: np.ndarray, video_context, audio_context, mask,
                         sigmas: Sequence[float], neg_video_context=None, neg_audio_context=None, neg_mask=None,
                         cfg_scale: float = 1.0, guidance_rescale: float = 0.0, image_latent: Optional[np.ndarray] = None,
-                        inject_noise: Optional[Sequence[np.ndarray]] = None, image_cond_noise_scale: float = 0.0):
+                        inject_noise: Optional[Sequence[np.ndarray]] = None, image_cond_noise_scale: float = 0.0,
+                        batched_cfg: bool = True):
     """The same loop on the device-resident session (ltx_av_denoise_begin / _step): latents, text caches and velocities stay
-    in HBM, the only per-step host traffic is the optional re-noised conditioning frame.  Returns (video latent [1,C,F,H,W],
-    audio latent [1,Ta,Ca])."""
+    in HBM, the only per-step host traffic is the optional re-noised conditioning frame.  batched_cfg: run the two guidance
+    passes as one B = 2 forward (same values).  Returns (video latent [1,C,F,H,W], audio latent [1,Ta,Ca])."""
     _, C, F, H, W = video_noise.shape
     ctx.av_denoise_begin(video_noise[0], audio_noise[0], (F, H, W), float(sigmas[0]), video_context, audio_context, mask,
                          neg_video_context, neg_audio_context, neg_mask)
@@ -144,6 +145,6 @@ def denoise_av_resident(ctx: LtxContext, video_noise: np.ndarray, audio_noise: n
         if i2v and image_cond_noise_scale > 0 and sg > 0 and inject_noise is not None:
             ctx.denoise_set_frame0(np.asarray(image_latent, dtype=np.float32) + np.float32(image_cond_noise_scale)
                                    * np.asarray(inject_noise[step], dtype=np.float32) * np.float32(sg * sg))
-        ctx.av_denoise_step(sg, sn, step, cfg_scale, guidance_rescale, i2v_frame0_conditioned=i2v)
+        ctx.av_denoise_step(sg, sn, step, cfg_scale, guidance_rescale, i2v_frame0_conditioned=i2v, batched_cfg=batched_cfg)
     v, a = ctx.av_denoise_get_latents()
     return v[None], a[None]
