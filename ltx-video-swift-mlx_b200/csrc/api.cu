@@ -1277,7 +1277,9 @@ int ltx_op_gemm_resid(ltx_ctx* c, const void* A, const void* B, const float* bia
     e.mode = EPI_GATE_RESID; e.resid = x; e.ldr = N; e.bias = bias; e.gate_a = gate_a; e.gate_b = gate_b; e.gate_ld = 0;
     e.rows_per_gate = M > 0 ? M : 1; e.shadow = reinterpret_cast<bf16*>(shadow); e.lds = N; e.scale = scale;
     if (M > 32 && M <= 512) gemm_attach_workspace(c, e);   // as the DiT forward does for few-row problems (swap-AB kernel)
-    launch_gemm(reinterpret_cast<const bf16*>(A), K, reinterpret_cast<const bf16*>(B), K, M, N, K, e, c->stream, 0, 0, 0,
+    // LTX_GEMM_FORCE_BN: a launch_gemm force_bn for this op, which has no argument for it (tools/gemm_bench.py's sweeps)
+    const char* fb = getenv("LTX_GEMM_FORCE_BN");
+    launch_gemm(reinterpret_cast<const bf16*>(A), K, reinterpret_cast<const bf16*>(B), K, M, N, K, e, c->stream, fb ? atoi(fb) : 0, 0, 0,
                 32 /* M <= 32: the weight-streaming kernel, as on the dual model's audio stream */);
     c->launches++;
   });

@@ -719,9 +719,8 @@ template <int BN, int MODE>
 void conv_launch(const CUtensorMap& tmX, const CUtensorMap& tmW, const ConvGeom& g, const ConvEpi& ep, cudaStream_t s, bool pair) {
   if (g.slab) { conv_launch_slab<BN, MODE>(tmX, tmW, g, ep, s); return; }
   // 128-channel stages where they fit: tiles up to 128 columns (3 / 4 stages of 64 / 48 KB stay in flight) and whole pairs of chunks
-  static const int ks_env = [] { const char* e = getenv("LTX_CONV_KS"); return e ? atoi(e) : 2; }();
   if (pair) conv_launch_pair<BN, MODE>(tmX, tmW, g, ep, s);
-  else if (BN <= 128 && ks_env == 2 && g.Cin % (2 * CBK) == 0) conv_launch_ks<BN, MODE, (BN <= 128 ? 2 : 1)>(tmX, tmW, g, ep, s);
+  else if (BN <= 128 && g.Cin % (2 * CBK) == 0) conv_launch_ks<BN, MODE, (BN <= 128 ? 2 : 1)>(tmX, tmW, g, ep, s);
   else conv_launch_ks<BN, MODE, 1>(tmX, tmW, g, ep, s);
 }
 

@@ -20,7 +20,7 @@ namespace {
 void gemm(ltx_ctx* c, const bf16* A, int64_t lda, const bf16* B, int64_t ldb, int M, int N, int K, const GemmEpi& e,
           int a_kblock = 0, int64_t a_kblock_stride = 0) {
   auto it = c->qw.empty() ? c->qw.end() : c->qw.find(B);
-  const bool panel = it != c->qw.end() && it->second.scratch != nullptr && M >= 257;
+  const bool panel = it != c->qw.end() && gemm_q_uses_panel(it->second, M);
   ProfScope ps(c, PROF_GEMM, 2.0 * M * N * K, 2.0 * (static_cast<double>(M) * K + static_cast<double>(N) * K + static_cast<double>(M) * N),
                panel ? 2 : 1);
   if (it != c->qw.end()) {   // weight was replaced by int8 / int4 codes: dequant-fused kernel, or panel + bf16 kernel for large M

@@ -224,7 +224,7 @@ __global__ void __launch_bounds__(256) qknorm_rope_hd_kernel(bf16* x, int64_t ld
 void gemm(ltx_ctx* c, const bf16* A, int64_t lda, const bf16* B, int64_t ldb, int M, int N, int K, const GemmEpi& e,
           int items = 1) {
   auto it = c->qw.empty() ? c->qw.end() : c->qw.find(B);
-  const bool panel = it != c->qw.end() && it->second.scratch != nullptr && M >= 257;
+  const bool panel = it != c->qw.end() && gemm_q_uses_panel(it->second, M);
   ProfScope ps(c, PROF_GEMM, 2.0 * M * N * K, 2.0 * (static_cast<double>(M) * K + static_cast<double>(N) * K + static_cast<double>(M) * N),
                panel ? 2 : 1);
   if (it != c->qw.end()) {   // int8 / int4 codes (quantize(model: ltx2, ...), Pipeline/LTXPipeline.swift:491): dequant-fused kernel

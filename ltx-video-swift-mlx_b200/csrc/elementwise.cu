@@ -1,11 +1,10 @@
 // HBM-bound row / elementwise kernels of the DiT step: AdaLN-modulated RMSNorm / LayerNorm, q/k RMSNorm-across-heads
 // fused with split RoPE, the timestep-embedding GEMV chain, patchify / unpatchify, and the fused
 // CFG + rescale + STG + GE + Euler update.  All vectorised 16-byte accesses, fp32 math.
-// The two row kernels of a DiT block have a streaming form for D = 4096 (rmsnorm_mod_stream_kernel, qknorm_rope_stream_kernel:
-// persistent CTAs whose rows arrive in shared memory by cp.async.bulk, all of a CTA's rows requested up front) and a
-// register-staged form for the same D (LTX_ROWS_STREAM=0) besides the generic one-row-per-CTA kernels for other widths.
+// The two row kernels of a DiT block take D = 4096 in a streaming form (rmsnorm_mod_stream_kernel, qknorm_rope_stream_kernel:
+// persistent CTAs whose rows arrive in shared memory by cp.async.bulk, all of a CTA's rows requested up front) and other
+// widths in the generic one-row-per-CTA kernels.
 #include <algorithm>
-#include <cstdlib>
 
 #include "ltx_internal.h"
 #include "ptx.cuh"
@@ -28,26 +27,6 @@ __device__ __forceinline__ float block_sum(float v, float* red) {
   }
   __syncthreads();
   return red[32];
-}
-
-// R independent sums at once (one barrier pair for all of them); every thread gets all totals; fixed summation order
-template <int R>
-__device__ __forceinline__ void block_sum_multi(float (&v)[R], float* red /* >= 8 * R floats, 256-thread CTAs */) {
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nw = blockDim.x >> 5;
-#pragma unroll
-  for (int r = 0; r < R; ++r) v[r] = warp_sum(v[r]);
-  __syncthreads();
-  if (lane == 0) {
-#pragma unroll
-    for (int r = 0; r < R; ++r) red[warp * R + r] = v[r];
-  }
-  __syncthreads();
-#pragma unroll
-  for (int r = 0; r < R; ++r) {
-    float t = 0.f;
-    for (int w = 0; w < nw; ++w) t += red[w * R + r];
-    v[r] = t;
-  }
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -100,105 +79,11 @@ __global__ void __launch_bounds__(256) rmsnorm_mod_kernel(const float* __restric
   }
 }
 
-// Fast path: D == 4 * VPT * 256.  A CTA owns ROWS rows: ALL their loads are issued up front (ROWS * VPT float4 per thread in
-// flight, one global read of x), the ROWS row statistics are reduced together (one barrier pair), and the combined
-// modulation vectors are fetched once per CTA -- the kernel is one memory latency + one reduction deep instead of ROWS.
-template <int VPT, int ROWS>
-__global__ void __launch_bounds__(256) rmsnorm_mod_fast_kernel(const float* x, bf16* out, int M,
-                                                                const float* __restrict__ tbl_shift,
-                                                                const float* __restrict__ tbl_scale,
-                                                                const float* ada_shift, const float* ada_scale, int64_t ada_ld,
-                                                                int rows_per_mod, float eps, int layernorm) {
-  __shared__ float red[8 * ROWS];
-  constexpr int D = 4 * VPT * 256;
-  const int row0 = blockIdx.x * ROWS;
-  // PDL: x and the ada vectors are written by preceding kernels that may still be running when this CTA starts, so their
-  // pointers must NOT be const __restrict__: the compiler hoists such "invariant" loads above griddepcontrol.wait
-  griddep_launch();
-  griddep_wait();
-  float4 v[ROWS][VPT];
-#pragma unroll
-  for (int rr = 0; rr < ROWS; ++rr) {
-    const float4* xr = reinterpret_cast<const float4*>(x + static_cast<int64_t>(row0 + rr) * D);
-#pragma unroll
-    for (int k = 0; k < VPT; ++k)
-      v[rr][k] = (row0 + rr < M) ? xr[threadIdx.x + k * 256] : make_float4(0.f, 0.f, 0.f, 0.f);
-  }
-  float mean[ROWS], rstd[ROWS];
-  if (layernorm) {
-    float s1[ROWS];
-#pragma unroll
-    for (int rr = 0; rr < ROWS; ++rr) {
-      s1[rr] = 0.f;
-#pragma unroll
-      for (int k = 0; k < VPT; ++k) s1[rr] += v[rr][k].x + v[rr][k].y + v[rr][k].z + v[rr][k].w;
-    }
-    block_sum_multi<ROWS>(s1, red);
-    float sv[ROWS];
-#pragma unroll
-    for (int rr = 0; rr < ROWS; ++rr) {
-      mean[rr] = s1[rr] / D;
-      sv[rr] = 0.f;
-#pragma unroll
-      for (int k = 0; k < VPT; ++k) {
-        const float a = v[rr][k].x - mean[rr], b = v[rr][k].y - mean[rr], c = v[rr][k].z - mean[rr], d = v[rr][k].w - mean[rr];
-        sv[rr] += a * a + b * b + c * c + d * d;
-      }
-    }
-    block_sum_multi<ROWS>(sv, red);
-#pragma unroll
-    for (int rr = 0; rr < ROWS; ++rr) rstd[rr] = rsqrtf(sv[rr] / D + eps);
-  } else {
-    float s2[ROWS];
-#pragma unroll
-    for (int rr = 0; rr < ROWS; ++rr) {
-      mean[rr] = 0.f;
-      s2[rr] = 0.f;
-#pragma unroll
-      for (int k = 0; k < VPT; ++k)
-        s2[rr] += v[rr][k].x * v[rr][k].x + v[rr][k].y * v[rr][k].y + v[rr][k].z * v[rr][k].z + v[rr][k].w * v[rr][k].w;
-    }
-    block_sum_multi<ROWS>(s2, red);
-#pragma unroll
-    for (int rr = 0; rr < ROWS; ++rr) rstd[rr] = rsqrtf(s2[rr] / D + eps);
-  }
-  int cur_mod = -1;
-  float4 sc[VPT], sh[VPT];
-#pragma unroll
-  for (int rr = 0; rr < ROWS; ++rr) {
-    const int row = row0 + rr;
-    if (row >= M) break;   // uniform across the CTA
-    const int mod = row / rows_per_mod;
-    if (mod != cur_mod) {
-      cur_mod = mod;
-      const int64_t aoff = static_cast<int64_t>(mod) * ada_ld;
-#pragma unroll
-      for (int k = 0; k < VPT; ++k) {
-        const int i = threadIdx.x + k * 256;
-        const float4 a = reinterpret_cast<const float4*>(tbl_scale)[i], b = reinterpret_cast<const float4*>(ada_scale + aoff)[i];
-        const float4 c = reinterpret_cast<const float4*>(tbl_shift)[i], d = reinterpret_cast<const float4*>(ada_shift + aoff)[i];
-        sc[k] = make_float4(1.f + a.x + b.x, 1.f + a.y + b.y, 1.f + a.z + b.z, 1.f + a.w + b.w);
-        sh[k] = make_float4(c.x + d.x, c.y + d.y, c.z + d.z, c.w + d.w);
-      }
-    }
-    uint2* orow = reinterpret_cast<uint2*>(out + static_cast<int64_t>(row) * D);
-#pragma unroll
-    for (int k = 0; k < VPT; ++k) {
-      const float y0 = (v[rr][k].x - mean[rr]) * rstd[rr] * sc[k].x + sh[k].x;
-      const float y1 = (v[rr][k].y - mean[rr]) * rstd[rr] * sc[k].y + sh[k].y;
-      const float y2 = (v[rr][k].z - mean[rr]) * rstd[rr] * sc[k].z + sh[k].z;
-      const float y3 = (v[rr][k].w - mean[rr]) * rstd[rr] * sc[k].w + sh[k].w;
-      orow[threadIdx.x + k * 256] = make_uint2(pack_bf16(y0, y1), pack_bf16(y2, y3));
-    }
-  }
-}
-
-
-// Streaming form (default for D = 4096): persistent CTAs, three per SM, each with a ring of NST row buffers in shared memory
+// Streaming form (D = 4096): persistent CTAs, three per SM, each with a ring of NST row buffers in shared memory
 // that ONE thread fills with 16 KB bulk copies (cp.async.bulk + mbarrier) -- every row a CTA will ever touch is requested
-// before the first one is reduced, at no register cost: 3 x NST x 16 KB in flight per SM against 64 KB for the register form
-// above (146 registers -> one CTA per SM: load phase, reduce phase, store phase in turn: 2.9 TB/s at M = 1536).  The
-// modulation vectors stay in registers for the CTA's whole life (one L2 read per CTA, not one per 4 rows).
+// before the first one is reduced, at no register cost: 3 x NST x 16 KB in flight per SM against 64 KB for a form that
+// staged 4 rows per CTA in registers (146 registers -> one CTA per SM: load phase, reduce phase, store phase in turn:
+// 2.9 TB/s at M = 1536).  The modulation vectors stay in registers for the CTA's whole life (one L2 read per CTA).
 // Reduction scratch alternates between two slots, so one __syncthreads per reduction is enough; the same barrier tells
 // the filling thread that every thread has taken its part of the stage out of shared memory.
 __device__ __forceinline__ float block_sum_256(float v, float* red, int& slot) {
@@ -371,110 +256,7 @@ __global__ void __launch_bounds__(256) qknorm_rope_kernel(bf16* __restrict__ x, 
   }
 }
 
-// Fast path: D == 16 * 256 -> exactly one (x1, x2) pair-chunk per thread and row, kept in registers between the reduction
-// and the rotation (one global read).  A CTA owns ROWS rows whose loads are all issued up front and whose sums of squares are
-// reduced together; the learned weight slice stays in registers; blockIdx.y selects the segment (q | k of the fused
-// projection: column offset seg * D, weight w0 / w1) so both norms are one launch.
-template <int ROWS>
-__global__ void __launch_bounds__(256) qknorm_rope_fast_kernel(bf16* __restrict__ x, int64_t ld, int M,
-                                                                const float* __restrict__ w0, const float* __restrict__ w1,
-                                                                const float* __restrict__ cosb, const float* __restrict__ sinb,
-                                                                int rows_per_rope, float eps, bf16* __restrict__ bout0,
-                                                                bf16* __restrict__ bout1, int hpb, int64_t bstride,
-                                                                int64_t bld, int use_peer, const PeerTable peer0,
-                                                                const PeerTable peer1) {
-  __shared__ float red[8 * ROWS];
-  constexpr int D = 4096;
-  const int seg = blockIdx.y;
-  const float* w = seg == 0 ? w0 : w1;
-  bf16* bout = seg == 0 ? bout0 : bout1;
-  const int hh = threadIdx.x >> 3, jc = (threadIdx.x & 7) * 8;
-  const int c1 = hh * 128 + jc, c2 = c1 + 64;
-  float wa[8], wb[8];
-#pragma unroll
-  for (int t = 0; t < 8; t += 4) {
-    const float4 a = *reinterpret_cast<const float4*>(w + c1 + t), b = *reinterpret_cast<const float4*>(w + c2 + t);
-    wa[t] = a.x; wa[t + 1] = a.y; wa[t + 2] = a.z; wa[t + 3] = a.w;
-    wb[t] = b.x; wb[t + 1] = b.y; wb[t + 2] = b.z; wb[t + 3] = b.w;
-  }
-  griddep_launch();
-  griddep_wait();   // the learned weights above are constants; x comes from the preceding GEMM
-  const int row0 = blockIdx.x * ROWS;
-  uint4 u1[ROWS], u2[ROWS];
-#pragma unroll
-  for (int rr = 0; rr < ROWS; ++rr) {
-    const bf16* xr = x + static_cast<int64_t>(row0 + rr) * ld + static_cast<int64_t>(seg) * D;
-    u1[rr] = (row0 + rr < M) ? *reinterpret_cast<const uint4*>(xr + c1) : make_uint4(0u, 0u, 0u, 0u);
-    u2[rr] = (row0 + rr < M) ? *reinterpret_cast<const uint4*>(xr + c2) : make_uint4(0u, 0u, 0u, 0u);
-  }
-  float ss[ROWS];
-#pragma unroll
-  for (int rr = 0; rr < ROWS; ++rr) {
-    const __nv_bfloat162* a2 = reinterpret_cast<const __nv_bfloat162*>(&u1[rr]);
-    const __nv_bfloat162* b2 = reinterpret_cast<const __nv_bfloat162*>(&u2[rr]);
-    ss[rr] = 0.f;
-#pragma unroll
-    for (int t = 0; t < 4; ++t) {
-      const float2 fa = __bfloat1622float2(a2[t]), fb = __bfloat1622float2(b2[t]);
-      ss[rr] += fa.x * fa.x + fa.y * fa.y + fb.x * fb.x + fb.y * fb.y;
-    }
-  }
-  block_sum_multi<ROWS>(ss, red);
-#pragma unroll
-  for (int rr = 0; rr < ROWS; ++rr) {
-    const int row = row0 + rr;
-    if (row >= M) break;
-    float cs[8], sn[8];
-    if (cosb) {
-      const int64_t fo = static_cast<int64_t>(row % rows_per_rope) * (D >> 1) + hh * 64 + jc;
-#pragma unroll
-      for (int t = 0; t < 8; t += 4) {
-        const float4 a = *reinterpret_cast<const float4*>(cosb + fo + t), b = *reinterpret_cast<const float4*>(sinb + fo + t);
-        cs[t] = a.x; cs[t + 1] = a.y; cs[t + 2] = a.z; cs[t + 3] = a.w;
-        sn[t] = b.x; sn[t + 1] = b.y; sn[t + 2] = b.z; sn[t + 3] = b.w;
-      }
-    }
-    const __nv_bfloat162* a2 = reinterpret_cast<const __nv_bfloat162*>(&u1[rr]);
-    const __nv_bfloat162* b2 = reinterpret_cast<const __nv_bfloat162*>(&u2[rr]);
-    const float rstd = rsqrtf(ss[rr] / D + eps);
-    float y1[8], y2[8];
-#pragma unroll
-    for (int t = 0; t < 4; ++t) {
-      const float2 fa = __bfloat1622float2(a2[t]), fb = __bfloat1622float2(b2[t]);
-      const float xa[2] = {fa.x, fa.y}, xb[2] = {fb.x, fb.y};
-#pragma unroll
-      for (int e = 0; e < 2; ++e) {
-        const int i = 2 * t + e;
-        const float a = xa[e] * rstd * wa[i], b = xb[e] * rstd * wb[i];
-        if (cosb) {
-          y1[i] = a * cs[i] - b * sn[i];
-          y2[i] = b * cs[i] + a * sn[i];
-        } else {
-          y1[i] = a; y2[i] = b;
-        }
-      }
-    }
-    bf16* xr = x + static_cast<int64_t>(row) * ld + static_cast<int64_t>(seg) * D;
-    bf16* o1 = xr + c1;
-    bf16* o2 = xr + c2;
-    if (use_peer) {   // Ulysses over peer memory: head block hh / hpb lives in that rank's receive buffer
-      bf16* base = reinterpret_cast<bf16*>(seg == 0 ? peer0.p[hh / hpb] : peer1.p[hh / hpb]);
-      bf16* ob = base + static_cast<int64_t>(row) * bld + (hh % hpb) * 128 + jc;
-      o1 = ob;
-      o2 = ob + 64;
-    } else if (bout) {
-      bf16* ob = bout + static_cast<int64_t>(hh / hpb) * bstride + static_cast<int64_t>(row) * bld + (hh % hpb) * 128 + jc;
-      o1 = ob;
-      o2 = ob + 64;
-    }
-    *reinterpret_cast<uint4*>(o1) =
-        make_uint4(pack_bf16(y1[0], y1[1]), pack_bf16(y1[2], y1[3]), pack_bf16(y1[4], y1[5]), pack_bf16(y1[6], y1[7]));
-    *reinterpret_cast<uint4*>(o2) =
-        make_uint4(pack_bf16(y2[0], y2[1]), pack_bf16(y2[2], y2[3]), pack_bf16(y2[4], y2[5]), pack_bf16(y2[6], y2[7]));
-  }
-}
-
-// Streaming form of the q/k norm (default for D = 4096): as rmsnorm_mod_stream_kernel.  A stage holds one row: the nseg
+// Streaming form of the q/k norm (D = 4096): as rmsnorm_mod_stream_kernel.  A stage holds one row: the nseg
 // (1 | 2) bf16 segments -- contiguous in the fused q|k projection output -- and, with RoPE, its cos and sin rows, so the
 // rotation tables are fetched once per row for both segments.  Two CTAs per SM, STAGES_BYTES of bulk copies in flight each.
 constexpr int QK_STREAM_BYTES = 96 * 1024;
@@ -840,41 +622,20 @@ inline int grid_for(int64_t work, int threads) {
   return static_cast<int>(blocks);
 }
 
-// rows per CTA of the fast row kernels (LTX_ROWS_PER_CTA = 2 | 4)
-int rows_per_cta() {
-  static const int r = [] { const char* e = getenv("LTX_ROWS_PER_CTA"); const int v = e ? atoi(e) : 4; return v == 2 ? 2 : 4; }();
-  return r;
-}
-
-// LTX_ROWS_STREAM=0: the register-staged row kernels instead of the bulk-copy streaming ones
-bool rows_stream() {
-  static const bool on = [] { const char* e = getenv("LTX_ROWS_STREAM"); return e ? atoi(e) != 0 : true; }();
-  return on;
-}
-
 }  // namespace
 
 void launch_rmsnorm_mod(const float* x, bf16* out, int M, int D, const float* tbl_shift, const float* tbl_scale,
                         const float* ada_shift, const float* ada_scale, int64_t ada_ld, int rows_per_mod, float eps,
                         int layernorm, cudaStream_t s) {
   LTX_CHECK(D % 4 == 0 && M > 0 && ada_ld % 4 == 0, 2, "rmsnorm_mod: D must be a multiple of 4");
-  if (D == 4096 && rows_stream() && (reinterpret_cast<uintptr_t>(x) & 15) == 0) {
+  if (D == 4096) {   // rows arrive by 16 KB bulk copies
+    LTX_CHECK((reinterpret_cast<uintptr_t>(x) & 15) == 0, 2, "rmsnorm_mod: x must be 16-byte aligned");
     constexpr int NST = 4;
     const size_t smem = NST * 4096 * 4 + NST * 8 + 64;
     auto kern = rmsnorm_mod_stream_kernel<NST>;
     ensure_dyn_smem(reinterpret_cast<const void*>(kern), smem);
     launch_pdl(PDL_ROWS, kern, dim3(std::min(M, 3 * device_sm_count())), dim3(256), smem, s, x, out, M, tbl_shift, tbl_scale,
                ada_shift, ada_scale, ada_ld, rows_per_mod > 0 ? rows_per_mod : 1, eps, layernorm);
-    return;
-  }
-  if (D == 4096) {
-    const int rpm = rows_per_mod > 0 ? rows_per_mod : 1;
-    if (rows_per_cta() == 2)
-      launch_pdl(PDL_ROWS, rmsnorm_mod_fast_kernel<4, 2>, dim3((M + 1) / 2), dim3(256), 0, s, x, out, M, tbl_shift, tbl_scale, ada_shift,
-                 ada_scale, ada_ld, rpm, eps, layernorm);
-    else
-      launch_pdl(PDL_ROWS, rmsnorm_mod_fast_kernel<4, 4>, dim3((M + 3) / 4), dim3(256), 0, s, x, out, M, tbl_shift, tbl_scale, ada_shift,
-                 ada_scale, ada_ld, rpm, eps, layernorm);
     return;
   }
   rmsnorm_mod_kernel<<<M, 256, 0, s>>>(x, out, D, tbl_shift, tbl_scale, ada_shift, ada_scale, ada_ld,
@@ -894,8 +655,10 @@ void launch_qknorm_rope(bf16* x, int64_t ld, int M, int D, const float* w, const
   const int use_peer = blocked ? blocked->use_peer : 0;
   const PeerTable pt0 = blocked ? blocked->peer[0] : PeerTable{}, pt1 = blocked ? blocked->peer[1] : PeerTable{};
   LTX_CHECK(!blocked || (hpb > 0 && (D / 128) % hpb == 0 && (use_peer || (b0 && (!w_second || b1)))), 2, "qknorm_rope: bad blocked output");
-  // streaming form: the segments of a row must be one contiguous, 16-byte aligned piece
-  if (D == 4096 && rows_stream() && (reinterpret_cast<uintptr_t>(x) & 15) == 0 && (!cosb || ((reinterpret_cast<uintptr_t>(cosb) | reinterpret_cast<uintptr_t>(sinb)) & 15) == 0)) {
+  if (D == 4096) {   // a row's segments and its cos / sin rows arrive by bulk copies: one contiguous, 16-byte aligned piece each
+    LTX_CHECK((reinterpret_cast<uintptr_t>(x) & 15) == 0 &&
+                  (!cosb || ((reinterpret_cast<uintptr_t>(cosb) | reinterpret_cast<uintptr_t>(sinb)) & 15) == 0),
+              2, "qknorm_rope: x, cos and sin must be 16-byte aligned");
     const size_t smem = QK_STREAM_BYTES + 8 * 8 + 128;
     const int nseg = w_second ? 2 : 1;
     const dim3 grid(std::min(M, 2 * device_sm_count()));
@@ -910,15 +673,6 @@ void launch_qknorm_rope(bf16* x, int64_t ld, int M, int D, const float* w, const
       launch_pdl(PDL_ROWS, kern, grid, dim3(256), smem, s, x, ld, M, nseg, w, w_second, cosb, sinb, rpr, eps, b0, b1, hpb, bs, bld,
                  use_peer, pt0, pt1);
     }
-    return;
-  }
-  if (D == 4096) {
-    if (rows_per_cta() == 2)
-      launch_pdl(PDL_ROWS, qknorm_rope_fast_kernel<2>, dim3((M + 1) / 2, w_second ? 2 : 1), dim3(256), 0, s, x, ld, M, w, w_second, cosb, sinb,
-                 rpr, eps, b0, b1, hpb, bs, bld, use_peer, pt0, pt1);
-    else
-      launch_pdl(PDL_ROWS, qknorm_rope_fast_kernel<4>, dim3((M + 3) / 4, w_second ? 2 : 1), dim3(256), 0, s, x, ld, M, w, w_second, cosb, sinb,
-                 rpr, eps, b0, b1, hpb, bs, bld, use_peer, pt0, pt1);
     return;
   }
   qknorm_rope_kernel<<<M, 256, 0, s>>>(x, ld, D, w, cosb, sinb, rpr, eps, b0, hpb, bs, bld, use_peer, pt0);

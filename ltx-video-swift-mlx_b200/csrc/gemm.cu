@@ -15,8 +15,6 @@
 // waves of 148 CTAs ("wave-fitted" tiles): at M = 1536 an N = 4096 GEMM runs as 12 x 24 tiles of 128x176 (2 waves, 97 %
 // full) instead of 12 x 16 tiles of 128x256 (2 waves, 65 % full); N = 8192 / 16384 use 128x224 (3 / 6 waves, 99 % full).
 // A stream-K variant (split last wave + fp32 partial fix-up) was measured slower than this on B200 and was dropped.
-#include <cstdlib>
-
 #include "gemm_epilogue.cuh"
 #include "ltx_internal.h"
 #include "ptx.cuh"
@@ -209,11 +207,7 @@ void launch_gemm(const bf16* A, int64_t lda, const bf16* B, int64_t ldb, int M, 
     LTX_CHECK(epi.ldo % (epi.mode == EPI_F32 ? 4 : 8) == 0, 2, "GEMM: output ld alignment");
   }
   // force_bn >= 1000 selects the 2-CTA pair kernel (gemm2.cu) with width force_bn - 1000 (0 = fitted); by default the
-  // pair kernel is used whenever the problem has more than one 128-row tile (LTX_GEMM_2CTA=0 disables it)
-  if (force_bn == 0) {  // experiment hook: LTX_GEMM_FORCE_BN is re-read on every call
-    const char* e = getenv("LTX_GEMM_FORCE_BN");
-    if (e) force_bn = atoi(e);
-  }
+  // pair kernel is used whenever the problem has more than one 128-row tile
   const bool skinny = allow_skinny && force_bn == 0 && gemm_skinny_eligible(lda, ldb, M, N, K, epi, a_kblock, allow_skinny);
   LTX_CHECK(epi.transpose_out == 0 || skinny, 2, "GEMM: transpose_out is served by the weight-streaming kernel only");
   if (skinny) {
@@ -226,8 +220,7 @@ void launch_gemm(const bf16* A, int64_t lda, const bf16* B, int64_t ldb, int M, 
     launch_gemm_swapab(A, lda, B, ldb, M, N, K, epi, stream, a_kblock, a_kblock_stride);
     return;
   }
-  static const bool pair_default = [] { const char* e = getenv("LTX_GEMM_2CTA"); return e ? atoi(e) != 0 : true; }();
-  if (force_bn >= 1000 || (force_bn == 0 && pair_default && M > 128)) {
+  if (force_bn >= 1000 || (force_bn == 0 && M > 128)) {
     launch_gemm_2cta(A, lda, B, ldb, M, N, K, epi, stream, force_bn >= 1000 ? force_bn - 1000 : 0, a_kblock, a_kblock_stride);
     return;
   }

@@ -3,7 +3,7 @@
 // Why: the 1-CTA kernel (gemm.cu) is bound by operand delivery L2 -> SM (48 KB per k-block per CTA at 128x256).  In pair
 // mode each CTA loads its own 128 rows of A but only HALF of the B tile (BN/2 rows); tcgen05.mma.cta_group::2 (M = 256)
 // reads both halves across the pair, so a CTA moves 16 + BN/4 KB per k-block (32 KB at BN = 256) for the same flops, and
-// the smem freed by the half-size B stage buys a deeper TMA ring (6 stages).
+// the smem freed by the half-size B stage buys a deeper TMA ring (3 stages of 128 k).
 //
 // Protocol (mirrors the CUTLASS / DeepGEMM 2-SM pattern):
 //   * both CTAs run every warp role; only the leader (cluster rank 0) issues tcgen05.mma
@@ -12,8 +12,6 @@
 //   * tcgen05.commit ... .multicast::cluster (mask 0b11) releases the smem stage / publishes the accumulator in BOTH CTAs
 //   * each CTA's epilogue drains its own 128 TMEM lanes and arrives remotely on the leader's tmem-empty barrier
 //   * TMEM is allocated with cta_group::2 by the same warp of both CTAs; cluster barriers bracket setup and teardown
-#include <cstdlib>
-
 #include "gemm_epilogue.cuh"
 #include "ltx_internal.h"
 #include "ptx.cuh"
@@ -23,27 +21,28 @@ namespace ltx {
 namespace {
 
 constexpr int BM2 = 128;          // rows per CTA (256 per pair)
-constexpr int BK2 = 64;
+constexpr int BK2 = 64;           // k of one 128-byte swizzle atom
 constexpr int G2_THREADS = 192;
-constexpr int G2_STAGES = 6;
 constexpr int G2_BN_MAX = 256;
-constexpr uint32_t G2_A_BYTES = BM2 * BK2 * 2;                 // 16 KB
-constexpr uint32_t G2_B_STRIDE = (G2_BN_MAX / 2) * BK2 * 2;    // 16 KB: half of the B tile
-constexpr size_t G2_SMEM = 1024 + G2_STAGES * (G2_A_BYTES + G2_B_STRIDE) + (2 * G2_STAGES + 4) * 8 + 16 + 128 + 4 * EPI_STAGE_BYTES;
+constexpr uint32_t G2_A_BYTES = BM2 * BK2 * 2;                 // 16 KB: one atom of A
+constexpr uint32_t G2_B_STRIDE = (G2_BN_MAX / 2) * BK2 * 2;    // 16 KB: one atom of half the B tile
+// A pipeline stage holds 128 k (two swizzle atoms per operand), so the issuing thread waits on / commits to half as many
+// barriers per k as with 64-wide stages and has 8 MMAs in flight per wait; 3 stages of 64 KB.  -4..7 % on every DiT GEMM
+// shape at M = 1536 against 64-wide stages on the same box (profiles/r02_gemm_kstage_sweep.txt).
+constexpr int G2_KSUB = 2;        // swizzle atoms per operand and stage
+constexpr int G2_STAGES = 3;
+constexpr uint32_t G2_A_STAGE = G2_KSUB * G2_A_BYTES, G2_B_STAGE = G2_KSUB * G2_B_STRIDE;
+constexpr size_t G2_SMEM = 1024 + G2_STAGES * (G2_A_STAGE + G2_B_STAGE) + (2 * G2_STAGES + 4) * 8 + 16 + 128 + 4 * EPI_STAGE_BYTES;
 
-// KS = 64-wide k sub-blocks per pipeline stage.  KS = 2: a stage holds 128 k (two swizzle atoms per operand), so the issuing
-// thread waits on / commits to half as many barriers per k and has 8 MMAs in flight per wait; 3 stages of 64 KB.
-template <int MODE, int KS>
+template <int MODE>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(G2_THREADS, 1)
 gemm_bf16_2cta(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, int M, int N, int K, int BN,
                int a_kblock, const GemmEpi ep) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~static_cast<uintptr_t>(1023));
-  constexpr int STAGES = G2_STAGES / KS;
-  constexpr uint32_t A_STAGE = KS * G2_A_BYTES, B_STAGE = KS * G2_B_STRIDE;
   uint8_t* sA = smem;
-  uint8_t* sB = smem + STAGES * A_STAGE;
-  uint64_t* full = reinterpret_cast<uint64_t*>(sB + STAGES * B_STAGE);
+  uint8_t* sB = smem + G2_STAGES * G2_A_STAGE;
+  uint64_t* full = reinterpret_cast<uint64_t*>(sB + G2_STAGES * G2_B_STAGE);
   uint64_t* empty = full + G2_STAGES;
   uint64_t* tfull = empty + G2_STAGES;
   uint64_t* tempty = tfull + 2;
@@ -57,14 +56,14 @@ gemm_bf16_2cta(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   const int num_mp = (M + 2 * BM2 - 1) / (2 * BM2);   // 256-row pair tiles
   const int num_n = (N + BN - 1) / BN;
   const int num_tiles = num_mp * num_n;
-  const int num_k = (K + KS * BK2 - 1) / (KS * BK2);   // pipeline steps of KS * 64 k
+  const int num_k = (K + G2_KSUB * BK2 - 1) / (G2_KSUB * BK2);   // pipeline steps of 128 k
   const int half_bn = BN >> 1;
   const uint32_t b_bytes = static_cast<uint32_t>(half_bn) * BK2 * 2;
 
   if (warp == 0 && lane == 0) {
     tma_prefetch_desc(&tmA);
     tma_prefetch_desc(&tmB);
-    for (int i = 0; i < STAGES; ++i) {
+    for (int i = 0; i < G2_STAGES; ++i) {
       mbar_init(&full[i], 2);    // leader's expect_tx arrive + the peer's remote arrive (only the leader's copy is used)
       mbar_init(&empty[i], 1);   // multicast tcgen05.commit
     }
@@ -93,18 +92,18 @@ gemm_bf16_2cta(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         const int n0 = n_blk * BN + static_cast<int>(rank) * half_bn;
         for (int kb = 0; kb < num_k; ++kb) {
           mbar_wait(&empty[stage], phase ^ 1);
-          if (leader) mbar_arrive_expect_tx(&full[stage], 2 * KS * (G2_A_BYTES + b_bytes));
+          if (leader) mbar_arrive_expect_tx(&full[stage], 2 * G2_KSUB * (G2_A_BYTES + b_bytes));
           else mbar_arrive_remote(&full[stage], 0);
 #pragma unroll
-          for (int ks = 0; ks < KS; ++ks) {   // k past K (a ragged tail) is zero-filled by TMA
-            const int k0 = (kb * KS + ks) * BK2;
+          for (int ks = 0; ks < G2_KSUB; ++ks) {   // k past K (a ragged tail) is zero-filled by TMA
+            const int k0 = (kb * G2_KSUB + ks) * BK2;
             if (a_kblock > 0)
-              tma_load_3d_2sm(sA + stage * A_STAGE + ks * G2_A_BYTES, &tmA, &full[stage], k0 % a_kblock, m0, k0 / a_kblock);
+              tma_load_3d_2sm(sA + stage * G2_A_STAGE + ks * G2_A_BYTES, &tmA, &full[stage], k0 % a_kblock, m0, k0 / a_kblock);
             else
-              tma_load_2d_2sm(sA + stage * A_STAGE + ks * G2_A_BYTES, &tmA, &full[stage], k0, m0);
-            tma_load_2d_2sm(sB + stage * B_STAGE + ks * G2_B_STRIDE, &tmB, &full[stage], k0, n0);
+              tma_load_2d_2sm(sA + stage * G2_A_STAGE + ks * G2_A_BYTES, &tmA, &full[stage], k0, m0);
+            tma_load_2d_2sm(sB + stage * G2_B_STAGE + ks * G2_B_STRIDE, &tmB, &full[stage], k0, n0);
           }
-          if (++stage == STAGES) { stage = 0; phase ^= 1; }
+          if (++stage == G2_STAGES) { stage = 0; phase ^= 1; }
         }
       }
     }
@@ -126,16 +125,16 @@ gemm_bf16_2cta(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
           tc_fence_after();
           // descriptors: stage base + a compile-time offset (the start-address field counts 16-byte units and cannot carry
           // out of its 14 bits: all operand buffers sit below 256 KB) -- the issuing thread spends one add per operand
-          const uint64_t a_desc = a_desc0 + static_cast<uint64_t>(stage) * (A_STAGE >> 4);
-          const uint64_t b_desc = b_desc0 + static_cast<uint64_t>(stage) * (B_STAGE >> 4);
+          const uint64_t a_desc = a_desc0 + static_cast<uint64_t>(stage) * (G2_A_STAGE >> 4);
+          const uint64_t b_desc = b_desc0 + static_cast<uint64_t>(stage) * (G2_B_STAGE >> 4);
 #pragma unroll
-          for (int ks = 0; ks < KS; ++ks)
+          for (int ks = 0; ks < G2_KSUB; ++ks)
 #pragma unroll
             for (int k = 0; k < BK2 / 16; ++k)
               umma_bf16_2cta(d_tmem, a_desc + ((ks * G2_A_BYTES + k * 32) >> 4), b_desc + ((ks * G2_B_STRIDE + k * 32) >> 4),
                              idesc, (kb | ks | k) != 0 ? 1u : 0u);
           umma_commit_2cta(&empty[stage]);
-          if (++stage == STAGES) { stage = 0; phase ^= 1; }
+          if (++stage == G2_STAGES) { stage = 0; phase ^= 1; }
         }
         umma_commit_2cta(&tfull[as]);
       }
@@ -165,18 +164,15 @@ gemm_bf16_2cta(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   }
 }
 
-template <int MODE, int KS>
+template <int MODE>
 void launch2(const CUtensorMap& tmA, const CUtensorMap& tmB, int M, int N, int K, int BN, int a_kblock, const GemmEpi& epi,
              cudaStream_t stream) {
-  auto kern = gemm_bf16_2cta<MODE, KS>;
+  auto kern = gemm_bf16_2cta<MODE>;
   ensure_dyn_smem(kern, G2_SMEM);
   const int tiles = ((M + 2 * BM2 - 1) / (2 * BM2)) * ((N + BN - 1) / BN);
   const int clusters = device_sm_count() / 2;
   const int grid = 2 * (tiles < clusters ? tiles : clusters);
-  static const int dbg = [] { const char* e = getenv("LTX_GEMM_DEBUG"); return e ? atoi(e) : 0; }();
-  GemmEpi ep2 = epi;
-  ep2.debug = dbg;
-  launch_pdl(PDL_GEMM, kern, dim3(grid), dim3(G2_THREADS), G2_SMEM, stream, tmA, tmB, M, N, K, BN, a_kblock, ep2);
+  launch_pdl(PDL_GEMM, kern, dim3(grid), dim3(G2_THREADS), G2_SMEM, stream, tmA, tmB, M, N, K, BN, a_kblock, epi);
 }
 
 }  // namespace
@@ -215,22 +211,14 @@ void launch_gemm_2cta(const bf16* A, int64_t lda, const bf16* B, int64_t ldb, in
     tmA = make_tmap_2d(A, M, K, lda, BM2);
   }
   CUtensorMap tmB = make_tmap_2d(B, N, K, ldb, bn / 2);
-  // 128-wide k stages by default: -4..7 % on every DiT GEMM shape at M = 1536 against 64-wide ones on the same box
-  // (profiles/r02_gemm_kstage_sweep.txt); LTX_GEMM_KS=1 selects the 64-wide pipeline
-  static const int ks_env = [] { const char* e = getenv("LTX_GEMM_KS"); return e ? atoi(e) : 2; }();
-  const bool ks2 = ks_env == 2;
-#define LTX_G2_LAUNCH(MODE_)                                                            \
-  if (ks2) launch2<MODE_, 2>(tmA, tmB, M, N, K, bn, a_kblock, epi, stream);             \
-  else launch2<MODE_, 1>(tmA, tmB, M, N, K, bn, a_kblock, epi, stream)
   switch (epi.mode) {
-    case EPI_BF16: LTX_G2_LAUNCH(EPI_BF16); break;
-    case EPI_GELU_BF16: LTX_G2_LAUNCH(EPI_GELU_BF16); break;
-    case EPI_GATE_RESID: LTX_G2_LAUNCH(EPI_GATE_RESID); break;
-    case EPI_F32: LTX_G2_LAUNCH(EPI_F32); break;
-    case EPI_SILU_BF16: LTX_G2_LAUNCH(EPI_SILU_BF16); break;
+    case EPI_BF16: launch2<EPI_BF16>(tmA, tmB, M, N, K, bn, a_kblock, epi, stream); break;
+    case EPI_GELU_BF16: launch2<EPI_GELU_BF16>(tmA, tmB, M, N, K, bn, a_kblock, epi, stream); break;
+    case EPI_GATE_RESID: launch2<EPI_GATE_RESID>(tmA, tmB, M, N, K, bn, a_kblock, epi, stream); break;
+    case EPI_F32: launch2<EPI_F32>(tmA, tmB, M, N, K, bn, a_kblock, epi, stream); break;
+    case EPI_SILU_BF16: launch2<EPI_SILU_BF16>(tmA, tmB, M, N, K, bn, a_kblock, epi, stream); break;
     default: LTX_CHECK(false, 2, "bad GEMM epilogue mode");
   }
-#undef LTX_G2_LAUNCH
 }
 
 }  // namespace ltx

@@ -37,7 +37,6 @@ __device__ __forceinline__ float4 ld4_guard(const float* p, int nvalid) {
 template <int MODE>
 __device__ __forceinline__ void epi_store_chunk(const float* stage, int lane, int row0, int col0, int ncols, int M, int N,
                                                 const GemmEpi& ep, const float4 (&xin)[8]) {
-  if (ep.debug & 1) return;
   const int cg = lane & 7, rs = lane >> 3;
   const int c = col0 + cg * 4;
   const int nlim = (col0 + ncols < N) ? col0 + ncols : N;   // never touch the next tile's columns from a 16-wide tail chunk
@@ -148,7 +147,6 @@ __device__ __forceinline__ void epi_store_chunk(const float* stage, int lane, in
 // contiguous bytes of row (n - tsplit_col) of the transposed output.
 __device__ __forceinline__ void epi_store_chunk_t(const float* stage, int lane, int row0, int col0, int ncols, int M, int N,
                                                   const GemmEpi& ep) {
-  if (ep.debug & 1) return;
   const int n = col0 + lane;
   if (lane >= ncols || n >= N || row0 >= M) return;
   const float b = (ep.bias && !ep.bias_per_row) ? ep.bias[n] : 0.f;
@@ -173,7 +171,7 @@ __device__ __forceinline__ void epi_prefetch_resid(float4 (&xin)[8], int lane, i
   const int cg = lane & 7, rs = lane >> 3;
   const int c = col0 + cg * 4;
   const int nlim = (col0 + ncols < N) ? col0 + ncols : N;
-  const int nvalid = (ep.debug & 1) ? 0 : nlim - c;
+  const int nvalid = nlim - c;
 #pragma unroll
   for (int i = 0; i < 8; ++i) {
     const int row = row0 + rs + 4 * i;

@@ -15,8 +15,6 @@
 //                                fence.proxy.async, arrive
 //   warp 1     : MMA issuer (tcgen05.mma, TMEM accumulators, two stages)      warps 2-5: epilogue
 // HBM / L2 traffic for weights drops 2x (int8) / 4x (int4); the tensor core still runs bf16 x bf16 -> fp32.
-#include <cstdlib>
-
 #include "gemm_epilogue.cuh"
 #include "ltx_internal.h"
 #include "ptx.cuh"
@@ -365,17 +363,18 @@ void launch_q_mode(const CUtensorMap& tmA, const CUtensorMap& tmQ, int M, int N,
 
 }  // namespace
 
+// Large M: the fused kernels redo the code -> bf16 conversion once per 128 / 256-row M tile (12x / 6x at M = 1536) and are
+// bound by its instruction issue (~450 TFLOP/s); converting the weight ONCE into the context's bf16 panel and running the
+// bf16 pair kernel on it is ~2x faster there.  The fused kernels keep the small-M regime, where weight bytes dominate.
+bool gemm_q_uses_panel(const QuantW& W, int M) { return W.scratch != nullptr && M >= 257; }
+
 void launch_gemm_q(const bf16* A, int64_t lda, const QuantW& W, int M, int N, int K, const GemmEpi& epi, cudaStream_t stream,
                    int force_bn, int a_kblock, int64_t a_kblock_stride) {
   LTX_CHECK(M > 0 && N > 0 && K > 0 && K % 64 == 0, 2, "quantised GEMM: K must be a multiple of the group size 64");
   LTX_CHECK(W.bits == 8 || W.bits == 4, 2, "quantised GEMM: 8 or 4 bits");
   LTX_CHECK(W.n == N && W.k == K && W.q && W.scales && W.biases, 2, "quantised GEMM: weight shape mismatch");
   LTX_CHECK(lda % 8 == 0, 2, "quantised GEMM: lda must be a multiple of 8");
-  // Large M: the fused kernels redo the code -> bf16 conversion once per 128 / 256-row M tile (12x / 6x at M = 1536) and are
-  // bound by its instruction issue (~450 TFLOP/s); converting the weight ONCE into the context's bf16 panel and running the
-  // bf16 pair kernel on it is ~2x faster there.  The fused kernels keep the small-M regime, where weight bytes dominate.
-  static const int panel_min_m = [] { const char* e = getenv("LTX_GEMMQ_PANEL_MIN_M"); return e ? atoi(e) : 257; }();
-  if (W.scratch != nullptr && force_bn == 0 && M >= panel_min_m) {
+  if (force_bn == 0 && gemm_q_uses_panel(W, M)) {
     launch_dequantize_panel(W, W.scratch, stream);
     launch_gemm(A, lda, W.scratch, K, M, N, K, epi, stream, 0, a_kblock, a_kblock_stride);
     return;

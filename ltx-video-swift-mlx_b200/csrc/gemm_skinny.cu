@@ -140,7 +140,6 @@ gemm_skinny_kernel(const bf16* A, int64_t lda, const bf16* W, int64_t ldb, int M
       part[warp][rb * 16 + g + 8][j * 8 + 2 * c + 1] = acc[rb][j][3];
     }
   __syncthreads();
-  if (ep.debug & 1) return;
   const int col = (threadIdx.x & 7) * 2;
 #pragma unroll
   for (int pass = 0; pass < RB / 2; ++pass) {   // 32 rows per pass
@@ -208,8 +207,7 @@ void launch_impl(const bf16* A, int64_t lda, const bf16* W, int64_t ldb, int M, 
 }  // namespace
 
 bool gemm_skinny_eligible(int64_t lda, int64_t ldb, int M, int N, int K, const GemmEpi& epi, int a_kblock, int max_rows) {
-  static const bool enabled = []() { const char* e = getenv("LTX_GEMM_SKINNY"); return !(e && e[0] == '0'); }();   // A/B switch
-  return enabled && M >= 1 && M <= max_rows && (max_rows == 32 || max_rows == 64) && a_kblock == 0 && K % 32 == 0 && N % SK_COLS == 0 && lda % 8 == 0 && ldb % 8 == 0 &&
+  return M >= 1 && M <= max_rows && (max_rows == 32 || max_rows == 64) && a_kblock == 0 && K % 32 == 0 && N % SK_COLS == 0 && lda % 8 == 0 && ldb % 8 == 0 &&
          epi.col_block == 0 && epi.tsplit_col == 0 && epi.mode >= EPI_BF16 && epi.mode <= EPI_SILU_BF16 &&
          (epi.transpose_out == 0 || epi.mode == EPI_BF16) && (epi.t_item_rows == 0 || (max_rows == 64 && epi.t_item_ld >= epi.t_item_rows));
 }

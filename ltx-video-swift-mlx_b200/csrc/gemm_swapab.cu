@@ -23,8 +23,6 @@
 //   * 8-stage TMA ring (224 KB), double-buffered accumulators, PDL prologue overlap, TMA zero-fill for ragged M / N / K
 // Same epilogue contract as launch_gemm (bias, GELU / SiLU, gate * residual + bf16 shadow, fp32, column-blocked and peer-memory
 // destinations, K-blocked A); transposed-column output (tsplit_col) stays with the tile kernels.
-#include <cstdlib>
-
 #include "ltx_internal.h"
 #include "ptx.cuh"
 
@@ -343,8 +341,7 @@ void launch_sw(const CUtensorMap& tmW, const CUtensorMap& tmA, const SwapParams&
 }  // namespace
 
 bool gemm_swapab_eligible(int64_t lda, int64_t ldb, int M, int N, int K, const GemmEpi& epi) {
-  static const bool on = [] { const char* e = getenv("LTX_GEMM_SWAPAB"); return e ? atoi(e) != 0 : true; }();
-  if (!on || M > 2 * SW_MC_MAX || M < 1 || N < 1 || K < 8) return false;
+  if (M > 2 * SW_MC_MAX || M < 1 || N < 1 || K < 8) return false;
   if (epi.tsplit_col != 0 || epi.transpose_out != 0) return false;
   if (K % 8 != 0 || lda % 8 != 0 || ldb % 8 != 0) return false;
   return true;

@@ -122,7 +122,6 @@ struct GemmEpi {
   // (m / t_item_rows) * t_item_ld + m % t_item_rows, so each item's V^T block starts at a padded column.  0 = off.
   int t_item_rows = 0;
   int64_t t_item_ld = 0;
-  int debug = 0;  // bit 0: skip the epilogue's global traffic (LTX_GEMM_DEBUG, timing experiments only)
   // Optional split-K workspace of the weight-streaming kernel for M <= 512 (gemm_swapab.cu): fp32 partial tiles + one zeroed
   // arrival counter per (weight tile, CTA).  Owned by the caller's context (one per stream); giving it is also the opt-in to
   // that kernel -- its summation order differs from the tile kernels' when K is split.
@@ -167,6 +166,8 @@ struct QuantW {
 // C[M,N] = A[M,K] * (s*q + beta)[N,K]^T with the epilogues of launch_gemm (group size 64)
 void launch_gemm_q(const bf16* A, int64_t lda, const QuantW& W, int M, int N, int K, const GemmEpi& epi, cudaStream_t stream,
                    int force_bn = 0, int a_kblock = 0, int64_t a_kblock_stride = 0);
+// whether launch_gemm_q (force_bn = 0) takes an M-row product through the bf16 panel: a dequantize launch + the bf16 GEMM
+bool gemm_q_uses_panel(const QuantW& W, int M);
 void launch_quantize(const bf16* w, int N, int K, int bits, uint8_t* q, float* scales, float* biases, cudaStream_t s);
 void launch_dequantize(const QuantW& W, bf16* w, cudaStream_t s);
 // vectorised, PDL-aware conversion of the whole weight into a bf16 panel (same rounding as the fused kernels)

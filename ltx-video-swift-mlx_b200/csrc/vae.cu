@@ -4,8 +4,6 @@
 // HBM layout: every activation is channels-last fp32 [T, H, W, C] (the residual stream stays fp32); each conv reads a
 // bf16 padded copy produced by the fused pixel-norm/scale-shift/SiLU prologue and writes fp32 through its epilogue
 // (+bias, +residual, depth-to-space scatter, or unpatchify+clip straight into the [F, H, W, 3] frame buffer).
-#include <cstdlib>
-
 #include "ctx.h"
 
 namespace ltx {
@@ -177,8 +175,7 @@ void vae_resgroup_fused(ltx_ctx* c, float* x, const std::vector<VaeResBlock>& bl
   const double cflops = 2.0 * 27.0 * C * C * vox, wbytes = 27.0 * C * C * 2.0;
   // conv2 -> next conv1 hand-over (mode 4, in the coalesced epilogue domain).  Measured: 25-frame decode 16.26 -> 16.14 ms
   // (prologue 3.1 -> 2.3 ms, convs +1.5 ms: the second epilogue pass is exposed at the short 128-channel main loops), 121 frames
-  // 76.7 -> 72.3 ms.  LTX_VAE_FUSE2=0 switches it off.
-  static const bool fuse2 = []() { const char* e = getenv("LTX_VAE_FUSE2"); return !(e && e[0] == '0'); }();
+  // 76.7 -> 72.3 ms.
   for (size_t j = 0; j < blocks.size(); ++j) {
     const VaeResBlock& rb = blocks[j];
     const float* tb = tables[j];
@@ -190,7 +187,7 @@ void vae_resgroup_fused(ltx_ctx* c, float* x, const std::vector<VaeResBlock>& bl
       launch_conv3d(padA, rb.c1.w, T, H, W, C, C, e, c->stream, 27);
     }
     halo(padB);
-    const bool last = j + 1 == blocks.size() || !fuse2;
+    const bool last = j + 1 == blocks.size();
     ConvEpi e;
     e.mode = last ? 0 : 4; e.out = x; e.bias = rb.c2.b; e.resid = x; e.Cin = C;
     if (!last) { e.next_pad = padA; e.next_scale = tables[j + 1] + C; e.next_shift = tables[j + 1]; e.next_tshift = tshift; }
@@ -375,10 +372,9 @@ void vae_decode_dev(ltx_ctx* c, const float* latent_dev, int Fp, int Hp, int Wp,
     // denormalise (x*std + mean, :379-381) fused into conv_in's padding prologue
     conv(c, hbuf, 1, v.std, v.mean, v.conv_in, T, H, W, causal, 0, x, nullptr, n_active);
     int64_t ch = g.vae_base_channels;
-    static const bool fuse_ok = []() { const char* e = getenv("LTX_VAE_FUSE"); return !(e && e[0] == '0'); }();   // LTX_VAE_FUSE=0: A/B switch
     for (int s = 0; s < 4; ++s) {
       if (timed) time_emb(v.stage_te[s], te_stage);   // one embedding per res-block group (:152-160)
-      const bool fuse = ch > 64 && ch <= 256 && ch % 32 == 0 && fuse_ok && !v.stages[s].empty();
+      const bool fuse = ch > 64 && ch <= 256 && ch % 32 == 0 && !v.stages[s].empty();
       if (fuse) {
         // every block's effective table is needed at once: a conv2 epilogue applies the NEXT block's scale1 / shift1
         std::vector<const float*> tabs;

@@ -57,7 +57,8 @@ def test_attention_guards(ctx, B, H, HD, Nq, Nk):
 
 @pytest.mark.parametrize("M,D", [(1, 4096), (3, 4096), (5, 4096), (193, 4096), (7, 512), (2, 256)])
 def test_row_kernels_guards(ctx, M, D):
-    """rmsnorm_mod and qknorm_rope with row counts that leave a CTA partly empty (4 rows per CTA at D = 4096)."""
+    """rmsnorm_mod and qknorm_rope with row counts below / not a multiple of the CTA count (persistent streaming CTAs at
+    D = 4096, one row per CTA otherwise): nothing is written behind the M rows and every row is written."""
     g = torch.Generator(device="cuda").manual_seed(M + D)
     pad = 5
     x = torch.full((M + pad, D), NAN, device="cuda")
@@ -87,6 +88,31 @@ def test_row_kernels_guards(ctx, M, D):
     c3, s3 = cos.view(M, heads, 64), sin.view(M, heads, 64)
     ref = torch.stack([n[:, :, 0] * c3 - n[:, :, 1] * s3, n[:, :, 1] * c3 + n[:, :, 0] * s3], 2).reshape(M, D)
     assert rel_l2(y[:M].float(), ref) <= 4e-3
+
+
+def test_row_kernels_refuse_misaligned_rows(ctx):
+    """At D = 4096 the rows (and the RoPE tables) reach the kernels by bulk copies, which need 16-byte aligned sources: a
+    pointer off that alignment is refused with code 2, and nothing is written."""
+    from ltx_video_swift_mlx_b200._lib import LtxError
+    M, D = 3, 4096
+    x = torch.randn(M * D + 4, device="cuda")
+    tb = torch.zeros(4, D, device="cuda")
+    out = torch.full((M, D), NAN, device="cuda", dtype=torch.bfloat16)
+    torch.cuda.synchronize()
+    with pytest.raises(LtxError) as e:
+        ctx._check(ctx.lib.ltx_op_rmsnorm_mod(ctx.handle, x.data_ptr() + 4, out.data_ptr(), M, D, tb[0].data_ptr(), tb[1].data_ptr(),
+                                              tb[2].data_ptr(), tb[3].data_ptr(), 1e-6, 0))
+    assert e.value.code == 2
+    y = torch.randn(M * D + 8, device="cuda").bfloat16()
+    y0 = y.clone()
+    w = torch.ones(D, device="cuda")
+    tabs = torch.rand(2, M * D // 2 + 4, device="cuda")
+    for yp, cp in ((y.data_ptr() + 2, tabs[0].data_ptr()), (y.data_ptr(), tabs[0].data_ptr() + 4)):
+        with pytest.raises(LtxError) as e:
+            ctx._check(ctx.lib.ltx_op_qknorm_rope(ctx.handle, yp, M, D, w.data_ptr(), cp, tabs[1].data_ptr(), M, 1e-6))
+        assert e.value.code == 2
+    ctx.sync()
+    assert torch.isnan(out.float()).all() and torch.equal(y, y0)
 
 
 @pytest.mark.parametrize("T,H,W,Cin,Cout", [(1, 3, 5, 64, 48), (2, 7, 9, 64, 64), (3, 5, 130, 128, 128), (1, 17, 3, 128, 256)])

@@ -1,5 +1,6 @@
 """Micro-benchmark of the attention kernel on the DiT shapes.  R launches queued behind a 1 GB memset on the library's stream
-(the host's issue latency is not in the number), CUDA events around the R.  LTX_ATT_NT=1 / 2 forces one / two query tiles per CTA."""
+(the host's issue latency is not in the number), CUDA events around the R.  ATT_SHAPES=a,b runs only those shapes;
+LTX_ATT_PAIR=0 / 1 forces one CTA per query tile / CTA pairs."""
 import os
 import math, sys, torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))

@@ -30,7 +30,8 @@ def bench_q(name, M, N, K, bits, bn=0):
 
 for nm, M, N, K in ([("qk", 1536, 8192, 4096), ("out", 1536, 4096, 4096), ("ffn_in", 1536, 16384, 4096), ("ffn_out", 1536, 4096, 16384)] if '--quant' in sys.argv else []):
     for bits in (8, 4):
-        for bn in (0, 1256, 1224, 1192, 1176, 256):    # 0 / 1xxx: pair kernel (fitted / forced width); 256: 1-CTA kernel
+        # the dequant-fused kernel (ltx_op_gemm_q gives no bf16 panel, so M = 1536 stays on it): 0 = wave-fitted width, else forced
+        for bn in (0, 256, 224, 192, 176, 128):
             bench_q(nm, M, N, K, bits, bn)
 
 # M = 1536 shapes of the DiT block: the pair kernel at forced widths (1000 + width, 1000 = fitted); 0 = the library's own choice.  Timed like the small-M sweep below: R launches on R cold weight

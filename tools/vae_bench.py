@@ -1,4 +1,5 @@
-"""VAE decode timing (25-frame and 121-frame clips, 768x512) with the per-class profile; LTX_CONV_KS=1 / 2 selects the k-stage width."""
+"""VAE decode timing (25-frame and 121-frame clips, 768x512) with the per-class profile; LTX_CONV_PAIR=0 runs one CTA per
+voxel tile, LTX_CONV_SLAB=0 per-tap stages."""
 import os, sys, torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import ltx_video_swift_mlx_b200  # noqa
