@@ -109,7 +109,14 @@ int ltx_fuse_lora(ltx_ctx* ctx, const char* key, const void* down, const void* u
  * accumulation / residual stream / norms / softmax; velocity within rel-L2 1e-2 of the fp32 graph.  32: fp32 mode -- DiT
  * matrices stay fp32, activations fp32, every Linear runs as a split-bf16 (3-term) tensor-core product that is exact to
  * fp32 rounding, attention in fp32; velocity within rel-L2 1e-4 (the mode BASELINE config 0, "random-init fp32", is checked
- * in).  Must be called before the DiT weights are loaded; single GPU, no quantisation; the VAE is unaffected. */
+ * in); single GPU, no quantisation.  8: FP8 mode -- at ltx_finalize_weights every Linear inside the transformer blocks
+ * (attn1 q|k|v and to_out, attn2 q, text k / v and to_out, FFN in / out) becomes e4m3 codes with one power-of-two scale per output channel (s = 2^ceil(log2(amax /
+ * 448)), q = e4m3_rn_satfinite(w / s); the bf16 copies are freed, about half the DiT's weight bytes), and each of those GEMMs
+ * quantises its activation rows by the same rule and runs e4m3 x e4m3 -> fp32 on the tensor cores (tcgen05 kind::f8f6f4),
+ * scaled back per row and column before the bias.  Patchify, caption projection, timestep MLPs / AdaLN and proj_out stay bf16.
+ * FP8 mode refuses quant_bits != 16, sequence parallelism (pass groups are fine) and the dual audio/video model
+ * (LTX_ERR_UNSUPPORTED).  Must be called before the DiT weights are loaded (8 after that: LTX_ERR_UNSUPPORTED); the VAE is
+ * unaffected in every mode. */
 int ltx_set_precision(ltx_ctx* ctx, int bits);
 /* Where quantised weights live (takes effect at the next ltx_finalize_weights with quant_bits 8 / 4).  0 (default): as codes --
  * 13 GB (int8) / 6.5 GB (int4) for the video DiT; every GEMM dequantises on the fly (fused kernel for M <= 256, a per-GEMM bf16
@@ -411,6 +418,20 @@ int ltx_op_quantize(ltx_ctx* ctx, const void* w_bf16, int N, int K, int bits, vo
 int ltx_op_dequantize(ltx_ctx* ctx, const void* q, const float* scales, const float* biases, int N, int K, int bits, void* w_bf16);
 int ltx_op_gemm_q(ltx_ctx* ctx, const void* A, const void* q, const float* scales, const float* biases, int bits,
                   const float* bias, void* C, int M, int N, int K, int mode, int force_bn);
+/* FP8 mode's per-row quantiser: x bf16 [M, K] (row pitch ld elements, ld % 8 == 0, K % 16 == 0) -> e4m3 codes [M, K] and fp32
+ * scales [M], s = 2^ceil(log2(amax / 448)) (1 for a zero row), q = e4m3_rn_satfinite(x / s). */
+int ltx_op_quantize_fp8(ltx_ctx* ctx, const void* x_bf16, int M, int K, int64_t ld, void* codes, float* scales);
+/* FP8 pair GEMM: C[M,N] = (Aq[M,K] Bq[N,K]^T) * sa[m] * sb[n] + bias[n] on e4m3 codes (K % 16 == 0, sb 16-byte aligned);
+ * mode as in ltx_op_gemm; force_bn 0 = fitted tile width, else a multiple of 16 in [64, 256]. */
+int ltx_op_gemm_fp8(ltx_ctx* ctx, const void* Aq, const float* sa, const void* Bq, const float* sb, const float* bias, void* C, int M,
+                    int N, int K, int mode, int force_bn);
+/* The same product with the fused q|k|v or residual epilogues.  C != NULL: bf16 output, columns n >= tsplit_col (> 0, a multiple
+ * of 32) stored transposed into Ct[(n - tsplit_col) * ldt + m], the others into C [M, tsplit_col] (tsplit_col = 0: C [M, N]).
+ * x != NULL (C == NULL): x[M,N] (fp32) += (product + bias) * (gate_a[n] + gate_b[n]) (gates nullable), shadow (bf16, nullable)
+ * = new x. */
+int ltx_op_gemm_fp8_ex(ltx_ctx* ctx, const void* Aq, const float* sa, const void* Bq, const float* sb, const float* bias, void* C,
+                       void* Ct, int tsplit_col, int64_t ldt, float* x, const float* gate_a, const float* gate_b, void* shadow,
+                       int M, int N, int K, int force_bn);
 /* O = softmax(Q K^T * scale + key_bias) V ; Q [B*Nq, H*128], K [B*Nk, H*128], Vt [H*128, B*ldvb] (batch b owns
  * columns [b*ldvb, b*ldvb + Nk), ldvb % 8 == 0), all bf16. */
 int ltx_op_attention(ltx_ctx* ctx, const void* Q, const void* K, const void* Vt, int64_t ldvb, const float* key_bias, void* O,

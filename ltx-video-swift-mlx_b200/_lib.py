@@ -111,6 +111,9 @@ SIGNATURES = {
     "ltx_op_quantize": (_I, [_P, _P, _I, _I, _I, _P, _P, _P]),
     "ltx_op_dequantize": (_I, [_P, _P, _P, _P, _I, _I, _I, _P]),
     "ltx_op_gemm_q": (_I, [_P, _P, _P, _P, _P, _I, _P, _P, _I, _I, _I, _I, _I]),
+    "ltx_op_quantize_fp8": (_I, [_P, _P, _I, _I, _I64, _P, _P]),
+    "ltx_op_gemm_fp8": (_I, [_P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I]),
+    "ltx_op_gemm_fp8_ex": (_I, [_P, _P, _P, _P, _P, _P, _P, _P, _I, _I64, _P, _P, _P, _P, _I, _I, _I, _I]),
     "ltx_op_attention": (_I, [_P, _P, _P, _P, _I64, _P, _P, _I, _I, _I, _I, _F]),
     "ltx_op_attention_hd": (_I, [_P, _P, _P, _P, _I64, _P, _P, _I, _I, _I, _I, _I, _F]),
     "ltx_op_attention_blocks": (_I, [_P, _P, _P, _P, _I64, _I, _I, _I, _F, C.POINTER(_P), _I, _I]),

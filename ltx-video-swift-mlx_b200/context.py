@@ -227,7 +227,9 @@ class LtxContext:
         self._check(self.lib.ltx_fuse_lora(self.handle, key.encode(), _ptr(d), _ptr(u), code, int(d.shape[0]), float(scale)))
 
     def set_precision(self, bits: int):
-        """16 = bf16 mode (default), 32 = fp32 mode (fp32 DiT weights, split-bf16 tensor-core GEMMs); before loading weights."""
+        """16 = bf16 mode (default), 32 = fp32 mode (fp32 DiT weights, split-bf16 tensor-core GEMMs), 8 = FP8 mode (the block
+        Linears run as e4m3 x e4m3 GEMMs with per-row power-of-two scales; no quantised weights, sequence parallelism or dual
+        audio/video model); before loading weights."""
         self._check(self.lib.ltx_set_precision(self.handle, int(bits)))
 
     def set_quant_storage(self, materialise: bool):

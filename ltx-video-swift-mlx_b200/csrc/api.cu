@@ -419,7 +419,10 @@ int ltx_init_random_weights(ltx_ctx* c, int which, uint64_t seed) {
 
 int ltx_set_precision(ltx_ctx* c, int bits) {
   return guarded(c, [&] {
-    LTX_CHECK(bits == 16 || bits == 32, LTX_ERR_UNSUPPORTED, "precision must be 16 (bf16 mode) or 32 (fp32 mode)");
+    LTX_CHECK(bits == 16 || bits == 32 || bits == 8, LTX_ERR_UNSUPPORTED,
+              "precision must be 16 (bf16 mode), 32 (fp32 mode) or 8 (FP8 mode)");
+    LTX_CHECK(bits != 8 || (!c->dit_ready && c->tensors.count("patchify_proj.weight") == 0), LTX_ERR_UNSUPPORTED,
+              "FP8 mode must be set before the DiT weights are loaded");
     LTX_CHECK(!c->dit_ready && c->tensors.count("patchify_proj.weight") == 0, LTX_ERR_INVALID_ARGUMENT,
               "ltx_set_precision must be called before the DiT weights are loaded");
     c->precision = bits;
@@ -434,17 +437,19 @@ int ltx_finalize_weights(ltx_ctx* c, int quant_bits, int group_size) {
   return guarded(c, [&] {
     LTX_CHECK(quant_bits == 16 || quant_bits == 8 || quant_bits == 4, LTX_ERR_UNSUPPORTED, "quant_bits must be 16, 8 or 4");
     LTX_CHECK(quant_bits == 16 || group_size == 64, LTX_ERR_UNSUPPORTED, "only group_size 64 is implemented");
-    LTX_CHECK(quant_bits == 16 || c->precision == 16, LTX_ERR_UNSUPPORTED, "fp32 mode cannot be combined with quantised weights");
+    LTX_CHECK(quant_bits == 16 || c->precision == 16, LTX_ERR_UNSUPPORTED,
+              "fp32 and FP8 modes cannot be combined with quantised weights");
     graphs_clear(c);
     // each component is packed once; a later call (after loading another component) only packs what is new
     if (c->tensors.count("patchify_proj.weight") && !c->dit_ready) {
       if (c->precision == 32) dit_finalize_f32(c);
       else dit_finalize(c);
       if (c->tensors.count("audio_patchify_proj.weight")) {
-        LTX_CHECK(c->precision == 16, LTX_ERR_UNSUPPORTED, "the dual audio/video model has no fp32 mode");
+        LTX_CHECK(c->precision == 16, LTX_ERR_UNSUPPORTED, "the dual audio/video model has no fp32 or FP8 mode");
         dit_av_finalize(c);
       }
       if (quant_bits != 16) dit_quantize(c, quant_bits);
+      if (c->precision == 8) dit_convert_fp8(c);
     }
     if (c->tensors.count("vae.conv_in.conv.weight") && !c->vae.ready) vae_finalize(c);
     if (c->tensors.count("vae_encoder.conv_in.conv.weight") && !c->enc.ready) vae_encoder_finalize(c);
@@ -494,12 +499,13 @@ int ltx_dit_forward(ltx_ctx* c, const void* latent, ltx_dtype latent_dtype, cons
     // steady state of a denoise loop at this seam (text cached under the key, RoPE table built): the forward is a fixed launch
     // sequence on fixed buffers -> replay it as a graph
     const TextCache* tcache = find_text(c->text, key, B, S);
-    const bool steady = tcache != nullptr && c->precision == 16 && c->rope_f == F && c->rope_h == H && c->rope_w == W && c->rope_cos.ptr;
+    const bool steady = tcache != nullptr && c->precision != 32 && c->rope_f == F && c->rope_h == H && c->rope_w == W && c->rope_cos.ptr;
     KeyBuilder kb;
     if (steady) {
       kb.add('F').add(B).add(N).add(S).add(F).add(H).add(W).add(static_cast<int>(latent_dtype)).add(static_cast<int>(context_dtype))
           .add(ts_per_token).add(mask_dev).add(lat.ptr).add(ctx.ptr).add(c->ts_in.ptr).add(c->vel.ptr).add(tcache->k.ptr).add(tcache->vt.ptr)
-          .add(tcache->has_bias).add(c->rope_cos.ptr).add(c->dist.sp).add(c->dist.sp_rank).add(c->dist.p2p).add(c->quant_bits);
+          .add(tcache->has_bias).add(c->rope_cos.ptr).add(c->dist.sp).add(c->dist.sp_rank).add(c->dist.p2p).add(c->quant_bits)
+          .add(c->precision);
       kb.add(flags->n_stg_blocks).add(flags->skip_self_attn).add(flags->skip_ff).add(flags->n_cas_blocks).add(flags->cross_attn_scale);
       for (int i = 0; i < flags->n_stg_blocks && i < LTX_MAX_FLAG_BLOCKS; ++i) kb.add(flags->stg_blocks[i]);
       for (int i = 0; i < flags->n_cas_blocks && i < LTX_MAX_FLAG_BLOCKS; ++i) kb.add(flags->cas_blocks[i]);
@@ -514,11 +520,17 @@ int ltx_dit_forward(ltx_ctx* c, const void* latent, ltx_dtype latent_dtype, cons
   });
 }
 
+// The dual model shares the video block weights, which FP8 mode converts to e4m3: its forwards and loop are refused there.
+static void av_precision_check(ltx_ctx* c) {
+  LTX_CHECK(c->precision != 8, LTX_ERR_UNSUPPORTED, "the dual audio/video model has no FP8 mode");
+}
+
 int ltx_av_forward_dev(ltx_ctx* c, const void* video_latent, ltx_dtype video_dtype, const void* audio_latent,
                        ltx_dtype audio_dtype, const void* video_context, const void* audio_context, ltx_dtype context_dtype,
                        const float* video_sigma, const float* audio_sigma, const int32_t* video_mask, const int32_t* audio_mask,
                        int N, int Ta, int S, int F, int H, int W, uint64_t context_key, float* out_video, float* out_audio) {
   return guarded(c, [&] {
+    av_precision_check(c);
     dit_av_forward_dev(c, video_latent, video_dtype, audio_latent, audio_dtype, video_context, audio_context, context_dtype,
                        video_sigma, 0, audio_sigma, video_mask, audio_mask, 1, N, Ta, S, F, H, W, context_key, out_video, out_audio);
   });
@@ -530,6 +542,7 @@ int ltx_av_forward_tokens_dev(ltx_ctx* c, const void* video_latent, ltx_dtype vi
                               const int32_t* audio_mask, int N, int Ta, int S, int F, int H, int W, uint64_t context_key,
                               float* out_video, float* out_audio) {
   return guarded(c, [&] {
+    av_precision_check(c);
     dit_av_forward_dev(c, video_latent, video_dtype, audio_latent, audio_dtype, video_context, audio_context, context_dtype,
                        video_sigmas, 1, audio_sigma, video_mask, audio_mask, 1, N, Ta, S, F, H, W, context_key, out_video, out_audio);
   });
@@ -538,6 +551,7 @@ int ltx_av_forward_tokens_dev(ltx_ctx* c, const void* video_latent, ltx_dtype vi
 // refusals of the batched dual forward that come before any work: B outside 1..2, B = 2 under Ulysses, null tensors
 static void av_batch_check(ltx_ctx* c, int B, const void* vl, const void* al, const void* vc, const void* ac, const float* vs,
                            const float* as, const void* ov, const void* oa) {
+  av_precision_check(c);
   LTX_CHECK(B >= 1, LTX_ERR_INVALID_ARGUMENT, "dual forward: B must be >= 1");
   LTX_CHECK(B <= 2, LTX_ERR_UNSUPPORTED, "dual forward: batches of 1 or 2 items");
   LTX_CHECK(B == 1 || !(c->dist.comm_world && c->dist.sp > 1), LTX_ERR_UNSUPPORTED, "the batched dual forward is single-GPU");
@@ -862,7 +876,7 @@ int ltx_denoise_step(ltx_ctx* c, const ltx_step_params* p) {
     // better (N = 4096 GEMMs: 192 tiles instead of 2 x 96 on 74 CTA pairs; attention: 768 CTAs instead of 2 x 384 on 296
     // slots) and the weights are read once.  Batch row 0 is the conditional pass, so the STG pass can still resume from its
     // stream.  Per batch row the arithmetic is that of the separate passes.
-    const bool batched = batched_cfg_env() && use_cfg && groups == 1 && !(c->dist.comm_world && c->dist.sp > 1) && c->precision == 16 &&
+    const bool batched = batched_cfg_env() && use_cfg && groups == 1 && !(c->dist.comm_world && c->dist.sp > 1) && c->precision != 32 &&
                          !p->disable_batched_cfg;
     const int stg_idx = use_stg ? n_pass - 1 : -1;
     const bool share = use_stg && !p->disable_stg_prefix_sharing && first_stg > 0 && first_stg < g.num_layers &&
@@ -905,10 +919,10 @@ int ltx_denoise_step(ltx_ctx* c, const ltx_step_params* p) {
     };
     // Steady state (every step of a session but the first): the projected text of each prompt this rank needs is cached and
     // the RoPE table is built, so the step is a fixed launch sequence on fixed buffers -> captured once, then replayed.
-    bool steady = c->precision == 16 && c->rope_f == F && c->rope_h == H && c->rope_w == W && c->rope_cos.ptr != nullptr;
+    bool steady = c->precision != 32 && c->rope_f == F && c->rope_h == H && c->rope_w == W && c->rope_cos.ptr != nullptr;
     KeyBuilder kb;
     kb.add('S').add(F).add(H).add(W).add(S).add(i2v).add(use_cfg).add(use_stg).add(share).add(first_stg).add(p->n_stg_blocks).add(batched)
-        .add(c->dist.world).add(c->dist.rank).add(c->dist.sp).add(groups).add(c->dist.p2p).add(c->quant_bits).add(c->s_ctx_dtype)
+        .add(c->dist.world).add(c->dist.rank).add(c->dist.sp).add(groups).add(c->dist.p2p).add(c->quant_bits).add(c->precision).add(c->s_ctx_dtype)
         .add(c->s_latent.ptr).add(c->s_tok.ptr).add(c->s_sigma.ptr).add(c->s_ts.ptr).add(c->vel.ptr).add(c->rope_cos.ptr);
     for (int i = 0; i < p->n_stg_blocks && i < LTX_MAX_FLAG_BLOCKS; ++i) kb.add(p->stg_blocks[i]);
     if (batched) {
@@ -960,6 +974,7 @@ int ltx_av_denoise_begin(ltx_ctx* c, const float* video_noise, const float* audi
                          const void* video_context, const void* audio_context, ltx_dtype context_dtype, const int32_t* mask,
                          const void* neg_video_context, const void* neg_audio_context, const int32_t* neg_mask, int S) {
   return guarded(c, [&] {
+    av_precision_check(c);
     LTX_CHECK(video_noise && audio_noise && video_context && audio_context && F > 0 && H > 0 && W > 0 && Ta > 0 && S > 0,
               LTX_ERR_INVALID_ARGUMENT, "bad av_denoise_begin arguments");
     LTX_CHECK((neg_video_context == nullptr) == (neg_audio_context == nullptr), LTX_ERR_INVALID_ARGUMENT,
@@ -1019,6 +1034,7 @@ int ltx_av_denoise_begin(ltx_ctx* c, const float* video_noise, const float* audi
 
 int ltx_av_denoise_step(ltx_ctx* c, const ltx_step_params* p) {
   return guarded(c, [&] {
+    av_precision_check(c);
     LTX_CHECK(p != nullptr && c->s_F > 0 && c->s_Ta > 0, LTX_ERR_INVALID_ARGUMENT, "av_denoise_step before av_denoise_begin");
     LTX_CHECK(p->sigma > 0.f, LTX_ERR_INVALID_ARGUMENT, "sigma must be > 0");
     LTX_CHECK(p->stg_scale == 0.f && p->ge_gamma == 0.f, LTX_ERR_UNSUPPORTED,
@@ -1335,6 +1351,48 @@ int ltx_op_gemm_q(ltx_ctx* c, const void* A, const void* q, const float* scales,
     GemmEpi e;
     e.mode = mode; e.out = C; e.ldo = N; e.bias = bias;
     launch_gemm_q(reinterpret_cast<const bf16*>(A), K, W, M, N, K, e, c->stream, force_bn);
+    c->launches++;
+  });
+}
+
+int ltx_op_quantize_fp8(ltx_ctx* c, const void* x_bf16, int M, int K, int64_t ld, void* codes, float* scales) {
+  return guarded(c, [&] {
+    LTX_CHECK(x_bf16 && codes && scales, LTX_ERR_INVALID_ARGUMENT, "null tensor");
+    launch_quantize_rows_fp8(reinterpret_cast<const bf16*>(x_bf16), ld, M, K, reinterpret_cast<uint8_t*>(codes), scales, c->stream);
+    c->launches++;
+  });
+}
+
+int ltx_op_gemm_fp8(ltx_ctx* c, const void* Aq, const float* sa, const void* Bq, const float* sb, const float* bias, void* C, int M,
+                    int N, int K, int mode, int force_bn) {
+  return guarded(c, [&] {
+    LTX_CHECK(Aq && sa && Bq && sb && C, LTX_ERR_INVALID_ARGUMENT, "null tensor");
+    LTX_CHECK(mode == EPI_BF16 || mode == EPI_GELU_BF16 || mode == EPI_F32 || mode == EPI_SILU_BF16, LTX_ERR_INVALID_ARGUMENT, "bad mode");
+    GemmEpi e;
+    e.mode = mode; e.out = C; e.ldo = N; e.bias = bias;
+    launch_gemm_fp8(reinterpret_cast<const uint8_t*>(Aq), K, sa, reinterpret_cast<const uint8_t*>(Bq), K, sb, M, N, K, e, c->stream,
+                    force_bn);
+    c->launches++;
+  });
+}
+
+int ltx_op_gemm_fp8_ex(ltx_ctx* c, const void* Aq, const float* sa, const void* Bq, const float* sb, const float* bias, void* C,
+                       void* Ct, int tsplit_col, int64_t ldt, float* x, const float* gate_a, const float* gate_b, void* shadow,
+                       int M, int N, int K, int force_bn) {
+  return guarded(c, [&] {
+    LTX_CHECK(Aq && sa && Bq && sb && (x != nullptr) != (C != nullptr), LTX_ERR_INVALID_ARGUMENT,
+              "bad FP8 GEMM arguments: one of C (bf16, with optional V^T split) or x (gate * residual)");
+    GemmEpi e;
+    e.bias = bias;
+    if (x) {
+      e.mode = EPI_GATE_RESID; e.resid = x; e.ldr = N; e.gate_a = gate_a; e.gate_b = gate_b; e.gate_ld = 0;
+      e.rows_per_gate = M; e.shadow = reinterpret_cast<bf16*>(shadow); e.lds = N;
+    } else {
+      e.mode = EPI_BF16; e.out = C; e.ldo = tsplit_col > 0 ? tsplit_col : N;
+      if (tsplit_col > 0) { e.tsplit_col = tsplit_col; e.out_t = reinterpret_cast<bf16*>(Ct); e.ldt = ldt; }
+    }
+    launch_gemm_fp8(reinterpret_cast<const uint8_t*>(Aq), K, sa, reinterpret_cast<const uint8_t*>(Bq), K, sb, M, N, K, e, c->stream,
+                    force_bn);
     c->launches++;
   });
 }

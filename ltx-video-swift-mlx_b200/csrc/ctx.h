@@ -254,7 +254,9 @@ struct ltx_ctx {
   int snap_rows = 0;
 
   // ---- fp32 mode (dit_f32.cu): fp32 weights + activations, split-bf16 GEMM operands
-  int precision = 16;   // 16: bf16 weights (default), 32: DiT matrices stay fp32 and the forward runs in fp32 mode
+  int precision = 16;   // 16: bf16 weights (default), 32: DiT matrices stay fp32 and the forward runs in fp32 mode,
+                        // 8: the block Linears run as e4m3 x e4m3 GEMMs (weights converted at finalize, dit_convert_fp8)
+  ltx::DevBuf fp8_act;  // mode 8: e4m3 codes + row scales of the current GEMM's A operand
   ltx::DevBuf f_asplit, f_wsplit, f_h, f_q, f_k, f_v, f_att, f_ffh, f_ctx, f_c1, f_c2, f_tk, f_tv, f_lat, f_bias;
 
   // ---- resident denoise session
@@ -309,6 +311,7 @@ void graphs_clear(ltx_ctx* c);
 // dit.cu
 void dit_finalize(ltx_ctx* c);
 void dit_quantize(ltx_ctx* c, int bits);
+void dit_convert_fp8(ltx_ctx* c);
 // snapshot_block >= 0: save the residual stream at the entry of that block (for a later resume);
 // resume_block >= 0: skip the embedding and blocks [0, resume_block) and continue from the saved stream (SURVEY H10:
 // the STG-perturbed pass shares every block before the first perturbed one with the conditional pass).

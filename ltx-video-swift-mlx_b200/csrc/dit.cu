@@ -16,9 +16,38 @@ namespace ltx {
 
 namespace {
 
+// the e4m3 replacement of a weight (precision mode 8), or nullptr
+const QuantW* fp8_weight(const ltx_ctx* c, const void* w) {
+  if (c->qw.empty()) return nullptr;
+  auto it = c->qw.find(w);
+  return (it != c->qw.end() && it->second.fmt == QF_E4M3) ? &it->second : nullptr;
+}
+
+// Precision mode 8: A's rows become e4m3 codes + power-of-two row scales in one reused scratch buffer, then the FP8 pair kernel
+// runs for every M (no weight-streaming, 1-CTA or swap-AB form), so each row's result depends on that row alone: a batched
+// forward equals its items' forwards bit for bit.  Rows [0, N) of the weight are used (the q|k rows of the packed q|k|v).
+void gemm_fp8(ltx_ctx* c, const bf16* A, int64_t lda, const QuantW& W, int M, int N, int K, const GemmEpi& e, int force_bn) {
+  LTX_CHECK(W.k == K && W.n >= N, LTX_ERR_INVALID_ARGUMENT, "FP8 GEMM: weight shape mismatch");
+  const size_t code_bytes = (static_cast<size_t>(M) * K + 15) / 16 * 16;
+  c->fp8_act.reserve(code_bytes + static_cast<size_t>(M) * 4);
+  uint8_t* q = c->fp8_act.as<uint8_t>();
+  float* s = reinterpret_cast<float*>(q + code_bytes);
+  {
+    ProfScope ps(c, PROF_ROW, 0.0, 3.0 * M * K + 4.0 * M);
+    launch_quantize_rows_fp8(A, lda, M, K, q, s, c->stream);
+  }
+  ProfScope ps(c, PROF_GEMM, 2.0 * M * N * K, static_cast<double>(M) * K + static_cast<double>(N) * K + 2.0 * M * N);
+  launch_gemm_fp8(q, K, s, W.q, W.k, W.scales, M, N, K, e, c->stream, force_bn);
+}
+
 // profiled launch helpers (flop / byte counts are the algorithmic ones used by bench.py's roofline)
 void gemm(ltx_ctx* c, const bf16* A, int64_t lda, const bf16* B, int64_t ldb, int M, int N, int K, const GemmEpi& e,
           int a_kblock = 0, int64_t a_kblock_stride = 0) {
+  if (const QuantW* w8 = fp8_weight(c, B)) {
+    LTX_CHECK(a_kblock == 0, LTX_ERR_UNSUPPORTED, "FP8 GEMM: no K-blocked A operand");
+    gemm_fp8(c, A, lda, *w8, M, N, K, e, 0);
+    return;
+  }
   auto it = c->qw.empty() ? c->qw.end() : c->qw.find(B);
   const bool panel = it != c->qw.end() && gemm_q_uses_panel(it->second, M);
   ProfScope ps(c, PROF_GEMM, 2.0 * M * N * K, 2.0 * (static_cast<double>(M) * K + static_cast<double>(N) * K + static_cast<double>(M) * N),
@@ -329,6 +358,16 @@ void dit_finalize(ltx_ctx* c) {
   c->dit_ready = true;
 }
 
+namespace {
+// frees a replaced weight: a loaded tensor or an allocation made by finalize
+void release_weight(ltx_ctx* c, const void* p) {
+  for (auto it = c->tensors.begin(); it != c->tensors.end(); ++it)
+    if (it->second.ptr == p) { cudaFree(it->second.ptr); c->tensors.erase(it); return; }
+  for (auto it = c->owned.begin(); it != c->owned.end(); ++it)
+    if (*it == p) { cudaFree(*it); c->owned.erase(it); return; }
+}
+}  // namespace
+
 // Replace every GEMM weight of the DiT by per-64-group affine codes (the reference quantises every Linear,
 // P/LTXPipeline.swift:323-333); the bf16 copies are freed.  The M = 1 timestep-MLP GEMVs keep bf16 weights.
 void dit_quantize(ltx_ctx* c, int bits) {
@@ -336,12 +375,7 @@ void dit_quantize(ltx_ctx* c, int bits) {
   LTX_CHECK(bits == 8 || bits == 4, LTX_ERR_UNSUPPORTED, "quant_bits must be 16, 8 or 4");
   const ltx_config& g = c->cfg;
   const int D = g.num_heads * g.head_dim, FF = g.ffn_mult * D;
-  auto release = [&](const void* p) {
-    for (auto it = c->tensors.begin(); it != c->tensors.end(); ++it)
-      if (it->second.ptr == p) { cudaFree(it->second.ptr); c->tensors.erase(it); return; }
-    for (auto it = c->owned.begin(); it != c->owned.end(); ++it)
-      if (*it == p) { cudaFree(*it); c->owned.erase(it); return; }
-  };
+  auto release = [&](const void* p) { release_weight(c, p); };
   // Each quantised weight gets a 16-byte device allocation whose address is its identity from now on: the struct field
   // is repointed to it and gemm() recognises it in c->qw (the freed bf16 address could be handed out again by cudaMalloc).
   std::vector<const void*> to_free;
@@ -417,6 +451,51 @@ void dit_quantize(ltx_ctx* c, int bits) {
   c->quant_bits = bits;
 }
 
+// Precision mode 8: every Linear inside the transformer blocks becomes e4m3 codes with one power-of-two scale per output
+// channel (launch_quantize_rows_fp8: the rule gemm() applies to the activation rows); the bf16 copies are freed.  Patchify,
+// caption projection, the timestep MLPs / AdaLN and proj_out stay bf16.  The weights are found through dit_quantize's
+// handles, with the e4m3 format in their map entry.
+void dit_convert_fp8(ltx_ctx* c) {
+  LTX_CHECK(c->dit_ready && c->qw.empty(), LTX_ERR_WEIGHTS, "FP8 conversion needs finalized, unquantised DiT weights");
+  const ltx_config& g = c->cfg;
+  const int D = g.num_heads * g.head_dim, FF = g.ffn_mult * D;
+  LTX_CHECK(D % 16 == 0 && FF % 16 == 0, LTX_ERR_INVALID_CONFIGURATION, "FP8 mode needs Linear widths that are multiples of 16");
+  std::vector<const void*> to_free;
+  auto handle_for = [&](const QuantW& r) {
+    void* handle = nullptr;
+    LTX_CUDA(cudaMalloc(&handle, 16));
+    c->owned.push_back(handle);
+    c->qw[handle] = r;
+    return reinterpret_cast<const bf16*>(handle);
+  };
+  auto conv = [&](const bf16*& w, int N, int K) {
+    uint8_t* q = nullptr;
+    float* s = nullptr;
+    LTX_CUDA(cudaMalloc(&q, static_cast<size_t>(N) * K));
+    LTX_CUDA(cudaMalloc(&s, static_cast<size_t>(N) * 4));
+    c->owned.push_back(q); c->owned.push_back(s);
+    launch_quantize_rows_fp8(w, K, N, K, q, s, c->stream);
+    QuantW r;
+    r.fmt = QF_E4M3; r.q = q; r.scales = s; r.bits = 8; r.n = N; r.k = K;
+    to_free.push_back(w);
+    w = handle_for(r);
+    return r;
+  };
+  for (auto& b : c->blocks) {
+    // the packed q|k|v [3D, D] as one matrix, so the fused projection with its V^T epilogue stays one launch; its v rows get
+    // a handle of their own (rows are independent) for the per-batch V^T projections
+    QuantW v = conv(b.a1.wq, 3 * D, D);
+    v.q += static_cast<size_t>(2) * D * D; v.scales += 2 * D; v.n = D;
+    b.a1.wk = nullptr;
+    b.a1.wv = handle_for(v);
+    conv(b.a1.wo, D, D);
+    conv(b.a2.wq, D, D); conv(b.a2.wk, D, D); conv(b.a2.wv, D, D); conv(b.a2.wo, D, D);
+    conv(b.w_in, FF, D); conv(b.w_out, D, FF);
+  }
+  LTX_CUDA(cudaStreamSynchronize(c->stream));
+  for (const void* p : to_free) release_weight(c, p);
+}
+
 void dit_forward_dev(ltx_ctx* c, const void* latent, int latent_dtype, const void* context, int context_dtype,
                      const float* timesteps_dev, int ts_per_token, const int32_t* mask_dev, int B, int N, int S, int F,
                      int H, int W, const ltx_dit_flags* flags, float* out_velocity_dev, int snapshot_block, int resume_block) {
@@ -434,6 +513,7 @@ void dit_forward_dev(ltx_ctx* c, const void* latent, int latent_dtype, const voi
   const int Cin = g.in_channels, Cout = g.out_channels;
   // ---- Ulysses sequence parallelism: this rank owns tokens [tok0, tok0 + Nl) for every row-wise op
   const int P = (c->dist.comm_world && c->dist.sp > 1) ? c->dist.sp : 1;
+  LTX_CHECK(P == 1 || c->precision != 8, LTX_ERR_UNSUPPORTED, "FP8 mode has no sequence-parallel forward");
   LTX_CHECK(P == 1 || (B == 1 && N % P == 0 && Hh % P == 0), LTX_ERR_INVALID_ARGUMENT,
             "sequence parallelism needs B == 1 and N, num_heads divisible by sp_size");
   const int Nl = N / P, tok0 = (P > 1 ? c->dist.sp_rank : 0) * Nl;
@@ -590,10 +670,14 @@ void dit_forward_dev(ltx_ctx* c, const void* latent, int latent_dtype, const voi
       // q|k|v in one GEMM (N = 3D, 256-wide tiles: 288 tiles = 3.9 rounds of 74 CTA pairs at M = 1536), the V columns stored
       // transposed by the epilogue; separate q|k and V^T GEMMs for batches, sequence parallelism and quantised weights
       // (batches: V^T row = feature, column = b * ldv + token -- the same as the GEMM row b * N + token when ldv == N)
-      const bool fused_qkv = P == 1 && (B == 1 || ldv == N) && c->qw.empty() && D % 32 == 0;
+      const QuantW* qkv8 = fp8_weight(c, bw.a1.wq);
+      const bool fused_qkv = P == 1 && (B == 1 || ldv == N) && (c->qw.empty() || qkv8) && D % 32 == 0;
       GemmEpi e;
       e.mode = EPI_BF16; e.out = qk; e.ldo = 2 * D; e.bias = bw.a1.bq;
-      if (fused_qkv) {
+      if (fused_qkv && qkv8) {
+        e.tsplit_col = 2 * D; e.out_t = vt; e.ldt = B * ldv;
+        gemm_fp8(c, h, D, *qkv8, R, 3 * D, D, e, 256);
+      } else if (fused_qkv) {
         e.tsplit_col = 2 * D; e.out_t = vt; e.ldt = B * ldv;
         ProfScope ps(c, PROF_GEMM, 2.0 * R * 3.0 * D * D, 2.0 * (static_cast<double>(R) * D + 3.0 * D * D + 3.0 * R * D));
         launch_gemm(h, D, bw.a1.wq, D, R, 3 * D, D, e, st, R > 128 ? 1256 : 256);

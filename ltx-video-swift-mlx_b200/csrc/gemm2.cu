@@ -21,7 +21,7 @@ namespace ltx {
 namespace {
 
 constexpr int BM2 = 128;          // rows per CTA (256 per pair)
-constexpr int BK2 = 64;           // k of one 128-byte swizzle atom
+constexpr int BK2 = 64;           // k of one 128-byte swizzle atom (bf16; 128 e4m3 codes fill the same atom)
 constexpr int G2_THREADS = 192;
 constexpr int G2_BN_MAX = 256;
 constexpr uint32_t G2_A_BYTES = BM2 * BK2 * 2;                 // 16 KB: one atom of A
@@ -34,10 +34,14 @@ constexpr int G2_STAGES = 3;
 constexpr uint32_t G2_A_STAGE = G2_KSUB * G2_A_BYTES, G2_B_STAGE = G2_KSUB * G2_B_STRIDE;
 constexpr size_t G2_SMEM = 1024 + G2_STAGES * (G2_A_STAGE + G2_B_STAGE) + (2 * G2_STAGES + 4) * 8 + 16 + 128 + 4 * EPI_STAGE_BYTES;
 
-template <int MODE>
+// FP8: the operands are e4m3 codes (kind::f8f6f4).  A swizzle atom then holds 128 k instead of 64, so a stage holds 256 k;
+// the byte layout of the stages, the four 32-byte MMA steps per atom and the barrier protocol are the same.  The epilogue
+// scales the accumulator by sa[m] * sb[n] (gemm_epilogue.cuh) before the epilogue of `ep`.
+template <int MODE, bool FP8>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(G2_THREADS, 1)
 gemm_bf16_2cta(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, int M, int N, int K, int BN,
-               int a_kblock, const GemmEpi ep) {
+               int a_kblock, const GemmEpi ep, const float* sa, const float* sb) {
+  constexpr int AK = FP8 ? 2 * BK2 : BK2;   // k of one swizzle atom
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~static_cast<uintptr_t>(1023));
   uint8_t* sA = smem;
@@ -56,7 +60,7 @@ gemm_bf16_2cta(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   const int num_mp = (M + 2 * BM2 - 1) / (2 * BM2);   // 256-row pair tiles
   const int num_n = (N + BN - 1) / BN;
   const int num_tiles = num_mp * num_n;
-  const int num_k = (K + G2_KSUB * BK2 - 1) / (G2_KSUB * BK2);   // pipeline steps of 128 k
+  const int num_k = (K + G2_KSUB * AK - 1) / (G2_KSUB * AK);   // pipeline steps of 128 k (256 k with FP8)
   const int half_bn = BN >> 1;
   const uint32_t b_bytes = static_cast<uint32_t>(half_bn) * BK2 * 2;
 
@@ -96,7 +100,7 @@ gemm_bf16_2cta(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
           else mbar_arrive_remote(&full[stage], 0);
 #pragma unroll
           for (int ks = 0; ks < G2_KSUB; ++ks) {   // k past K (a ragged tail) is zero-filled by TMA
-            const int k0 = (kb * G2_KSUB + ks) * BK2;
+            const int k0 = (kb * G2_KSUB + ks) * AK;
             if (a_kblock > 0)
               tma_load_3d_2sm(sA + stage * G2_A_STAGE + ks * G2_A_BYTES, &tmA, &full[stage], k0 % a_kblock, m0, k0 / a_kblock);
             else
@@ -109,7 +113,7 @@ gemm_bf16_2cta(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     }
   } else if (warp == 1) {
     if (leader && lane == 0) {
-      const uint32_t idesc = umma_idesc_bf16(2 * BM2, BN);
+      const uint32_t idesc = FP8 ? umma_idesc_e4m3(2 * BM2, BN) : umma_idesc_bf16(2 * BM2, BN);
       const uint64_t a_desc0 = umma_desc_sw128(smem_u32(sA)), b_desc0 = umma_desc_sw128(smem_u32(sB));
       int stage = 0;
       uint32_t phase = 0;
@@ -130,9 +134,11 @@ gemm_bf16_2cta(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
 #pragma unroll
           for (int ks = 0; ks < G2_KSUB; ++ks)
 #pragma unroll
-            for (int k = 0; k < BK2 / 16; ++k)
-              umma_bf16_2cta(d_tmem, a_desc + ((ks * G2_A_BYTES + k * 32) >> 4), b_desc + ((ks * G2_B_STRIDE + k * 32) >> 4),
-                             idesc, (kb | ks | k) != 0 ? 1u : 0u);
+            for (int k = 0; k < BK2 / 16; ++k) {
+              const uint64_t ad = a_desc + ((ks * G2_A_BYTES + k * 32) >> 4), bd = b_desc + ((ks * G2_B_STRIDE + k * 32) >> 4);
+              if (FP8) umma_f8_2cta(d_tmem, ad, bd, idesc, (kb | ks | k) != 0 ? 1u : 0u);
+              else umma_bf16_2cta(d_tmem, ad, bd, idesc, (kb | ks | k) != 0 ? 1u : 0u);
+            }
           umma_commit_2cta(&empty[stage]);
           if (++stage == G2_STAGES) { stage = 0; phase ^= 1; }
         }
@@ -149,8 +155,8 @@ gemm_bf16_2cta(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       mbar_wait(&tfull[as], aphase);
       tc_fence_after();
       const uint32_t taddr = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + as * G2_BN_MAX;
-      epilogue_tile<MODE>(taddr, BN, epi_stage + (warp - 2) * (EPI_STAGE_BYTES / 4), lane,
-                          (mp * 2 + static_cast<int>(rank)) * BM2 + q * 32, n_blk * BN, M, N, ep);
+      epilogue_tile<MODE, FP8>(taddr, BN, epi_stage + (warp - 2) * (EPI_STAGE_BYTES / 4), lane,
+                               (mp * 2 + static_cast<int>(rank)) * BM2 + q * 32, n_blk * BN, M, N, ep, sa, sb);
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive_remote(&tempty[as], 0);
@@ -164,15 +170,34 @@ gemm_bf16_2cta(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   }
 }
 
-template <int MODE>
+template <int MODE, bool FP8 = false>
 void launch2(const CUtensorMap& tmA, const CUtensorMap& tmB, int M, int N, int K, int BN, int a_kblock, const GemmEpi& epi,
-             cudaStream_t stream) {
-  auto kern = gemm_bf16_2cta<MODE>;
+             cudaStream_t stream, const float* sa = nullptr, const float* sb = nullptr) {
+  auto kern = gemm_bf16_2cta<MODE, FP8>;
   ensure_dyn_smem(kern, G2_SMEM);
   const int tiles = ((M + 2 * BM2 - 1) / (2 * BM2)) * ((N + BN - 1) / BN);
   const int clusters = device_sm_count() / 2;
   const int grid = 2 * (tiles < clusters ? tiles : clusters);
-  launch_pdl(PDL_GEMM, kern, dim3(grid), dim3(G2_THREADS), G2_SMEM, stream, tmA, tmB, M, N, K, BN, a_kblock, epi);
+  launch_pdl(PDL_GEMM, kern, dim3(grid), dim3(G2_THREADS), G2_SMEM, stream, tmA, tmB, M, N, K, BN, a_kblock, epi, sa, sb);
+}
+
+template <bool FP8>
+void launch2_mode(const CUtensorMap& tmA, const CUtensorMap& tmB, int M, int N, int K, int bn, int a_kblock, const GemmEpi& epi,
+                  cudaStream_t stream, const float* sa, const float* sb) {
+  switch (epi.mode) {
+    case EPI_BF16: launch2<EPI_BF16, FP8>(tmA, tmB, M, N, K, bn, a_kblock, epi, stream, sa, sb); break;
+    case EPI_GELU_BF16: launch2<EPI_GELU_BF16, FP8>(tmA, tmB, M, N, K, bn, a_kblock, epi, stream, sa, sb); break;
+    case EPI_GATE_RESID: launch2<EPI_GATE_RESID, FP8>(tmA, tmB, M, N, K, bn, a_kblock, epi, stream, sa, sb); break;
+    case EPI_F32: launch2<EPI_F32, FP8>(tmA, tmB, M, N, K, bn, a_kblock, epi, stream, sa, sb); break;
+    case EPI_SILU_BF16: launch2<EPI_SILU_BF16, FP8>(tmA, tmB, M, N, K, bn, a_kblock, epi, stream, sa, sb); break;
+    default: LTX_CHECK(false, 2, "bad GEMM epilogue mode");
+  }
+}
+
+void check_tsplit(const GemmEpi& epi, int bn) {
+  LTX_CHECK(epi.tsplit_col == 0 || (epi.mode == EPI_BF16 && bn % 32 == 0 && epi.tsplit_col % 32 == 0 && epi.out_t != nullptr &&
+                                    epi.ldt % 8 == 0 && epi.col_block == 0),
+            2, "GEMM: transposed-column output needs the bf16 epilogue, a tile width and split column that are multiples of 32");
 }
 
 }  // namespace
@@ -200,9 +225,7 @@ void launch_gemm_2cta(const bf16* A, int64_t lda, const bf16* B, int64_t ldb, in
                       cudaStream_t stream, int force_bn, int a_kblock, int64_t a_kblock_stride) {
   int bn = force_bn ? force_bn : gemm2_fit_tile_width(M, N);
   LTX_CHECK(bn >= 64 && bn <= 256 && bn % 16 == 0, 2, "2-CTA GEMM: tile width must be a multiple of 16 in [64, 256]");
-  LTX_CHECK(epi.tsplit_col == 0 || (epi.mode == EPI_BF16 && bn % 32 == 0 && epi.tsplit_col % 32 == 0 && epi.out_t != nullptr &&
-                                    epi.ldt % 8 == 0 && epi.col_block == 0),
-            2, "GEMM: transposed-column output needs the bf16 epilogue, a tile width and split column that are multiples of 32");
+  check_tsplit(epi, bn);
   CUtensorMap tmA;
   if (a_kblock > 0) {
     LTX_CHECK(a_kblock % BK2 == 0 && K % a_kblock == 0 && lda == a_kblock, 2, "GEMM: bad K-blocked A layout");
@@ -211,14 +234,30 @@ void launch_gemm_2cta(const bf16* A, int64_t lda, const bf16* B, int64_t ldb, in
     tmA = make_tmap_2d(A, M, K, lda, BM2);
   }
   CUtensorMap tmB = make_tmap_2d(B, N, K, ldb, bn / 2);
-  switch (epi.mode) {
-    case EPI_BF16: launch2<EPI_BF16>(tmA, tmB, M, N, K, bn, a_kblock, epi, stream); break;
-    case EPI_GELU_BF16: launch2<EPI_GELU_BF16>(tmA, tmB, M, N, K, bn, a_kblock, epi, stream); break;
-    case EPI_GATE_RESID: launch2<EPI_GATE_RESID>(tmA, tmB, M, N, K, bn, a_kblock, epi, stream); break;
-    case EPI_F32: launch2<EPI_F32>(tmA, tmB, M, N, K, bn, a_kblock, epi, stream); break;
-    case EPI_SILU_BF16: launch2<EPI_SILU_BF16>(tmA, tmB, M, N, K, bn, a_kblock, epi, stream); break;
-    default: LTX_CHECK(false, 2, "bad GEMM epilogue mode");
+  launch2_mode<false>(tmA, tmB, M, N, K, bn, a_kblock, epi, stream, nullptr, nullptr);
+}
+
+void launch_gemm_fp8(const uint8_t* A, int64_t lda, const float* sa, const uint8_t* B, int64_t ldb, const float* sb, int M, int N,
+                     int K, const GemmEpi& epi, cudaStream_t stream, int force_bn) {
+  LTX_CHECK(M > 0 && N > 0 && K > 0, 2, "GEMM: empty problem");
+  LTX_CHECK(K % 16 == 0 && lda % 16 == 0 && ldb % 16 == 0 && lda >= K && ldb >= K, 2,
+            "FP8 GEMM: K and the row pitches must be multiples of 16 bytes");
+  LTX_CHECK(sa != nullptr && sb != nullptr && (reinterpret_cast<uintptr_t>(sb) & 15) == 0, 2,
+            "FP8 GEMM: row scales of both operands needed (sb 16-byte aligned)");
+  LTX_CHECK(epi.col_block == 0 && epi.transpose_out == 0, 2, "FP8 GEMM: no column-blocked or transposed-row output");
+  if (epi.mode == EPI_GATE_RESID) {
+    LTX_CHECK(epi.resid != nullptr && epi.ldr % 4 == 0, 2, "GEMM: residual epilogue needs fp32 resid with ld % 4 == 0");
+    LTX_CHECK(epi.shadow == nullptr || epi.lds % 4 == 0, 2, "GEMM: shadow ld must be a multiple of 4");
+  } else {
+    LTX_CHECK(epi.out != nullptr, 2, "GEMM: missing output");
+    LTX_CHECK(epi.ldo % (epi.mode == EPI_F32 ? 4 : 8) == 0, 2, "GEMM: output ld alignment");
   }
+  const int bn = force_bn ? force_bn : gemm2_fit_tile_width(M, N);
+  LTX_CHECK(bn >= 64 && bn <= 256 && bn % 16 == 0, 2, "2-CTA GEMM: tile width must be a multiple of 16 in [64, 256]");
+  check_tsplit(epi, bn);
+  const CUtensorMap tmA = make_tmap_u8_sw128(A, M, K, lda, BM2);
+  const CUtensorMap tmB = make_tmap_u8_sw128(B, N, K, ldb, bn / 2);
+  launch2_mode<true>(tmA, tmB, M, N, K, bn, 0, epi, stream, sa, sb);
 }
 
 }  // namespace ltx

@@ -180,11 +180,29 @@ __device__ __forceinline__ void epi_prefetch_resid(float4 (&xin)[8], int lane, i
   }
 }
 
+// SCALED (the FP8 pair kernel): this thread's accumulator row times sa[row], then times sb[column], in fp32 and in that order,
+// before anything else of the epilogue.  Columns past N read no scale (their results are never stored).
+__device__ __forceinline__ void epi_scale_chunk(uint32_t (&r)[32], float sa, const float* sb, int col0, int N) {
+  float s[32];
+  if (col0 + 32 <= N) {
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+      const float4 t = reinterpret_cast<const float4*>(sb + col0)[j];
+      s[4 * j] = t.x; s[4 * j + 1] = t.y; s[4 * j + 2] = t.z; s[4 * j + 3] = t.w;
+    }
+  } else {
+#pragma unroll
+    for (int j = 0; j < 32; ++j) s[j] = col0 + j < N ? sb[col0 + j] : 0.f;
+  }
+#pragma unroll
+  for (int j = 0; j < 32; ++j) r[j] = __float_as_uint((__uint_as_float(r[j]) * sa) * s[j]);
+}
+
 // Whole-tile epilogue of one warp: accumulator lanes [taddr.lane, +32) x BN columns starting at TMEM address `taddr`;
 // output rows [row0, row0+32), columns [col_base, col_base+BN).  BN is a multiple of 16.  Must be called by all 32 lanes.
-template <int MODE>
+template <int MODE, bool SCALED = false>
 __device__ __forceinline__ void epilogue_tile(uint32_t taddr, int BN, float* stage, int lane, int row0, int col_base, int M,
-                                              int N, const GemmEpi& ep) {
+                                              int N, const GemmEpi& ep, const float* sa = nullptr, const float* sb = nullptr) {
   const int nfull = BN >> 5;
   const int nch = nfull + ((BN & 16) ? 1 : 0);
   uint32_t r[32];
@@ -192,9 +210,12 @@ __device__ __forceinline__ void epilogue_tile(uint32_t taddr, int BN, float* sta
   if (nfull > 0) tmem_ld32(taddr, r);
   else tmem_ld16(taddr, r);
   if (MODE == EPI_GATE_RESID) epi_prefetch_resid(xcur, lane, row0, col_base, nfull > 0 ? 32 : 16, M, N, ep);
+  float row_s = 0.f;
+  if (SCALED && row0 + lane < M) row_s = sa[row0 + lane];
 #pragma unroll 1
   for (int c = 0; c < nch; ++c) {
     tmem_ld_wait();
+    if (SCALED) epi_scale_chunk(r, row_s, sb, col_base + c * 32, N);
     epi_stage_write(stage, lane, r);
     __syncwarp();
     if (c + 1 < nch) {   // next chunk's TMEM read and residual loads overlap this chunk's global traffic

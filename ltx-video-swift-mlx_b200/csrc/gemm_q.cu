@@ -15,6 +15,8 @@
 //                                fence.proxy.async, arrive
 //   warp 1     : MMA issuer (tcgen05.mma, TMEM accumulators, two stages)      warps 2-5: epilogue
 // HBM / L2 traffic for weights drops 2x (int8) / 4x (int4); the tensor core still runs bf16 x bf16 -> fp32.
+#include <cuda_fp8.h>
+
 #include "gemm_epilogue.cuh"
 #include "ltx_internal.h"
 #include "ptx.cuh"
@@ -361,7 +363,73 @@ void launch_q_mode(const CUtensorMap& tmA, const CUtensorMap& tmQ, int M, int N,
   }
 }
 
+// ---------------------------------------------------------------- per-row e4m3 quantiser (precision mode 8)
+// One CTA per row.  Pass 1 takes the row's amax, pass 2 writes the codes; both read 8 bf16 per thread and step.  The scale is
+// a power of two, so x / s is exact and each code is a function of its element and the row's amax alone: the codes do not
+// depend on the launch shape, and a row's codes do not depend on the other rows.
+constexpr int QF8_THREADS = 256;
+
+__global__ void __launch_bounds__(QF8_THREADS) quantize_rows_fp8_kernel(const bf16* x, int64_t ld, int K, uint8_t* q, float* s) {
+  __shared__ float red[QF8_THREADS / 32];
+  __shared__ float row_scale;
+  griddep_wait();
+  griddep_launch();
+  const int m = blockIdx.x, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const bf16* xr = x + static_cast<int64_t>(m) * ld;
+  const int nvec = K / 8;
+  float amax = 0.f;
+  for (int v = threadIdx.x; v < nvec; v += QF8_THREADS) {
+    const uint4 u = *reinterpret_cast<const uint4*>(xr + v * 8);
+    const __nv_bfloat162* h = reinterpret_cast<const __nv_bfloat162*>(&u);
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      const float2 f = __bfloat1622float2(h[j]);
+      amax = fmaxf(amax, fmaxf(fabsf(f.x), fabsf(f.y)));
+    }
+  }
+  amax = warp_max(amax);
+  if (lane == 0) red[warp] = amax;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    float a = 0.f;
+#pragma unroll
+    for (int w = 0; w < QF8_THREADS / 32; ++w) a = fmaxf(a, red[w]);
+    // the least power of two 2^e with a <= 448 * 2^e: a = f * 2^E (f in [0.5, 1)), 448 = 0.875 * 2^9
+    float sc = 1.f;
+    if (a > 0.f) {
+      int E;
+      const float f = frexpf(a, &E);
+      sc = ldexpf(1.f, f <= 0.875f ? E - 9 : E - 8);
+    }
+    row_scale = sc;
+    s[m] = sc;
+  }
+  __syncthreads();
+  const float sc = row_scale;
+  uint8_t* qr = q + static_cast<int64_t>(m) * K;
+  for (int v = threadIdx.x; v < nvec; v += QF8_THREADS) {
+    const uint4 u = *reinterpret_cast<const uint4*>(xr + v * 8);
+    const __nv_bfloat162* h = reinterpret_cast<const __nv_bfloat162*>(&u);
+    uint32_t packed[2];
+#pragma unroll
+    for (int j = 0; j < 2; ++j) {
+      const float2 f0 = __bfloat1622float2(h[2 * j]), f1 = __bfloat1622float2(h[2 * j + 1]);
+      const uint32_t lo = __nv_cvt_float2_to_fp8x2(make_float2(f0.x / sc, f0.y / sc), __NV_SATFINITE, __NV_E4M3);
+      const uint32_t hi = __nv_cvt_float2_to_fp8x2(make_float2(f1.x / sc, f1.y / sc), __NV_SATFINITE, __NV_E4M3);
+      packed[j] = lo | (hi << 16);
+    }
+    *reinterpret_cast<uint2*>(qr + v * 8) = make_uint2(packed[0], packed[1]);
+  }
+}
+
 }  // namespace
+
+void launch_quantize_rows_fp8(const bf16* x, int64_t ld, int M, int K, uint8_t* q, float* s, cudaStream_t stream) {
+  LTX_CHECK(M > 0 && K > 0 && K % 16 == 0 && ld % 8 == 0 && ld >= K, 2, "FP8 quantiser: K % 16 == 0, ld % 8 == 0, ld >= K");
+  LTX_CHECK((reinterpret_cast<uintptr_t>(x) & 15) == 0 && (reinterpret_cast<uintptr_t>(q) & 15) == 0, 2,
+            "FP8 quantiser: 16-byte aligned input and codes");
+  launch_pdl(PDL_ROWS, quantize_rows_fp8_kernel, dim3(M), dim3(QF8_THREADS), 0, stream, x, ld, K, q, s);
+}
 
 // Large M: the fused kernels redo the code -> bf16 conversion once per 128 / 256-row M tile (12x / 6x at M = 1536) and are
 // bound by its instruction issue (~450 TFLOP/s); converting the weight ONCE into the context's bf16 panel and running the

@@ -153,15 +153,28 @@ void launch_gemm_swapab(const bf16* A, int64_t lda, const bf16* W, int64_t ldb, 
 void launch_gemm_2cta(const bf16* A, int64_t lda, const bf16* B, int64_t ldb, int M, int N, int K, const GemmEpi& epi,
                       cudaStream_t stream, int force_bn, int a_kblock, int64_t a_kblock_stride);
 int gemm2_fit_tile_width(int M, int N);
+// FP8 form of the pair kernel: C[M,N] = (A[M,K] * B[N,K]^T) * sa[m] * sb[n] (fp32, in that order) + the epilogue of `epi`.
+// A, B: e4m3 codes, K-major, row pitch lda / ldb bytes (multiples of 16; K % 16 == 0, the K tail is zero-filled by TMA);
+// sa [M], sb [N] fp32 row scales.  force_bn: 0 = gemm2_fit_tile_width, else a multiple of 16 in [64, 256].
+void launch_gemm_fp8(const uint8_t* A, int64_t lda, const float* sa, const uint8_t* B, int64_t ldb, const float* sb, int M, int N,
+                     int K, const GemmEpi& epi, cudaStream_t stream, int force_bn = 0);
+// Per-row e4m3 quantiser (gemm_q.cu): s[m] = 2^ceil(log2(amax_m / 448)) (1 for a zero row), q[m,k] = e4m3_rn_satfinite(x / s).
+// x bf16 [M, K] with row pitch ld (elements, multiple of 8; K % 16 == 0); q [M, K] (pitch K), s [M].
+void launch_quantize_rows_fp8(const bf16* x, int64_t ld, int M, int K, uint8_t* q, float* s, cudaStream_t stream);
 // ---------------------------------------------------------------- quantised weights (gemm_q.cu)
+enum QuantFormat : int {
+  QF_AFFINE = 0,   // per-64-group affine codes s * q + beta (8 or 4 bit): dequant-fused / panel kernels
+  QF_E4M3 = 1,     // e4m3 codes with one power-of-two scale per row (precision mode 8): the FP8 pair kernel
+};
 struct QuantW {
-  const uint8_t* q = nullptr;    // [N, K] codes (8-bit) or [N, K/2] packed nibbles (4-bit)
-  const float* scales = nullptr; // [K/64, N]
-  const float* biases = nullptr; // [K/64, N]
+  const uint8_t* q = nullptr;    // [N, K] codes (8-bit, e4m3) or [N, K/2] packed nibbles (4-bit)
+  const float* scales = nullptr; // affine: [K/64, N]; e4m3: [N]
+  const float* biases = nullptr; // affine: [K/64, N]; e4m3: unused
   int bits = 0, n = 0, k = 0;
   // optional bf16 [n, k] scratch panel shared by all quantised weights of a context: for M > 256 the weight is converted
   // once per GEMM into it (it stays in the 126 MB L2 for the D x D projections) and the bf16 pair kernel runs on the panel
   bf16* scratch = nullptr;
+  int fmt = QF_AFFINE;
 };
 // C[M,N] = A[M,K] * (s*q + beta)[N,K]^T with the epilogues of launch_gemm (group size 64)
 void launch_gemm_q(const bf16* A, int64_t lda, const QuantW& W, int M, int N, int K, const GemmEpi& epi, cudaStream_t stream,
@@ -174,6 +187,8 @@ void launch_dequantize(const QuantW& W, bf16* w, cudaStream_t s);
 void launch_dequantize_panel(const QuantW& W, bf16* w, cudaStream_t s);
 // uint8 matrix [rows, row_bytes], box [box_rows, box_bytes], no swizzle
 CUtensorMap make_tmap_u8(const void* base, uint64_t rows, uint64_t row_bytes, uint32_t box_rows, uint32_t box_bytes);
+// uint8 matrix [rows, cols] with row pitch row_bytes; box [box_rows, 128 bytes], 128-byte swizzle (the e4m3 GEMM operands)
+CUtensorMap make_tmap_u8_sw128(const void* base, uint64_t rows, uint64_t cols, uint64_t row_bytes, uint32_t box_rows);
 // bf16 [R, C] (row pitch ld_in) -> [C, R] (row pitch ld_out)
 void launch_transpose_bf16(const bf16* in, int64_t ld_in, int R, int C, bf16* out, int64_t ld_out, cudaStream_t s);
 

@@ -158,6 +158,11 @@ __device__ __forceinline__ uint64_t umma_desc_sw128(uint32_t smem_addr) {
 __host__ __device__ constexpr uint32_t umma_idesc_bf16(uint32_t M, uint32_t N) {
   return (1u << 4) | (1u << 7) | (1u << 10) | ((N >> 3) << 17) | ((M >> 4) << 24);
 }
+// Instruction descriptor, kind::f8f6f4, e4m3 x e4m3 -> fp32, both operands K-major: the same fields, a_format = b_format = 0
+// (E4M3).  One MMA covers 32 k (32 bytes per row), as one kind::f16 MMA covers 16 bf16.
+__host__ __device__ constexpr uint32_t umma_idesc_e4m3(uint32_t M, uint32_t N) {
+  return (1u << 4) | ((N >> 3) << 17) | ((M >> 4) << 24);
+}
 
 __device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accum) {
   asm volatile(
@@ -237,6 +242,16 @@ __device__ __forceinline__ void umma_bf16_2cta(uint32_t tmem_d, uint64_t adesc, 
       ".reg .pred p;\n"
       "setp.ne.b32 p, %4, 0;\n"
       "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n"
+      "}\n" ::"r"(tmem_d),
+      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accum)
+      : "memory");
+}
+__device__ __forceinline__ void umma_f8_2cta(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accum) {
+  asm volatile(
+      "{\n"
+      ".reg .pred p;\n"
+      "setp.ne.b32 p, %4, 0;\n"
+      "tcgen05.mma.cta_group::2.kind::f8f6f4 [%0], %1, %2, %3, p;\n"
       "}\n" ::"r"(tmem_d),
       "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accum)
       : "memory");

@@ -99,6 +99,21 @@ CUtensorMap make_tmap_u8(const void* base, uint64_t rows, uint64_t row_bytes, ui
   return m;
 }
 
+CUtensorMap make_tmap_u8_sw128(const void* base, uint64_t rows, uint64_t cols, uint64_t row_bytes, uint32_t box_rows) {
+  LTX_CHECK((reinterpret_cast<uintptr_t>(base) & 15) == 0 && row_bytes % 16 == 0 && cols % 16 == 0, 2, "TMA u8: 16-byte alignment");
+  LTX_CHECK(box_rows <= 256, 2, "TMA u8 box: <= 256 rows");
+  CUtensorMap m;
+  cuuint64_t dims[2] = {cols, rows};
+  cuuint64_t strides[1] = {row_bytes};
+  cuuint32_t box[2] = {128, box_rows};
+  cuuint32_t estr[2] = {1, 1};
+  CUresult r = encode_fn()(&m, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, const_cast<void*>(base), dims, strides, box, estr,
+                           CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                           CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  LTX_CHECK(r == CUDA_SUCCESS, 3, "cuTensorMapEncodeTiled(u8, sw128) failed: " + std::to_string(static_cast<int>(r)));
+  return m;
+}
+
 // Per-device caches (one process may hold contexts on several GPUs, each driven by its own host thread): the SM count and the
 // set of kernels that already opted in to more than 48 KB of dynamic shared memory -- cudaFuncSetAttribute is per device.
 namespace {
