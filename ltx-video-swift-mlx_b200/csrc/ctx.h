@@ -3,7 +3,6 @@
 #include <atomic>
 #include <map>
 #include <string>
-#include <unordered_map>
 #include <vector>
 
 #include "../../include/ltxcuda.h"
@@ -51,8 +50,30 @@ struct DevBuf {
   T* as() const { return reinterpret_cast<T*>(ptr); }
 };
 
+// The weight of a transformer Linear [n, k] in one of three formats.  dit_quantize / dit_convert_fp8 replace the bf16 matrix
+// by its codes in place (w becomes nullptr); linear() in dit.cu picks the kernels from fmt.
+enum LinearFormat : int {
+  LW_BF16 = 0,     // w: bf16 [n, k] row-major
+  LW_AFFINE = 1,   // q: per-64-group affine codes s * q + beta (8 or 4 bit): dequant-fused / panel kernels
+  LW_E4M3 = 2,     // q: e4m3 codes with one power-of-two scale per row (precision mode 8): the FP8 pair kernel
+};
+struct LinearW {
+  int fmt = LW_BF16;
+  int n = 0, k = 0;
+  const bf16* w = nullptr;
+  QuantW q;
+};
+
+struct AdaLnW {   // AdaLayerNormSingle: Linear(256, dim) -> SiLU -> Linear(dim, dim) ; SiLU -> Linear(dim, n * dim)
+  const bf16 *w1 = nullptr, *w2 = nullptr, *wl = nullptr;
+  const float *b1 = nullptr, *b2 = nullptr, *bl = nullptr;
+  int dim = 0, n = 0;
+};
+
 struct AttnWeights {
-  const bf16 *wq = nullptr, *wk = nullptr, *wv = nullptr, *wo = nullptr;  // [D, D]; attn1: wq points at the packed [2D, D] q|k
+  // [inner, cdim] (wo: [qdim, inner]).  Video attn1: wq is the packed q|k|v [3D, D] and wv its v rows; wk is unused.  With
+  // affine codes wq holds only the q|k rows [2D, D] and wv the v rows as a matrix of their own.
+  LinearW wq, wk, wv, wo;
   const float *bq = nullptr, *bk = nullptr, *bv = nullptr, *bo = nullptr;
   const float *q_norm = nullptr, *k_norm = nullptr;
 };
@@ -60,7 +81,7 @@ struct AttnWeights {
 struct BlockWeights {
   const float* sst = nullptr;  // scale_shift_table [6, D]
   AttnWeights a1, a2;
-  const bf16 *w_in = nullptr, *w_out = nullptr;
+  LinearW w_in, w_out;
   const float *b_in = nullptr, *b_out = nullptr;
 };
 
@@ -77,7 +98,7 @@ struct TextCache {  // caption projection + per-block cross-attention K / V^T (s
 
 // what dit_prepare_text needs to build a stream's text cache: caption projection + per-block cross-attention K / V weights
 struct TextProjW {
-  const bf16 *w_c1 = nullptr, *w_c2 = nullptr;
+  LinearW w_c1, w_c2;
   const float *b_c1 = nullptr, *b_c2 = nullptr;
   int D = 0;
   const void* user = nullptr;
@@ -113,16 +134,11 @@ struct VaeWeights {
 
 // dual audio / video model (T/LTX2Transformer.swift, T/LTX2TransformerBlock.swift): the audio stream, the learned norms and the
 // cross-modal attentions on top of the video weights held in ltx_ctx::blocks
-struct AdaLnW {   // AdaLayerNormSingle: Linear(256, dim) -> SiLU -> Linear(dim, dim) ; SiLU -> Linear(dim, n * dim)
-  const bf16 *w1 = nullptr, *w2 = nullptr, *wl = nullptr;
-  const float *b1 = nullptr, *b2 = nullptr, *bl = nullptr;
-  int dim = 0, n = 0;
-};
 struct AvBlockW {
   const float *norm1 = nullptr, *norm2 = nullptr, *norm3 = nullptr, *a2v_norm = nullptr;        // video, [D]
   const float *anorm1 = nullptr, *anorm2 = nullptr, *anorm3 = nullptr, *v2a_norm = nullptr;     // audio, [Da]
   AttnWeights aa1, aa2, a2v, v2a;   // audio self / audio text-cross / audio->video / video->audio
-  const bf16 *w_in = nullptr, *w_out = nullptr;
+  LinearW w_in, w_out;
   const float *b_in = nullptr, *b_out = nullptr;
   const float *asst = nullptr;      // audio_scale_shift_table [6, Da]
   const float *sst_ca_v = nullptr;  // scale_shift_table_a2v_ca_video [5, D]
@@ -131,7 +147,7 @@ struct AvBlockW {
 struct AvWeights {
   bool ready = false;
   int Da = 0, Ha = 0, hd = 0, Cin = 0;
-  const bf16 *w_patch = nullptr, *w_c1 = nullptr, *w_c2 = nullptr, *w_out = nullptr;
+  LinearW w_patch, w_c1, w_c2, w_out;
   const float *b_patch = nullptr, *b_c1 = nullptr, *b_c2 = nullptr, *b_out = nullptr, *sst_out = nullptr;
   AdaLnW ada_a, cv_ss, cv_g, ca_ss, ca_g;
   std::vector<AvBlockW> blocks;
@@ -221,7 +237,6 @@ struct ltx_ctx {
   uint64_t launches = 0;
 
   std::map<std::string, ltx::DevTensor> tensors;  // raw tensors by post-mapping key
-  std::unordered_map<const void*, ltx::QuantW> qw;  // quantised replacements, keyed by the bf16 weight pointer they replace
   int quant_bits = 16;
   int quant_materialise = 0;                      // 1: dequantised bf16 values replace the weights at finalize (ltx_set_quant_storage)
   ltx::DevBuf q_panel;                            // bf16 conversion panel of the large-M quantised GEMM path
@@ -229,10 +244,9 @@ struct ltx_ctx {
   std::vector<void*> owned;                       // packed allocations made by finalize
   bool dit_ready = false;
   std::vector<ltx::BlockWeights> blocks;
-  const ltx::bf16 *w_patch = nullptr, *w_t1 = nullptr, *w_t2 = nullptr, *w_ada = nullptr, *w_c1 = nullptr, *w_c2 = nullptr,
-                  *w_out = nullptr;
-  const float *b_patch = nullptr, *b_t1 = nullptr, *b_t2 = nullptr, *b_ada = nullptr, *b_c1 = nullptr, *b_c2 = nullptr,
-              *b_out = nullptr, *sst_out = nullptr;
+  ltx::LinearW w_patch, w_c1, w_c2, w_out;
+  const float *b_patch = nullptr, *b_c1 = nullptr, *b_c2 = nullptr, *b_out = nullptr, *sst_out = nullptr;
+  ltx::AdaLnW adaln;   // timestep embedder + AdaLN-single (bf16 weights in every format)
   ltx::VaeWeights vae;
   ltx::AvWeights av;
   ltx::EncWeights enc;
@@ -308,7 +322,43 @@ struct ProfScope {
 };
 // api.cu: drop every captured graph (weights, communicators or precision changed)
 void graphs_clear(ltx_ctx* c);
-// dit.cu
+// dit.cu: the transformer Linears.  What a caller's rows imply for the bf16 kernels:
+struct LinearOpts {
+  int allow_skinny = 0;          // products of up to this many rows may take the weight-streaming kernel (launch_gemm)
+  bool split_k = false;          // M <= 512: opt in to the swap-AB kernel by giving it the context's split-K workspace
+  int tile_n = 0;                // bf16 / e4m3: forced tile width, 0: fitted (bf16: pair kernel for M > 128; e4m3: always pairs)
+  int a_kblock = 0;              // K-blocked A operand (Ulysses receive layout, see launch_gemm); not for e4m3 codes
+  int64_t a_kblock_stride = 0;
+};
+// epi(A[M, K] W[:N]^T): the only place that launches a transformer Linear.  Picks the kernels from W.fmt (e4m3: row quantiser +
+// FP8 pair kernel; affine: dequant-fused or panel kernel; bf16: launch_gemm with `o`) and profiles them.  N <= W.n: the first
+// N rows of the weight (the q|k rows of a packed q|k|v).
+void linear(ltx_ctx* c, const bf16* A, int64_t lda, const LinearW& W, int M, int N, int K, const GemmEpi& e, const LinearOpts& o);
+// V^T = (A W^T + bias)^T for `items` batch items of `rows` rows each (A [items * rows, W.k], pitch W.k): item i's [W.n, rows]
+// block starts at column i * item_ld of `out` (row pitch ld_out).  bf16: the weight-streaming kernel stores V^T directly when
+// o.allow_skinny admits the rows, otherwise the weight is the A operand so the product lands transposed; codes must be the B
+// operand: project into tmp [items * rows, W.n], then transpose each item.
+void linear_vt(ltx_ctx* c, const bf16* A, int rows, int items, const LinearW& W, const float* bias, bf16* out, int64_t ld_out,
+               int64_t item_ld, bf16* tmp, const LinearOpts& o);
+// Q [B*Nq, ldq], K [B*Nk, ldk], V^T [D, B*ldv] (item b at column b * ldv), key bias [B, Nk]; head_dim D / H
+void attention(ltx_ctx* c, const bf16* Q, int64_t ldq, const bf16* K, int64_t ldk, const bf16* Vt, int64_t ldv, const float* bias,
+               bf16* O, int64_t ldo, int B, int H, int Nq, int Nk, int D, const PeerTable* o_blocks = nullptr,
+               int rows_per_block = 0);
+// AdaLayerNormSingle (T/LTXTimestepEmbedding.swift:96-124) for one sigma per batch item (B rows): emb = L2(silu(L1(se))),
+// lin = L(silu(emb)), row pitches dim and n * dim.  se = sincos(sigma * mult) is shared by every embedder of the same stream;
+// given `sigma`, it is computed into se first.
+void adaln_single(ltx_ctx* c, const AdaLnW& a, float* se, float* t1, float* emb, float* lin, int B, const float* sigma = nullptr,
+                  float mult = 0.f);
+// The same for R sigmas (one per token): the three Linears as tensor-core GEMMs over the R rows, bf16 operands, the SiLUs in
+// the first epilogue / a cast pass.  se_bf [R, 256] bf16; t1_bf [R, dim] bf16 scratch; emb [R, dim] fp32; lin [R, n * dim]
+// fp32 with row pitch ld_lin.
+void adaln_single_rows(ltx_ctx* c, const AdaLnW& a, const bf16* se_bf, int R, bf16* t1_bf, float* emb, float* lin, int64_t ld_lin,
+                       const LinearOpts& o);
+// finalize helpers: shape-checked weights by key
+const bf16* wbf(ltx_ctx* c, const std::string& k, int64_t r, int64_t cc);
+const float* wf(ltx_ctx* c, const std::string& k, int64_t n);
+LinearW wlin(ltx_ctx* c, const std::string& k, int64_t n, int64_t kk);
+AdaLnW adaln_w(ltx_ctx* c, const std::string& p, int64_t dim, int n);
 void dit_finalize(ltx_ctx* c);
 void dit_quantize(ltx_ctx* c, int bits);
 void dit_convert_fp8(ltx_ctx* c);

@@ -16,87 +16,111 @@ namespace ltx {
 
 namespace {
 
-// the e4m3 replacement of a weight (precision mode 8), or nullptr
-const QuantW* fp8_weight(const ltx_ctx* c, const void* w) {
-  if (c->qw.empty()) return nullptr;
-  auto it = c->qw.find(w);
-  return (it != c->qw.end() && it->second.fmt == QF_E4M3) ? &it->second : nullptr;
+double gemm_bytes(int M, int N, int K) {
+  return 2.0 * (static_cast<double>(M) * K + static_cast<double>(N) * K + static_cast<double>(M) * N);
+}
+// the bf16 kernels (B: the weight, or the activation rows when a V^T projection makes the weight the A operand)
+void gemm_bf16(ltx_ctx* c, const bf16* A, int64_t lda, const bf16* B, int64_t ldb, int M, int N, int K, const GemmEpi& e,
+               const LinearOpts& o) {
+  ProfScope ps(c, PROF_GEMM, 2.0 * M * N * K, gemm_bytes(M, N, K));
+  GemmEpi ew = e;
+  if (o.split_k && M <= 512) gemm_attach_workspace(c, ew);
+  const int force_bn = o.tile_n == 0 ? 0 : M > 128 ? 1000 + o.tile_n : o.tile_n;
+  launch_gemm(A, lda, B, ldb, M, N, K, ew, c->stream, force_bn, o.a_kblock, o.a_kblock_stride, o.allow_skinny);
 }
 
-// Precision mode 8: A's rows become e4m3 codes + power-of-two row scales in one reused scratch buffer, then the FP8 pair kernel
-// runs for every M (no weight-streaming, 1-CTA or swap-AB form), so each row's result depends on that row alone: a batched
-// forward equals its items' forwards bit for bit.  Rows [0, N) of the weight are used (the q|k rows of the packed q|k|v).
-void gemm_fp8(ltx_ctx* c, const bf16* A, int64_t lda, const QuantW& W, int M, int N, int K, const GemmEpi& e, int force_bn) {
-  LTX_CHECK(W.k == K && W.n >= N, LTX_ERR_INVALID_ARGUMENT, "FP8 GEMM: weight shape mismatch");
-  const size_t code_bytes = (static_cast<size_t>(M) * K + 15) / 16 * 16;
-  c->fp8_act.reserve(code_bytes + static_cast<size_t>(M) * 4);
-  uint8_t* q = c->fp8_act.as<uint8_t>();
-  float* s = reinterpret_cast<float*>(q + code_bytes);
-  {
-    ProfScope ps(c, PROF_ROW, 0.0, 3.0 * M * K + 4.0 * M);
-    launch_quantize_rows_fp8(A, lda, M, K, q, s, c->stream);
-  }
-  ProfScope ps(c, PROF_GEMM, 2.0 * M * N * K, static_cast<double>(M) * K + static_cast<double>(N) * K + 2.0 * M * N);
-  launch_gemm_fp8(q, K, s, W.q, W.k, W.scales, M, N, K, e, c->stream, force_bn);
-}
+}  // namespace
 
 // profiled launch helpers (flop / byte counts are the algorithmic ones used by bench.py's roofline)
-void gemm(ltx_ctx* c, const bf16* A, int64_t lda, const bf16* B, int64_t ldb, int M, int N, int K, const GemmEpi& e,
-          int a_kblock = 0, int64_t a_kblock_stride = 0) {
-  if (const QuantW* w8 = fp8_weight(c, B)) {
-    LTX_CHECK(a_kblock == 0, LTX_ERR_UNSUPPORTED, "FP8 GEMM: no K-blocked A operand");
-    gemm_fp8(c, A, lda, *w8, M, N, K, e, 0);
+void linear(ltx_ctx* c, const bf16* A, int64_t lda, const LinearW& W, int M, int N, int K, const GemmEpi& e, const LinearOpts& o) {
+  LTX_CHECK(W.k == K && N >= 1 && N <= W.n, LTX_ERR_INVALID_ARGUMENT, "Linear: weight shape mismatch");
+  if (W.fmt == LW_BF16) {
+    gemm_bf16(c, A, lda, W.w, K, M, N, K, e, o);
+  } else if (W.fmt == LW_AFFINE) {   // dequant-fused kernel, or panel + bf16 kernel for large M
+    ProfScope ps(c, PROF_GEMM, 2.0 * M * N * K, gemm_bytes(M, N, K), gemm_q_uses_panel(W.q, M) ? 2 : 1);
+    launch_gemm_q(A, lda, W.q, M, N, K, e, c->stream, 0, o.a_kblock, o.a_kblock_stride);
+  } else {
+    // A's rows become e4m3 codes + power-of-two row scales in one reused scratch buffer, then the FP8 pair kernel runs for
+    // every M (no weight-streaming, 1-CTA or swap-AB form), so each row's result depends on that row alone: a batched forward
+    // equals its items' forwards bit for bit
+    LTX_CHECK(o.a_kblock == 0, LTX_ERR_UNSUPPORTED, "FP8 GEMM: no K-blocked A operand");
+    const size_t code_bytes = (static_cast<size_t>(M) * K + 15) / 16 * 16;
+    c->fp8_act.reserve(code_bytes + static_cast<size_t>(M) * 4);
+    uint8_t* q = c->fp8_act.as<uint8_t>();
+    float* s = reinterpret_cast<float*>(q + code_bytes);
+    {
+      ProfScope ps(c, PROF_ROW, 0.0, 3.0 * M * K + 4.0 * M);
+      launch_quantize_rows_fp8(A, lda, M, K, q, s, c->stream);
+    }
+    ProfScope ps(c, PROF_GEMM, 2.0 * M * N * K, static_cast<double>(M) * K + static_cast<double>(N) * K + 2.0 * M * N);
+    launch_gemm_fp8(q, K, s, W.q.q, W.q.k, W.q.scales, M, N, K, e, c->stream, o.tile_n);
+  }
+}
+
+void linear_vt(ltx_ctx* c, const bf16* A, int rows, int items, const LinearW& W, const float* bias, bf16* out, int64_t ld_out,
+               int64_t item_ld, bf16* tmp, const LinearOpts& o) {
+  const int N = W.n, K = W.k;
+  GemmEpi e;
+  e.mode = EPI_BF16; e.bias = bias;
+  if (W.fmt != LW_BF16) {
+    e.out = tmp; e.ldo = N;
+    linear(c, A, K, W, items * rows, N, K, e, o);
+    ProfScope ps(c, PROF_OTHER, 0.0, 4.0 * items * rows * N, items);
+    for (int i = 0; i < items; ++i)
+      launch_transpose_bf16(tmp + static_cast<int64_t>(i) * rows * N, N, rows, N, out + i * item_ld, ld_out, c->stream);
     return;
   }
-  auto it = c->qw.empty() ? c->qw.end() : c->qw.find(B);
-  const bool panel = it != c->qw.end() && gemm_q_uses_panel(it->second, M);
-  ProfScope ps(c, PROF_GEMM, 2.0 * M * N * K, 2.0 * (static_cast<double>(M) * K + static_cast<double>(N) * K + static_cast<double>(M) * N),
-               panel ? 2 : 1);
-  if (it != c->qw.end()) {   // weight was replaced by int8 / int4 codes: dequant-fused kernel, or panel + bf16 kernel for large M
-    launch_gemm_q(A, lda, it->second, M, N, K, e, c->stream, 0, a_kblock, a_kblock_stride);
+  e.out = out; e.ldo = ld_out;
+  if (items > 1) { e.t_item_rows = rows; e.t_item_ld = item_ld; }
+  if (gemm_skinny_eligible(K, K, items * rows, N, K, e, 0, o.allow_skinny)) {
+    e.transpose_out = 1;
+    linear(c, A, K, W, items * rows, N, K, e, o);
     return;
   }
-  if (M <= 512) {   // few rows (an Ulysses shard, a small clip): opt in to the weight-streaming kernel
-    GemmEpi ew = e;
-    gemm_attach_workspace(c, ew);
-    launch_gemm(A, lda, B, ldb, M, N, K, ew, c->stream, 0, a_kblock, a_kblock_stride);
+  e.t_item_rows = 0;
+  e.bias_per_row = 1;
+  if (items == 1 || rows == item_ld) {   // the items' column blocks are contiguous
+    gemm_bf16(c, W.w, K, A, K, N, items * rows, K, e, o);
     return;
   }
-  launch_gemm(A, lda, B, ldb, M, N, K, e, c->stream, 0, a_kblock, a_kblock_stride);
-}
-// V^T [D, ncols] (row pitch ld_out) = (h Wv^T + bv)^T for one batch.  bf16 weights: run the projection with the weight as
-// the A operand so the result lands transposed; quantised weights must be the B operand: project into `tmp`, transpose.
-void v_transposed(ltx_ctx* c, const bf16* wv, const float* bv, const bf16* hrows, int rows, int D, bf16* out, int64_t ld_out,
-                  bf16* tmp) {
-  if (c->qw.empty() || c->qw.find(wv) == c->qw.end()) {
-    GemmEpi ev;
-    ev.mode = EPI_BF16; ev.out = out; ev.ldo = ld_out; ev.bias = bv; ev.bias_per_row = 1;
-    gemm(c, wv, D, hrows, D, D, rows, D, ev);
-    return;
+  for (int i = 0; i < items; ++i) {
+    e.out = out + i * item_ld;
+    gemm_bf16(c, W.w, K, A + static_cast<int64_t>(i) * rows * K, K, N, rows, K, e, o);
   }
-  GemmEpi ev;
-  ev.mode = EPI_BF16; ev.out = tmp; ev.ldo = D; ev.bias = bv;
-  gemm(c, hrows, D, wv, D, rows, D, D, ev);
-  ProfScope ps(c, PROF_OTHER, 0.0, 4.0 * rows * D);
-  launch_transpose_bf16(tmp, D, rows, D, out, ld_out, c->stream);
 }
-void attention(ltx_ctx* c, const bf16* Q, int64_t ldq, const bf16* K, int64_t ldk, const bf16* Vt, int64_t ldvb,
-               const float* bias, bf16* O, int64_t ldo, int B, int H, int Nq, int Nk, int D, float scale,
-               const PeerTable* o_blocks = nullptr, int rows_per_block = 0) {
-  ProfScope ps(c, PROF_ATTN, 4.0 * B * H * static_cast<double>(Nq) * Nk * 128.0,
-               2.0 * B * (2.0 * Nq + 2.0 * Nk) * D);
-  launch_attention(Q, ldq, K, ldk, Vt, ldvb, bias, O, ldo, B, H, Nq, Nk, D, scale, c->stream, o_blocks, rows_per_block);
+
+void attention(ltx_ctx* c, const bf16* Q, int64_t ldq, const bf16* K, int64_t ldk, const bf16* Vt, int64_t ldv, const float* bias,
+               bf16* O, int64_t ldo, int B, int H, int Nq, int Nk, int D, const PeerTable* o_blocks, int rows_per_block) {
+  const int hd = D / H;
+  ProfScope ps(c, PROF_ATTN, 4.0 * B * H * static_cast<double>(Nq) * Nk * hd, 2.0 * B * (2.0 * Nq + 2.0 * Nk) * D);
+  launch_attention(Q, ldq, K, ldk, Vt, ldv, bias, O, ldo, B, H, Nq, Nk, D, 1.0f / sqrtf(static_cast<float>(hd)), c->stream, o_blocks,
+                   rows_per_block);
 }
-void norm_mod(ltx_ctx* c, const float* x, bf16* out, int M, int D, const float* ts, const float* tsc, const float* as,
-              const float* asc, int64_t ada_ld, int rows_per_mod, float eps, int ln) {
-  ProfScope ps(c, PROF_ROW, 0.0, static_cast<double>(M) * D * 6.0);
-  launch_rmsnorm_mod(x, out, M, D, ts, tsc, as, asc, ada_ld, rows_per_mod, eps, ln, c->stream);
+
+void adaln_single(ltx_ctx* c, const AdaLnW& a, float* se, float* t1, float* emb, float* lin, int B, const float* sigma, float mult) {
+  ProfScope ps(c, PROF_OTHER, 2.0 * B * a.dim * (256.0 + (1.0 + a.n) * a.dim), 2.0 * a.dim * (256.0 + (1.0 + a.n) * a.dim),
+               sigma ? 4 : 3);
+  if (sigma) launch_sincos_embed(sigma, mult, se, B, 256, c->stream);
+  launch_gemv(a.w1, a.b1, se, t1, B, a.dim, 256, 0, c->stream);
+  launch_gemv(a.w2, a.b2, t1, emb, B, a.dim, a.dim, 1, c->stream);
+  launch_gemv(a.wl, a.bl, emb, lin, B, a.n * a.dim, a.dim, 1, c->stream);
 }
-void qknorm(ltx_ctx* c, bf16* x, int64_t ld, int M, int D, const float* w, const float* cs, const float* sn, int rpr,
-            float eps, const float* w_second = nullptr, const QkOut* blocked = nullptr) {
-  const int segs = w_second ? 2 : 1;
-  ProfScope ps(c, PROF_ROW, 0.0, segs * static_cast<double>(M) * D * (4.0 + (cs ? 4.0 : 0.0)), (D == 4096) ? 1 : segs);
-  launch_qknorm_rope(x, ld, M, D, w, cs, sn, rpr, eps, c->stream, w_second, blocked);
+
+void adaln_single_rows(ltx_ctx* c, const AdaLnW& a, const bf16* se_bf, int R, bf16* t1_bf, float* emb, float* lin, int64_t ld_lin,
+                       const LinearOpts& o) {
+  GemmEpi e1;
+  e1.mode = EPI_SILU_BF16; e1.out = t1_bf; e1.ldo = a.dim; e1.bias = a.b1;
+  gemm_bf16(c, se_bf, 256, a.w1, 256, R, a.dim, 256, e1, o);
+  GemmEpi e2;
+  e2.mode = EPI_F32; e2.out = emb; e2.ldo = a.dim; e2.bias = a.b2;
+  gemm_bf16(c, t1_bf, a.dim, a.w2, a.dim, R, a.dim, a.dim, e2, o);
+  {
+    ProfScope ps(c, PROF_OTHER, 0.0, 6.0 * R * a.dim);
+    launch_silu_cast(emb, t1_bf, static_cast<int64_t>(R) * a.dim, c->stream);
+  }
+  GemmEpi e3;
+  e3.mode = EPI_F32; e3.out = lin; e3.ldo = ld_lin; e3.bias = a.bl;
+  gemm_bf16(c, t1_bf, a.dim, a.wl, a.dim, R, a.n * a.dim, a.dim, e3, o);
 }
 
 const bf16* wbf(ltx_ctx* c, const std::string& k, int64_t r, int64_t cc) {
@@ -109,6 +133,33 @@ const float* wf(ltx_ctx* c, const std::string& k, int64_t n) {
   const DevTensor& t = get_tensor(c, k);
   LTX_CHECK(t.dtype == LTX_F32 && t.numel() == n, LTX_ERR_WEIGHTS, "bad shape for '" + k + "'");
   return reinterpret_cast<const float*>(t.ptr);
+}
+LinearW wlin(ltx_ctx* c, const std::string& k, int64_t n, int64_t kk) {
+  LinearW w;
+  w.n = static_cast<int>(n); w.k = static_cast<int>(kk); w.w = wbf(c, k, n, kk);
+  return w;
+}
+AdaLnW adaln_w(ltx_ctx* c, const std::string& p, int64_t dim, int n) {
+  AdaLnW a;
+  a.w1 = wbf(c, p + ".emb.linear_1.weight", dim, 256); a.b1 = wf(c, p + ".emb.linear_1.bias", dim);
+  a.w2 = wbf(c, p + ".emb.linear_2.weight", dim, dim); a.b2 = wf(c, p + ".emb.linear_2.bias", dim);
+  a.wl = wbf(c, p + ".linear.weight", n * dim, dim); a.bl = wf(c, p + ".linear.bias", n * dim);
+  a.dim = static_cast<int>(dim); a.n = n;
+  return a;
+}
+
+namespace {
+
+void norm_mod(ltx_ctx* c, const float* x, bf16* out, int M, int D, const float* ts, const float* tsc, const float* as,
+              const float* asc, int64_t ada_ld, int rows_per_mod, float eps, int ln) {
+  ProfScope ps(c, PROF_ROW, 0.0, static_cast<double>(M) * D * 6.0);
+  launch_rmsnorm_mod(x, out, M, D, ts, tsc, as, asc, ada_ld, rows_per_mod, eps, ln, c->stream);
+}
+void qknorm(ltx_ctx* c, bf16* x, int64_t ld, int M, int D, const float* w, const float* cs, const float* sn, int rpr,
+            float eps, const float* w_second = nullptr, const QkOut* blocked = nullptr) {
+  const int segs = w_second ? 2 : 1;
+  ProfScope ps(c, PROF_ROW, 0.0, segs * static_cast<double>(M) * D * (4.0 + (cs ? 4.0 : 0.0)), (D == 4096) ? 1 : segs);
+  launch_qknorm_rope(x, ld, M, D, w, cs, sn, rpr, eps, c->stream, w_second, blocked);
 }
 
 // Host fp64 RoPE table, token-major [N, D/2] (T/LTXRoPE.swift:375-488, 552-610; see oracle.rope_table).
@@ -210,22 +261,24 @@ TextCache& dit_prepare_text(ltx_ctx* c, TextCache* slots, int* rr, const TextPro
   }
   c->c1.reserve(static_cast<size_t>(R) * D * 2);
   c->c2.reserve(static_cast<size_t>(R) * D * 2);
+  LinearOpts o;   // both models build their text caches with the video model's rule: split-K for few rows
+  o.split_k = true;
   GemmEpi e;
   e.mode = EPI_GELU_BF16; e.out = c->c1.ptr; e.ldo = D; e.bias = src.b_c1;
-  gemm(c, ctx_bf, Cc, src.w_c1, Cc, static_cast<int>(R), D, Cc, e);
+  linear(c, ctx_bf, Cc, src.w_c1, static_cast<int>(R), D, Cc, e, o);
   e.mode = EPI_BF16; e.out = c->c2.ptr; e.bias = src.b_c2;
-  gemm(c, c->c1.as<bf16>(), D, src.w_c2, D, static_cast<int>(R), D, D, e);
+  linear(c, c->c1.as<bf16>(), D, src.w_c2, static_cast<int>(R), D, D, e, o);
   for (int i = 0; i < L; ++i) {
     const AttnWeights& a = src.layer(src.user, i);
     bf16* kd = tc.k.as<bf16>() + static_cast<int64_t>(i) * R * D;
     bf16* vd = tc.vt.as<bf16>() + static_cast<int64_t>(i) * D * B * tc.ldv;
     GemmEpi ek;
     ek.mode = EPI_BF16; ek.out = kd; ek.ldo = D; ek.bias = a.bk;
-    gemm(c, c->c2.as<bf16>(), D, a.wk, D, static_cast<int>(R), D, D, ek);
+    linear(c, c->c2.as<bf16>(), D, a.wk, static_cast<int>(R), D, D, ek, o);
     qknorm(c, kd, D, static_cast<int>(R), D, a.k_norm, nullptr, nullptr, 1, g.norm_eps);
     for (int b = 0; b < B; ++b)  // V^T[D, S] per batch, one column block each
-      v_transposed(c, a.wv, a.bv, c->c2.as<bf16>() + static_cast<int64_t>(b) * S * D, S, D, vd + b * tc.ldv, B * tc.ldv,
-                   c->c1.as<bf16>());
+      linear_vt(c, c->c2.as<bf16>() + static_cast<int64_t>(b) * S * D, S, 1, a.wv, a.bv, vd + b * tc.ldv, B * tc.ldv, tc.ldv,
+                c->c1.as<bf16>(), o);
   }
   // An all-ones mask (what the real text connector emits, LTXTextEncoder.swift:514-520) adds a zero bias: skip it.
   bool any_masked = false;
@@ -284,20 +337,15 @@ void dit_finalize(ltx_ctx* c) {
   const int64_t D = static_cast<int64_t>(g.num_heads) * g.head_dim, FF = g.ffn_mult * D;
   LTX_CHECK(g.in_channels % 8 == 0 && g.caption_channels % 8 == 0 && g.out_channels % 8 == 0, LTX_ERR_INVALID_CONFIGURATION,
             "channel counts must be multiples of 8");
-  c->w_patch = wbf(c, "patchify_proj.weight", D, g.in_channels);
+  c->w_patch = wlin(c, "patchify_proj.weight", D, g.in_channels);
   c->b_patch = wf(c, "patchify_proj.bias", D);
-  c->w_t1 = wbf(c, "adaln_single.emb.linear_1.weight", D, 256);
-  c->b_t1 = wf(c, "adaln_single.emb.linear_1.bias", D);
-  c->w_t2 = wbf(c, "adaln_single.emb.linear_2.weight", D, D);
-  c->b_t2 = wf(c, "adaln_single.emb.linear_2.bias", D);
-  c->w_ada = wbf(c, "adaln_single.linear.weight", 6 * D, D);
-  c->b_ada = wf(c, "adaln_single.linear.bias", 6 * D);
-  c->w_c1 = wbf(c, "caption_projection.linear_1.weight", D, g.caption_channels);
+  c->adaln = adaln_w(c, "adaln_single", D, 6);
+  c->w_c1 = wlin(c, "caption_projection.linear_1.weight", D, g.caption_channels);
   c->b_c1 = wf(c, "caption_projection.linear_1.bias", D);
-  c->w_c2 = wbf(c, "caption_projection.linear_2.weight", D, D);
+  c->w_c2 = wlin(c, "caption_projection.linear_2.weight", D, D);
   c->b_c2 = wf(c, "caption_projection.linear_2.bias", D);
   c->sst_out = wf(c, "scale_shift_table", 2 * D);
-  c->w_out = wbf(c, "proj_out.weight", g.out_channels, D);
+  c->w_out = wlin(c, "proj_out.weight", g.out_channels, D);
   c->b_out = wf(c, "proj_out.bias", g.out_channels);
   c->blocks.assign(g.num_layers, BlockWeights());
   for (int i = 0; i < g.num_layers; ++i) {
@@ -305,7 +353,7 @@ void dit_finalize(ltx_ctx* c) {
     BlockWeights& b = c->blocks[i];
     b.sst = wf(c, p + "scale_shift_table", 6 * D);
     // attn1: pack q|k|v into one [3D, D] operand: the three projections of the block run as ONE GEMM (N = 3D; V leaves its
-    // epilogue transposed); the Ulysses / quantised paths address the q|k rows and the v rows of the same buffer separately
+    // epilogue transposed); the other paths address the q|k rows (wq, N = 2D) and the v rows (wv) of the same buffer
     {
       const bf16* wq = wbf(c, p + "attn1.to_q.weight", D, D);
       const bf16* wk = wbf(c, p + "attn1.to_k.weight", D, D);
@@ -332,26 +380,27 @@ void dit_finalize(ltx_ctx* c) {
         cudaFree(it->second.ptr);
         c->tensors.erase(it);
       }
-      b.a1.wq = wqkv; b.a1.wk = wqkv + D * D; b.a1.wv = wqkv + 2 * D * D;
+      b.a1.wq.n = 3 * D; b.a1.wq.k = D; b.a1.wq.w = wqkv;
+      b.a1.wv.n = D; b.a1.wv.k = D; b.a1.wv.w = wqkv + 2 * D * D;
       b.a1.bq = bqkv; b.a1.bk = bqkv + D; b.a1.bv = bqkv + 2 * D;
     }
-    b.a1.wo = wbf(c, p + "attn1.to_out.weight", D, D);
+    b.a1.wo = wlin(c, p + "attn1.to_out.weight", D, D);
     b.a1.bo = wf(c, p + "attn1.to_out.bias", D);
     b.a1.q_norm = wf(c, p + "attn1.q_norm.weight", D);
     b.a1.k_norm = wf(c, p + "attn1.k_norm.weight", D);
-    b.a2.wq = wbf(c, p + "attn2.to_q.weight", D, D);
+    b.a2.wq = wlin(c, p + "attn2.to_q.weight", D, D);
     b.a2.bq = wf(c, p + "attn2.to_q.bias", D);
-    b.a2.wk = wbf(c, p + "attn2.to_k.weight", D, D);
+    b.a2.wk = wlin(c, p + "attn2.to_k.weight", D, D);
     b.a2.bk = wf(c, p + "attn2.to_k.bias", D);
-    b.a2.wv = wbf(c, p + "attn2.to_v.weight", D, D);
+    b.a2.wv = wlin(c, p + "attn2.to_v.weight", D, D);
     b.a2.bv = wf(c, p + "attn2.to_v.bias", D);
-    b.a2.wo = wbf(c, p + "attn2.to_out.weight", D, D);
+    b.a2.wo = wlin(c, p + "attn2.to_out.weight", D, D);
     b.a2.bo = wf(c, p + "attn2.to_out.bias", D);
     b.a2.q_norm = wf(c, p + "attn2.q_norm.weight", D);
     b.a2.k_norm = wf(c, p + "attn2.k_norm.weight", D);
-    b.w_in = wbf(c, p + "ff.project_in.proj.weight", FF, D);
+    b.w_in = wlin(c, p + "ff.project_in.proj.weight", FF, D);
     b.b_in = wf(c, p + "ff.project_in.proj.bias", FF);
-    b.w_out = wbf(c, p + "ff.project_out.weight", D, FF);
+    b.w_out = wlin(c, p + "ff.project_out.weight", D, FF);
     b.b_out = wf(c, p + "ff.project_out.bias", D);
   }
   c->scratch.reserve(64 * sizeof(double));
@@ -374,123 +423,99 @@ void dit_quantize(ltx_ctx* c, int bits) {
   LTX_CHECK(c->dit_ready, LTX_ERR_WEIGHTS, "DiT weights not finalized");
   LTX_CHECK(bits == 8 || bits == 4, LTX_ERR_UNSUPPORTED, "quant_bits must be 16, 8 or 4");
   const ltx_config& g = c->cfg;
-  const int D = g.num_heads * g.head_dim, FF = g.ffn_mult * D;
-  auto release = [&](const void* p) { release_weight(c, p); };
-  // Each quantised weight gets a 16-byte device allocation whose address is its identity from now on: the struct field
-  // is repointed to it and gemm() recognises it in c->qw (the freed bf16 address could be handed out again by cudaMalloc).
-  std::vector<const void*> to_free;
-  auto qf = [&](const bf16*& w, int N, int K) {
+  const int D = g.num_heads * g.head_dim;
+  std::vector<const void*> to_free;   // freed at the end: attn1's v rows live in the allocation of its packed q|k|v
+  std::vector<LinearW*> coded;
+  // rows: quantise only the leading rows of the matrix (0: all of them)
+  auto qf = [&](LinearW& w, int rows = 0) {
+    const int N = rows ? rows : w.n, K = w.k;
+    LTX_CHECK(w.fmt == LW_BF16, LTX_ERR_WEIGHTS, "quantisation needs bf16 weights");
     LTX_CHECK(K % 64 == 0, LTX_ERR_INVALID_CONFIGURATION, "quantisation needs every Linear input width to be a multiple of 64");
     uint8_t* q = nullptr;
     float *s = nullptr, *b = nullptr;
-    void* handle = nullptr;
     const size_t qbytes = static_cast<size_t>(N) * K * bits / 8, sbytes = static_cast<size_t>(K / 64) * N * 4;
     LTX_CUDA(cudaMalloc(&q, qbytes));
     LTX_CUDA(cudaMalloc(&s, sbytes));
     LTX_CUDA(cudaMalloc(&b, sbytes));
-    LTX_CUDA(cudaMalloc(&handle, 16));
-    c->owned.push_back(q); c->owned.push_back(s); c->owned.push_back(b); c->owned.push_back(handle);
-    launch_quantize(w, N, K, bits, q, s, b, c->stream);
+    c->owned.push_back(q); c->owned.push_back(s); c->owned.push_back(b);
+    launch_quantize(w.w, N, K, bits, q, s, b, c->stream);
     QuantW r;
     r.q = q; r.scales = s; r.biases = b; r.bits = bits; r.n = N; r.k = K;
     if (c->quant_materialise) {
       // materialised storage: the weight keeps its place and dtype, its values become s * q + beta (the panel conversion's
       // arithmetic and rounding, i.e. exactly what the fused kernels would feed the tensor cores); the codes are dropped
-      launch_dequantize_panel(r, const_cast<bf16*>(w), c->stream);
+      launch_dequantize_panel(r, const_cast<bf16*>(w.w), c->stream);
       LTX_CUDA(cudaStreamSynchronize(c->stream));
-      for (void* ptr : {static_cast<void*>(q), static_cast<void*>(s), static_cast<void*>(b), handle}) {
+      for (void* ptr : {static_cast<void*>(q), static_cast<void*>(s), static_cast<void*>(b)}) {
         cudaFree(ptr);
         c->owned.erase(std::find(c->owned.begin(), c->owned.end(), ptr));
       }
       return;
     }
     LTX_CUDA(cudaStreamSynchronize(c->stream));
-    c->qw[handle] = r;
-    to_free.push_back(w);
-    w = reinterpret_cast<const bf16*>(handle);
+    to_free.push_back(w.w);
+    w.fmt = LW_AFFINE; w.n = N; w.w = nullptr; w.q = r;
+    coded.push_back(&w);
   };
-  const bool codes = !c->quant_materialise;
-  qf(c->w_patch, D, g.in_channels);
-  qf(c->w_c1, D, g.caption_channels);
-  qf(c->w_c2, D, D);
-  qf(c->w_out, g.out_channels, D);
+  qf(c->w_patch); qf(c->w_c1); qf(c->w_c2); qf(c->w_out);
   for (auto& b : c->blocks) {
-    qf(b.a1.wq, 2 * D, D);            // packed q|k (the v rows behind them are quantised by the next call: rows are independent)
-    if (codes) b.a1.wk = nullptr;
-    qf(b.a1.wv, D, D); qf(b.a1.wo, D, D);
-    qf(b.a2.wq, D, D); qf(b.a2.wk, D, D); qf(b.a2.wv, D, D); qf(b.a2.wo, D, D);
-    qf(b.w_in, FF, D); qf(b.w_out, D, FF);
+    qf(b.a1.wq, 2 * D);   // the q|k rows of the packed q|k|v (its v rows are quantised by the next call: rows are independent)
+    qf(b.a1.wv); qf(b.a1.wo);
+    qf(b.a2.wq); qf(b.a2.wk); qf(b.a2.wv); qf(b.a2.wo);
+    qf(b.w_in); qf(b.w_out);
   }
   if (c->av.ready) {
     // the dual model's Linears (quantize(model: ltx2, groupSize: 64, bits:), Pipeline/LTXPipeline.swift:491); the AdaLN-single
     // embedders stay bf16 like the video model's timestep MLP
     AvWeights& a = c->av;
-    const int Da = a.Da, FFa = g.ffn_mult * Da, Ca = a.Cin;
-    qf(a.w_patch, Da, Ca);
-    qf(a.w_c1, Da, g.caption_channels);
-    qf(a.w_c2, Da, Da);
-    qf(a.w_out, Ca, Da);
-    auto qattn = [&](AttnWeights& w, int qdim, int cdim, int inner) {
-      qf(w.wq, inner, qdim); qf(w.wk, inner, cdim); qf(w.wv, inner, cdim); qf(w.wo, qdim, inner);
-    };
+    qf(a.w_patch); qf(a.w_c1); qf(a.w_c2); qf(a.w_out);
     for (auto& b : a.blocks) {
-      qattn(b.aa1, Da, Da, Da);
-      qattn(b.aa2, Da, Da, Da);
-      qattn(b.a2v, D, Da, Da);
-      qattn(b.v2a, Da, D, Da);
-      qf(b.w_in, FFa, Da); qf(b.w_out, Da, FFa);
+      for (AttnWeights* w : {&b.aa1, &b.aa2, &b.a2v, &b.v2a}) { qf(w->wq); qf(w->wk); qf(w->wv); qf(w->wo); }
+      qf(b.w_in); qf(b.w_out);
     }
   }
-  if (!codes) { c->quant_bits = bits; return; }   // materialised: the structs still point at (now dequantised) bf16 weights
-  for (const void* p : to_free) release(p);
+  c->quant_bits = bits;
+  if (c->quant_materialise) return;   // the weights stay bf16 (now dequantised)
+  for (const void* p : to_free) release_weight(c, p);
   // one bf16 panel for the large-M path of launch_gemm_q, sized for the largest weight (the FFN matrices)
   size_t max_elems = 0;
-  for (auto& kv : c->qw) max_elems = std::max(max_elems, static_cast<size_t>(kv.second.n) * kv.second.k);
+  for (const LinearW* w : coded) max_elems = std::max(max_elems, static_cast<size_t>(w->n) * w->k);
   c->q_panel.reserve(max_elems * 2);
-  for (auto& kv : c->qw) kv.second.scratch = c->q_panel.as<bf16>();
-  c->quant_bits = bits;
+  for (LinearW* w : coded) w->q.scratch = c->q_panel.as<bf16>();
 }
 
 // Precision mode 8: every Linear inside the transformer blocks becomes e4m3 codes with one power-of-two scale per output
-// channel (launch_quantize_rows_fp8: the rule gemm() applies to the activation rows); the bf16 copies are freed.  Patchify,
-// caption projection, the timestep MLPs / AdaLN and proj_out stay bf16.  The weights are found through dit_quantize's
-// handles, with the e4m3 format in their map entry.
+// channel (launch_quantize_rows_fp8: the rule linear() applies to the activation rows); the bf16 copies are freed.  Patchify,
+// caption projection, the timestep MLPs / AdaLN and proj_out stay bf16.
 void dit_convert_fp8(ltx_ctx* c) {
-  LTX_CHECK(c->dit_ready && c->qw.empty(), LTX_ERR_WEIGHTS, "FP8 conversion needs finalized, unquantised DiT weights");
+  LTX_CHECK(c->dit_ready, LTX_ERR_WEIGHTS, "DiT weights not finalized");
   const ltx_config& g = c->cfg;
   const int D = g.num_heads * g.head_dim, FF = g.ffn_mult * D;
   LTX_CHECK(D % 16 == 0 && FF % 16 == 0, LTX_ERR_INVALID_CONFIGURATION, "FP8 mode needs Linear widths that are multiples of 16");
   std::vector<const void*> to_free;
-  auto handle_for = [&](const QuantW& r) {
-    void* handle = nullptr;
-    LTX_CUDA(cudaMalloc(&handle, 16));
-    c->owned.push_back(handle);
-    c->qw[handle] = r;
-    return reinterpret_cast<const bf16*>(handle);
-  };
-  auto conv = [&](const bf16*& w, int N, int K) {
+  auto conv = [&](LinearW& w) {
+    LTX_CHECK(w.fmt == LW_BF16, LTX_ERR_WEIGHTS, "FP8 conversion needs unquantised DiT weights");
+    const int N = w.n, K = w.k;
     uint8_t* q = nullptr;
     float* s = nullptr;
     LTX_CUDA(cudaMalloc(&q, static_cast<size_t>(N) * K));
     LTX_CUDA(cudaMalloc(&s, static_cast<size_t>(N) * 4));
     c->owned.push_back(q); c->owned.push_back(s);
-    launch_quantize_rows_fp8(w, K, N, K, q, s, c->stream);
-    QuantW r;
-    r.fmt = QF_E4M3; r.q = q; r.scales = s; r.bits = 8; r.n = N; r.k = K;
-    to_free.push_back(w);
-    w = handle_for(r);
-    return r;
+    launch_quantize_rows_fp8(w.w, K, N, K, q, s, c->stream);
+    to_free.push_back(w.w);
+    w.fmt = LW_E4M3; w.w = nullptr;
+    w.q.q = q; w.q.scales = s; w.q.bits = 8; w.q.n = N; w.q.k = K;
   };
   for (auto& b : c->blocks) {
-    // the packed q|k|v [3D, D] as one matrix, so the fused projection with its V^T epilogue stays one launch; its v rows get
-    // a handle of their own (rows are independent) for the per-batch V^T projections
-    QuantW v = conv(b.a1.wq, 3 * D, D);
-    v.q += static_cast<size_t>(2) * D * D; v.scales += 2 * D; v.n = D;
-    b.a1.wk = nullptr;
-    b.a1.wv = handle_for(v);
-    conv(b.a1.wo, D, D);
-    conv(b.a2.wq, D, D); conv(b.a2.wk, D, D); conv(b.a2.wv, D, D); conv(b.a2.wo, D, D);
-    conv(b.w_in, FF, D); conv(b.w_out, D, FF);
+    // the packed q|k|v [3D, D] as one matrix, so the fused projection with its V^T epilogue stays one launch; its v rows are a
+    // view of it (rows are independent) for the per-batch V^T projections
+    conv(b.a1.wq);
+    b.a1.wv = b.a1.wq;
+    b.a1.wv.n = b.a1.wv.q.n = D;
+    b.a1.wv.q.q += static_cast<size_t>(2) * D * D; b.a1.wv.q.scales += 2 * D;
+    conv(b.a1.wo);
+    conv(b.a2.wq); conv(b.a2.wk); conv(b.a2.wv); conv(b.a2.wo);
+    conv(b.w_in); conv(b.w_out);
   }
   LTX_CUDA(cudaStreamSynchronize(c->stream));
   for (const void* p : to_free) release_weight(c, p);
@@ -521,8 +546,9 @@ void dit_forward_dev(ltx_ctx* c, const void* latent, int latent_dtype, const voi
   const int Nq = (P > 1) ? Nl : N;         // local query rows per batch
   const int Csp = D / P, Hl = Hh / P;      // per-rank feature slice / heads inside self-attention
   const float eps = g.norm_eps;
-  const float att_scale = 1.0f / sqrtf(static_cast<float>(g.head_dim));
   cudaStream_t st = c->stream;
+  LinearOpts o;   // few rows (an Ulysses shard, a small clip): opt in to the weight-streaming kernel
+  o.split_k = true;
   ltx_dit_flags noflags = {};
   noflags.cross_attn_scale = 1.0f;
   if (!flags) flags = &noflags;
@@ -609,7 +635,7 @@ void dit_forward_dev(ltx_ctx* c, const void* latent, int latent_dtype, const voi
   if (resume_block < 0) {
     GemmEpi e;
     e.mode = EPI_BF16; e.out = xb; e.ldo = D; e.bias = c->b_patch;
-    gemm(c, lat_bf, Cin, c->w_patch, Cin, R, D, Cin, e);
+    linear(c, lat_bf, Cin, c->w_patch, R, D, Cin, e, o);
     ProfScope ps(c, PROF_OTHER, 0.0, 6.0 * R * D);
     launch_cast_bf16_f32(xb, x, static_cast<int64_t>(R) * D, st);
   } else {
@@ -622,33 +648,15 @@ void dit_forward_dev(ltx_ctx* c, const void* latent, int latent_dtype, const voi
   }
   // ---- timestep path (T/LTXTimestepEmbedding.swift:62-124): fp32 activations, bf16 weights
   if (!ts_per_token) {
-    ProfScope ps(c, PROF_OTHER, 2.0 * B * D * (256.0 + 7.0 * D), 2.0 * D * (256.0 + 7.0 * D), 4);
-    launch_sincos_embed(timesteps_dev, g.timestep_scale_multiplier, c->se.as<float>(), B, 256, st);
-    launch_gemv(c->w_t1, c->b_t1, c->se.as<float>(), c->t1.as<float>(), B, D, 256, 0, st);
-    launch_gemv(c->w_t2, c->b_t2, c->t1.as<float>(), emb, B, D, D, 1, st);
-    launch_gemv(c->w_ada, c->b_ada, emb, ada, B, 6 * D, D, 1, st);
+    adaln_single(c, c->adaln, c->se.as<float>(), c->t1.as<float>(), emb, ada, B, timesteps_dev, g.timestep_scale_multiplier);
   } else {
-    // one embedding per token: the same three Linears as tensor-core GEMMs over the R local rows (bf16 operands, the
-    // SiLUs fused into the first epilogue / a cast pass); timesteps [B, N] are indexed from this rank's first token
+    // one embedding per token over the R local rows; timesteps [B, N] are indexed from this rank's first token
     bf16* se_bf = reinterpret_cast<bf16*>(c->se.ptr);      // [R, 256] bf16
-    bf16* t1_bf = reinterpret_cast<bf16*>(c->t1.ptr);      // [R, D] bf16 = silu(linear_1), later silu(emb)
     {
       ProfScope ps(c, PROF_OTHER, 0.0, 4.0 * R + 512.0 * R);
       launch_sincos_embed(timesteps_dev + tok0, g.timestep_scale_multiplier, nullptr, R, 256, st, se_bf);
     }
-    GemmEpi e1;
-    e1.mode = EPI_SILU_BF16; e1.out = t1_bf; e1.ldo = D; e1.bias = c->b_t1;
-    gemm(c, se_bf, 256, c->w_t1, 256, R, D, 256, e1);
-    GemmEpi e2;
-    e2.mode = EPI_F32; e2.out = emb; e2.ldo = D; e2.bias = c->b_t2;
-    gemm(c, t1_bf, D, c->w_t2, D, R, D, D, e2);
-    {
-      ProfScope ps(c, PROF_OTHER, 0.0, 6.0 * R * D);
-      launch_silu_cast(emb, t1_bf, static_cast<int64_t>(R) * D, st);
-    }
-    GemmEpi e3;
-    e3.mode = EPI_F32; e3.out = ada; e3.ldo = 6 * D; e3.bias = c->b_ada;
-    gemm(c, t1_bf, D, c->w_ada, D, R, 6 * D, D, e3);
+    adaln_single_rows(c, c->adaln, se_bf, R, reinterpret_cast<bf16*>(c->t1.ptr), emb, ada, 6 * D, o);
   }
 
   const int64_t ada_ld = 6 * static_cast<int64_t>(D);
@@ -670,25 +678,23 @@ void dit_forward_dev(ltx_ctx* c, const void* latent, int latent_dtype, const voi
       // q|k|v in one GEMM (N = 3D, 256-wide tiles: 288 tiles = 3.9 rounds of 74 CTA pairs at M = 1536), the V columns stored
       // transposed by the epilogue; separate q|k and V^T GEMMs for batches, sequence parallelism and quantised weights
       // (batches: V^T row = feature, column = b * ldv + token -- the same as the GEMM row b * N + token when ldv == N)
-      const QuantW* qkv8 = fp8_weight(c, bw.a1.wq);
-      const bool fused_qkv = P == 1 && (B == 1 || ldv == N) && (c->qw.empty() || qkv8) && D % 32 == 0;
+      const bool packed_qkv = bw.a1.wq.fmt != LW_AFFINE;   // the q|k|v rows are one matrix
+      const bool fused_qkv = P == 1 && (B == 1 || ldv == N) && packed_qkv && D % 32 == 0;
       GemmEpi e;
       e.mode = EPI_BF16; e.out = qk; e.ldo = 2 * D; e.bias = bw.a1.bq;
-      if (fused_qkv && qkv8) {
+      if (fused_qkv) {
         e.tsplit_col = 2 * D; e.out_t = vt; e.ldt = B * ldv;
-        gemm_fp8(c, h, D, *qkv8, R, 3 * D, D, e, 256);
-      } else if (fused_qkv) {
-        e.tsplit_col = 2 * D; e.out_t = vt; e.ldt = B * ldv;
-        ProfScope ps(c, PROF_GEMM, 2.0 * R * 3.0 * D * D, 2.0 * (static_cast<double>(R) * D + 3.0 * D * D + 3.0 * R * D));
-        launch_gemm(h, D, bw.a1.wq, D, R, 3 * D, D, e, st, R > 128 ? 1256 : 256);
+        LinearOpts ow;
+        ow.tile_n = 256;
+        linear(c, h, D, bw.a1.wq, R, 3 * D, D, e, ow);
       } else if (P == 1) {
-        gemm(c, h, D, bw.a1.wq, D, R, 2 * D, D, e);  // fused q|k projection
+        linear(c, h, D, bw.a1.wq, R, 2 * D, D, e, o);  // fused q|k projection
       }
       if (P == 1) {
         for (int b = 0; b < B && !fused_qkv; ++b)  // V^T, one column block per batch
-          v_transposed(c, bw.a1.wv, bw.a1.bv, h + static_cast<int64_t>(b) * N * D, N, D, vt + b * ldv, B * ldv, q2);
+          linear_vt(c, h + static_cast<int64_t>(b) * N * D, N, 1, bw.a1.wv, bw.a1.bv, vt + b * ldv, B * ldv, ldv, q2, o);
         qknorm(c, qk, 2 * D, R, D, bw.a1.q_norm, cos_l, sin_l, rope_period, eps, bw.a1.k_norm);
-        attention(c, qk, 2 * D, qk + D, 2 * D, vt, ldv, nullptr, att, D, B, Hh, N, N, D, att_scale);
+        attention(c, qk, 2 * D, qk + D, 2 * D, vt, ldv, nullptr, att, D, B, Hh, N, N, D);
       } else {
         // ---- Ulysses: q/k (normed + RoPE'd, which needs the full feature row) and v leave in a head-blocked layout,
         // one all-to-all turns [Nl tokens, all heads] into [all tokens, Hl heads]; attention runs on the local heads;
@@ -708,17 +714,17 @@ void dit_forward_dev(ltx_ctx* c, const void* latent, int latent_dtype, const voi
             ot.p[d] = peer_base[d] + static_cast<int64_t>(3 * P + me) * blk;
           }
         }
-        if (c->qw.empty()) {
-          // bf16 weights: q | k | v as ONE projection over the packed [3D, D] operand (one launch instead of two at a row count
-          // where every launch is latency-bound): q | k stay local (row-major, pitch 2D), the v columns go column-blocked to
-          // their destination ranks
+        if (packed_qkv) {
+          // q | k | v as ONE projection over the packed [3D, D] operand (one launch instead of two at a row count where every
+          // launch is latency-bound): q | k stay local (row-major, pitch 2D), the v columns go column-blocked to their
+          // destination ranks
           GemmEpi eqkv = ev;
           eqkv.out = qk; eqkv.ldo = 2 * D; eqkv.bias = bw.a1.bq;
           eqkv.col_block_from = 2 * D; eqkv.blocked_out = ev.out; eqkv.blocked_ld = Csp;
-          gemm(c, h, D, bw.a1.wq, D, R, 3 * D, D, eqkv);
+          linear(c, h, D, bw.a1.wq, R, 3 * D, D, eqkv, o);
         } else {
-          gemm(c, h, D, bw.a1.wq, D, R, 2 * D, D, e);  // fused q|k projection
-          gemm(c, h, D, bw.a1.wv, D, R, D, D, ev);
+          linear(c, h, D, bw.a1.wq, R, 2 * D, D, e, o);  // fused q|k projection
+          linear(c, h, D, bw.a1.wv, R, D, D, ev, o);
         }
         qknorm(c, qk, 2 * D, R, D, bw.a1.q_norm, cos_l, sin_l, rope_period, eps, bw.a1.k_norm, &qo);
         if (p2p) {
@@ -735,11 +741,11 @@ void dit_forward_dev(ltx_ctx* c, const void* latent, int latent_dtype, const voi
           launch_transpose_bf16(vrecv, Csp, N, Csp, vt_sp, ldv, st);
         }
         if (p2p) {
-          attention(c, qrecv, Csp, krecv, Csp, vt_sp, ldv, nullptr, osend, Csp, 1, Hl, N, N, Csp, att_scale, &ot, Nl);
+          attention(c, qrecv, Csp, krecv, Csp, vt_sp, ldv, nullptr, osend, Csp, 1, Hl, N, N, Csp, &ot, Nl);
           ProfScope ps(c, PROF_COMM, 0.0, 2.0 * P * blk * 2.0);
           dist_p2p_barrier(c, 1);   // every rank's attention rows for our tokens have landed in the o region
         } else {
-          attention(c, qrecv, Csp, krecv, Csp, vt_sp, ldv, nullptr, osend, Csp, 1, Hl, N, N, Csp, att_scale);
+          attention(c, qrecv, Csp, krecv, Csp, vt_sp, ldv, nullptr, osend, Csp, 1, Hl, N, N, Csp);
           ProfScope ps(c, PROF_COMM, 0.0, 2.0 * P * blk * 2.0);
           const void* sb[1] = {osend};
           void* rb[1] = {orecv};
@@ -750,46 +756,49 @@ void dit_forward_dev(ltx_ctx* c, const void* latent, int latent_dtype, const voi
       eo.mode = EPI_GATE_RESID; eo.resid = x; eo.ldr = D; eo.bias = bw.a1.bo;
       eo.gate_a = ada + 2 * D; eo.gate_b = bw.sst + 2 * D; eo.gate_ld = ada_ld; eo.rows_per_gate = rows_per_b;
       eo.shadow = xb; eo.lds = D;
-      if (P == 1)
-        gemm(c, att, D, bw.a1.wo, D, R, D, D, eo);
-      else
-        gemm(c, orecv, Csp, bw.a1.wo, D, R, D, D, eo, Csp, blk);
+      if (P == 1) {
+        linear(c, att, D, bw.a1.wo, R, D, D, eo, o);
+      } else {   // the exchanged attention rows arrive K-blocked
+        LinearOpts ok = o;
+        ok.a_kblock = Csp; ok.a_kblock_stride = blk;
+        linear(c, orecv, Csp, bw.a1.wo, R, D, D, eo, ok);
+      }
     }
     {
       // cross-attention on the UN-normalised stream (T/LTXTransformerBlock.swift:205-214)
       GemmEpi e;
       e.mode = EPI_BF16; e.out = q2; e.ldo = D; e.bias = bw.a2.bq;
-      gemm(c, xb, D, bw.a2.wq, D, R, D, D, e);
+      linear(c, xb, D, bw.a2.wq, R, D, D, e, o);
       qknorm(c, q2, D, R, D, bw.a2.q_norm, nullptr, nullptr, 1, eps);
       const bf16* k2 = tc.k.as<bf16>() + static_cast<int64_t>(i) * B * S * D;
       const bf16* v2 = tc.vt.as<bf16>() + static_cast<int64_t>(i) * D * B * tc.ldv;
-      attention(c, q2, D, k2, D, v2, tc.ldv, key_bias, att, D, B, Hh, Nq, S, D, att_scale);
+      attention(c, q2, D, k2, D, v2, tc.ldv, key_bias, att, D, B, Hh, Nq, S, D);
       GemmEpi eo;
       eo.mode = EPI_GATE_RESID; eo.resid = x; eo.ldr = D; eo.bias = bw.a2.bo; eo.scale = cas;
       const bool next_needs_shadow = skip_ff && (i + 1 < L) &&
                                      in_list(i + 1, flags->stg_blocks, flags->n_stg_blocks) && flags->skip_self_attn;
       if (next_needs_shadow) { eo.shadow = xb; eo.lds = D; }
-      gemm(c, att, D, bw.a2.wo, D, R, D, D, eo);
+      linear(c, att, D, bw.a2.wo, R, D, D, eo, o);
     }
     if (!skip_ff) {
       norm_mod(c, x, h, R, D, bw.sst + 3 * D, bw.sst + 4 * D, ada + 3 * D, ada + 4 * D, ada_ld, rows_per_b, eps, 0);
       GemmEpi e;
       e.mode = EPI_GELU_BF16; e.out = ffh; e.ldo = FFD; e.bias = bw.b_in;
-      gemm(c, h, D, bw.w_in, D, R, FFD, D, e);
+      linear(c, h, D, bw.w_in, R, FFD, D, e, o);
       GemmEpi eo;
       eo.mode = EPI_GATE_RESID; eo.resid = x; eo.ldr = D; eo.bias = bw.b_out;
       eo.gate_a = ada + 5 * D; eo.gate_b = bw.sst + 5 * D; eo.gate_ld = ada_ld; eo.rows_per_gate = rows_per_b;
       const bool next_needs_shadow =
           (i + 1 < L) && in_list(i + 1, flags->stg_blocks, flags->n_stg_blocks) && flags->skip_self_attn;
       if (next_needs_shadow) { eo.shadow = xb; eo.lds = D; }
-      gemm(c, ffh, FFD, bw.w_out, FFD, R, D, FFD, eo);
+      linear(c, ffh, FFD, bw.w_out, R, D, FFD, eo, o);
     }
   }
   // ---- output head (T/LTXTransformer.swift:208-224): LayerNorm(no affine) * (1 + scale) + shift ; proj_out
   norm_mod(c, x, h, R, D, c->sst_out, c->sst_out + D, emb, emb, D, rows_per_b, eps, 1);
   GemmEpi e;
   e.mode = EPI_F32; e.out = (P > 1) ? c->sp_vel.ptr : out_velocity_dev; e.ldo = Cout; e.bias = c->b_out;
-  gemm(c, h, D, c->w_out, D, R, Cout, D, e);
+  linear(c, h, D, c->w_out, R, Cout, D, e, o);
   if (P > 1) {  // every rank receives the full velocity [N, Cout]
     ProfScope ps(c, PROF_COMM, 0.0, 4.0 * N * Cout);
     dist_allgather_sp(c, c->sp_vel.ptr, out_velocity_dev, static_cast<size_t>(Nl) * Cout * 4);

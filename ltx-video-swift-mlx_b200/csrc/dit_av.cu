@@ -219,76 +219,21 @@ __global__ void __launch_bounds__(256) qknorm_rope_hd_kernel(bf16* x, int64_t ld
 }
 
 // ---------------------------------------------------------------- profiled launch helpers
-// items: batch items whose rows make up M (1 or 2).  The weight-streaming kernel takes up to 32 rows per item, so a row of a
-// two-item product runs on the kernel its one-item product runs on.
-void gemm(ltx_ctx* c, const bf16* A, int64_t lda, const bf16* B, int64_t ldb, int M, int N, int K, const GemmEpi& e,
-          int items = 1) {
-  auto it = c->qw.empty() ? c->qw.end() : c->qw.find(B);
-  const bool panel = it != c->qw.end() && gemm_q_uses_panel(it->second, M);
-  ProfScope ps(c, PROF_GEMM, 2.0 * M * N * K, 2.0 * (static_cast<double>(M) * K + static_cast<double>(N) * K + static_cast<double>(M) * N),
-               panel ? 2 : 1);
-  if (it != c->qw.end()) {   // int8 / int4 codes (quantize(model: ltx2, ...), Pipeline/LTXPipeline.swift:491): dequant-fused kernel
-    launch_gemm_q(A, lda, it->second, M, N, K, e, c->stream);
-    return;
-  }
-  launch_gemm(A, lda, B, ldb, M, N, K, e, c->stream, 0, 0, 0, 32 * items);   // the audio stream's Linears stream their weights
-}
 // out_bf16[M, N] = A W^T + b
-void linear(ltx_ctx* c, const bf16* A, int M, int K, const bf16* W, const float* b, int N, bf16* out, int mode = EPI_BF16,
-            int items = 1) {
+void proj(ltx_ctx* c, const bf16* A, int M, int K, const LinearW& W, const float* b, int N, bf16* out, int mode,
+          const LinearOpts& o) {
   GemmEpi e;
   e.mode = mode; e.out = out; e.ldo = N; e.bias = b;
-  gemm(c, A, K, W, K, M, N, K, e, items);
+  linear(c, A, K, W, M, N, K, e, o);
 }
 // x[M, N] (fp32) += (A W^T + b) * (gate_a[(m / gate_rows) * gate_ld + n] + gate_b[n])   (null gates: 1); gate_ld = 0: one
 // gate row for all M rows
-void linear_resid(ltx_ctx* c, const bf16* A, int M, int K, const bf16* W, const float* b, int N, float* x, const float* gate_a,
-                  const float* gate_b, int64_t gate_ld = 0, int gate_rows = 1, int items = 1) {
+void proj_resid(ltx_ctx* c, const bf16* A, int M, int K, const LinearW& W, const float* b, int N, float* x, const float* gate_a,
+                const float* gate_b, int64_t gate_ld, int gate_rows, const LinearOpts& o) {
   GemmEpi e;
   e.mode = EPI_GATE_RESID; e.resid = x; e.ldr = N; e.bias = b; e.gate_a = gate_a; e.gate_b = gate_b; e.gate_ld = gate_ld;
   e.rows_per_gate = gate_ld > 0 ? gate_rows : (M > 0 ? M : 1);
-  gemm(c, A, K, W, K, M, N, K, e, items);
-}
-// V^T of `items` batch items: item i's [Nout, rows] block starts at column i * item_ld of `out` (row pitch items * item_ld)
-// = (h W^T + b)^T.  The weight is the A operand, so the product lands transposed.  Quantised weights must be the B operand:
-// project into `tmp` [items * rows, Nout], then transpose.
-void linear_t(ltx_ctx* c, const bf16* W, const float* b, int Nout, int K, const bf16* hrows, int rows, int items, bf16* out,
-              int64_t item_ld, bf16* tmp) {
-  const int64_t ld_out = items * item_ld;
-  if (c->qw.empty() || c->qw.find(W) == c->qw.end()) {
-    GemmEpi e;
-    e.mode = EPI_BF16; e.out = out; e.ldo = ld_out; e.bias = b;
-    if (items > 1) { e.t_item_rows = rows; e.t_item_ld = item_ld; }
-    if (rows <= 32 && gemm_skinny_eligible(K, K, items * rows, Nout, K, e, 0, 32 * items)) {   // audio rows: stream the weight
-      e.transpose_out = 1;
-      gemm(c, hrows, K, W, K, items * rows, Nout, K, e, items);
-      return;
-    }
-    e.t_item_rows = 0;
-    e.bias_per_row = 1;
-    if (items == 1 || rows == item_ld) {   // the items' column blocks are contiguous
-      gemm(c, W, K, hrows, K, Nout, items * rows, K, e);
-      return;
-    }
-    for (int i = 0; i < items; ++i) {
-      e.out = out + i * item_ld;
-      gemm(c, W, K, hrows + static_cast<int64_t>(i) * rows * K, K, Nout, rows, K, e);
-    }
-    return;
-  }
-  GemmEpi e;
-  e.mode = EPI_BF16; e.out = tmp; e.ldo = Nout; e.bias = b;
-  gemm(c, hrows, K, W, K, items * rows, Nout, K, e, items);
-  ProfScope ps(c, PROF_OTHER, 0.0, 4.0 * items * rows * Nout, items);
-  for (int i = 0; i < items; ++i)
-    launch_transpose_bf16(tmp + static_cast<int64_t>(i) * rows * Nout, Nout, rows, Nout, out + i * item_ld, ld_out, c->stream);
-}
-// B items: Q [B*Nq, D], K [B*Nk, ldk], V^T [D, B*ldv] (item b at column b * ldv), key bias [B, Nk]
-void attention(ltx_ctx* c, const bf16* Q, const bf16* K, int64_t ldk, const bf16* Vt, int64_t ldv, const float* bias, bf16* O, int H,
-               int hd, int B, int Nq, int Nk) {
-  const int D = H * hd;
-  ProfScope ps(c, PROF_ATTN, 4.0 * B * H * static_cast<double>(Nq) * Nk * hd, 2.0 * B * (2.0 * Nq + 2.0 * Nk) * D);
-  launch_attention(Q, D, K, ldk, Vt, ldv, bias, O, D, B, H, Nq, Nk, D, 1.0f / sqrtf(static_cast<float>(hd)), c->stream);
+  linear(c, A, K, W, M, N, K, e, o);
 }
 // a_ld > 0: row r takes its modulation rows sc_a / sh_a + (r / a_rpr) * a_ld (one per token, or one per batch item)
 void normw(ltx_ctx* c, const float* x, bf16* out, int M, int D, const float* w, const float* sc_t, const float* sc_a,
@@ -329,65 +274,16 @@ void qknorm_hd(ltx_ctx* c, bf16* x, int M, int D, int hd, const float* w, const 
   LTX_CUDA(cudaGetLastError());
 }
 
-const bf16* wbf(ltx_ctx* c, const std::string& k, int64_t r, int64_t cc) {
-  const DevTensor& t = get_tensor(c, k);
-  LTX_CHECK(t.dtype == LTX_BF16 && t.shape.size() == 2 && t.shape[0] == r && t.shape[1] == cc, LTX_ERR_WEIGHTS,
-            "bad shape for '" + k + "'");
-  return reinterpret_cast<const bf16*>(t.ptr);
-}
-const float* wf(ltx_ctx* c, const std::string& k, int64_t n) {
-  const DevTensor& t = get_tensor(c, k);
-  LTX_CHECK(t.dtype == LTX_F32 && t.numel() == n, LTX_ERR_WEIGHTS, "bad shape for '" + k + "'");
-  return reinterpret_cast<const float*>(t.ptr);
-}
 AttnWeights attn_w(ltx_ctx* c, const std::string& p, int64_t qdim, int64_t cdim, int64_t inner) {
   AttnWeights a;
-  a.wq = wbf(c, p + ".to_q.weight", inner, qdim); a.bq = wf(c, p + ".to_q.bias", inner);
-  a.wk = wbf(c, p + ".to_k.weight", inner, cdim); a.bk = wf(c, p + ".to_k.bias", inner);
-  a.wv = wbf(c, p + ".to_v.weight", inner, cdim); a.bv = wf(c, p + ".to_v.bias", inner);
-  a.wo = wbf(c, p + ".to_out.weight", qdim, inner); a.bo = wf(c, p + ".to_out.bias", qdim);
+  a.wq = wlin(c, p + ".to_q.weight", inner, qdim); a.bq = wf(c, p + ".to_q.bias", inner);
+  a.wk = wlin(c, p + ".to_k.weight", inner, cdim); a.bk = wf(c, p + ".to_k.bias", inner);
+  a.wv = wlin(c, p + ".to_v.weight", inner, cdim); a.bv = wf(c, p + ".to_v.bias", inner);
+  a.wo = wlin(c, p + ".to_out.weight", qdim, inner); a.bo = wf(c, p + ".to_out.bias", qdim);
   a.q_norm = wf(c, p + ".q_norm.weight", inner);
   a.k_norm = wf(c, p + ".k_norm.weight", inner);
   return a;
 }
-AdaLnW adaln_w(ltx_ctx* c, const std::string& p, int64_t dim, int n) {
-  AdaLnW a;
-  a.w1 = wbf(c, p + ".emb.linear_1.weight", dim, 256); a.b1 = wf(c, p + ".emb.linear_1.bias", dim);
-  a.w2 = wbf(c, p + ".emb.linear_2.weight", dim, dim); a.b2 = wf(c, p + ".emb.linear_2.bias", dim);
-  a.wl = wbf(c, p + ".linear.weight", n * dim, dim); a.bl = wf(c, p + ".linear.bias", n * dim);
-  a.dim = static_cast<int>(dim); a.n = n;
-  return a;
-}
-
-// AdaLayerNormSingle (T/LTXTimestepEmbedding.swift:96-124) for one sigma per batch item (B rows): se = sincos(sigma * mult)
-// is shared by every embedder of the same stream; emb = L2(silu(L1(se))), lin = L(silu(emb)), row pitches dim and n * dim.
-void adaln_single(ltx_ctx* c, const AdaLnW& a, const float* se, float* t1, float* emb, float* lin, int B = 1) {
-  ProfScope ps(c, PROF_OTHER, 2.0 * B * a.dim * (256.0 + (1.0 + a.n) * a.dim), 2.0 * a.dim * (256.0 + (1.0 + a.n) * a.dim), 3);
-  launch_gemv(a.w1, a.b1, se, t1, B, a.dim, 256, 0, c->stream);
-  launch_gemv(a.w2, a.b2, t1, emb, B, a.dim, a.dim, 1, c->stream);
-  launch_gemv(a.wl, a.bl, emb, lin, B, a.n * a.dim, a.dim, 1, c->stream);
-}
-
-// The same for R sigmas (one per video token): the three Linears as tensor-core GEMMs over the R rows, bf16 operands, the
-// SiLUs in the first epilogue / a cast pass (the video-only model's per-token path, dit.cu).  se_bf [R, 256] bf16;
-// t1_bf [R, dim] bf16 scratch; emb [R, dim] fp32; lin [R, n * dim] fp32 with row pitch ld_lin.
-void adaln_single_rows(ltx_ctx* c, const AdaLnW& a, const bf16* se_bf, int R, bf16* t1_bf, float* emb, float* lin, int64_t ld_lin,
-                       int items) {
-  GemmEpi e1;
-  e1.mode = EPI_SILU_BF16; e1.out = t1_bf; e1.ldo = a.dim; e1.bias = a.b1;
-  gemm(c, se_bf, 256, a.w1, 256, R, a.dim, 256, e1, items);
-  GemmEpi e2;
-  e2.mode = EPI_F32; e2.out = emb; e2.ldo = a.dim; e2.bias = a.b2;
-  gemm(c, t1_bf, a.dim, a.w2, a.dim, R, a.dim, a.dim, e2, items);
-  {
-    ProfScope ps(c, PROF_OTHER, 0.0, 6.0 * R * a.dim);
-    launch_silu_cast(emb, t1_bf, static_cast<int64_t>(R) * a.dim, c->stream);
-  }
-  GemmEpi e3;
-  e3.mode = EPI_F32; e3.out = lin; e3.ldo = ld_lin; e3.bias = a.bl;
-  gemm(c, t1_bf, a.dim, a.wl, a.dim, R, a.n * a.dim, a.dim, e3, items);
-}
-
 // 1-D RoPE table, token-major [T, dim/2] (precomputeFreqsCis with a [1, T] grid, T/LTXRoPE.swift:375-488): all dim/2
 // frequencies come from the single axis, no identity padding.
 void build_rope_1d(ltx_ctx* c, DevBuf& cosb, DevBuf& sinb, const std::vector<float>& pos, int dim, float theta, int max_pos) {
@@ -420,7 +316,7 @@ int64_t round_up8(int64_t v) { return (v + 7) / 8 * 8; }
 
 void dit_av_finalize(ltx_ctx* c) {
   const ltx_config& g = c->cfg;
-  LTX_CHECK(c->dit_ready && c->precision == 16 && c->qw.empty(), LTX_ERR_WEIGHTS,
+  LTX_CHECK(c->dit_ready && c->precision == 16 && c->w_patch.fmt == LW_BF16, LTX_ERR_WEIGHTS,
             "the dual model is finalized on the bf16 video weights (quantisation follows)");
   AvWeights& a = c->av;
   const int64_t D = static_cast<int64_t>(g.num_heads) * g.head_dim;
@@ -430,13 +326,13 @@ void dit_av_finalize(ltx_ctx* c) {
   LTX_CHECK(Da % 128 == 0, LTX_ERR_INVALID_CONFIGURATION, "audio inner dim must be a multiple of 128");
   const int Ca = g.audio_in_channels > 0 ? g.audio_in_channels : 128;
   a.Da = static_cast<int>(Da); a.Ha = Ha; a.hd = hd; a.Cin = Ca;
-  a.w_patch = wbf(c, "audio_patchify_proj.weight", Da, Ca); a.b_patch = wf(c, "audio_patchify_proj.bias", Da);
-  a.w_c1 = wbf(c, "audio_caption_projection.linear_1.weight", Da, g.caption_channels);
+  a.w_patch = wlin(c, "audio_patchify_proj.weight", Da, Ca); a.b_patch = wf(c, "audio_patchify_proj.bias", Da);
+  a.w_c1 = wlin(c, "audio_caption_projection.linear_1.weight", Da, g.caption_channels);
   a.b_c1 = wf(c, "audio_caption_projection.linear_1.bias", Da);
-  a.w_c2 = wbf(c, "audio_caption_projection.linear_2.weight", Da, Da);
+  a.w_c2 = wlin(c, "audio_caption_projection.linear_2.weight", Da, Da);
   a.b_c2 = wf(c, "audio_caption_projection.linear_2.bias", Da);
   a.sst_out = wf(c, "audio_scale_shift_table", 2 * Da);
-  a.w_out = wbf(c, "audio_proj_out.weight", Ca, Da); a.b_out = wf(c, "audio_proj_out.bias", Ca);
+  a.w_out = wlin(c, "audio_proj_out.weight", Ca, Da); a.b_out = wf(c, "audio_proj_out.bias", Ca);
   a.ada_a = adaln_w(c, "audio_adaln_single", Da, 6);
   a.cv_ss = adaln_w(c, "av_ca_video_scale_shift_adaln_single", D, 4);
   a.cv_g = adaln_w(c, "av_ca_a2v_gate_adaln_single", D, 1);
@@ -454,8 +350,8 @@ void dit_av_finalize(ltx_ctx* c) {
     b.aa2 = attn_w(c, p + "audio_attn2", Da, Da, Da);
     b.a2v = attn_w(c, p + "audio_to_video_attn", D, Da, Da);
     b.v2a = attn_w(c, p + "video_to_audio_attn", Da, D, Da);
-    b.w_in = wbf(c, p + "audio_ff.project_in.proj.weight", FFa, Da); b.b_in = wf(c, p + "audio_ff.project_in.proj.bias", FFa);
-    b.w_out = wbf(c, p + "audio_ff.project_out.weight", Da, FFa); b.b_out = wf(c, p + "audio_ff.project_out.bias", Da);
+    b.w_in = wlin(c, p + "audio_ff.project_in.proj.weight", FFa, Da); b.b_in = wf(c, p + "audio_ff.project_in.proj.bias", FFa);
+    b.w_out = wlin(c, p + "audio_ff.project_out.weight", Da, FFa); b.b_out = wf(c, p + "audio_ff.project_out.bias", Da);
     b.asst = wf(c, p + "audio_scale_shift_table", 6 * Da);
     b.sst_ca_v = wf(c, p + "scale_shift_table_a2v_ca_video", 5 * D);
     b.sst_ca_a = wf(c, p + "scale_shift_table_a2v_ca_audio", 5 * Da);
@@ -484,6 +380,8 @@ void dit_av_forward_dev(ltx_ctx* c, const void* v_latent, int v_dtype, const voi
   cudaStream_t st = c->stream;
   const int64_t ldv = round_up8(N), lda = round_up8(Ta);   // per-item column pitches of the V^T operands
   const int R = B * N, Ra = B * Ta;                         // rows of the two streams
+  LinearOpts o;   // the weight-streaming kernel takes up to 32 rows per item: a row of a two-item product runs on the kernel its
+  o.allow_skinny = 32 * B;   // one-item product runs on (the audio stream's Linears stream their weights)
 
   // ---- workspaces: the video stream reuses the video-only model's buffers
   c->x.reserve(static_cast<size_t>(R) * D * 4);
@@ -509,7 +407,7 @@ void dit_av_forward_dev(ltx_ctx* c, const void* v_latent, int v_dtype, const voi
                 cag_ld = per_item ? static_cast<int64_t>(Da) : 0;
   // audio / cross-modal workspace carved out of one allocation
   size_t off = 0;
-  auto carve = [&](size_t bytes) { const size_t o = off; off += (bytes + 255) / 256 * 256; return o; };
+  auto carve = [&](size_t bytes) { const size_t at = off; off += (bytes + 255) / 256 * 256; return at; };
   const size_t o_ax = carve(static_cast<size_t>(Ra) * Da * 4), o_ah = carve(static_cast<size_t>(Ra) * Da * 2),
                o_ah2 = carve(static_cast<size_t>(Ra) * Da * 2), o_aq = carve(static_cast<size_t>(Ra) * Da * 2),
                o_ak = carve(static_cast<size_t>(Ra) * Da * 2), o_avt = carve(static_cast<size_t>(Da) * B * lda * 2),
@@ -522,7 +420,7 @@ void dit_av_forward_dev(ltx_ctx* c, const void* v_latent, int v_dtype, const voi
                o_vada = carve(static_cast<size_t>(VR) * 6 * D * 4), o_aada = carve(static_cast<size_t>(B) * 6 * Da * 4),
                o_cv = carve(static_cast<size_t>(VR) * 5 * D * 4), o_ca = carve(static_cast<size_t>(B) * 5 * Da * 4),
                o_scr = carve(static_cast<size_t>(VR) * D * 4),
-               o_tq = carve(c->qw.empty() ? 0 : static_cast<size_t>(std::max(R, Ra)) * D * 2),   // projection before the V^T transpose
+               o_tq = carve(c->w_patch.fmt == LW_BF16 ? 0 : static_cast<size_t>(std::max(R, Ra)) * D * 2),   // codes: projection before the V^T transpose
                o_sev = carve(v_ts_per_token ? static_cast<size_t>(R) * 256 * 2 : 0),
                o_t1v = carve(v_ts_per_token ? static_cast<size_t>(R) * D * 2 : 0);
   wsb.reserve(off);
@@ -579,7 +477,7 @@ void dit_av_forward_dev(ltx_ctx* c, const void* v_latent, int v_dtype, const voi
   const float* abias = tca.has_bias ? tca.bias.as<float>() : nullptr;
 
   // ---- patchify projections (T/LTX2Transformer.swift:255, 262); the reference's bf16 Linear output is rounded to bf16
-  auto embed = [&](const void* lat, int dt, int rows, int Cin, const bf16* w, const float* b, int Dout, float* xout, bf16* tmp) {
+  auto embed = [&](const void* lat, int dt, int rows, int Cin, const LinearW& w, const float* b, int Dout, float* xout, bf16* tmp) {
     const bf16* src = reinterpret_cast<const bf16*>(lat);
     if (dt == LTX_F32) {
       LTX_CHECK((static_cast<int64_t>(rows) * Cin) % 4 == 0, LTX_ERR_INVALID_ARGUMENT, "latent size");
@@ -587,7 +485,7 @@ void dit_av_forward_dev(ltx_ctx* c, const void* v_latent, int v_dtype, const voi
       launch_cast_f32_bf16(reinterpret_cast<const float*>(lat), lat_bf, static_cast<int64_t>(rows) * Cin, st);
       src = lat_bf;
     }
-    linear(c, src, rows, Cin, w, b, Dout, tmp, EPI_BF16, B);
+    proj(c, src, rows, Cin, w, b, Dout, tmp, EPI_BF16, o);
     ProfScope ps(c, PROF_OTHER, 0.0, 6.0 * rows * Dout);
     launch_cast_bf16_f32(tmp, xout, static_cast<int64_t>(rows) * Dout, st);
   };
@@ -601,13 +499,10 @@ void dit_av_forward_dev(ltx_ctx* c, const void* v_latent, int v_dtype, const voi
     launch_sincos_embed(v_ts_dev, g.timestep_scale_multiplier, se, B, 256, st);
     launch_sincos_embed(a_ts_dev, g.timestep_scale_multiplier, se_a, B, 256, st);
   }
-  AdaLnW vmain;
-  vmain.w1 = c->w_t1; vmain.b1 = c->b_t1; vmain.w2 = c->w_t2; vmain.b2 = c->b_t2; vmain.wl = c->w_ada; vmain.bl = c->b_ada;
-  vmain.dim = D; vmain.n = 6;
   float* cvg = v_ts_per_token ? cv + 4 * D : cv + static_cast<int64_t>(B) * 4 * D;   // gate rows (see the pitches above)
   float* cag = ca + static_cast<int64_t>(B) * 4 * Da;
   if (!v_ts_per_token) {
-    adaln_single(c, vmain, se, t1, vemb, vada, B);
+    adaln_single(c, c->adaln, se, t1, vemb, vada, B);
     adaln_single(c, av.cv_ss, se, t1, scr, cv, B);              // rows 0-3: a2v scale, a2v shift, v2a scale, v2a shift
     adaln_single(c, av.cv_g, se, t1, scr, cvg, B);              // row 4: a2v gate
   } else {
@@ -616,9 +511,9 @@ void dit_av_forward_dev(ltx_ctx* c, const void* v_latent, int v_dtype, const voi
       ProfScope ps(c, PROF_OTHER, 0.0, 4.0 * R + 512.0 * R);
       launch_sincos_embed(v_ts_dev, g.timestep_scale_multiplier, nullptr, R, 256, st, sev);
     }
-    adaln_single_rows(c, vmain, sev, R, t1v, vemb, vada, vada_ld, B);
-    adaln_single_rows(c, av.cv_ss, sev, R, t1v, scr, cv, cv_ld, B);         // [R, 5, D]: rows 0-3 of every token
-    adaln_single_rows(c, av.cv_g, sev, R, t1v, scr, cvg, cvg_ld, B);        // row 4 of every token
+    adaln_single_rows(c, c->adaln, sev, R, t1v, vemb, vada, vada_ld, o);
+    adaln_single_rows(c, av.cv_ss, sev, R, t1v, scr, cv, cv_ld, o);         // [R, 5, D]: rows 0-3 of every token
+    adaln_single_rows(c, av.cv_g, sev, R, t1v, scr, cvg, cvg_ld, o);        // row 4 of every token
   }
   adaln_single(c, av.ada_a, se_a, t1, aemb, aada, B);
   adaln_single(c, av.ca_ss, se_a, t1, scr, ca, B);
@@ -629,75 +524,68 @@ void dit_av_forward_dev(ltx_ctx* c, const void* v_latent, int v_dtype, const voi
     const AvBlockW& ba = av.blocks[i];
     // ---- 1: video self-attention (T/LTX2TransformerBlock.swift:208-211)
     normw(c, x, h, R, D, ba.norm1, bv.sst + D, vada + D, bv.sst, vada, eps, vada_ld, v_rpr);
-    {
-      GemmEpi e;
-      e.mode = EPI_BF16; e.out = qk; e.ldo = 2 * D; e.bias = bv.a1.bq;
-      gemm(c, h, D, bv.a1.wq, D, R, 2 * D, D, e, B);   // packed q|k projection
-    }
-    linear_t(c, bv.a1.wv, bv.a1.bv, D, D, h, N, B, vt, ldv, tq);
+    proj(c, h, R, D, bv.a1.wq, bv.a1.bq, 2 * D, qk, EPI_BF16, o);   // packed q|k projection
+    linear_vt(c, h, N, B, bv.a1.wv, bv.a1.bv, vt, B * ldv, ldv, tq, o);
     {
       ProfScope ps(c, PROF_ROW, 0.0, 2.0 * R * D * 8.0, (D == 4096) ? 1 : 2);
       launch_qknorm_rope(qk, 2 * D, R, D, bv.a1.q_norm, cos_v, sin_v, N, eps, st, bv.a1.k_norm);
     }
-    {
-      ProfScope ps(c, PROF_ATTN, 4.0 * B * Hv * static_cast<double>(N) * N * hdv, 2.0 * 4.0 * R * D);
-      launch_attention(qk, 2 * D, qk + D, 2 * D, vt, ldv, nullptr, att, D, B, Hv, N, N, D, 1.0f / sqrtf(static_cast<float>(hdv)), st);
-    }
-    linear_resid(c, att, R, D, bv.a1.wo, bv.a1.bo, D, x, vada + 2 * D, bv.sst + 2 * D, vada_ld, v_rpr, B);
+    attention(c, qk, 2 * D, qk + D, 2 * D, vt, ldv, nullptr, att, D, B, Hv, N, N, D);
+    proj_resid(c, att, R, D, bv.a1.wo, bv.a1.bo, D, x, vada + 2 * D, bv.sst + 2 * D, vada_ld, v_rpr, o);
     // ---- 2: audio self-attention (:213-216)
     normw(c, ax, ah, Ra, Da, ba.anorm1, ba.asst + Da, aada + Da, ba.asst, aada, eps, aada_ld, Ta);
-    linear(c, ah, Ra, Da, ba.aa1.wq, ba.aa1.bq, Da, aq, EPI_BF16, B);
-    linear(c, ah, Ra, Da, ba.aa1.wk, ba.aa1.bk, Da, ak, EPI_BF16, B);
-    linear_t(c, ba.aa1.wv, ba.aa1.bv, Da, Da, ah, Ta, B, avt, lda, tq);
+    proj(c, ah, Ra, Da, ba.aa1.wq, ba.aa1.bq, Da, aq, EPI_BF16, o);
+    proj(c, ah, Ra, Da, ba.aa1.wk, ba.aa1.bk, Da, ak, EPI_BF16, o);
+    linear_vt(c, ah, Ta, B, ba.aa1.wv, ba.aa1.bv, avt, B * lda, lda, tq, o);
     qknorm_hd(c, aq, Ra, Da, hda, ba.aa1.q_norm, cos_a, sin_a, Ta, eps);
     qknorm_hd(c, ak, Ra, Da, hda, ba.aa1.k_norm, cos_a, sin_a, Ta, eps);
-    attention(c, aq, ak, Da, avt, lda, nullptr, aatt, Ha, hda, B, Ta, Ta);
-    linear_resid(c, aatt, Ra, Da, ba.aa1.wo, ba.aa1.bo, Da, ax, aada + 2 * Da, ba.asst + 2 * Da, aada_ld, Ta, B);
+    attention(c, aq, Da, ak, Da, avt, lda, nullptr, aatt, Da, B, Ha, Ta, Ta, Da);
+    proj_resid(c, aatt, Ra, Da, ba.aa1.wo, ba.aa1.bo, Da, ax, aada + 2 * Da, ba.asst + 2 * Da, aada_ld, Ta, o);
     // ---- 3: video text cross-attention on norm2(x), no RoPE, no gate (:218-221)
     normw(c, x, h, R, D, ba.norm2, nullptr, nullptr, nullptr, nullptr, eps);
-    linear(c, h, R, D, bv.a2.wq, bv.a2.bq, D, q2, EPI_BF16, B);
+    proj(c, h, R, D, bv.a2.wq, bv.a2.bq, D, q2, EPI_BF16, o);
     qknorm_hd(c, q2, R, D, hdv, bv.a2.q_norm, nullptr, nullptr, 1, eps);
-    attention(c, q2, tcv.k.as<bf16>() + static_cast<int64_t>(i) * B * S * D, D,
-              tcv.vt.as<bf16>() + static_cast<int64_t>(i) * D * B * tcv.ldv, tcv.ldv, vbias, att, Hv, hdv, B, N, S);
-    linear_resid(c, att, R, D, bv.a2.wo, bv.a2.bo, D, x, nullptr, nullptr, 0, 1, B);
+    attention(c, q2, D, tcv.k.as<bf16>() + static_cast<int64_t>(i) * B * S * D, D,
+              tcv.vt.as<bf16>() + static_cast<int64_t>(i) * D * B * tcv.ldv, tcv.ldv, vbias, att, D, B, Hv, N, S, D);
+    proj_resid(c, att, R, D, bv.a2.wo, bv.a2.bo, D, x, nullptr, nullptr, 0, 1, o);
     // ---- 4: audio text cross-attention (:223-226)
     normw(c, ax, ah, Ra, Da, ba.anorm2, nullptr, nullptr, nullptr, nullptr, eps);
-    linear(c, ah, Ra, Da, ba.aa2.wq, ba.aa2.bq, Da, aq, EPI_BF16, B);
+    proj(c, ah, Ra, Da, ba.aa2.wq, ba.aa2.bq, Da, aq, EPI_BF16, o);
     qknorm_hd(c, aq, Ra, Da, hda, ba.aa2.q_norm, nullptr, nullptr, 1, eps);
-    attention(c, aq, tca.k.as<bf16>() + static_cast<int64_t>(i) * B * S * Da, Da,
-              tca.vt.as<bf16>() + static_cast<int64_t>(i) * Da * B * tca.ldv, tca.ldv, abias, aatt, Ha, hda, B, Ta, S);
-    linear_resid(c, aatt, Ra, Da, ba.aa2.wo, ba.aa2.bo, Da, ax, nullptr, nullptr, 0, 1, B);
+    attention(c, aq, Da, tca.k.as<bf16>() + static_cast<int64_t>(i) * B * S * Da, Da,
+              tca.vt.as<bf16>() + static_cast<int64_t>(i) * Da * B * tca.ldv, tca.ldv, abias, aatt, Da, B, Ha, Ta, S, Da);
+    proj_resid(c, aatt, Ra, Da, ba.aa2.wo, ba.aa2.bo, Da, ax, nullptr, nullptr, 0, 1, o);
     // ---- 5-6: cross-modal attention; both directions read the streams as they are here (:228-271).  Table / embedding
     // rows: 0 a2v scale, 1 a2v shift, 2 v2a scale, 3 v2a shift, 4 gate.  Each item attends within itself only.
     normw2(c, x, h, h2, R, D, ba.a2v_norm, ba.sst_ca_v, cv, eps, cv_ld, v_rpr);   // video as a2v query (h) and v2a context (h2)
     normw2(c, ax, ah, ah2, Ra, Da, ba.v2a_norm, ba.sst_ca_a, ca, eps, ca_ld, Ta);  // audio as a2v context (ah) and v2a query (ah2)
     // A2V: Q from video (temporal RoPE of the video frames), K / V from audio
-    linear(c, h, R, D, ba.a2v.wq, ba.a2v.bq, Da, cq, EPI_BF16, B);
-    linear(c, ah, Ra, Da, ba.a2v.wk, ba.a2v.bk, Da, ak, EPI_BF16, B);
-    linear_t(c, ba.a2v.wv, ba.a2v.bv, Da, Da, ah, Ta, B, avt, lda, tq);
+    proj(c, h, R, D, ba.a2v.wq, ba.a2v.bq, Da, cq, EPI_BF16, o);
+    proj(c, ah, Ra, Da, ba.a2v.wk, ba.a2v.bk, Da, ak, EPI_BF16, o);
+    linear_vt(c, ah, Ta, B, ba.a2v.wv, ba.a2v.bv, avt, B * lda, lda, tq, o);
     qknorm_hd(c, cq, R, Da, hda, ba.a2v.q_norm, cos_xv, sin_xv, N, eps);
     qknorm_hd(c, ak, Ra, Da, hda, ba.a2v.k_norm, cos_a, sin_a, Ta, eps);
-    attention(c, cq, ak, Da, avt, lda, nullptr, catt, Ha, hda, B, N, Ta);
+    attention(c, cq, Da, ak, Da, avt, lda, nullptr, catt, Da, B, Ha, N, Ta, Da);
     // V2A: Q from audio, K / V from video (projected before the a2v update lands in x: h2 was taken above)
-    linear(c, ah2, Ra, Da, ba.v2a.wq, ba.v2a.bq, Da, aq, EPI_BF16, B);
-    linear(c, h2, R, D, ba.v2a.wk, ba.v2a.bk, Da, cq, EPI_BF16, B);
-    linear_t(c, ba.v2a.wv, ba.v2a.bv, Da, D, h2, N, B, vt2, ldv, tq);
+    proj(c, ah2, Ra, Da, ba.v2a.wq, ba.v2a.bq, Da, aq, EPI_BF16, o);
+    proj(c, h2, R, D, ba.v2a.wk, ba.v2a.bk, Da, cq, EPI_BF16, o);
+    linear_vt(c, h2, N, B, ba.v2a.wv, ba.v2a.bv, vt2, B * ldv, ldv, tq, o);
     qknorm_hd(c, aq, Ra, Da, hda, ba.v2a.q_norm, cos_a, sin_a, Ta, eps);
     qknorm_hd(c, cq, R, Da, hda, ba.v2a.k_norm, cos_xv, sin_xv, N, eps);
-    attention(c, aq, cq, Da, vt2, ldv, nullptr, aatt, Ha, hda, B, Ta, N);
-    linear_resid(c, catt, R, Da, ba.a2v.wo, ba.a2v.bo, D, x, cvg, ba.sst_ca_v + 4 * D, cvg_ld, v_rpr, B);
-    linear_resid(c, aatt, Ra, Da, ba.v2a.wo, ba.v2a.bo, Da, ax, cag, ba.sst_ca_a + 4 * Da, cag_ld, Ta, B);
+    attention(c, aq, Da, cq, Da, vt2, ldv, nullptr, aatt, Da, B, Ha, Ta, N, Da);
+    proj_resid(c, catt, R, Da, ba.a2v.wo, ba.a2v.bo, D, x, cvg, ba.sst_ca_v + 4 * D, cvg_ld, v_rpr, o);
+    proj_resid(c, aatt, Ra, Da, ba.v2a.wo, ba.v2a.bo, Da, ax, cag, ba.sst_ca_a + 4 * Da, cag_ld, Ta, o);
     // ---- 7-8: feed-forward on both streams (:273-281)
     normw(c, x, h, R, D, ba.norm3, bv.sst + 4 * D, vada + 4 * D, bv.sst + 3 * D, vada + 3 * D, eps, vada_ld, v_rpr);
-    linear(c, h, R, D, bv.w_in, bv.b_in, FFD, ffh, EPI_GELU_BF16, B);
-    linear_resid(c, ffh, R, FFD, bv.w_out, bv.b_out, D, x, vada + 5 * D, bv.sst + 5 * D, vada_ld, v_rpr, B);
+    proj(c, h, R, D, bv.w_in, bv.b_in, FFD, ffh, EPI_GELU_BF16, o);
+    proj_resid(c, ffh, R, FFD, bv.w_out, bv.b_out, D, x, vada + 5 * D, bv.sst + 5 * D, vada_ld, v_rpr, o);
     normw(c, ax, ah, Ra, Da, ba.anorm3, ba.asst + 4 * Da, aada + 4 * Da, ba.asst + 3 * Da, aada + 3 * Da, eps, aada_ld, Ta);
-    linear(c, ah, Ra, Da, ba.w_in, ba.b_in, FFa, affh, EPI_GELU_BF16, B);
-    linear_resid(c, affh, Ra, FFa, ba.w_out, ba.b_out, Da, ax, aada + 5 * Da, ba.asst + 5 * Da, aada_ld, Ta, B);
+    proj(c, ah, Ra, Da, ba.w_in, ba.b_in, FFa, affh, EPI_GELU_BF16, o);
+    proj_resid(c, affh, Ra, FFa, ba.w_out, ba.b_out, Da, ax, aada + 5 * Da, ba.asst + 5 * Da, aada_ld, Ta, o);
   }
   // ---- output heads (T/LTX2Transformer.swift:370-388): LayerNorm(no affine) * (1 + scale) + shift ; proj_out
   // emb: one row per item (rpr = rows of an item) or per token (rpr = 1)
-  auto head = [&](const float* xs, int rows, int Dx, const float* sst, const float* emb, int rpr, bf16* tmp, const bf16* w,
+  auto head = [&](const float* xs, int rows, int Dx, const float* sst, const float* emb, int rpr, bf16* tmp, const LinearW& w,
                   const float* b, int Cout, float* out) {
     {
       ProfScope ps(c, PROF_ROW, 0.0, static_cast<double>(rows) * Dx * 6.0);
@@ -705,7 +593,7 @@ void dit_av_forward_dev(ltx_ctx* c, const void* v_latent, int v_dtype, const voi
     }
     GemmEpi e;
     e.mode = EPI_F32; e.out = out; e.ldo = Cout; e.bias = b;
-    gemm(c, tmp, Dx, w, Dx, rows, Cout, Dx, e, B);
+    linear(c, tmp, Dx, w, rows, Cout, Dx, e, o);
   };
   head(x, R, D, c->sst_out, vemb, v_rpr, h, c->w_out, c->b_out, g.out_channels, out_v_dev);
   head(ax, Ra, Da, av.sst_out, aemb, Ta, ah, av.w_out, av.b_out, Ca, out_a_dev);

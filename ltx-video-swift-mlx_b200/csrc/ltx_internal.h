@@ -162,10 +162,7 @@ void launch_gemm_fp8(const uint8_t* A, int64_t lda, const float* sa, const uint8
 // x bf16 [M, K] with row pitch ld (elements, multiple of 8; K % 16 == 0); q [M, K] (pitch K), s [M].
 void launch_quantize_rows_fp8(const bf16* x, int64_t ld, int M, int K, uint8_t* q, float* s, cudaStream_t stream);
 // ---------------------------------------------------------------- quantised weights (gemm_q.cu)
-enum QuantFormat : int {
-  QF_AFFINE = 0,   // per-64-group affine codes s * q + beta (8 or 4 bit): dequant-fused / panel kernels
-  QF_E4M3 = 1,     // e4m3 codes with one power-of-two scale per row (precision mode 8): the FP8 pair kernel
-};
+// affine codes (launch_gemm_q) or e4m3 codes (launch_gemm_fp8); which one is the LinearW's format (ctx.h)
 struct QuantW {
   const uint8_t* q = nullptr;    // [N, K] codes (8-bit, e4m3) or [N, K/2] packed nibbles (4-bit)
   const float* scales = nullptr; // affine: [K/64, N]; e4m3: [N]
@@ -174,7 +171,6 @@ struct QuantW {
   // optional bf16 [n, k] scratch panel shared by all quantised weights of a context: for M > 256 the weight is converted
   // once per GEMM into it (it stays in the 126 MB L2 for the D x D projections) and the bf16 pair kernel runs on the panel
   bf16* scratch = nullptr;
-  int fmt = QF_AFFINE;
 };
 // C[M,N] = A[M,K] * (s*q + beta)[N,K]^T with the epilogues of launch_gemm (group size 64)
 void launch_gemm_q(const bf16* A, int64_t lda, const QuantW& W, int M, int N, int K, const GemmEpi& epi, cudaStream_t stream,
