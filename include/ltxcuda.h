@@ -94,16 +94,35 @@ int ltx_load_tensor(ltx_ctx* ctx, const char* key, const void* host_data, ltx_dt
  * 5 = dual audio/video transformer (loadTransformerWeights(includeAudio: true), :605-639: the audio_*, av_ca_* and
  * cross-modal tensors are kept under their own names).  ltx_map_weight_key also accepts which = 6: a LoRA layer key ->
  * the model weight it patches (LoRAKeyMapper.loraKeyToModelKey, LoRA/LoRALoader.swift:209-243).
- * F32 / BF16 / F16 tensors are accepted.  n_loaded (nullable) receives the number of tensors taken.  Follow with
- * ltx_finalize_weights.  ltx_map_weight_key exposes the name mapping alone (no context, no GPU): it writes the mapped name,
- * or an empty string for a tensor the loader skips, into out[cap]. */
+ * F32 / BF16 / F16 tensors are accepted, and for which = 1 and 5 also scaled-FP8 Linears (the layout of ltx_load_tensor_e4m3,
+ * assumed from the ".weight_scale" / ".input_scale" side keys the reference's loader filters): "X.weight" in F8_E4M3
+ * (e4m3fn) [N, K] with "X.weight_scale" in F32 / BF16 of shape [] / [1] / [N] / [N, 1]; "X.input_scale" is ignored (FP8 mode
+ * quantises activations per token row at run time).  Mixed files are fine.  Refused with LTX_ERR_WEIGHTS: F8_E4M3 without a
+ * valid scale (or with a scale that is not finite and > 0), F8_E5M2, F8_E4M3 on anything but a 2-D transformer ".weight"
+ * (and in the VAE / encoder / upscaler files), NaN codes.  The whole header is validated before anything is uploaded; the NaN
+ * check runs during the upload, and a refused file leaves none of its tensors in the context.  n_loaded (nullable) receives
+ * the number of tensors taken.  Follow with ltx_finalize_weights.  ltx_map_weight_key exposes the name mapping alone (no
+ * context, no GPU): it writes the mapped name, or an empty string for a tensor the loader skips, into out[cap]. */
 int ltx_load_safetensors(ltx_ctx* ctx, const char* path, int which, int* n_loaded);
+/* The code-carrying twin of ltx_load_tensor, for callers that parse scaled-FP8 checkpoints themselves: the transformer Linear
+ * weight `key` (post-mapping name, ending in ".weight") of shape[ndim = 2] = [N, K] given as e4m3 (e4m3fn) codes[N * K] and
+ * fp32 scales[n_scales], n_scales = 1 (one scale per tensor) or N (one per output channel): w[n][k] = e4m3(code) * scale.
+ * bf16 and int8 / int4 modes store the decoded bf16 values (the rounding an fp32 file of w gets), fp32 mode the fp32 products.
+ * FP8 mode keeps the codes of the Linears inside the transformer blocks as they are, with their scales as the GEMM's row
+ * scales (no second rounding, half the bytes of bf16); the other Linears are decoded to bf16.  (The dual audio/video model
+ * has no FP8 mode; ltx_load_safetensors with which = 5 decodes its tensors in every mode.)  n_scales other than 1 or N, ndim != 2 or null pointers:
+ * LTX_ERR_INVALID_ARGUMENT; a key outside the transformer, a scale that is not finite and > 0, or a NaN code (0x7F / 0xFF,
+ * checked on the device; the tensor is then not loaded): LTX_ERR_WEIGHTS. */
+int ltx_load_tensor_e4m3(ltx_ctx* ctx, const char* key, const uint8_t* codes, const float* scales, int64_t n_scales,
+                         const int64_t* shape, int ndim);
 int ltx_map_weight_key(int which, const char* file_key, char* out, size_t cap);
 /* LoRA fuse at load time -- LoRAAdapter.fuseWeights (LoRA/LoRAAdapter.swift:64-166) with the delta of LoRAWeights.getDelta
  * (LoRA/LoRALoader.swift:162-178): W[out, in] += scale * up[out, rank] @ down[rank, in] on the loaded tensor `key` (post-mapping
  * name; ltx_map_weight_key(6, loraLayerKey) is LoRAKeyMapper.loraKeyToModelKey :209-243).  Call after loading the base weights
  * and BEFORE ltx_finalize_weights: quantisation then sees the merged weight (the reference dequantises, merges, requantises).
- * rank must be a multiple of 8; scale = user scale * alpha / rank as computed by the reference's loader. */
+ * rank must be a multiple of 8; scale = user scale * alpha / rank as computed by the reference's loader.  A weight held as
+ * e4m3 codes (FP8 mode, loaded from a scaled-FP8 checkpoint) is decoded to bf16 first and the delta added there; finalize then
+ * converts it by FP8 mode's per-row rule: "merge, then quantise", as for int8. */
 int ltx_fuse_lora(ltx_ctx* ctx, const char* key, const void* down, const void* up, ltx_dtype dtype, int rank, float scale);
 /* Precision of the DiT path.  16 (default): the reference's "bf16" mode -- bf16 weights and tensor-core operands, fp32
  * accumulation / residual stream / norms / softmax; velocity within rel-L2 1e-2 of the fp32 graph.  32: fp32 mode -- DiT
@@ -113,7 +132,10 @@ int ltx_fuse_lora(ltx_ctx* ctx, const char* key, const void* down, const void* u
  * (attn1 q|k|v and to_out, attn2 q, text k / v and to_out, FFN in / out) becomes e4m3 codes with one power-of-two scale per output channel (s = 2^ceil(log2(amax /
  * 448)), q = e4m3_rn_satfinite(w / s); the bf16 copies are freed, about half the DiT's weight bytes), and each of those GEMMs
  * quantises its activation rows by the same rule and runs e4m3 x e4m3 -> fp32 on the tensor cores (tcgen05 kind::f8f6f4),
- * scaled back per row and column before the bias.  Patchify, caption projection, timestep MLPs / AdaLN and proj_out stay bf16.
+ * scaled back per row and column before the bias.  Those Linears that arrive as e4m3 codes (a scaled-FP8 checkpoint through
+ * ltx_load_safetensors or ltx_load_tensor_e4m3) keep the file's codes and take the file's scale (per tensor, broadcast, or
+ * per output channel) as their row scale instead: nothing is rounded twice and no bf16 copy of them is ever made.
+ * Patchify, caption projection, timestep MLPs / AdaLN and proj_out stay bf16 (decoded when they arrive as codes).
  * FP8 mode refuses quant_bits != 16, sequence parallelism (pass groups are fine) and the dual audio/video model
  * (LTX_ERR_UNSUPPORTED).  Must be called before the DiT weights are loaded (8 after that: LTX_ERR_UNSUPPORTED); the VAE is
  * unaffected in every mode. */

@@ -51,6 +51,7 @@ SIGNATURES = {
     "ltx_last_error": (C.c_char_p, [_P]),
     "ltx_sync": (_I, [_P]),
     "ltx_load_tensor": (_I, [_P, C.c_char_p, _P, _I, C.POINTER(_I64), _I]),
+    "ltx_load_tensor_e4m3": (_I, [_P, C.c_char_p, _P, _P, _I64, C.POINTER(_I64), _I]),
     "ltx_load_safetensors": (_I, [_P, C.c_char_p, _I, C.POINTER(_I)]),
     "ltx_map_weight_key": (_I, [_I, C.c_char_p, C.c_char_p, _SZ]),
     "ltx_fuse_lora": (_I, [_P, C.c_char_p, _P, _P, _I, _I, _F]),

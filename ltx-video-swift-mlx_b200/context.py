@@ -207,6 +207,24 @@ class LtxContext:
         shape = (C.c_int64 * max(1, a.ndim))(*a.shape)
         self._check(self.lib.ltx_load_tensor(self.handle, key.encode(), _ptr(a), code, shape, a.ndim))
 
+    def load_tensor_e4m3(self, key: str, codes, scale):
+        """A transformer Linear weight [N, K] of a scaled-FP8 checkpoint: codes as a torch.float8_e4m3fn tensor or uint8 codes
+        (numpy or torch), scale one value (per tensor) or N values (per output channel); w = e4m3(code) * scale.  Decoded to the
+        mode's storage, or kept as codes for the block Linears in FP8 mode (ltx_load_tensor_e4m3)."""
+        if hasattr(codes, "detach"):
+            import torch
+            t = codes.detach().cpu().contiguous()
+            if t.dtype == torch.float8_e4m3fn:
+                t = t.view(torch.uint8)
+            codes = t.numpy()
+        q = np.ascontiguousarray(codes)
+        if q.dtype != np.uint8 or q.ndim != 2:
+            raise LtxError(2, "load_tensor_e4m3: codes must be a 2-D float8_e4m3fn or uint8 tensor")
+        s = np.ascontiguousarray(np.asarray(scale.detach().cpu().float() if hasattr(scale, "detach") else scale,
+                                            dtype=np.float32).reshape(-1))
+        shape = (C.c_int64 * 2)(*q.shape)
+        self._check(self.lib.ltx_load_tensor_e4m3(self.handle, key.encode(), _ptr(q), _ptr(s), s.size, shape, 2))
+
     def load_weights(self, weights: Dict[str, object], prefix: str = ""):
         for k, v in weights.items():
             self.load_tensor(prefix + k, v)

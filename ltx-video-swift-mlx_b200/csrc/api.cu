@@ -1,5 +1,6 @@
 // extern "C" surface of libltxcuda.so (include/ltxcuda.h).  Every entry point catches C++ exceptions and maps
 // them to the integer status + ltx_last_error() contract.
+#include <cmath>
 #include <cstring>
 
 #include "ctx.h"
@@ -244,7 +245,7 @@ int ltx_ctx_destroy(ltx_ctx* c) {
   graphs_clear(c);
   try { dist_destroy(c); } catch (...) {}
   for (auto& kv : c->tensors)
-    if (kv.second.ptr) cudaFree(kv.second.ptr);
+    kv.second.free_storage();
   for (void* p : c->owned) cudaFree(p);
   DevBuf* bufs[] = {&c->sp_send, &c->sp_recv, &c->sp_vt, &c->sp_vel, &c->api_lat, &c->api_ctx, &c->lat_in, &c->ctx_in, &c->ts_in, &c->mask_in, &c->x, &c->xb, &c->h, &c->qk, &c->vt, &c->att, &c->q2,
                     &c->ffh, &c->vel, &c->se, &c->t1, &c->emb, &c->ada, &c->c1, &c->c2, &c->rope_cos, &c->rope_sin,
@@ -377,6 +378,22 @@ int ltx_load_tensor(ltx_ctx* c, const char* key, const void* host_data, ltx_dtyp
   return guarded(c, [&] {
     LTX_CHECK(key != nullptr, LTX_ERR_INVALID_ARGUMENT, "null key");
     load_tensor_host(c, key, host_data, dtype, shape, ndim);
+  });
+}
+
+int ltx_load_tensor_e4m3(ltx_ctx* c, const char* key, const uint8_t* codes, const float* scales, int64_t n_scales,
+                         const int64_t* shape, int ndim) {
+  return guarded(c, [&] {
+    LTX_CHECK(key && codes && scales && shape && ndim == 2 && shape[0] > 0 && shape[1] > 0, LTX_ERR_INVALID_ARGUMENT,
+              "load_tensor_e4m3: bad arguments");
+    LTX_CHECK(n_scales == 1 || n_scales == shape[0], LTX_ERR_INVALID_ARGUMENT, "load_tensor_e4m3: n_scales must be 1 or shape[0]");
+    const std::string k = key;
+    const bool other_model = k.compare(0, 4, "vae.") == 0 || k.compare(0, 12, "vae_encoder.") == 0 || k.compare(0, 9, "upscaler.") == 0;
+    LTX_CHECK(!other_model && k.size() > 7 && k.compare(k.size() - 7, 7, ".weight") == 0, LTX_ERR_WEIGHTS,
+              "'" + k + "': e4m3 codes are only accepted for the weight of a transformer Linear");
+    for (int64_t i = 0; i < n_scales; ++i)
+      LTX_CHECK(std::isfinite(scales[i]) && scales[i] > 0.f, LTX_ERR_WEIGHTS, "'" + k + "': every scale must be finite and > 0");
+    load_tensor_e4m3_host(c, k, codes, scales, n_scales, shape, true);
   });
 }
 

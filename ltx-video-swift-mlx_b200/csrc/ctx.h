@@ -10,14 +10,27 @@
 
 namespace ltx {
 
+// Storage of a transformer Linear held as the e4m3 codes of a scaled-FP8 checkpoint (FP8 mode only; never an ltx_dtype): codes
+// [N, K] in ptr, fp32 row scales [N] in scales, w[n][k] = e4m3(code) * scales[n].  Two allocations: the scales appended to
+// the codes would push every codes allocation past a multiple of the allocator's 2 MB granule.
+constexpr int DT_E4M3 = 100;
+
 struct DevTensor {
   void* ptr = nullptr;
-  int dtype = LTX_F32;  // storage dtype on the device: LTX_BF16 or LTX_F32
+  int dtype = LTX_F32;     // storage dtype on the device: LTX_BF16, LTX_F32 or DT_E4M3
+  float* scales = nullptr; // DT_E4M3 only
   std::vector<int64_t> shape;
   int64_t numel() const {
     int64_t n = 1;
     for (auto d : shape) n *= d;
     return n;
+  }
+  const uint8_t* codes() const { return static_cast<const uint8_t*>(ptr); }
+  void free_storage() {
+    if (ptr) cudaFree(ptr);
+    if (scales) cudaFree(scales);
+    ptr = nullptr;
+    scales = nullptr;
   }
 };
 
@@ -55,7 +68,8 @@ struct DevBuf {
 enum LinearFormat : int {
   LW_BF16 = 0,     // w: bf16 [n, k] row-major
   LW_AFFINE = 1,   // q: per-64-group affine codes s * q + beta (8 or 4 bit): dequant-fused / panel kernels
-  LW_E4M3 = 2,     // q: e4m3 codes with one power-of-two scale per row (precision mode 8): the FP8 pair kernel
+  LW_E4M3 = 2,     // q: e4m3 codes with one fp32 scale per row (precision mode 8): the FP8 pair kernel.  A power of two when
+                   // dit_convert_fp8 made the codes, the checkpoint's scale when they were loaded from a scaled-FP8 file
 };
 struct LinearW {
   int fmt = LW_BF16;
@@ -428,6 +442,13 @@ int load_safetensors(ltx_ctx* c, const char* path, int which);
 // weights.cu
 const DevTensor& get_tensor(ltx_ctx* c, const std::string& key);
 void load_tensor_host(ltx_ctx* c, const std::string& key, const void* host, int dtype, const int64_t* shape, int ndim);
+// A transformer Linear [N, K] from e4m3 codes and fp32 scales (n_scales: 1 = per tensor, N = per output channel; validated by the
+// caller).  FP8 mode with keep_codes keeps the codes of the block Linears dit_convert_fp8 would convert (DT_E4M3); every other
+// case decodes to the storage dtype of the mode.  NaN codes: LTX_ERR_WEIGHTS, and the tensor is not left in the context.
+void load_tensor_e4m3_host(ltx_ctx* c, const std::string& key, const uint8_t* codes, const float* scales, int64_t n_scales,
+                           const int64_t* shape, bool keep_codes);
+// A DT_E4M3 tensor's codes decoded to bf16 storage in place (ltx_fuse_lora merges into the decoded values)
+void decode_e4m3_tensor(ltx_ctx* c, DevTensor& t);
 void init_random_weights(ltx_ctx* c, int which, uint64_t seed);
 void fuse_lora(ltx_ctx* c, const std::string& key, const void* down_host, const void* up_host, int dtype, int rank, float scale);
 std::string map_lora_key(const std::string& lora_key);

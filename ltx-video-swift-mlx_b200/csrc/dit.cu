@@ -136,7 +136,15 @@ const float* wf(ltx_ctx* c, const std::string& k, int64_t n) {
 }
 LinearW wlin(ltx_ctx* c, const std::string& k, int64_t n, int64_t kk) {
   LinearW w;
-  w.n = static_cast<int>(n); w.k = static_cast<int>(kk); w.w = wbf(c, k, n, kk);
+  w.n = static_cast<int>(n); w.k = static_cast<int>(kk);
+  const DevTensor& t = get_tensor(c, k);
+  if (t.dtype == DT_E4M3) {   // codes of a scaled-FP8 checkpoint, kept in FP8 mode
+    LTX_CHECK(t.shape.size() == 2 && t.shape[0] == n && t.shape[1] == kk, LTX_ERR_WEIGHTS, "bad shape for '" + k + "'");
+    w.fmt = LW_E4M3;
+    w.q.q = t.codes(); w.q.scales = t.scales; w.q.bits = 8; w.q.n = w.n; w.q.k = w.k;
+    return w;
+  }
+  w.w = wbf(c, k, n, kk);
   return w;
 }
 AdaLnW adaln_w(ltx_ctx* c, const std::string& p, int64_t dim, int n) {
@@ -355,33 +363,52 @@ void dit_finalize(ltx_ctx* c) {
     // attn1: pack q|k|v into one [3D, D] operand: the three projections of the block run as ONE GEMM (N = 3D; V leaves its
     // epilogue transposed); the other paths address the q|k rows (wq, N = 2D) and the v rows (wv) of the same buffer
     {
-      const bf16* wq = wbf(c, p + "attn1.to_q.weight", D, D);
-      const bf16* wk = wbf(c, p + "attn1.to_k.weight", D, D);
-      const bf16* wv = wbf(c, p + "attn1.to_v.weight", D, D);
+      const LinearW ws[3] = {wlin(c, p + "attn1.to_q.weight", D, D), wlin(c, p + "attn1.to_k.weight", D, D),
+                             wlin(c, p + "attn1.to_v.weight", D, D)};
       const float* bq = wf(c, p + "attn1.to_q.bias", D);
       const float* bk = wf(c, p + "attn1.to_k.bias", D);
       const float* bvv = wf(c, p + "attn1.to_v.bias", D);
-      bf16* wqkv = nullptr;
       float* bqkv = nullptr;
-      LTX_CUDA(cudaMalloc(&wqkv, static_cast<size_t>(3) * D * D * 2));
-      c->owned.push_back(wqkv);
       LTX_CUDA(cudaMalloc(&bqkv, static_cast<size_t>(3) * D * 4));
       c->owned.push_back(bqkv);
-      const bf16* ws[3] = {wq, wk, wv};
       const float* bs[3] = {bq, bk, bvv};
-      for (int t = 0; t < 3; ++t) {
-        LTX_CUDA(cudaMemcpyAsync(wqkv + static_cast<size_t>(t) * D * D, ws[t], static_cast<size_t>(D) * D * 2, cudaMemcpyDeviceToDevice, c->stream));
+      for (int t = 0; t < 3; ++t)
         LTX_CUDA(cudaMemcpyAsync(bqkv + static_cast<size_t>(t) * D, bs[t], static_cast<size_t>(D) * 4, cudaMemcpyDeviceToDevice, c->stream));
+      if (ws[0].fmt == LW_E4M3 || ws[1].fmt == LW_E4M3 || ws[2].fmt == LW_E4M3) {
+        // FP8 mode with sources held as e4m3 codes: the packed q|k|v is made as codes + row scales [3D] one [D, D] block per
+        // source -- codes and scales copied, a bf16 source converted by dit_convert_fp8's per-row rule (rows are independent)
+        uint8_t* q = nullptr;
+        float* s = nullptr;
+        LTX_CUDA(cudaMalloc(&q, static_cast<size_t>(3) * D * D));
+        LTX_CUDA(cudaMalloc(&s, static_cast<size_t>(3) * D * 4));
+        c->owned.push_back(q); c->owned.push_back(s);
+        for (int t = 0; t < 3; ++t) {
+          uint8_t* qt = q + static_cast<size_t>(t) * D * D;
+          if (ws[t].fmt == LW_E4M3) {
+            LTX_CUDA(cudaMemcpyAsync(qt, ws[t].q.q, static_cast<size_t>(D) * D, cudaMemcpyDeviceToDevice, c->stream));
+            LTX_CUDA(cudaMemcpyAsync(s + t * D, ws[t].q.scales, static_cast<size_t>(D) * 4, cudaMemcpyDeviceToDevice, c->stream));
+          } else {
+            launch_quantize_rows_fp8(ws[t].w, D, static_cast<int>(D), static_cast<int>(D), qt, s + t * D, c->stream);
+          }
+        }
+        b.a1.wq.fmt = LW_E4M3; b.a1.wq.n = 3 * D; b.a1.wq.k = D;
+        b.a1.wq.q.q = q; b.a1.wq.q.scales = s; b.a1.wq.q.bits = 8; b.a1.wq.q.n = 3 * D; b.a1.wq.q.k = D;
+      } else {
+        bf16* wqkv = nullptr;
+        LTX_CUDA(cudaMalloc(&wqkv, static_cast<size_t>(3) * D * D * 2));
+        c->owned.push_back(wqkv);
+        for (int t = 0; t < 3; ++t)
+          LTX_CUDA(cudaMemcpyAsync(wqkv + static_cast<size_t>(t) * D * D, ws[t].w, static_cast<size_t>(D) * D * 2, cudaMemcpyDeviceToDevice, c->stream));
+        b.a1.wq.n = 3 * D; b.a1.wq.k = D; b.a1.wq.w = wqkv;
+        b.a1.wv.n = D; b.a1.wv.k = D; b.a1.wv.w = wqkv + 2 * D * D;
       }
       LTX_CUDA(cudaStreamSynchronize(c->stream));
       // the unpacked copies are no longer needed
       for (const char* k : {"attn1.to_q.weight", "attn1.to_k.weight", "attn1.to_v.weight"}) {
         auto it = c->tensors.find(p + k);
-        cudaFree(it->second.ptr);
+        it->second.free_storage();
         c->tensors.erase(it);
       }
-      b.a1.wq.n = 3 * D; b.a1.wq.k = D; b.a1.wq.w = wqkv;
-      b.a1.wv.n = D; b.a1.wv.k = D; b.a1.wv.w = wqkv + 2 * D * D;
       b.a1.bq = bqkv; b.a1.bk = bqkv + D; b.a1.bv = bqkv + 2 * D;
     }
     b.a1.wo = wlin(c, p + "attn1.to_out.weight", D, D);
@@ -486,7 +513,8 @@ void dit_quantize(ltx_ctx* c, int bits) {
 
 // Precision mode 8: every Linear inside the transformer blocks becomes e4m3 codes with one power-of-two scale per output
 // channel (launch_quantize_rows_fp8: the rule linear() applies to the activation rows); the bf16 copies are freed.  Patchify,
-// caption projection, the timestep MLPs / AdaLN and proj_out stay bf16.
+// caption projection, the timestep MLPs / AdaLN and proj_out stay bf16.  Linears loaded as the codes of a scaled-FP8 checkpoint
+// (wlin: LW_E4M3 already) keep them and their scales.
 void dit_convert_fp8(ltx_ctx* c) {
   LTX_CHECK(c->dit_ready, LTX_ERR_WEIGHTS, "DiT weights not finalized");
   const ltx_config& g = c->cfg;
@@ -494,6 +522,7 @@ void dit_convert_fp8(ltx_ctx* c) {
   LTX_CHECK(D % 16 == 0 && FF % 16 == 0, LTX_ERR_INVALID_CONFIGURATION, "FP8 mode needs Linear widths that are multiples of 16");
   std::vector<const void*> to_free;
   auto conv = [&](LinearW& w) {
+    if (w.fmt == LW_E4M3) return;
     LTX_CHECK(w.fmt == LW_BF16, LTX_ERR_WEIGHTS, "FP8 conversion needs unquantised DiT weights");
     const int N = w.n, K = w.k;
     uint8_t* q = nullptr;

@@ -8,11 +8,18 @@
 // File format (safetensors): u64 little-endian header length, a flat JSON object {name: {"dtype", "shape", "data_offsets"}}
 // (+ "__metadata__"), then the raw little-endian tensor bytes.  The file is mmap'ed; each selected tensor goes through
 // load_tensor_host (H2D copy + the fp32 -> bf16 cast of :1005-1012 on the device).
+//
+// Scaled-FP8 transformer files (the convention the reference's ".weight_scale" / ".input_scale" filter implies, :617-629; no
+// such file was at hand, so anything else is refused rather than guessed at): a Linear weight "X.weight" in F8_E4M3 (e4m3fn)
+// of shape [N, K] with "X.weight_scale" beside it, F32 or BF16 of shape [] / [1] (per tensor) or [N] / [N, 1] (per output
+// channel), finite and > 0: w[n][k] = e4m3(code) * scale.  "X.input_scale" is ignored: FP8 mode quantises the activation rows
+// at run time.  Those go through load_tensor_e4m3_host.
 #include <fcntl.h>
 #include <sys/mman.h>
 #include <sys/stat.h>
 #include <unistd.h>
 
+#include <cmath>
 #include <cstring>
 
 #include "ctx.h"
@@ -180,6 +187,22 @@ struct MappedFile {
   }
 };
 
+// The header is untrusted input: bound the rank, reject negative dims and an element count that overflows, and only then
+// compare the byte count with the data offsets.  Returns the element count.
+uint64_t checked_numel(const std::string& key, const TensorInfo& t, size_t esz, uint64_t data_size) {
+  LTX_CHECK(t.shape.size() <= 8, LTX_ERR_WEIGHTS, "tensor '" + key + "': more than 8 dimensions");
+  LTX_CHECK(t.begin <= t.end && t.end <= data_size, LTX_ERR_WEIGHTS, "tensor '" + key + "': data_offsets outside the file");
+  const uint64_t span = t.end - t.begin;
+  uint64_t n_u = 1;
+  for (int64_t d : t.shape) {
+    LTX_CHECK(d >= 0, LTX_ERR_WEIGHTS, "tensor '" + key + "': negative dimension");
+    LTX_CHECK(d == 0 || n_u <= UINT64_MAX / static_cast<uint64_t>(d), LTX_ERR_WEIGHTS, "tensor '" + key + "': element count overflows");
+    n_u *= static_cast<uint64_t>(d);
+  }
+  LTX_CHECK(n_u <= span / esz && n_u * esz == span, LTX_ERR_WEIGHTS, "tensor '" + key + "': data_offsets do not match its shape");
+  return n_u;
+}
+
 }  // namespace
 
 // Transformer key of the checkpoint -> name the context expects, or "" when the tensor is not part of the video-only DiT.
@@ -310,7 +333,17 @@ int load_safetensors(ltx_ctx* c, const char* path, int which) {
   bool unified = false;
   if (which != 4)
     for (const auto& kv : header) unified = unified || starts_with(kv.first, want);
-  int loaded = 0;
+  const bool transformer = which == 1 || which == 5;
+  // Pass 1 validates every tensor the call takes (and pairs each e4m3 weight with its scale) before anything is uploaded, so a
+  // refused file loads nothing.
+  struct Item {
+    std::string name;
+    const uint8_t* bytes;
+    int dtype;                   // an ltx_dtype, or DT_E4M3: codes of a scaled-FP8 Linear
+    std::vector<int64_t> shape;
+    std::vector<float> scales;   // DT_E4M3: 1 (per tensor) or shape[0] (per output channel) values, finite and > 0
+  };
+  std::vector<Item> items;
   for (const auto& kv : header) {
     if (unified && !starts_with(kv.first, want)) continue;
     const std::string name = which == 1   ? map_transformer_key(kv.first)
@@ -320,35 +353,74 @@ int load_safetensors(ltx_ctx* c, const char* path, int which) {
                                           : map_transformer_key(kv.first, true);
     if (name.empty()) continue;
     const TensorInfo& t = kv.second;
-    int dtype;
-    size_t esz;
-    if (t.dtype == "F32") { dtype = LTX_F32; esz = 4; }
-    else if (t.dtype == "BF16") { dtype = LTX_BF16; esz = 2; }
-    else if (t.dtype == "F16") { dtype = LTX_F16; esz = 2; }
-    else LTX_CHECK(false, LTX_ERR_WEIGHTS, "tensor '" + kv.first + "' has unsupported dtype " + t.dtype);
-    // the header is untrusted input: bound the rank, reject negative dims and an element count that overflows, and only then
-    // compare the byte count with the (already range-checked) data offsets
-    LTX_CHECK(t.shape.size() <= 8, LTX_ERR_WEIGHTS, "tensor '" + kv.first + "': more than 8 dimensions");
-    LTX_CHECK(t.begin <= t.end && t.end <= data_size, LTX_ERR_WEIGHTS, "tensor '" + kv.first + "': data_offsets outside the file");
-    const uint64_t span = t.end - t.begin;
-    uint64_t n_u = 1;
-    for (int64_t d : t.shape) {
-      LTX_CHECK(d >= 0, LTX_ERR_WEIGHTS, "tensor '" + kv.first + "': negative dimension");
-      LTX_CHECK(d == 0 || n_u <= UINT64_MAX / static_cast<uint64_t>(d), LTX_ERR_WEIGHTS,
-                "tensor '" + kv.first + "': element count overflows");
-      n_u *= static_cast<uint64_t>(d);
+    Item it;
+    it.name = name;
+    it.dtype = DT_E4M3;
+    size_t esz = 1;
+    if (t.dtype == "F32") { it.dtype = LTX_F32; esz = 4; }
+    else if (t.dtype == "BF16") { it.dtype = LTX_BF16; esz = 2; }
+    else if (t.dtype == "F16") { it.dtype = LTX_F16; esz = 2; }
+    else LTX_CHECK(t.dtype == "F8_E4M3", LTX_ERR_WEIGHTS, "tensor '" + kv.first + "' has unsupported dtype " + t.dtype);
+    const uint64_t n_u = checked_numel(kv.first, t, esz, data_size);
+    if (it.dtype == DT_E4M3) {
+      // scaled FP8: only the 2-D weight of a transformer Linear, with its weight_scale beside it
+      LTX_CHECK(transformer && ends_with(kv.first, ".weight") && t.shape.size() == 2 && n_u > 0, LTX_ERR_WEIGHTS,
+                "tensor '" + kv.first + "': F8_E4M3 is only accepted for the 2-D weight of a transformer Linear");
+      const std::string skey = kv.first + "_scale";
+      const auto s = header.find(skey);
+      LTX_CHECK(s != header.end(), LTX_ERR_WEIGHTS, "tensor '" + kv.first + "': F8_E4M3 without '" + skey + "'");
+      const TensorInfo& st = s->second;
+      LTX_CHECK(st.dtype == "F32" || st.dtype == "BF16", LTX_ERR_WEIGHTS, "'" + skey + "': scale dtype must be F32 or BF16");
+      const int64_t N = t.shape[0];
+      const std::vector<int64_t>& ss = st.shape;
+      const bool per_tensor = ss.empty() || (ss.size() == 1 && ss[0] == 1);
+      const bool per_row = (ss.size() == 1 && ss[0] == N) || (ss.size() == 2 && ss[0] == N && ss[1] == 1);
+      LTX_CHECK(per_tensor || per_row, LTX_ERR_WEIGHTS, "'" + skey + "': scale shape must be [], [1], [N] or [N, 1]");
+      const size_t sesz = st.dtype == "F32" ? 4 : 2;
+      const uint64_t ns = checked_numel(skey, st, sesz, data_size);
+      const uint8_t* sp = data + st.begin;
+      for (uint64_t i = 0; i < ns; ++i) {
+        uint32_t u = 0;
+        if (sesz == 4) memcpy(&u, sp + 4 * i, 4);
+        else { uint16_t h; memcpy(&h, sp + 2 * i, 2); u = static_cast<uint32_t>(h) << 16; }
+        float v;
+        memcpy(&v, &u, 4);
+        LTX_CHECK(std::isfinite(v) && v > 0.f, LTX_ERR_WEIGHTS, "'" + skey + "': every scale must be finite and > 0");
+        it.scales.push_back(v);
+      }
     }
-    LTX_CHECK(n_u <= span / esz && n_u * esz == span, LTX_ERR_WEIGHTS,
-              "tensor '" + kv.first + "': data_offsets do not match its shape");
     if (n_u == 0) continue;   // empty tensor: nothing to load
     const int64_t n = static_cast<int64_t>(n_u);
-    std::vector<int64_t> shape = t.shape;
-    if (name == "vae.mean_of_means" || name == "vae.std_of_means") shape.assign(1, n);   // .squeezed() (:833, :837)
-    if (shape.empty()) shape.assign(1, 1);                                                  // scalars (timestep_scale_multiplier)
-    load_tensor_host(c, name, data + t.begin, dtype, shape.data(), static_cast<int>(shape.size()));
-    ++loaded;
+    it.bytes = data + t.begin;
+    it.shape = t.shape;
+    if (name == "vae.mean_of_means" || name == "vae.std_of_means") it.shape.assign(1, n);   // .squeezed() (:833, :837)
+    if (it.shape.empty()) it.shape.assign(1, 1);                                              // scalars (timestep_scale_multiplier)
+    items.push_back(std::move(it));
   }
-  return loaded;
+  // Pass 2 uploads.  The NaN check of e4m3 codes runs on the device during the upload; when it (or anything else) fails, every
+  // tensor this call loaded is removed again.
+  std::vector<std::string> done;
+  try {
+    for (const Item& it : items) {
+      if (it.dtype == DT_E4M3)
+        // the dual audio/video model has no FP8 mode: its tensors are always decoded
+        load_tensor_e4m3_host(c, it.name, it.bytes, it.scales.data(), static_cast<int64_t>(it.scales.size()), it.shape.data(),
+                              which == 1);
+      else
+        load_tensor_host(c, it.name, it.bytes, it.dtype, it.shape.data(), static_cast<int>(it.shape.size()));
+      done.push_back(it.name);
+    }
+  } catch (...) {
+    cudaStreamSynchronize(c->stream);
+    for (const std::string& k : done) {
+      auto t = c->tensors.find(k);
+      if (t == c->tensors.end()) continue;
+      t->second.free_storage();
+      c->tensors.erase(t);
+    }
+    throw;
+  }
+  return static_cast<int>(items.size());
 }
 
 }  // namespace ltx

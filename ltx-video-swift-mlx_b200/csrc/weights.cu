@@ -1,7 +1,12 @@
 // Weight ingestion for libltxcuda: host tensors under the reference's post-mapping key names
 // (Utils/ModelDownloader.swift:756-899) are copied to the device as bf16 (matrices / conv kernels, mirroring the
-// loader's fp32->bf16 cast at :1005-1012) or fp32 (biases, norm weights, scale-shift tables).
+// loader's fp32->bf16 cast at :1005-1012) or fp32 (biases, norm weights, scale-shift tables).  Transformer Linears of a
+// scaled-FP8 checkpoint (e4m3 codes + scales) are decoded on the device to the same storage, or kept as codes in FP8 mode.
 #include <cuda_fp16.h>
+#include <cuda_fp8.h>
+
+#include <cstring>
+#include <type_traits>
 
 #include "ctx.h"
 
@@ -43,6 +48,78 @@ void convert_to(const void* src, void* dst, int dst_dtype, int64_t n, cudaStream
   LTX_CUDA(cudaGetLastError());
 }
 
+// Scaled-FP8 decode: w[i] = e4m3(codes[i]) * scales[i / K] (K = n for one scale per tensor), stored as bf16
+// (__float2bfloat16_rn of the fp32 product: what an fp32 checkpoint of the same values gets) or as the fp32 product; D = void
+// only scans.  Every thread reads 16 codes per 16-byte load; the n % 16 tail is read byte by byte.  Each thread that met a NaN
+// code (0x7F / 0xFF) adds one to *nan_count.
+template <typename D>
+__global__ void decode_e4m3_kernel(const uint8_t* __restrict__ codes, const float* __restrict__ scales, int64_t K, int64_t n,
+                                   D* __restrict__ out, unsigned int* __restrict__ nan_count) {
+  const int64_t chunks = n / 16, stride = static_cast<int64_t>(gridDim.x) * blockDim.x;
+  const int64_t tid = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x;
+  bool nan = false;
+  auto value = [&](uint8_t b, float s) {
+    nan |= (b & 0x7F) == 0x7F;
+    return __half2float(__half(__nv_cvt_fp8_to_halfraw(b, __NV_E4M3))) * s;
+  };
+  for (int64_t t = tid; t < chunks; t += stride) {
+    const uint4 v = reinterpret_cast<const uint4*>(codes)[t];
+    const uint8_t* b = reinterpret_cast<const uint8_t*>(&v);
+    const int64_t e0 = t * 16;
+    int64_t row = e0 / K, col = e0 - row * K;
+    float s = scales[row];
+    float f[16];
+#pragma unroll
+    for (int j = 0; j < 16; ++j) {
+      if (col == K) { ++row; col = 0; s = scales[row]; }
+      f[j] = value(b[j], s);
+      ++col;
+    }
+    if constexpr (std::is_same<D, bf16>::value) {
+      alignas(16) bf16 h[16];
+#pragma unroll
+      for (int j = 0; j < 16; ++j) h[j] = __float2bfloat16_rn(f[j]);
+      uint4* o = reinterpret_cast<uint4*>(out + e0);
+      o[0] = reinterpret_cast<const uint4*>(h)[0];
+      o[1] = reinterpret_cast<const uint4*>(h)[1];
+    } else if constexpr (std::is_same<D, float>::value) {
+      float4* o = reinterpret_cast<float4*>(out + e0);
+#pragma unroll
+      for (int j = 0; j < 4; ++j) o[j] = make_float4(f[4 * j], f[4 * j + 1], f[4 * j + 2], f[4 * j + 3]);
+    }
+  }
+  for (int64_t i = chunks * 16 + tid; i < n; i += stride) {
+    const float f = value(codes[i], scales[i / K]);
+    if constexpr (std::is_same<D, bf16>::value) out[i] = __float2bfloat16_rn(f);
+    else if constexpr (std::is_same<D, float>::value) out[i] = f;
+  }
+  if (nan) atomicAdd(nan_count, 1u);
+}
+
+// codes / scales on the device (codes 16-byte aligned); out: bf16, fp32 or nullptr (scan only).  Returns how many threads met a
+// NaN code (0: none).
+unsigned int decode_e4m3(ltx_ctx* c, const uint8_t* codes, const float* scales, int64_t K, int64_t n, int out_dtype, void* out) {
+  unsigned int* nan_count = nullptr;
+  LTX_CUDA(cudaMalloc(&nan_count, sizeof(unsigned int)));
+  LTX_CUDA(cudaMemsetAsync(nan_count, 0, sizeof(unsigned int), c->stream));
+  int64_t blocks = (n / 16 + 255) / 256;
+  blocks = blocks < 1 ? 1 : blocks > 8192 ? 8192 : blocks;
+  const dim3 grid(static_cast<unsigned>(blocks)), block(256);
+  if (!out)
+    decode_e4m3_kernel<void><<<grid, block, 0, c->stream>>>(codes, scales, K, n, nullptr, nan_count);
+  else if (out_dtype == LTX_BF16)
+    decode_e4m3_kernel<bf16><<<grid, block, 0, c->stream>>>(codes, scales, K, n, static_cast<bf16*>(out), nan_count);
+  else
+    decode_e4m3_kernel<float><<<grid, block, 0, c->stream>>>(codes, scales, K, n, static_cast<float*>(out), nan_count);
+  LTX_CUDA(cudaGetLastError());
+  unsigned int h = 0;
+  LTX_CUDA(cudaMemcpyAsync(&h, nan_count, sizeof(h), cudaMemcpyDeviceToHost, c->stream));
+  LTX_CUDA(cudaStreamSynchronize(c->stream));
+  LTX_CUDA(cudaFree(nan_count));
+  c->launches += 1;
+  return h;
+}
+
 size_t dtype_size(int dt) { return dt == LTX_F32 ? 4 : 2; }
 
 bool ends_with(const std::string& s, const std::string& suf) {
@@ -58,19 +135,49 @@ int storage_dtype(const ltx_ctx* c, const std::string& key, int ndim) {
   return LTX_BF16;
 }
 
-DevTensor& alloc_tensor(ltx_ctx* c, const std::string& key, const std::vector<int64_t>& shape) {
+void erase_tensor(ltx_ctx* c, const std::string& key) {
   auto it = c->tensors.find(key);
-  if (it != c->tensors.end()) {
-    if (it->second.ptr) cudaFree(it->second.ptr);
-    c->tensors.erase(it);
-  }
+  if (it == c->tensors.end()) return;
+  it->second.free_storage();
+  c->tensors.erase(it);
+}
+
+// dtype -1: the storage dtype of the mode (storage_dtype)
+DevTensor& alloc_tensor(ltx_ctx* c, const std::string& key, const std::vector<int64_t>& shape, int dtype = -1) {
+  erase_tensor(c, key);
   DevTensor t;
   t.shape = shape;
-  t.dtype = storage_dtype(c, key, static_cast<int>(shape.size()));
-  size_t bytes = static_cast<size_t>(t.numel()) * dtype_size(t.dtype);
+  t.dtype = dtype >= 0 ? dtype : storage_dtype(c, key, static_cast<int>(shape.size()));
+  size_t bytes = static_cast<size_t>(t.numel()) * (t.dtype == DT_E4M3 ? 1 : dtype_size(t.dtype));
   LTX_CUDA(cudaMalloc(&t.ptr, bytes < 16 ? 16 : bytes));
-  return c->tensors[key] = t;
+  DevTensor& r = c->tensors[key] = t;
+  if (r.dtype == DT_E4M3) LTX_CUDA(cudaMalloc(&r.scales, static_cast<size_t>(shape[0]) * 4));
+  return r;
 }
+
+// The Linears FP8 mode runs on e4m3 codes (dit_convert_fp8): "transformer_blocks.<i>." + one of kLinears.
+bool fp8_block_linear(const std::string& key) {
+  static const char* kPrefix = "transformer_blocks.";
+  static const char* kLinears[] = {"attn1.to_q.weight", "attn1.to_k.weight", "attn1.to_v.weight", "attn1.to_out.weight",
+                                   "attn2.to_q.weight", "attn2.to_k.weight", "attn2.to_v.weight", "attn2.to_out.weight",
+                                   "ff.project_in.proj.weight", "ff.project_out.weight"};
+  const size_t np = strlen(kPrefix);
+  if (key.compare(0, np, kPrefix) != 0) return false;
+  size_t i = np;
+  while (i < key.size() && key[i] >= '0' && key[i] <= '9') ++i;
+  if (i == np || i >= key.size() || key[i] != '.') return false;
+  const std::string rest = key.substr(i + 1);
+  for (const char* l : kLinears)
+    if (rest == l) return true;
+  return false;
+}
+
+// device allocation freed on every exit path
+struct DevScratch {
+  void* p = nullptr;
+  explicit DevScratch(size_t bytes) { LTX_CUDA(cudaMalloc(&p, bytes)); }
+  ~DevScratch() { cudaFree(p); }
+};
 
 void fill(ltx_ctx* c, const std::string& key, const std::vector<int64_t>& shape, float stdv, float mean, uint64_t& seed) {
   DevTensor& t = alloc_tensor(c, key, shape);
@@ -113,6 +220,44 @@ void load_tensor_host(ltx_ctx* c, const std::string& key, const void* host, int 
     convert_to<__half>(stage, t.ptr, t.dtype, n, c->stream);
   LTX_CUDA(cudaStreamSynchronize(c->stream));
   LTX_CUDA(cudaFree(stage));
+}
+
+void load_tensor_e4m3_host(ltx_ctx* c, const std::string& key, const uint8_t* codes, const float* scales, int64_t n_scales,
+                           const int64_t* shape, bool keep_codes) {
+  const int64_t N = shape[0], K = shape[1], n = N * K;
+  unsigned int nan = 0;
+  if (keep_codes && c->precision == 8 && fp8_block_linear(key)) {
+    // the codes go straight into their final allocation; a per-tensor scale is broadcast to the row scales the GEMM reads
+    DevTensor& t = alloc_tensor(c, key, {N, K}, DT_E4M3);
+    std::vector<float> rows(static_cast<size_t>(N));
+    for (int64_t r = 0; r < N; ++r) rows[r] = scales[n_scales == 1 ? 0 : r];
+    LTX_CUDA(cudaMemcpyAsync(t.ptr, codes, static_cast<size_t>(n), cudaMemcpyHostToDevice, c->stream));
+    LTX_CUDA(cudaMemcpyAsync(t.scales, rows.data(), static_cast<size_t>(N) * 4, cudaMemcpyHostToDevice, c->stream));
+    nan = decode_e4m3(c, t.codes(), t.scales, K, n, 0, nullptr);
+  } else {
+    DevTensor& t = alloc_tensor(c, key, {N, K});
+    const size_t code_bytes = (static_cast<size_t>(n) + 15) / 16 * 16;   // the scales start 16-byte aligned
+    DevScratch stage(code_bytes + static_cast<size_t>(n_scales) * 4);
+    uint8_t* sc = static_cast<uint8_t*>(stage.p);
+    float* ss = reinterpret_cast<float*>(sc + code_bytes);
+    LTX_CUDA(cudaMemcpyAsync(sc, codes, static_cast<size_t>(n), cudaMemcpyHostToDevice, c->stream));
+    LTX_CUDA(cudaMemcpyAsync(ss, scales, static_cast<size_t>(n_scales) * 4, cudaMemcpyHostToDevice, c->stream));
+    nan = decode_e4m3(c, sc, ss, n_scales == 1 ? n : K, n, t.dtype, t.ptr);
+  }
+  if (nan) {
+    erase_tensor(c, key);
+    LTX_CHECK(false, LTX_ERR_WEIGHTS, "tensor '" + key + "': NaN e4m3 code (0x7F / 0xFF)");
+  }
+}
+
+void decode_e4m3_tensor(ltx_ctx* c, DevTensor& t) {
+  LTX_CHECK(t.dtype == DT_E4M3 && t.shape.size() == 2, LTX_ERR_WEIGHTS, "decode_e4m3_tensor: not an e4m3 matrix");
+  bf16* w = nullptr;
+  LTX_CUDA(cudaMalloc(&w, static_cast<size_t>(t.numel()) * 2));
+  decode_e4m3(c, t.codes(), t.scales, t.shape[1], t.numel(), LTX_BF16, w);
+  t.free_storage();
+  t.ptr = w;
+  t.dtype = LTX_BF16;
 }
 
 namespace {
@@ -180,7 +325,10 @@ void fuse_lora(ltx_ctx* c, const std::string& key, const void* down_host, const 
             "LoRA target '" + key + "' is not loaded (fuse before ltx_finalize_weights, after loading the base weights)");
   DevTensor& w = it->second;
   LTX_CHECK(w.shape.size() == 2 && rank > 0, LTX_ERR_INVALID_ARGUMENT, "LoRA: 2-D target and a positive rank");
+  // a weight held as e4m3 codes (FP8 mode, scaled-FP8 checkpoint) is merged in bf16 and converted again at finalize by the
+  // per-row rule: "merge, then quantise", as for int8
   LTX_CHECK(down_host && up_host && (dtype == LTX_F32 || dtype == LTX_BF16 || dtype == LTX_F16), LTX_ERR_INVALID_ARGUMENT, "LoRA: bad factors");
+  if (w.dtype == DT_E4M3) decode_e4m3_tensor(c, w);
   const int64_t out = w.shape[0], in = w.shape[1];
   // the tensor-core GEMM wants K (= rank) to be a multiple of 8: ranks such as 4 are zero-padded, which adds exact zeros
   const int64_t rpad = (static_cast<int64_t>(rank) + 7) / 8 * 8;
