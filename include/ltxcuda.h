@@ -322,6 +322,38 @@ int ltx_vae_decode_tiled_dev(ltx_ctx* ctx, const float* latent, int Fp, int Hp, 
                              const float* decode_noise, int causal, int tile_size, int tile_overlap, float* out_frames,
                              int* out_num_frames);
 
+/* 8-bit frames.  The value v of a sample is what the fp32 entry points return: clip01((x + 1) / 2).
+ *   LTX_FRAMES_RGB8: [F, H, W, 3] uint8, q = (uint8_t)(v * 255.0f) -- one fp32 multiply, then truncation.  This is
+ *                    tensorToImages (U/VideoExporter.swift:543-580: clip, x 255, to uint8) as SURVEY section 2 row 21
+ *                    describes it, with MLX's float -> uint8 cast; the rounding rule is taken from that description.
+ *   LTX_FRAMES_I420: planar 4:2:0, BT.709, limited range; per frame Y [H][W] | U [H/2][W/2] | V [H/2][W/2], frames one
+ *                    after another.  Y = rint(16 + 219 Y'), Y' = 0.2126 R + 0.7152 G + 0.0722 B per pixel;
+ *                    Cb = rint(128 + 224 (B_m - Y'_m) / 1.8556), Cr = rint(128 + 224 (R_m - Y'_m) / 1.5748), where m is
+ *                    the mean colour of the 2x2 cell (((p00 + p01) + p10) + p11) * 0.25 per component and Y'_m its luma.
+ *                    fp32 arithmetic, round to nearest, ties to even. */
+typedef enum { LTX_FRAMES_RGB8 = 1, LTX_FRAMES_I420 = 2 } ltx_frames_format;
+/* Bytes of F frames of H x W pixels in `format`; 0 for a bad format, a non-positive size, or odd H / W in I420.  Host only. */
+size_t ltx_frames_u8_bytes(int F, int H, int W, int format);
+/* decodeVideo -> tensorToImages (U/VideoExporter.swift:543-580) as one call: the arguments of ltx_vae_decode /
+ * ltx_vae_decode_tiled, and `out` holds ltx_frames_u8_bytes(frames, 32H', 32W', format) bytes.  The untiled decode writes
+ * the 8-bit frames from conv_out's epilogue (no fp32 frame buffer; a temporally sharded decode gathers the 8-bit planes);
+ * the tiled one converts after its blend and clip.  Same bytes as ltx_frames_to_u8 of the fp32 decode.  A bad format or
+ * out == NULL returns LTX_ERR_INVALID_ARGUMENT before anything is written.  _dev: device pointers, `out` 4-byte aligned. */
+int ltx_vae_decode_u8(ltx_ctx* ctx, const float* latent, int Fp, int Hp, int Wp, float timestep, const float* decode_noise,
+                      int causal, int format, uint8_t* out);
+int ltx_vae_decode_u8_dev(ltx_ctx* ctx, const float* latent, int Fp, int Hp, int Wp, float timestep,
+                          const float* decode_noise, int causal, int format, uint8_t* out);
+int ltx_vae_decode_tiled_u8(ltx_ctx* ctx, const float* latent, int Fp, int Hp, int Wp, float timestep,
+                            const float* decode_noise, int causal, int tile_size, int tile_overlap, int format, uint8_t* out,
+                            int* out_num_frames);
+int ltx_vae_decode_tiled_u8_dev(ltx_ctx* ctx, const float* latent, int Fp, int Hp, int Wp, float timestep,
+                                const float* decode_noise, int causal, int tile_size, int tile_overlap, int format,
+                                uint8_t* out, int* out_num_frames);
+/* tensorToImages (U/VideoExporter.swift:543-580) for frames already decoded: fp32 [F, H, W, 3] (clipped to [0, 1] first)
+ * -> `format`, the same arithmetic as the fused decode.  Refusals as above; I420 needs even H and W. */
+int ltx_frames_to_u8(ltx_ctx* ctx, const float* frames, int F, int H, int W, int format, uint8_t* out);
+int ltx_frames_to_u8_dev(ltx_ctx* ctx, const float* frames, int F, int H, int W, int format, uint8_t* out);
+
 /* VideoEncoder.callAsFunction (Models/VAE/VideoEncoder.swift:270-312), the encoder half of encodeImage
  * (Pipeline/LTXPipeline.swift:1902-1932): pixels [3, T, H, W] fp32 (the reference feeds [-1, 1]), H and W multiples of 32
  * -> latent mean [128, ceil(T/8), H/32, W/32] fp32 (T = 8k+1 frames -> k+1 latent frames; an image is T = 1).

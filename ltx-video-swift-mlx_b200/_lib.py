@@ -10,6 +10,7 @@ LIB_PATH = os.path.join(_HERE, "libltxcuda.so")
 
 LTX_F32, LTX_BF16, LTX_F16 = 0, 1, 2
 LTX_MAX_FLAG_BLOCKS = 64
+LTX_FRAMES_RGB8, LTX_FRAMES_I420 = 1, 2     # ltx_frames_format
 
 
 class LtxConfig(C.Structure):
@@ -82,6 +83,13 @@ SIGNATURES = {
     "ltx_vae_tiled_frames": (_I, [_I, _I, _I]),
     "ltx_vae_decode_tiled": (_I, [_P, _P, _I, _I, _I, _F, _P, _I, _I, _I, _P, _P]),
     "ltx_vae_decode_tiled_dev": (_I, [_P, _P, _I, _I, _I, _F, _P, _I, _I, _I, _P, _P]),
+    "ltx_frames_u8_bytes": (_SZ, [_I, _I, _I, _I]),
+    "ltx_vae_decode_u8": (_I, [_P, _P, _I, _I, _I, _F, _P, _I, _I, _P]),
+    "ltx_vae_decode_u8_dev": (_I, [_P, _P, _I, _I, _I, _F, _P, _I, _I, _P]),
+    "ltx_vae_decode_tiled_u8": (_I, [_P, _P, _I, _I, _I, _F, _P, _I, _I, _I, _I, _P, _P]),
+    "ltx_vae_decode_tiled_u8_dev": (_I, [_P, _P, _I, _I, _I, _F, _P, _I, _I, _I, _I, _P, _P]),
+    "ltx_frames_to_u8": (_I, [_P, _P, _I, _I, _I, _I, _P]),
+    "ltx_frames_to_u8_dev": (_I, [_P, _P, _I, _I, _I, _I, _P]),
     "ltx_vae_encode": (_I, [_P, _P, _I, _I, _I, _I, _P]),
     "ltx_vae_encode_dev": (_I, [_P, _P, _I, _I, _I, _I, _P]),
     "ltx_upscale_latent": (_I, [_P, _P, _I, _I, _I, _P]),

@@ -9,7 +9,8 @@ from typing import Dict, Optional, Sequence, Tuple
 import numpy as np
 
 from . import _lib
-from ._lib import LTX_BF16, LTX_F16, LTX_F32, LtxConfig, LtxDitFlags, LtxError, LtxStepParams
+from ._lib import (LTX_BF16, LTX_F16, LTX_F32, LTX_FRAMES_I420, LTX_FRAMES_RGB8, LtxConfig, LtxDitFlags, LtxError,
+                   LtxStepParams)
 
 
 @dataclass
@@ -82,6 +83,13 @@ def _dtype_code(a) -> int:
 
 def _ptr(a: Optional[np.ndarray]):
     return None if a is None else a.ctypes.data_as(C.c_void_p)
+
+
+def _frames_format(format) -> int:
+    """Frame format code from "rgb8" / "i420" or an ltx_frames_format code (other codes go to the library, which refuses them)."""
+    if isinstance(format, str):
+        return {"rgb8": LTX_FRAMES_RGB8, "i420": LTX_FRAMES_I420}[format.lower()]
+    return int(format)
 
 
 def make_flags(stg_blocks: Sequence[int] = (), skip_self_attn: bool = False, skip_ff: bool = False,
@@ -524,6 +532,72 @@ class LtxContext:
     def vae_decode_dev(self, latent_ptr: int, fhw, out_ptr: int, causal: bool = False):
         Fp, Hp, Wp = fhw
         self._check(self.lib.ltx_vae_decode_dev(self.handle, latent_ptr, Fp, Hp, Wp, -1.0, None, int(causal), out_ptr))
+
+    # ------------------------------------------------------------------ 8-bit frames (decodeVideo -> tensorToImages)
+    @staticmethod
+    def frames_u8_shape(F: int, H: int, W: int, format) -> Tuple[int, ...]:
+        """Array shape of 8-bit frames: RGB8 (F, H, W, 3); I420 (F, 3H/2, W) -- each frame's Y, U and V planes one after
+        another, the usual two-dimensional view of I420."""
+        return (F, H, W, 3) if _frames_format(format) == LTX_FRAMES_RGB8 else (F, H * 3 // 2, W)
+
+    def vae_decode_u8(self, latent, format="rgb8", timestep: Optional[float] = None, decode_noise=None, causal: bool = False,
+                      out: Optional[np.ndarray] = None) -> np.ndarray:
+        """vae_decode straight to 8-bit frames, written by conv_out's epilogue; format "rgb8" or "i420" (ltxcuda.h)."""
+        fmt = _frames_format(format)
+        lat = _host(latent, np.float32)
+        if lat.ndim == 5:
+            lat = lat[0]
+        Cc, Fp, Hp, Wp = lat.shape
+        lat = np.ascontiguousarray(lat)
+        nz = None if decode_noise is None else _host(decode_noise, np.float32)
+        shape = self.frames_u8_shape(8 * (Fp - 1) + 1, 32 * Hp, 32 * Wp, fmt)
+        if out is None:
+            out = np.empty(shape, dtype=np.uint8)
+        assert out.shape == shape and out.dtype == np.uint8 and out.flags["C_CONTIGUOUS"]
+        self._check(self.lib.ltx_vae_decode_u8(self.handle, _ptr(lat), Fp, Hp, Wp, -1.0 if timestep is None else float(timestep),
+                                               _ptr(nz), int(causal), fmt, _ptr(out)))
+        return out
+
+    def vae_decode_tiled_u8(self, latent, tile_size: int, tile_overlap: int = 1, format="rgb8",
+                            timestep: Optional[float] = None, decode_noise=None, causal: bool = False) -> np.ndarray:
+        """vae_decode_tiled, then the 8-bit conversion of the blended and clipped frames."""
+        fmt = _frames_format(format)
+        lat = _host(latent, np.float32)
+        if lat.ndim == 5:
+            lat = lat[0]
+        Cc, Fp, Hp, Wp = lat.shape
+        lat = np.ascontiguousarray(lat)
+        nz = None if decode_noise is None else np.ascontiguousarray(_host(decode_noise, np.float32).reshape(lat.shape))
+        nf = self.lib.ltx_vae_tiled_frames(Fp, int(tile_size), int(tile_overlap))
+        if nf <= 0:
+            raise LtxError(2, "temporal tile overlap must be in [0, tile size)")
+        out = np.empty(self.frames_u8_shape(nf, 32 * Hp, 32 * Wp, fmt), dtype=np.uint8)
+        got = C.c_int(0)
+        self._check(self.lib.ltx_vae_decode_tiled_u8(self.handle, _ptr(lat), Fp, Hp, Wp,
+                                                     -1.0 if timestep is None else float(timestep), _ptr(nz), int(causal),
+                                                     int(tile_size), int(tile_overlap), fmt, _ptr(out), C.byref(got)))
+        assert got.value == nf
+        return out
+
+    def vae_decode_u8_dev(self, latent_ptr: int, fhw, out_ptr: int, format="rgb8", causal: bool = False,
+                          timestep: Optional[float] = None, noise_ptr: Optional[int] = None):
+        """Device pointers; out_ptr holds ltx_frames_u8_bytes(8(F'-1)+1, 32H', 32W', format) bytes, 4-byte aligned."""
+        Fp, Hp, Wp = fhw
+        self._check(self.lib.ltx_vae_decode_u8_dev(self.handle, latent_ptr, Fp, Hp, Wp, -1.0 if timestep is None else float(timestep),
+                                                   noise_ptr, int(causal), _frames_format(format), out_ptr))
+
+    def frames_to_u8(self, frames, format="rgb8") -> np.ndarray:
+        """fp32 frames [F, H, W, 3] (clipped to [0, 1]) -> 8-bit frames, the arithmetic of the fused decode."""
+        fmt = _frames_format(format)
+        fr = _host(frames, np.float32)
+        F, H, W, _ = fr.shape
+        out = np.empty(self.frames_u8_shape(F, H, W, fmt), dtype=np.uint8)
+        self._check(self.lib.ltx_frames_to_u8(self.handle, _ptr(fr), F, H, W, fmt, _ptr(out)))
+        return out
+
+    def frames_to_u8_dev(self, frames_ptr: int, fhw, out_ptr: int, format="rgb8"):
+        F, H, W = fhw
+        self._check(self.lib.ltx_frames_to_u8_dev(self.handle, frames_ptr, F, H, W, _frames_format(format), out_ptr))
 
     # ------------------------------------------------------------------ VAE encoder / latent upscaler / AdaIN
     def vae_encode(self, pixels, normalize: bool = True) -> np.ndarray:

@@ -254,7 +254,7 @@ int ltx_ctx_destroy(ltx_ctx* c) {
                     &c->v_lat, &c->v_noise, &c->v_frames, &c->v_mix, &c->v_te, &c->v_split, &c->v_pad2, &c->snap_x, &c->s_ts, &c->f_asplit, &c->f_wsplit, &c->f_h,
                     &c->f_q, &c->f_k, &c->f_v, &c->f_att, &c->f_ffh, &c->f_ctx, &c->f_c1, &c->f_c2, &c->f_tk, &c->f_tv, &c->f_lat,
                     &c->f_bias, &c->q_panel, &c->gemm_ws, &c->u_part, &c->u_ab, &c->u_stats, &c->u_in, &c->u_out, &c->u_ref, &c->av.ws, &c->av.a_cos, &c->av.a_sin, &c->av.xv_cos, &c->av.xv_sin, &c->av_in[0], &c->av_in[1], &c->av_in[2], &c->av_in[3], &c->av_in[4], &c->av_in[5], &c->av_in[6], &c->av_in[7],
-                    &c->v_tile_lat, &c->v_tile_noise, &c->v_tile_frames, &c->s_alat, &c->s_avc, &c->s_avu, &c->s_actx_pos, &c->s_actx_neg, &c->s_alat_pair, &c->s_actx_pair};
+                    &c->v_tile_lat, &c->v_tile_noise, &c->v_tile_frames, &c->v_frames_f32, &c->s_alat, &c->s_avc, &c->s_avu, &c->s_actx_pos, &c->s_actx_neg, &c->s_alat_pair, &c->s_actx_pair};
   for (DevBuf* b : bufs) b->release();
   for (auto& t : c->text) { t.k.release(); t.vt.release(); t.bias.release(); }
   for (auto& t : c->av.text) { t.k.release(); t.vt.release(); t.bias.release(); }
@@ -1202,6 +1202,100 @@ int ltx_vae_decode_tiled(ltx_ctx* c, const float* latent, int Fp, int Hp, int Wp
     LTX_CHECK(got == nf, LTX_ERR_CUDA, "tiled decode frame count mismatch");
     if (out_num_frames) *out_num_frames = got;
     LTX_CUDA(cudaMemcpyAsync(out_frames, c->v_frames.ptr, static_cast<size_t>(got) * fe * 4, cudaMemcpyDeviceToHost, c->stream));
+    LTX_CUDA(cudaStreamSynchronize(c->stream));
+  });
+}
+
+// ---------------------------------------------------------------- 8-bit frames
+size_t ltx_frames_u8_bytes(int F, int H, int W, int format) { return frames_u8_bytes(F, H, W, format); }
+
+namespace {
+void check_u8_out(int format, const void* out) {
+  LTX_CHECK(format == LTX_FRAMES_RGB8 || format == LTX_FRAMES_I420, LTX_ERR_INVALID_ARGUMENT, "bad frame format");
+  LTX_CHECK(out != nullptr, LTX_ERR_INVALID_ARGUMENT, "no output buffer");
+}
+}  // namespace
+
+int ltx_vae_decode_u8_dev(ltx_ctx* c, const float* latent, int Fp, int Hp, int Wp, float timestep, const float* decode_noise,
+                          int causal, int format, uint8_t* out) {
+  return guarded(c, [&] {
+    check_u8_out(format, out);
+    vae_decode_dev(c, latent, Fp, Hp, Wp, timestep, decode_noise, causal, out, format);
+  });
+}
+
+int ltx_vae_decode_u8(ltx_ctx* c, const float* latent, int Fp, int Hp, int Wp, float timestep, const float* decode_noise,
+                      int causal, int format, uint8_t* out) {
+  return guarded(c, [&] {
+    check_u8_out(format, out);
+    LTX_CHECK(latent && Fp > 0 && Hp > 0 && Wp > 0, LTX_ERR_INVALID_ARGUMENT, "bad vae_decode arguments");
+    const size_t n = static_cast<size_t>(c->cfg.vae_latent_channels) * Fp * Hp * Wp;
+    h2d(c, c->v_lat, latent, n * 4);
+    const float* nz = nullptr;
+    if (timestep >= 0.f) {
+      LTX_CHECK(decode_noise != nullptr, LTX_ERR_INVALID_ARGUMENT, "decode_noise is required when timestep >= 0");
+      h2d(c, c->v_noise, decode_noise, n * 4);
+      nz = c->v_noise.as<float>();
+    }
+    const size_t bytes = frames_u8_bytes(8 * (Fp - 1) + 1, 32 * Hp, 32 * Wp, format);
+    c->v_frames.reserve(bytes);
+    vae_decode_dev(c, c->v_lat.as<float>(), Fp, Hp, Wp, timestep, nz, causal, c->v_frames.ptr, format);
+    LTX_CUDA(cudaMemcpyAsync(out, c->v_frames.ptr, bytes, cudaMemcpyDeviceToHost, c->stream));
+    LTX_CUDA(cudaStreamSynchronize(c->stream));
+  });
+}
+
+int ltx_vae_decode_tiled_u8_dev(ltx_ctx* c, const float* latent, int Fp, int Hp, int Wp, float timestep, const float* decode_noise,
+                                int causal, int tile_size, int tile_overlap, int format, uint8_t* out, int* out_num_frames) {
+  return guarded(c, [&] {
+    check_u8_out(format, out);
+    const int n = vae_decode_tiled_dev(c, latent, Fp, Hp, Wp, timestep, decode_noise, causal, tile_size, tile_overlap, out, format);
+    if (out_num_frames) *out_num_frames = n;
+  });
+}
+
+int ltx_vae_decode_tiled_u8(ltx_ctx* c, const float* latent, int Fp, int Hp, int Wp, float timestep, const float* decode_noise,
+                            int causal, int tile_size, int tile_overlap, int format, uint8_t* out, int* out_num_frames) {
+  return guarded(c, [&] {
+    check_u8_out(format, out);
+    LTX_CHECK(latent && Fp > 0 && Hp > 0 && Wp > 0, LTX_ERR_INVALID_ARGUMENT, "bad vae_decode arguments");
+    const int nf = ltx_vae_tiled_frames(Fp, tile_size, tile_overlap);
+    LTX_CHECK(nf > 0, LTX_ERR_INVALID_ARGUMENT, "temporal tile overlap must be in [0, tile size)");
+    const size_t n = static_cast<size_t>(c->cfg.vae_latent_channels) * Fp * Hp * Wp;
+    h2d(c, c->v_lat, latent, n * 4);
+    const float* nz = nullptr;
+    if (timestep >= 0.f) {
+      LTX_CHECK(decode_noise != nullptr, LTX_ERR_INVALID_ARGUMENT, "decode_noise is required when timestep >= 0");
+      h2d(c, c->v_noise, decode_noise, n * 4);
+      nz = c->v_noise.as<float>();
+    }
+    const size_t bytes = frames_u8_bytes(nf, 32 * Hp, 32 * Wp, format);
+    c->v_frames.reserve(bytes);
+    const int got = vae_decode_tiled_dev(c, c->v_lat.as<float>(), Fp, Hp, Wp, timestep, nz, causal, tile_size, tile_overlap,
+                                         c->v_frames.ptr, format);
+    LTX_CHECK(got == nf, LTX_ERR_CUDA, "tiled decode frame count mismatch");
+    if (out_num_frames) *out_num_frames = got;
+    LTX_CUDA(cudaMemcpyAsync(out, c->v_frames.ptr, bytes, cudaMemcpyDeviceToHost, c->stream));
+    LTX_CUDA(cudaStreamSynchronize(c->stream));
+  });
+}
+
+int ltx_frames_to_u8_dev(ltx_ctx* c, const float* frames, int F, int H, int W, int format, uint8_t* out) {
+  return guarded(c, [&] {
+    check_u8_out(format, out);
+    frames_to_u8_dev(c, frames, F, H, W, format, out);
+  });
+}
+
+int ltx_frames_to_u8(ltx_ctx* c, const float* frames, int F, int H, int W, int format, uint8_t* out) {
+  return guarded(c, [&] {
+    check_u8_out(format, out);
+    const size_t bytes = frames_u8_bytes(F, H, W, format);
+    LTX_CHECK(frames != nullptr && bytes > 0, LTX_ERR_INVALID_ARGUMENT, "frames_to_u8: bad size or buffer (I420 needs even H and W)");
+    h2d(c, c->v_frames_f32, frames, static_cast<size_t>(F) * H * W * 3 * 4);
+    c->v_frames.reserve(bytes);
+    frames_to_u8_dev(c, c->v_frames_f32.as<float>(), F, H, W, format, c->v_frames.as<uint8_t>());
+    LTX_CUDA(cudaMemcpyAsync(out, c->v_frames.ptr, bytes, cudaMemcpyDeviceToHost, c->stream));
     LTX_CUDA(cudaStreamSynchronize(c->stream));
   });
 }

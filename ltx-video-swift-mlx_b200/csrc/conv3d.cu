@@ -17,6 +17,7 @@
 // than the rest, so those two choices never look at T (a temporal shard must round like the whole clip).
 #include <cstdlib>
 
+#include "frames_u8.cuh"
 #include "gemm_epilogue.cuh"
 #include "ltx_internal.h"
 #include "ptx.cuh"
@@ -121,6 +122,62 @@ __device__ __forceinline__ void conv_epilogue_chunk(const uint32_t (&r)[32], int
       const int c = co >> 4, pa = (co >> 2) & 3, pb = co & 3;
       const float v = (__uint_as_float(r[j]) + ep.bias[co] + 1.0f) * 0.5f;
       ep.out[((static_cast<int64_t>(t) * Ho + (4 * h + pb)) * Wo + (4 * w + pa)) * 3 + c] = ep.no_clip ? v : clip01(v);
+    }
+  }
+}
+
+// Modes 5 / 6: the voxel's 48 conv channels are 3 colours x one 4x4 pixel block (co = c*16 + pa*4 + pb -> pixel row pb,
+// column pa); r0 holds channels 0-31, r1 channels 32-47.  The values are mode 2's, clipped; the block is four whole 2x2
+// chroma cells, so I420 needs nothing from a neighbouring voxel.
+template <int MODE>
+__device__ __forceinline__ void conv_store_frames_u8(const uint32_t (&r0)[32], const uint32_t (&r1)[32], int t, int h, int w,
+                                                     const ConvGeom& g, const ConvEpi& ep) {
+  const int Ho = 4 * g.H, Wo = 4 * g.W;
+  float px[4][4][3];   // [row pb][column pa][colour]
+#pragma unroll
+  for (int co = 0; co < 48; ++co) {
+    const float v = (__uint_as_float(co < 32 ? r0[co] : r1[co - 32]) + ep.bias[co] + 1.0f) * 0.5f;
+    px[co & 3][(co >> 2) & 3][co >> 4] = clip01(v);
+  }
+  if (MODE == CONV_EPI_RGB8) {
+#pragma unroll
+    for (int pb = 0; pb < 4; ++pb) {   // 12 bytes per pixel row: 3 aligned words
+      uint32_t b[12];
+#pragma unroll
+      for (int i = 0; i < 12; ++i) b[i] = rgb8_code(px[pb][i / 3][i % 3]);
+      uint32_t* o = reinterpret_cast<uint32_t*>(ep.out_u8 + ((static_cast<int64_t>(t) * Ho + 4 * h + pb) * Wo + 4 * w) * 3);
+#pragma unroll
+      for (int k = 0; k < 3; ++k) o[k] = b[4 * k] | (b[4 * k + 1] << 8) | (b[4 * k + 2] << 16) | (b[4 * k + 3] << 24);
+    }
+  } else {
+    const int64_t plane = static_cast<int64_t>(Ho) * Wo;
+    uint8_t* yp = ep.out_u8 + static_cast<int64_t>(t) * (plane + plane / 2);
+    uint8_t* up = yp + plane;
+    uint8_t* vp = up + plane / 4;
+    uint32_t y[4][4], cb[2][2], cr[2][2];
+#pragma unroll
+    for (int cy = 0; cy < 2; ++cy)
+#pragma unroll
+      for (int cx = 0; cx < 2; ++cx) {
+        float p[4][3];
+        uint32_t yc[4];
+#pragma unroll
+        for (int i = 0; i < 4; ++i)
+#pragma unroll
+          for (int c = 0; c < 3; ++c) p[i][c] = px[2 * cy + (i >> 1)][2 * cx + (i & 1)][c];
+        i420_cell(p, yc, cb[cy][cx], cr[cy][cx]);
+#pragma unroll
+        for (int i = 0; i < 4; ++i) y[2 * cy + (i >> 1)][2 * cx + (i & 1)] = yc[i];
+      }
+#pragma unroll
+    for (int pb = 0; pb < 4; ++pb)
+      *reinterpret_cast<uint32_t*>(yp + static_cast<int64_t>(4 * h + pb) * Wo + 4 * w) =
+          y[pb][0] | (y[pb][1] << 8) | (y[pb][2] << 16) | (y[pb][3] << 24);
+#pragma unroll
+    for (int cy = 0; cy < 2; ++cy) {
+      const int64_t off = static_cast<int64_t>(2 * h + cy) * (Wo / 2) + 2 * w;
+      *reinterpret_cast<uint16_t*>(up + off) = static_cast<uint16_t>(cb[cy][0] | (cb[cy][1] << 8));
+      *reinterpret_cast<uint16_t*>(vp + off) = static_cast<uint16_t>(cr[cy][0] | (cr[cy][1] << 8));
     }
   }
 }
@@ -444,6 +501,13 @@ __device__ __forceinline__ void conv3d_body(const CUtensorMap& tmX, const CUtens
               *reinterpret_cast<uint4*>(dst + c * 32 + q4 * 8) = make_uint4(pk[4 * q4], pk[4 * q4 + 1], pk[4 * q4 + 2], pk[4 * q4 + 3]);
           }
         }
+      } else if (MODE == CONV_EPI_RGB8 || MODE == CONV_EPI_I420) {
+        // the first column chunk stays in registers until the second (channels 32-47) is in: one voxel = one whole pixel block
+        uint32_t r0[32], r1[32];
+        tmem_ld32(taddr, r0);
+        tmem_ld32(taddr + 32, r1);
+        tmem_ld_wait();
+        if (valid) conv_store_frames_u8<MODE>(r0, r1, vt, vh, vw, g, ep);
       } else {
 #pragma unroll 1
         for (int c = 0; c < BN / 32; ++c) {
@@ -732,6 +796,16 @@ void conv_launch_mode(const CUtensorMap& tmX, const CUtensorMap& tmW, const Conv
     case 2: conv_launch<BN, 2>(tmX, tmW, g, ep, s, pair); break;
     case 3: conv_launch<BN, 3>(tmX, tmW, g, ep, s, pair); break;
     case 4: conv_launch<BN, 4>(tmX, tmW, g, ep, s, pair); break;
+    case CONV_EPI_RGB8:
+    case CONV_EPI_I420:
+      // Cout = 48 always plans 64-wide tiles: the 8-bit stores are only instantiated there
+      if constexpr (BN == 64) {
+        if (ep.mode == CONV_EPI_RGB8) conv_launch<BN, CONV_EPI_RGB8>(tmX, tmW, g, ep, s, pair);
+        else conv_launch<BN, CONV_EPI_I420>(tmX, tmW, g, ep, s, pair);
+      } else {
+        LTX_CHECK(false, 2, "conv3d: 8-bit frame stores need 64-wide tiles");
+      }
+      break;
     default: LTX_CHECK(false, 2, "bad conv epilogue mode");
   }
 }
@@ -805,8 +879,11 @@ void launch_conv3d(const bf16* x_pad, const bf16* w, int T, int H, int W, int Ci
   LTX_CHECK(T > 0 && H > 1 && W > 1, 2, "conv3d: bad volume (reflect padding needs H, W >= 2)");
   LTX_CHECK(ntaps == 27 || ntaps == 9, 2, "conv3d: 27 taps (3x3x3) or 9 taps (per-frame 3x3)");
   LTX_CHECK(Cin > 0 && Cin % 64 == 0 && Cout > 0, 2, "conv3d: Cin must be a positive multiple of 64");
-  LTX_CHECK(epi.mode >= 0 && epi.mode <= 4, 2, "bad conv epilogue mode");
-  LTX_CHECK(epi.mode == 3 || epi.out != nullptr, 2, "conv3d: no output buffer");
+  LTX_CHECK(epi.mode >= 0 && epi.mode <= CONV_EPI_I420, 2, "bad conv epilogue mode");
+  const bool u8 = epi.mode == CONV_EPI_RGB8 || epi.mode == CONV_EPI_I420;
+  LTX_CHECK(epi.mode == 3 || (u8 ? epi.out_u8 != nullptr : epi.out != nullptr), 2, "conv3d: no output buffer");
+  LTX_CHECK(!u8 || (Cout == 48 && ntaps == 27 && reinterpret_cast<uintptr_t>(epi.out_u8) % 4 == 0), 2,
+            "conv3d: 8-bit frame stores need Cout = 48 and a 4-byte aligned output");
   LTX_CHECK(epi.mode != 0 || Cout % 4 == 0, 2, "conv3d: Cout must be a multiple of 4");
   LTX_CHECK(epi.mode != 1 || (Cout % 32 == 0 && Cin % 8 == 0 && epi.resid != nullptr && (epi.t_shift == 0 || epi.t_shift == 1)), 2,
             "conv3d: bad d2s configuration");

@@ -302,6 +302,7 @@ struct ltx_ctx {
   // ---- VAE workspaces
   ltx::DevBuf v_a, v_b, v_h, v_pad, v_lat, v_noise, v_frames, v_mix, v_te, v_split, v_pad2;
   ltx::DevBuf v_tile_lat, v_tile_noise, v_tile_frames;   // temporally tiled decode: one gathered chunk and its frames
+  ltx::DevBuf v_frames_f32;   // fp32 frames before the 8-bit conversion (tiled u8 decode, host-buffer ltx_frames_to_u8)
   int vae_no_clip = 0;                                    // conv_out stores (x+1)/2 unclipped (tiles are clipped after blending)
   ltx::DevBuf av_in[8];   // host-API staging of the dual model's inputs / outputs
   ltx::DevBuf u_part, u_ab, u_stats, u_in, u_out, u_ref;   // encoder / upscaler / AdaIN scratch and host-API staging
@@ -401,16 +402,23 @@ void dit_forward_f32(ltx_ctx* c, const void* latent, int latent_dtype, const voi
 // vae.cu
 void vae_finalize(ltx_ctx* c);
 int vae_tiled_frames(int Fp, int tile_size, int overlap);
+// Output formats of the decode: FRAMES_F32 = fp32 [F, H, W, 3] in [0, 1]; otherwise LTX_FRAMES_RGB8 / LTX_FRAMES_I420.
+constexpr int FRAMES_F32 = 0;
+// bytes of F frames of H x W in an 8-bit format; 0 for a bad format or size (I420: H and W even)
+size_t frames_u8_bytes(int64_t F, int64_t H, int64_t W, int format);
+// fp32 frames [F, H, W, 3] (clipped to [0, 1] on the way) -> 8-bit frames; the arithmetic of the fused conv_out store
+void frames_to_u8_dev(ltx_ctx* c, const float* frames_dev, int F, int H, int W, int format, uint8_t* out_dev);
 // returns the number of frames written
 int vae_decode_tiled_dev(ltx_ctx* c, const float* latent_dev, int Fp, int Hp, int Wp, float timestep, const float* noise_dev,
-                         int causal, int tile_size, int tile_overlap, float* frames_dev);
+                         int causal, int tile_size, int tile_overlap, void* frames_dev, int format = FRAMES_F32);
 void vae_decode_dev(ltx_ctx* c, const float* latent_dev, int Fp, int Hp, int Wp, float timestep, const float* noise_dev,
-                    int causal, float* frames_dev);
+                    int causal, void* frames_dev, int format = FRAMES_F32);
 ConvW vae_pack_conv_keys(ltx_ctx* c, const std::string& wkey, const std::string& bkey, int64_t cout, int64_t cin,
                          int64_t cout_use, int taps);
 const float* vae_vec(ltx_ctx* c, const std::string& key, int64_t n);
+// out: fp32, or the 8-bit frames of epilogue modes CONV_EPI_RGB8 / CONV_EPI_I420
 void vae_conv(ltx_ctx* c, const float* x, int prep_mode, const float* a, const float* b, const ConvW& w, int T, int H, int W,
-              int pad, int epi_mode, float* out, const float* resid, int n_active = 1, int t_shift = 0);
+              int pad, int epi_mode, void* out, const float* resid, int n_active = 1, int t_shift = 0);
 // vae_extra.cu: VAE encoder (V/VideoEncoder.swift), latent upscaler (Models/Upscaler/SpatialUpscaler.swift), AdaIN, re-noise
 void vae_encoder_finalize(ltx_ctx* c);
 void vae_encode_dev(ltx_ctx* c, const float* pixels_dev, int T, int H, int W, int normalize, float* latent_dev);

@@ -257,6 +257,7 @@ void launch_fill_normal_f32(float* p, int64_t n, float std, float mean, uint64_t
 // ---------------------------------------------------------------- VAE kernels (conv3d.cu)
 struct ConvEpi {
   int mode;                 // 0: out_f32 = acc + bias (+ resid) ; 1: depth-to-space scatter (+ tiled d2s residual) ; 2: unpatchify+clip to frames
+                            // 3 / 4: hand-over to the next conv (below) ; 5 / 6: unpatchify+clip to 8-bit frames (below)
   float* out;               // mode 0: [T,H,W,Cout] fp32 ; mode 1: [2T-1,2H,2W,Cout/8] fp32 ; mode 2: [T,4H,4W,3] fp32
   const float* bias;        // [Cout]
   const float* resid;       // mode 0: nullable [T,H,W,Cout] ; mode 1: conv input x fp32 [T,H,W,Cin]
@@ -274,7 +275,11 @@ struct ConvEpi {
   const float* next_shift = nullptr;
   int next_tshift = 1;
   int no_clip = 0;          // mode 2: store (x+1)/2 unclipped (temporal tiles are blended before the clip)
+  // modes 5 / 6: the values of mode 2, clipped, stored as 8-bit frames (frames_u8.cuh) -- 5: RGB8 [T,4H,4W,3];
+  // 6: I420, per frame Y [4H][4W] | U [2H][2W] | V [2H][2W].  Needs Cout = 48 in one tile and a 4-byte aligned out_u8.
+  uint8_t* out_u8 = nullptr;
 };
+enum { CONV_EPI_RGB8 = 5, CONV_EPI_I420 = 6 };
 // x_pad: bf16 [T+2, H+2, W+2, Cin] (already padded), w: bf16 [ntaps][Cout][Cin]; 3x3x3 cross-correlation (ntaps = 27) or a
 // per-frame 3x3 one (ntaps = 9: only the dt = 1 taps, the upscaler's Conv2d).
 bool conv3d_wants_tap_split(int H, int W, int Cin, int Cout);

@@ -5,6 +5,7 @@
 // bf16 padded copy produced by the fused pixel-norm/scale-shift/SiLU prologue and writes fp32 through its epilogue
 // (+bias, +residual, depth-to-space scatter, or unpatchify+clip straight into the [F, H, W, 3] frame buffer).
 #include "ctx.h"
+#include "frames_u8.cuh"
 
 namespace ltx {
 
@@ -56,7 +57,56 @@ __global__ void clip01_kernel(float* __restrict__ x, int64_t n4) {
   }
 }
 
+// fp32 frames -> 8-bit frames (frames_u8.cuh), the converter beside the fused conv_out store: one sample (RGB8) or one 2x2
+// chroma cell (I420) per thread and iteration
+__global__ void frames_rgb8_kernel(const float* __restrict__ x, uint8_t* __restrict__ out, int64_t n) {
+  for (int64_t i = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x; i < n; i += static_cast<int64_t>(gridDim.x) * blockDim.x)
+    out[i] = static_cast<uint8_t>(rgb8_code(fminf(fmaxf(x[i], 0.f), 1.f)));
+}
+__global__ void frames_i420_kernel(const float* __restrict__ x, uint8_t* __restrict__ out, int F, int H, int W) {
+  const int Hc = H / 2, Wc = W / 2;
+  const int64_t plane = static_cast<int64_t>(H) * W, ncell = static_cast<int64_t>(F) * Hc * Wc;
+  for (int64_t i = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x; i < ncell; i += static_cast<int64_t>(gridDim.x) * blockDim.x) {
+    const int cx = static_cast<int>(i % Wc), cy = static_cast<int>((i / Wc) % Hc);
+    const int64_t f = i / (static_cast<int64_t>(Wc) * Hc);
+    float p[4][3];
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+      const float* src = x + ((f * H + 2 * cy + (k >> 1)) * W + 2 * cx + (k & 1)) * 3;
+#pragma unroll
+      for (int c = 0; c < 3; ++c) p[k][c] = fminf(fmaxf(src[c], 0.f), 1.f);
+    }
+    uint32_t y[4], cb, cr;
+    i420_cell(p, y, cb, cr);
+    uint8_t* yp = out + f * (plane + plane / 2);
+#pragma unroll
+    for (int k = 0; k < 4; ++k) yp[static_cast<int64_t>(2 * cy + (k >> 1)) * W + 2 * cx + (k & 1)] = static_cast<uint8_t>(y[k]);
+    const int64_t off = static_cast<int64_t>(cy) * Wc + cx;
+    yp[plane + off] = static_cast<uint8_t>(cb);
+    yp[plane + plane / 4 + off] = static_cast<uint8_t>(cr);
+  }
+}
+
 }  // namespace
+
+size_t frames_u8_bytes(int64_t F, int64_t H, int64_t W, int format) {
+  if (F <= 0 || H <= 0 || W <= 0) return 0;
+  if (format == LTX_FRAMES_RGB8) return static_cast<size_t>(F * H * W * 3);
+  if (format == LTX_FRAMES_I420 && H % 2 == 0 && W % 2 == 0) return static_cast<size_t>(F * (H * W + H * W / 2));
+  return 0;
+}
+
+void frames_to_u8_dev(ltx_ctx* c, const float* frames_dev, int F, int H, int W, int format, uint8_t* out_dev) {
+  const size_t bytes = frames_u8_bytes(F, H, W, format);
+  LTX_CHECK(bytes > 0 && frames_dev != nullptr && out_dev != nullptr, LTX_ERR_INVALID_ARGUMENT,
+            "frames_to_u8: bad format, size or buffer (I420 needs even H and W)");
+  const int64_t work = format == LTX_FRAMES_RGB8 ? static_cast<int64_t>(bytes) : static_cast<int64_t>(F) * (H / 2) * (W / 2);
+  const int grid = static_cast<int>(std::min<int64_t>((work + 255) / 256, 148 * 16));
+  ProfScope ps(c, PROF_OTHER, 0.0, 4.0 * F * H * W * 3 + static_cast<double>(bytes));
+  if (format == LTX_FRAMES_RGB8) frames_rgb8_kernel<<<grid, 256, 0, c->stream>>>(frames_dev, out_dev, work);
+  else frames_i420_kernel<<<grid, 256, 0, c->stream>>>(frames_dev, out_dev, F, H, W);
+  LTX_CUDA(cudaGetLastError());
+}
 
 // Repacks a conv kernel stored in the checkpoint layout (O, I, 3, 3, 3) -- or (O, I, 3, 3) for the per-frame Conv2d of the
 // upscaler -- into the implicit GEMM's [taps][Cout][Cin] bf16 matrix.  cout_use < cout keeps the leading output channels
@@ -109,7 +159,7 @@ const float* vae_vec(ltx_ctx* c, const std::string& k, int64_t n) {
 // pad: VAE_PAD_* bits.  n_active > 1: this rank holds a temporal slab; the two time-padding frames of the conv input come
 // from the neighbouring ranks (the global first / last slab keep the replicated frame the prologue wrote).
 void vae_conv(ltx_ctx* c, const float* x, int prep_mode, const float* a, const float* b, const ConvW& w, int T, int H, int W,
-              int pad, int epi_mode, float* out, const float* resid, int n_active, int t_shift) {
+              int pad, int epi_mode, void* out, const float* resid, int n_active, int t_shift) {
   c->v_pad.reserve(static_cast<size_t>(T + 2) * (H + 2) * (W + 2) * w.cin * 2);
   const double vox = static_cast<double>(T) * H * W;
   {
@@ -124,7 +174,9 @@ void vae_conv(ltx_ctx* c, const float* x, int prep_mode, const float* a, const f
                        frame * 2, n_active);
   }
   ConvEpi e;
-  e.mode = epi_mode; e.out = out; e.bias = w.b; e.resid = resid; e.Cin = w.cin; e.t_shift = t_shift;
+  e.mode = epi_mode; e.bias = w.b; e.resid = resid; e.Cin = w.cin; e.t_shift = t_shift;
+  if (epi_mode == CONV_EPI_RGB8 || epi_mode == CONV_EPI_I420) e.out_u8 = static_cast<uint8_t*>(out);
+  else e.out = static_cast<float*>(out);
   e.no_clip = c->vae_no_clip;
   ProfScope ps(c, PROF_CONV, 2.0 * w.taps * w.cin * w.cout * vox,
                vox * (w.cin * 2.0 + w.cout * 4.0) + static_cast<double>(w.taps) * w.cin * w.cout * 2.0);
@@ -210,7 +262,7 @@ void vae_resgroup_fused(ltx_ctx* c, float* x, const std::vector<VaeResBlock>& bl
 namespace {
 inline const float* vf(ltx_ctx* c, const std::string& k, int64_t n) { return vae_vec(c, k, n); }
 inline void conv(ltx_ctx* c, const float* x, int prep_mode, const float* a, const float* b, const ConvW& w, int T, int H, int W,
-                 int causal, int epi_mode, float* out, const float* resid, int n_active = 1, int t_shift = 0) {
+                 int causal, int epi_mode, void* out, const float* resid, int n_active = 1, int t_shift = 0) {
   vae_conv(c, x, prep_mode, a, b, w, T, H, W, causal ? VAE_PAD_CAUSAL : 0, epi_mode, out, resid, n_active, t_shift);
 }
 }  // namespace
@@ -281,10 +333,14 @@ void vae_finalize(ltx_ctx* c) {
 }
 
 void vae_decode_dev(ltx_ctx* c, const float* latent_dev, int Fp, int Hp, int Wp, float timestep, const float* noise_dev,
-                    int causal, float* frames_dev) {
+                    int causal, void* frames_dev, int format) {
   VaeWeights& v = c->vae;
+  LTX_CHECK(format == FRAMES_F32 || format == LTX_FRAMES_RGB8 || format == LTX_FRAMES_I420, LTX_ERR_INVALID_ARGUMENT,
+            "bad frame format");
   LTX_CHECK(v.ready, LTX_ERR_WEIGHTS, "VAE weights not finalized");
   LTX_CHECK(latent_dev && frames_dev && Fp > 0 && Hp > 1 && Wp > 1, LTX_ERR_INVALID_ARGUMENT, "bad vae_decode arguments");
+  LTX_CHECK(format == FRAMES_F32 || reinterpret_cast<uintptr_t>(frames_dev) % 4 == 0, LTX_ERR_INVALID_ARGUMENT,
+            "8-bit frames need a 4-byte aligned output buffer");
   const bool timed = timestep >= 0.f;
   LTX_CHECK(!timed || v.has_time, LTX_ERR_WEIGHTS, "timestep-conditioned decode needs the VAE time-embedder weights");
   LTX_CHECK(!timed || noise_dev != nullptr, LTX_ERR_INVALID_ARGUMENT, "decode_noise is required when timestep >= 0");
@@ -342,7 +398,8 @@ void vae_decode_dev(ltx_ctx* c, const float* latent_dev, int Fp, int Hp, int Wp,
   if (n_active > 1 && rank < n_active) slab(rank, f0, f1);
   const bool active = rank < n_active;
   const int Ho = 32 * Hp, Wo = 32 * Wp;
-  const size_t frame_elems = static_cast<size_t>(Ho) * Wo * 3;
+  const size_t frame_bytes = format == FRAMES_F32 ? static_cast<size_t>(Ho) * Wo * 3 * 4 : frames_u8_bytes(1, Ho, Wo, format);
+  uint8_t* frames = static_cast<uint8_t*>(frames_dev);
   if (active) {
     int T = f1 - f0, H = Hp, W = Wp;
     const int t_shift = (n_active > 1 && rank > 0) ? 1 : 0;
@@ -403,21 +460,23 @@ void vae_decode_dev(ltx_ctx* c, const float* latent_dev, int Fp, int Hp, int Wp,
         T = 2 * T - 1 + t_shift; H *= 2; W *= 2; ch /= 2;
       }
     }
-    // pn * (1 + scale) + shift -> SiLU -> conv_out -> unpatchify -> (x+1)/2 clip -> [F, H, W, 3]   (:419-444, 501-505)
+    // pn * (1 + scale) + shift -> SiLU -> conv_out -> unpatchify -> (x+1)/2 clip -> [F, H, W, 3]   (:419-444, 501-505),
+    // or straight on to 8-bit frames (tensorToImages, U/VideoExporter.swift:543-580, or I420) in the same store
     const int out_f0 = f0 == 0 ? 0 : 8 * (f0 - 1) + 1;
     if (timed) time_emb(v.last_te, te_stage);
     const float* lt = eff_table(v.last_sst, static_cast<int>(2 * ch));
-    conv(c, x, 2, lt + ch, lt, v.conv_out, T, H, W, causal, 2, frames_dev + static_cast<size_t>(out_f0) * frame_elems,
+    const int out_mode = format == LTX_FRAMES_RGB8 ? CONV_EPI_RGB8 : (format == LTX_FRAMES_I420 ? CONV_EPI_I420 : 2);
+    conv(c, x, 2, lt + ch, lt, v.conv_out, T, H, W, causal, out_mode, frames + static_cast<size_t>(out_f0) * frame_bytes,
          nullptr, n_active);
   }
   if (n_active > 1) {
     // all ranks receive every slab (an all-gather with unequal counts, as one broadcast per owner)
-    ProfScope ps(c, PROF_COMM, 0.0, 4.0 * frame_elems * (8.0 * (Fp - 1) + 1), n_active);
+    ProfScope ps(c, PROF_COMM, 0.0, static_cast<double>(frame_bytes) * (8.0 * (Fp - 1) + 1), n_active);
     for (int r = 0; r < n_active; ++r) {
       int a0, a1;
       slab(r, a0, a1);
       const int o0 = a0 == 0 ? 0 : 8 * (a0 - 1) + 1, o1 = 8 * (a1 - 1) + 1;
-      dist_broadcast(c, frames_dev + static_cast<size_t>(o0) * frame_elems, static_cast<size_t>(o1 - o0) * frame_elems * 4, r);
+      dist_broadcast(c, frames + static_cast<size_t>(o0) * frame_bytes, static_cast<size_t>(o1 - o0) * frame_bytes, r);
     }
   }
 }
@@ -439,11 +498,14 @@ int vae_tiled_frames(int Fp, int tile_size, int overlap) {
   return total;
 }
 
+// 8-bit formats: the fp32 chunks are blended and clipped in v_frames_f32 and converted at the end (frames_to_u8_dev).
 int vae_decode_tiled_dev(ltx_ctx* c, const float* latent_dev, int Fp, int Hp, int Wp, float timestep, const float* noise_dev,
-                         int causal, int tile_size, int overlap, float* frames_dev) {
-  LTX_CHECK(latent_dev && frames_dev && Fp > 0 && Hp > 1 && Wp > 1, LTX_ERR_INVALID_ARGUMENT, "bad vae_decode arguments");
+                         int causal, int tile_size, int overlap, void* out_dev, int format) {
+  LTX_CHECK(format == FRAMES_F32 || format == LTX_FRAMES_RGB8 || format == LTX_FRAMES_I420, LTX_ERR_INVALID_ARGUMENT,
+            "bad frame format");
+  LTX_CHECK(latent_dev && out_dev && Fp > 0 && Hp > 1 && Wp > 1, LTX_ERR_INVALID_ARGUMENT, "bad vae_decode arguments");
   if (tile_size <= 0 || Fp <= tile_size) {   // decodeVideo's single-pass branch (:482, 496)
-    vae_decode_dev(c, latent_dev, Fp, Hp, Wp, timestep, noise_dev, causal, frames_dev);
+    vae_decode_dev(c, latent_dev, Fp, Hp, Wp, timestep, noise_dev, causal, out_dev, format);
     return 8 * (Fp - 1) + 1;
   }
   LTX_CHECK(overlap >= 0 && overlap < tile_size, LTX_ERR_INVALID_ARGUMENT, "temporal tile overlap must be in [0, tile size)");
@@ -455,6 +517,11 @@ int vae_decode_tiled_dev(ltx_ctx* c, const float* latent_dev, int Fp, int Hp, in
   c->v_tile_lat.reserve(static_cast<size_t>(C0) * tile_size * hw * 4);
   if (timed) c->v_tile_noise.reserve(static_cast<size_t>(C0) * tile_size * hw * 4);
   c->v_tile_frames.reserve(static_cast<size_t>(8 * (tile_size - 1) + 1) * fe * 4);
+  float* frames_dev = static_cast<float*>(out_dev);
+  if (format != FRAMES_F32) {
+    c->v_frames_f32.reserve(static_cast<size_t>(vae_tiled_frames(Fp, tile_size, overlap)) * fe * 4);
+    frames_dev = c->v_frames_f32.as<float>();
+  }
   struct NoClip {   // the chunk decodes leave the clip to the end; restored on every exit path
     ltx_ctx* c;
     explicit NoClip(ltx_ctx* cc) : c(cc) { c->vae_no_clip = 1; }
@@ -499,6 +566,7 @@ int vae_decode_tiled_dev(ltx_ctx* c, const float* latent_dev, int Fp, int Hp, in
     clip01_kernel<<<grid_for(n4), 256, 0, st>>>(frames_dev, n4);
     LTX_CUDA(cudaGetLastError());
   }
+  if (format != FRAMES_F32) frames_to_u8_dev(c, frames_dev, total, 32 * Hp, 32 * Wp, format, static_cast<uint8_t*>(out_dev));
   return total;
 }
 

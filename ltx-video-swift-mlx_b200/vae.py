@@ -30,6 +30,18 @@ def decode_video(latent, decoder: VideoDecoder, timestep: Optional[float] = None
     return decoder.ctx.vae_decode(lat, timestep, decode_noise, decoder.causal)
 
 
+def decode_video_u8(latent, decoder: VideoDecoder, format="rgb8", timestep: Optional[float] = None, temporal_tile_size: int = 0,
+                    temporal_tile_overlap: int = 1, decode_noise=None) -> np.ndarray:
+    """decode_video followed by tensorToImages (U/VideoExporter.swift:543-580) in one call: 8-bit frames, "rgb8" [F,H,W,3]
+    or "i420" [F,3H/2,W] (BT.709 limited range), as include/ltxcuda.h defines them.  Only the 8-bit frames cross PCIe."""
+    lat = np.asarray(latent, dtype=np.float32)
+    frames_lat = lat.shape[-3]
+    if temporal_tile_size > 0 and frames_lat > temporal_tile_size:
+        return decoder.ctx.vae_decode_tiled_u8(lat, temporal_tile_size, temporal_tile_overlap, format, timestep, decode_noise,
+                                               decoder.causal)
+    return decoder.ctx.vae_decode_u8(lat, format, timestep, decode_noise, decoder.causal)
+
+
 class VideoEncoder:
     """Handle on the encoder weights held by an LtxContext (VideoEncoder(causal: true), Models/VAE/VideoEncoder.swift:211)."""
 
